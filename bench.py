@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- inflow cell-updates/s per filter() step (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one DIGITAL_FILTER::filter(dt) (df.cpp:449-468) over one synthetic plane: noise generation,
 y-sweep, z-sweep, temporal blend, RST scaling, SRA -- all five outputs of every cell.
@@ -261,15 +261,14 @@ def facade_e2e(plane, steps, device):
 
 
 def batched_planes(dfb, torch, local, nplanes=8, steps=300):
-    """BASELINE config 5 on one GPU: `nplanes` planes of the reference's default 510x400 geometry behind ONE handle
+    """BASELINE config 5 on one GPU: `nplanes` planes of the reference's default 510x400 geometry (its stored setup tables) behind ONE handle
     (dfb_create_batch: one launch set per step for all of them), dt = 1e-5; resident and with the five fields of every plane
     delivered to pinned host memory."""
-    rst, ln = os.path.join(ROOT, "oracle", "_ref", "files", "RST.dat"), os.path.join(ROOT, "oracle", "_ref", "line.dat")
-    if not (os.path.exists(rst) and os.path.exists(ln)):
-        return dict(skipped="the reference's data files (oracle/_ref) did not travel")
+    from oracle import oracle as O
+    plane = O.stored_default_plane()
     out = {}
     for P in (1, nplanes):
-        d = dfb.DIGITAL_FILTER(dfb.DFConfig(vel_fluc_file=rst, line_file=ln, seed=1, device=local, plane_id=100 * local), fetch=False, nplanes=P)
+        d = dfb.DIGITAL_FILTER(dfb.DFConfig.from_plane(plane, seed=1, device=local, plane_id=100 * local), fetch=False, nplanes=P)
         st = torch.cuda.ExternalStream(d.stream(), device=local)
         for _ in range(10):
             d.filter(1e-5)
@@ -398,6 +397,24 @@ def slab_job(dfb, torch, dist, rank, world, local, steps=20):
     return rec
 
 
+DUMP_BYTES = 64 * 10 ** 6        # all files of --dump-outputs together, .npy headers included
+
+
+def dump_outputs(dfb, df, out_dir):
+    """The five fields a caller of filter(dt) receives after the last timed step, as <out_dir>/<field>.npy (float64).  With
+    several GPUs only rank 0's plane (plane_id 0) is written; the other ranks' planes differ only in their noise streams.  When all
+    five do not fit in DUMP_BYTES, every field is sampled at the same cells: a fixed-seed draw without replacement, in
+    ascending row-major order."""
+    names = dict(u_fluc=dfb.U_FLUC, v_fluc=dfb.V_FLUC, w_fluc=dfb.W_FLUC, T_fluc=dfb.T_FLUC, rho_fluc=dfb.RHO_FLUC)
+    cells = df.n_cells
+    n = min(cells, (DUMP_BYTES // len(names) - 1024) // 8)
+    idx = None if n == cells else np.sort(np.random.default_rng(0).choice(cells, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, which in names.items():
+        a = df.get(which).ravel()
+        np.save(os.path.join(out_dir, name + ".npy"), a if idx is None else a[idx])
+
+
 def run_b200(args, plane):
     import torch
     import _dfb_import  # noqa: F401
@@ -456,6 +473,8 @@ def run_b200(args, plane):
     t_wall = time.perf_counter() - t_wall0
     ms = sum(a.elapsed_time(b) for a, b in ev)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(dfb, df, args.dump_outputs)
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -604,12 +623,11 @@ def run_b200(args, plane):
             batched = dict(error=str(e)[:200])
     if world == 1 and not args.no_sweep:
         from digital_filtering_b200 import workloads as WL
+        from oracle import oracle as O
         sweep = {}
         cases = [("1024x2048_saturated_N128", lambda: dfb.DFConfig.from_plane(WL.NAMED["1024x2048_saturated_N128"](), seed=1, device=local)),
-                 ("512x512_N32", lambda: dfb.DFConfig.from_plane(WL.NAMED["512x512_N32"](), seed=1, device=local))]
-        rst, ln = os.path.join(ROOT, "oracle", "_ref", "files", "RST.dat"), os.path.join(ROOT, "oracle", "_ref", "line.dat")
-        if os.path.exists(rst) and os.path.exists(ln):
-            cases.append(("reference_default_plane_510x400", lambda: dfb.DFConfig(vel_fluc_file=rst, line_file=ln, seed=1, device=local)))
+                 ("512x512_N32", lambda: dfb.DFConfig.from_plane(WL.NAMED["512x512_N32"](), seed=1, device=local)),
+                 ("reference_default_plane_510x400", lambda: dfb.DFConfig.from_plane(O.stored_default_plane(), seed=1, device=local))]
         for name, mk in cases:
             try:
                 d2 = dfb.DIGITAL_FILTER(mk(), fetch=False)
@@ -665,6 +683,8 @@ def main():
     ap.add_argument("--no-slab", action="store_true", help="N > 1: skip the config-4 slab job")
     ap.add_argument("--no-facade", action="store_true", help="skip the C++ facade end-to-end leg")
     ap.add_argument("--no-full-plane", action="store_true", help="reference arm: skip the one whole-plane step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write u', v', w', T', rho' of the last timed step to DIR/<field>.npy "
+                    "(float64, at most 64 MB in all: a fixed sample of the cells when the plane is larger; rank 0's plane only)")
     args = ap.parse_args()
     import _dfb_import  # noqa: F401
     from digital_filtering_b200 import workloads as W
@@ -672,6 +692,8 @@ def main():
         raise SystemExit(f"unknown workload {args.workload}; choose from {sorted(W.NAMED)}")
     plane = W.NAMED[args.workload]()
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes what the B200 arm computed; the reference arm does not support it")
         run_reference_arm(args, plane)
     else:
         run_b200(args, plane)

@@ -4,8 +4,8 @@ ctypes front-end to the two CPU checkers:
   * libdforacle.so      our plain-C restatement (df_oracle.c, pcg32_oracle.c, normal_oracle.c)
   * _ref/libdfref.so    the reference's own df.cpp compiled from /root/reference (ref_shim.cpp);
                         prebuilt here, travels to the GPU box, absent -> RefFilter unavailable.
-Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import
-this module.  The product (digital-filtering_b200/) never does.
+Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference / default-plane legs may
+import this module.  The product (digital-filtering_b200/) never does.
 """
 import ctypes as C
 import os
@@ -182,6 +182,20 @@ def _read_zone_file(path):
         n = int(float(zone.split("i=")[1].split()[0]))
         rows = [[float(x) for x in ln.split()] for ln in fh if ln.strip()]
     return np.array(rows[:n])
+
+
+DEFAULT_TABLES = os.path.join(os.path.dirname(HERE), "tests", "golden", "default_tables.npz")
+
+
+def stored_default_plane(path=DEFAULT_TABLES):
+    """The reference's default 510x400 plane as its own setup left it (tests/golden/default_tables.npz, written from the running
+    reference object by tests/golden/make_golden.py): geometry, row tables, integral scales and half-widths, in the workload form
+    DFConfig.from_plane takes.  d_i and the uniform spanwise spacing are the reference's constants (df.cpp:7-16)."""
+    g = np.load(path)
+    Ny, Nz = int(g["Ny"]), int(g["Nz"])
+    return dict(name="reference_default_plane_510x400", Ny=Ny, Nz=Nz, d_i=0.0013, yc=g["yc"], dy=g["dy"], dz=np.full(Ny, 0.000133),
+                rows=g["rows"], scales=g["scales"], N_y=np.repeat(g["N_y"][:, :, None], Nz, axis=2),
+                N_z=np.repeat(g["N_z"][:, :, None], Nz, axis=2), Ny_max=[int(x) for x in g["Ny_max"]], Nz_max=[int(x) for x in g["Nz_max"]])
 
 
 def default_plane(rst_path=RST_DAT, line_path=LINE_DAT):

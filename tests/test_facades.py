@@ -2,7 +2,8 @@
   C++      include/digital_filter.hpp, used exactly like the reference's test/cpp-main.cpp
   Fortran  fortran/digital_filtering.f90 -- no Fortran compiler in the image, so its binding is
            exercised by tests/fortran_abi_mimic.c (same struct image, same by-reference calls)
-CPU: both compile and link against libdfb200.so.  GPU: both run on the reference's default plane."""
+CPU: both compile and link against libdfb200.so.  GPU: both run on the reference's default plane, read from files in the
+reference's formats that the `default_data` fixture writes from the stored tables."""
 import os
 import subprocess
 
@@ -80,12 +81,9 @@ def test_fortran_module_mirrors_the_c_struct():
 
 
 @pytest.mark.gpu
-def test_cpp_facade_runs_the_reference_example(dfb, O):
-    if not O.have_ref():
-        pytest.skip("needs the data files under oracle/_ref")
+def test_cpp_facade_runs_the_reference_example(dfb, default_data):
     _build(dfb)
-    os.makedirs(O.REF_RUN, exist_ok=True)
-    r = subprocess.run([os.path.join(BIN, "cpp-test")], cwd=O.REF_RUN, capture_output=True, text=True, timeout=300)
+    r = subprocess.run([os.path.join(BIN, "cpp-test")], cwd=default_data / "run", capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr
     assert "Ny=510 Nz=400" in r.stdout
     rms = float(r.stdout.split("=")[-1].split()[0])
@@ -117,11 +115,10 @@ def test_reference_main_runs_unchanged(dfb, O):
 
 
 @pytest.mark.gpu
-def test_fortran_calling_convention(dfb, O):
-    if not O.have_ref():
-        pytest.skip("needs the data files under oracle/_ref")
+def test_fortran_calling_convention(dfb, default_data):
     _build(dfb)
-    r = subprocess.run([os.path.join(BIN, "fortran_abi_mimic"), O.RST_DAT, O.LINE_DAT], capture_output=True, text=True, timeout=300)
+    r = subprocess.run([os.path.join(BIN, "fortran_abi_mimic"), str(default_data / "files" / "RST.dat"), str(default_data / "line.dat")],
+                       capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, (r.stdout, r.stderr)
     tok = r.stdout.split()
     assert tok[0] == "OK" and (int(tok[1]), int(tok[2])) == (510, 400) and float(tok[3]) > 1.0

@@ -14,7 +14,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, normwise_close
+from conftest import GOLDEN, default_plane, normwise_close
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-12
@@ -144,38 +144,52 @@ def test_G2_golden_small_plane_from_reference_object_code(dfb, O):
         df.close()
 
 
+def _default_plane_reference_step(dfb, O):
+    """The reference's default plane from its stored setup tables, and the one injected step whose reference outputs
+    tests/golden/default_step_digest.json records (sha256 + probes, tests/golden/make_golden.py): noise of step 1 and filt_old
+    from the oracle's counter-based stream (seed 20261018), dt = 1e-5.  The oracle's output of that step is checked against the
+    reference's sha256 here, so what the GPU is compared with below is the reference's own output, bit for bit.
+    Returns (df after the step, oracle output, plane, digest)."""
+    import hashlib
+    import json
+    d = json.load(open(os.path.join(GOLDEN, "default_step_digest.json")))
+    P = default_plane()
+    Ny, Nz, seed = P["Ny"], P["Nz"], d["seed"]
+    rys = [O.noise_rys(seed, 0, f, 1, Ny, P["Ny_max"][f], Nz) for f in range(3)]
+    hal = [O.noise_halo(seed, 0, f, 1, Ny, P["Nz_max"][f]) for f in range(3)]
+    fo = np.stack([O.noise_elements(seed, 100 + f, 0, Ny * Nz, 0, Ny * Nz).reshape(Ny, Nz) for f in range(3)])
+    o = O.step(P, rys, hal, fo, d["dt"])
+    for k, rec in d["outputs"].items():
+        assert hashlib.sha256(np.ascontiguousarray(o[k]).tobytes()).hexdigest() == rec["sha256"], k
+    df = dfb.DIGITAL_FILTER(dfb.DFConfig.from_plane(P, noise_mode=dfb.NOISE_INJECT))
+    df.set_state(fo, 1)
+    for f in range(3):
+        df.set_noise(f, rys[f], hal[f])
+    df.filter(d["dt"])
+    df.fetch()
+    return df, o, P, d
+
+
 def test_G2_default_plane_against_reference_object_code(dfb, O):
-    """config 1: the reference's own default plane (RST.dat + line.dat), its own filter() call
-    (own random_device noise) replayed on the GPU."""
-    if not O.have_ref():
-        pytest.skip("oracle/_ref did not travel")
-    ref = O.RefFilter()
-    cfg = dfb.DFConfig(vel_fluc_file=O.RST_DAT, line_file=O.LINE_DAT, noise_mode=dfb.NOISE_INJECT)
-    df = dfb.DIGITAL_FILTER(cfg)
-    P = ref.plane()
+    """config 1: the reference's own default plane (its setup tables, stored) and one step of its filter() on stored-noise
+    inputs whose outputs are recorded from the reference's object code: setup tables, half-widths, coefficients and all
+    five outputs on the GPU against them."""
+    df, o, P, d = _default_plane_reference_step(dfb, O)
     assert (df.Ny, df.Nz) == (510, 400)
-    assert np.array_equal(df.rows(), P["rows"])                 # setup tables bit-identical
+    assert np.array_equal(df.rows(), P["rows"])
     for f in range(3):
         assert np.array_equal(df.half_widths(f, 0), P["N_y"][f]) and np.array_equal(df.half_widths(f, 1), P["N_z"][f])
     for N in (2, 6, 28, 212):
         assert np.array_equal(df.table(11, N), O.coeffs(N))
     assert np.array_equal(df.table(10), P["scales"][:, 2])
-    for step in range(3):
-        fo = ref.outputs()["filt_old"].copy()
-        ref.filter(1e-5)                                        # DIGITAL_FILTER::filter, df.cpp:449-468
-        df.set_state(fo, 1 + step)
-        for f in range(3):
-            df.set_noise_ref_layout(f, ref.fvec(f, "r_ys"), ref.fvec(f, "r_zs"))
-        df.filter(1e-5)
-        df.fetch()
-        r = ref.outputs()
-        for f, F in enumerate((df.u, df.v, df.w)):
-            ok, ratio = normwise_close(F.fluc, r["fluc"][f], TOL)
-            assert ok, (step, f, ratio)
-            assert normwise_close(F.filt, r["filt"][f], TOL)[0]
-        assert normwise_close(df.T_fluc, r["T"], TOL)[0] and normwise_close(df.rho_fluc, r["rho"], TOL)[0]
+    got = dict(filt=np.stack([df.u.filt, df.v.filt, df.w.filt]), fluc=np.stack([df.u.fluc, df.v.fluc, df.w.fluc]), T=df.T_fluc, rho=df.rho_fluc)
+    for k, rec in d["outputs"].items():
+        for f in range(3 if k in ("filt", "fluc") else 1):
+            ok, ratio = normwise_close(got[k][f] if k in ("filt", "fluc") else got[k], o[k][f] if k in ("filt", "fluc") else o[k], TOL)
+            assert ok, (k, f, ratio)
+        probe = got[k].ravel()[[0, 12345, 99999, got[k].size - 1]]   # the reference's values at the recorded cells
+        assert np.all(np.abs(probe - rec["probe"]) <= TOL * np.maximum(np.abs(rec["probe"]), rec["rms"])), (k, probe, rec["probe"])
     df.close()
-    ref.close()
 
 
 def test_G2_generate_mode_equals_oracle_on_the_same_stream(dfb, O, W):
@@ -258,12 +272,11 @@ def test_inject_mode_requires_noise(dfb, W):
     df.close()
 
 
-def test_dns_statistics_file_layout(dfb, O, tmp_path):
+def test_dns_statistics_file_layout(dfb, default_data, tmp_path):
     """N1: the Fortran caller's configuration (vel_file_offset = 142 header lines + the DNS statistics
     layout, fortran-main.f90:17-19) gives the same tables as the preprocessed RST.dat (RST.cpp:43-50)."""
-    if not O.have_ref():
-        pytest.skip("needs the data files under oracle/_ref")
-    rst = [ln.split() for ln in open(O.RST_DAT).read().splitlines()[2:] if ln.strip()]
+    RST_DAT, LINE_DAT = str(default_data / "files" / "RST.dat"), str(default_data / "line.dat")
+    rst = [ln.split() for ln in open(RST_DAT).read().splitlines()[2:] if ln.strip()]
     stat = tmp_path / "Stat.dat"
     with open(stat, "w") as fh:
         for i in range(142):
@@ -272,8 +285,8 @@ def test_dns_statistics_file_layout(dfb, O, tmp_path):
             cols = ["0"] * 20
             cols[0], cols[1], cols[8], cols[10], cols[9], cols[15] = r[0], r[1], r[2], r[3], r[4], r[5]
             fh.write(" ".join(cols) + "\n")
-    a = dfb.DIGITAL_FILTER(dfb.DFConfig(vel_fluc_file=O.RST_DAT, line_file=O.LINE_DAT, seed=1))
-    b = dfb.DIGITAL_FILTER(dfb.DFConfig(vel_fluc_file=str(stat), line_file=O.LINE_DAT, seed=1, vel_file_offset=142, vel_file_N_values=330))
+    a = dfb.DIGITAL_FILTER(dfb.DFConfig(vel_fluc_file=RST_DAT, line_file=LINE_DAT, seed=1))
+    b = dfb.DIGITAL_FILTER(dfb.DFConfig(vel_fluc_file=str(stat), line_file=LINE_DAT, seed=1, vel_file_offset=142, vel_file_N_values=330))
     assert (a.Ny, a.Nz) == (b.Ny, b.Nz) == (510, 400)
     assert np.array_equal(a.rows(), b.rows())
     assert np.array_equal(a.u.fluc, b.u.fluc)
@@ -375,30 +388,30 @@ def test_N2_running_statistics_match_rms_add(dfb, W):
 
 
 def test_N4_csv_matches_reference_writer(dfb, O, tmp_path):
-    """write_csv (df.cpp:764-803): same header, same fixed 15-decimal format, same coordinates and (within the
-    fp64 gate) the same numbers as the file the reference's own filter() call writes."""
-    if not O.have_ref():
-        pytest.skip("oracle/_ref did not travel")
-    ref = O.RefFilter()
-    df = dfb.DIGITAL_FILTER(dfb.DFConfig(vel_fluc_file=O.RST_DAT, line_file=O.LINE_DAT, noise_mode=dfb.NOISE_INJECT))
-    fo = ref.outputs()["filt_old"].copy()
-    ref.filter(1e-5)                                   # writes <run>/../files/cpp_vel_fluc.csv (df.cpp:466-467)
-    df.set_state(fo, 1)
-    for f in range(3):
-        df.set_noise_ref_layout(f, ref.fvec(f, "r_ys"), ref.fvec(f, "r_zs"))
-    df.filter(1e-5)
+    """write_csv (df.cpp:764-803): same header, same fixed 15-decimal format, the reference's cell-centre coordinates
+    (df.cpp:776-786 on its own grid, read_grid df.cpp:71-118) and, within the fp64 gate, the reference's outputs of the
+    stored default-plane step (_default_plane_reference_step)."""
+    import ctypes as C
+    df, o, P, _ = _default_plane_reference_step(dfb, O)
     mine = tmp_path / "b200_vel_fluc.csv"
     df.write_csv(mine)
-    a = open(os.path.join(O.REF_FILES, "cpp_vel_fluc.csv")).read().splitlines()
     b = open(mine).read().splitlines()
-    assert a[0] == b[0] == "z,y,u_fluc,v_fluc,w_fluc,T_fluc,rho_fluc" and len(a) == len(b) == 1 + 510 * 400
-    for la, lb in list(zip(a[1:], b[1:]))[::997]:
-        ta, tb = la.split(","), lb.split(",")
-        assert ta[:2] == tb[:2]                        # coordinates print identically
+    Ny, Nz = P["Ny"], P["Nz"]
+    assert b[0] == "z,y,u_fluc,v_fluc,w_fluc,T_fluc,rho_fluc" and len(b) == 1 + Ny * Nz
+    yv, yc, dy = np.zeros(561), np.zeros(560), np.zeros(560)
+    O.lib().orc_default_grid(C.c_int(560), C.c_double(P["d_i"]), O._d(yv), O._d(yc), O._d(dy))
+    assert np.array_equal(yc[:Ny], P["yc"])
+    ref = np.stack([o["fluc"][0], o["fluc"][1], o["fluc"][2], o["T"], o["rho"]]).reshape(5, -1)
+    rms = np.sqrt((ref ** 2).mean(1))
+    for n in range(0, Ny * Nz, 997):
+        j, k = divmod(n, Nz)                           # one row per cell, j-major
+        tb = b[1 + n].split(",")
         assert all(len(x.split(".")[1]) == 15 for x in tb)
-        for x, y in zip(ta[2:], tb[2:]):
-            assert abs(float(x) - float(y)) <= 1e-12 * max(abs(float(x)), 1.0) + 2e-15
-    df.close(); ref.close()
+        assert tb[0] == "%.15f" % (0.25 * (k * 0.000133 + (k + 1) * 0.000133 + k * 0.000133 + (k + 1) * 0.000133))
+        assert tb[1] == "%.15f" % (0.25 * (yv[j] + yv[j] + yv[j + 1] + yv[j + 1]))
+        for x, r, s in zip(tb[2:], ref[:, n], rms):
+            assert abs(float(x) - r) <= TOL * max(abs(r), s) + 5e-16, (n, x, r)
+    df.close()
 
 
 # ---------------------------------------------------------------------------------------------
@@ -538,14 +551,15 @@ def test_timing_mode_does_not_change_results(dfb, W):
     a.close(); b.close()
 
 
-def test_G3_config1_default_plane_100_steps(dfb, O):
-    """BASELINE.json configs[0]: the reference's own default plane (RST.dat + line.dat), u'/v'/w' over 100 filter(dt)
+def test_G3_config1_default_plane_100_steps(dfb):
+    """BASELINE.json configs[0]: the reference's own default plane (the tables its setup built from RST.dat + line.dat), u'/v'/w' over 100 filter(dt)
     steps with dt = 1e-5 (cpp-main.cpp:15).  Reynolds stresses averaged over the steps and the 400 spanwise cells against
     the target RST the setup interpolated from the DNS file.  Stated tolerance (n_eff ~ 100*400/13 ~ 3000 per row):
     diagonal terms median < 3 %, p95 < 8 %; the reference itself shows median 0.5 %, max 2-3 % (BASELINE.md section 2)."""
-    if not O.have_ref():
-        pytest.skip("needs the data files under oracle/_ref")
-    df = dfb.DIGITAL_FILTER(dfb.DFConfig(vel_fluc_file=O.RST_DAT, line_file=O.LINE_DAT, seed=11), fetch=False)
+    P = default_plane()
+    df = dfb.DIGITAL_FILTER(dfb.DFConfig.from_plane(P, seed=11), fetch=False)
+    for f in range(3):                                       # the library derives the reference's half-widths from the stored geometry
+        assert np.array_equal(df.half_widths(f, 0), P["N_y"][f]) and np.array_equal(df.half_widths(f, 1), P["N_z"][f])
     rows = df.rows()
     acc = np.zeros((4, df.Ny))
     for _ in range(100):
@@ -802,16 +816,14 @@ def test_config5_batch_equals_independent_handles_bitwise(dfb, W, shape):
         d.close()
 
 
-def test_config5_default_plane_batch_against_single_plane(dfb, O):
+def test_config5_default_plane_batch_against_single_plane(dfb):
     """BASELINE config 5 proper: 8 planes of the reference's default geometry behind one handle.  The batch has 8 times the tiles
     and takes the run-recursive y-sweep on the row blocks where it pays (dfb_info 10 == 3), a single such plane stays on the band
     matrices (0): plane p of the batch and the single-plane handle with plane_id + p then agree to rounding (<= 1e-13 of the rms,
     far inside the 1e-12 gate each form passes against the oracle); bit for bit if they happen to run the same form."""
-    if not O.have_ref():
-        pytest.skip("needs the data files under oracle/_ref")
     P, p = 8, 5
-    batch = dfb.DIGITAL_FILTER(dfb.DFConfig(vel_fluc_file=O.RST_DAT, line_file=O.LINE_DAT, seed=21, plane_id=2), fetch=False, nplanes=P)
-    cfg1 = dfb.DFConfig(vel_fluc_file=O.RST_DAT, line_file=O.LINE_DAT, seed=21, plane_id=2 + p)
+    batch = dfb.DIGITAL_FILTER(dfb.DFConfig.from_plane(default_plane(), seed=21, plane_id=2), fetch=False, nplanes=P)
+    cfg1 = dfb.DFConfig.from_plane(default_plane(), seed=21, plane_id=2 + p)
     single = dfb.DIGITAL_FILTER(cfg1, fetch=False)
     same_form = batch.info(10) == single.info(10)
     for dt in (1e-5, 1e-5, 2e-5):

@@ -9,7 +9,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import GOLDEN
+from conftest import GOLDEN, default_plane
 
 
 def test_default_plane_tables_match_golden(O):
@@ -47,10 +47,12 @@ def test_small_plane_three_steps_match_golden_bitwise(O, W):
 
 
 def test_default_plane_step_digest(O):
-    if not O.have_ref():
-        pytest.skip("default-plane setup needs the data files under oracle/_ref")
     d = json.load(open(os.path.join(GOLDEN, "default_step_digest.json")))
-    P = O.default_plane()
+    P = default_plane()
+    # the half-widths the restatement derives from the stored geometry are the reference's own (default_tables.npz)
+    G = O.half_widths(dict(P))
+    assert np.array_equal(G["N_y"], P["N_y"]) and np.array_equal(G["N_z"], P["N_z"])
+    assert G["Ny_max"] == P["Ny_max"] == [212, 160, 212] and G["Nz_max"] == P["Nz_max"] == [6, 4, 6]
     Ny, Nz, seed = P["Ny"], P["Nz"], d["seed"]
     rys = [O.noise_rys(seed, 0, f, 1, Ny, P["Ny_max"][f], Nz) for f in range(3)]
     hal = [O.noise_halo(seed, 0, f, 1, Ny, P["Nz_max"][f]) for f in range(3)]
