@@ -50,6 +50,7 @@ class dfb_config(C.Structure):
         ("N_y", c_ip), ("N_z", c_ip),
         ("seed", C.c_uint64), ("noise_mode", C.c_int), ("device", C.c_int), ("plane_id", C.c_int),
         ("k_begin", C.c_int), ("k_end", C.c_int), ("skip_first_step", C.c_int), ("kernel_variant", C.c_int),
+        ("periodic_z", C.c_int),
     ]
 
 
@@ -167,6 +168,7 @@ class DFConfig:
         self.k_begin = self.k_end = 0
         self.skip_first_step = 0
         self.kernel_variant = 0
+        self.periodic_z = 0              # 1: spanwise-periodic plane (the z filter wraps around it; include/dfb200.h)
         for k, v in kw.items():
             if not hasattr(self, k):
                 raise TypeError(f"DFConfig has no field {k!r}")
@@ -251,6 +253,7 @@ class DIGITAL_FILTER:
         c.seed, c.noise_mode, c.device, c.plane_id = config.seed, config.noise_mode, config.device, config.plane_id
         c.k_begin, c.k_end = config.k_begin, config.k_end
         c.skip_first_step, c.kernel_variant = config.skip_first_step, config.kernel_variant
+        c.periodic_z = config.periodic_z
         self._h = C.c_void_p()
         self.nplanes = int(nplanes)
         if self.nplanes == 1:
@@ -365,6 +368,11 @@ class DIGITAL_FILTER:
         return bool(self.info(3))
 
     @property
+    def periodic_z(self):
+        """True when the plane is spanwise-periodic (dfb_config.periodic_z; dfb_info 13)"""
+        return bool(self.info(13))
+
+    @property
     def taps_per_step(self):
         return self.info(4)
 
@@ -383,20 +391,22 @@ class DIGITAL_FILTER:
         return out
 
     # ---- noise ----
-    def set_noise(self, field, r_ys, halo):
+    def set_noise(self, field, r_ys, halo=None):
+        """r_ys (Ny + 2 Ny_max, Nz) and the r_zs halo (Ny, 2 Nz_max); a periodic plane takes r_ys alone (halo=None)."""
         r_ys = np.ascontiguousarray(r_ys, dtype=np.float64)
         halo = np.ascontiguousarray(halo, dtype=np.float64) if halo is not None else None
         _check(lib().dfb_set_noise(self._h, field, _dptr(r_ys), _dptr(halo)))
 
     def set_noise_ref_layout(self, field, r_ys, r_zs):
         r_ys = np.ascontiguousarray(r_ys, dtype=np.float64)
-        r_zs = np.ascontiguousarray(r_zs, dtype=np.float64)
+        r_zs = np.ascontiguousarray(r_zs, dtype=np.float64) if r_zs is not None else None
         _check(lib().dfb_set_noise_ref_layout(self._h, field, _dptr(r_ys), _dptr(r_zs)))
 
     def get_noise(self, field):
+        """(r_ys, halo) of the last step's noise; (r_ys, None) on a periodic plane, which draws no halo."""
         F = (self.u, self.v, self.w)[field]
         r_ys = np.zeros((self.Ny + 2 * F.Ny_max, self.Nz))
-        halo = np.zeros((self.Ny, 2 * F.Nz_max))
+        halo = None if self.periodic_z else np.zeros((self.Ny, 2 * F.Nz_max))
         _check(lib().dfb_get_noise(self._h, field, _dptr(r_ys), _dptr(halo)))
         return r_ys, halo
 

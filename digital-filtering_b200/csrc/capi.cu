@@ -42,7 +42,7 @@ struct NoiseHost {            // one logical array of the noise contract
     int field, kind;
     uint64_t inc, state0, npairs;
     int n_seg;
-    void *d_jump = nullptr, *d_off = nullptr, *d_np = nullptr;
+    void *d_jump = nullptr, *d_off = nullptr, *d_np = nullptr, *d_win = nullptr;
 };
 
 }  // namespace
@@ -89,6 +89,7 @@ struct dfb_filter_s {
     // noise
     std::vector<NoiseHost> noise;
     NoiseParams np{};
+    NoiseWindows nwin{};              // periodic_z: segment windows of the r_ys arrays whose extended rows wrap (else all nullptr)
     unsigned long long* tl = nullptr; // development aid (DFB_TIMELINE): 64 steps x {noise, y, z} x {start, end}
     // N2: running statistics (opt-in)
     double* stats = nullptr;          // [P][6][Ny*W]: sum u'^2, v'^2, w'^2, T'^2, rho'^2, u'v'
@@ -249,8 +250,10 @@ void build_device(dfb_filter_s& H) {
         F.Ny_max = FP.Ny_max; F.Nz_max = FP.Nz_max;
         maxNz = std::max(maxNz, FP.Nz_max);
         F.rows_y = Ny + 2 * FP.Ny_max;
-        F.xk0 = std::max(0, P.k0 - FP.Nz_max);
-        const int xk1 = std::min(NzG, P.k1 + FP.Nz_max);
+        // periodic_z: the extended range is not clipped to the plane -- its columns beyond an edge are the plane's own columns,
+        // wrapped (Nz_max <= NzG: at most once), y-filtered like the others, so that the z-sweep needs no change at all
+        F.xk0 = P.periodic ? P.k0 - FP.Nz_max : std::max(0, P.k0 - FP.Nz_max);
+        const int xk1 = P.periodic ? P.k1 + FP.Nz_max : std::min(NzG, P.k1 + FP.Nz_max);
         F.We = xk1 - F.xk0;
         F.pitch_y = round_up(F.We, 16);
         F.zoff = (16 - FP.Nz_max % 16) % 16;
@@ -850,17 +853,30 @@ void build_device(dfb_filter_s& H) {
             A.inc = (stream << 1) | 1u;
             A.state0 = pcg_lcg(H.seed + A.inc, A.inc);
             std::vector<Jump> jumps;
-            std::vector<int> offv;         // r_ys: extended column of the segment's first pair (0 or -1); halo: 0
+            std::vector<int> offv;         // r_ys: extended column of the segment's first pair (its first column, or one less); halo: 0
             std::vector<int> npv;
+            std::vector<int4> winv;        // periodic_z, extended rows that wrap: {padded row, first, end extended column} per piece
             if (kind == 0) {
                 A.npairs = ((uint64_t)F.rows_y * (uint64_t)NzG + 1u) / 2u;
+                const int xk1 = F.xk0 + F.We;
+                const bool wraps = F.xk0 < 0 || xk1 > NzG;   // periodic_z only
                 for (int r = 0; r < F.rows_y; ++r) {
-                    const long long ea = (long long)r * NzG + F.xk0, eb = ea + F.We - 1;
-                    const long long qa = ea >> 1, qb = eb >> 1;
-                    offv.push_back((int)(2 * qa - ea)); npv.push_back((int)(qb - qa + 1));
-                    jumps.push_back(pcg_jump(4u * (uint64_t)qa, 1u));
+                    // the row's extended range as contiguous pieces of the stream: global columns [g0, g1) at extended column x0
+                    // (left of the plane: its last columns; the plane part; right of it: its first columns)
+                    const int pieces[3][3] = {{NzG + F.xk0, NzG, 0},
+                                              {std::max(F.xk0, 0), std::min(xk1, NzG), std::max(F.xk0, 0) - F.xk0},
+                                              {0, xk1 - NzG, NzG - F.xk0}};
+                    for (const auto& pc : pieces) {
+                        if (pc[1] <= pc[0]) continue;
+                        const long long ea = (long long)r * NzG + pc[0], eb = (long long)r * NzG + pc[1] - 1;
+                        const long long qa = ea >> 1, qb = eb >> 1;
+                        offv.push_back((int)(2 * qa - ea) + pc[2]); npv.push_back((int)(qb - qa + 1));
+                        jumps.push_back(pcg_jump(4u * (uint64_t)qa, 1u));
+                        if (wraps) winv.push_back(make_int4(r, pc[2], pc[2] + pc[1] - pc[0], 0));
+                    }
                 }
-            } else {
+                if (wraps && offv.size() > 65535u) throw Error{DFB_ERR_ARG, "periodic_z: too many padded rows for the noise kernel's grid"};
+            } else if (!P.periodic) {      // periodic_z: the z filter reads no raw noise, array 1 is not drawn
                 const int M = F.Nz_max;
                 A.npairs = (uint64_t)Ny * (uint64_t)M;
                 const bool touches = (P.k0 - M < 0) || (P.k1 + M > NzG);
@@ -874,6 +890,7 @@ void build_device(dfb_filter_s& H) {
             for (int v : npv) max_np = std::max(max_np, v);
             if (A.n_seg) {
                 A.d_jump = H.upload(jumps); A.d_off = H.upload(offv); A.d_np = H.upload(npv);
+                if (!winv.empty()) A.d_win = H.upload(winv);
             }
             H.noise.push_back(A);
         }
@@ -893,6 +910,7 @@ void fill_noise_params(dfb_filter_s& H, int64_t step) {
         if (!A.n_seg) continue;
         NoiseArray& a = H.np.a[n];
         a.seg_jump = A.d_jump; a.seg_off = static_cast<const int*>(A.d_off); a.seg_np = static_cast<const int*>(A.d_np);
+        H.nwin.seg_win[n] = static_cast<const int4*>(A.d_win);
         a.n_seg = A.n_seg; a.kind = A.kind; a.field = A.field;
         for (int p = 0; p < H.nplanes; ++p) {
             // stream ((plane*3 + field)*2 + array) of include/dfb_rng_spec.h; plane p of a batch is plane_id + p
@@ -918,7 +936,7 @@ void launch_noise_for(dfb_filter_s& H, int64_t step, int b, cudaStream_t st) {
     H.ybuf_step[b] = -1;                 // new noise invalidates whatever y-sweep result the set held
     fill_noise_params(H, step);
     H.np.tl = H.tl ? H.tl + (step % 64) * 8 : nullptr;
-    CUDA_TRY(launch_noise(H.np, H.D[b], st));
+    CUDA_TRY(launch_noise(H.np, H.nwin, H.D[b], st));
     CUDA_TRY(cudaEventRecord(H.ev_noise[b], st));
     H.buf_step[b] = step;
 }
@@ -1130,6 +1148,7 @@ int dfb_info(dfb_handle h, int what, int field, int64_t* out64) {
         case 10: *out64 = h->tuned ? h->y_form : -1; break;
         case 12: *out64 = h->transport; break;
         case 11: *out64 = h->tuned ? h->yp[0].n_rtiles : 0; break;
+        case 13: *out64 = h->plan.periodic ? 1 : 0; break;
         default: return fail(DFB_ERR_ARG, "unknown info selector");
     }
     return DFB_OK;
@@ -1308,13 +1327,22 @@ static int set_noise_impl(dfb_handle h, int field, const double* r_ys, const dou
     if (!h || !r_ys || field < 0 || field > 2) return fail(DFB_ERR_ARG, "bad argument");
     if (h->noise_mode != DFB_NOISE_INJECT) return fail(DFB_ERR_STATE, "handle was not created with noise_mode = DFB_NOISE_INJECT");
     if (h->nplanes != 1) return fail(DFB_ERR_STATE, "noise injection is defined for single-plane handles");
+    if (h->plan.periodic && (left || right)) return fail(DFB_ERR_ARG, "periodic_z: the noise is r_ys alone, the r_zs halo must be NULL");
     return guarded([&] {
         CUDA_TRY(cudaSetDevice(h->device));
         const FieldDev& F = h->D[h->step & 1].f[field];      // the set the next step reads
         const int W = h->D[0].W, M = F.Nz_max;
-        CUDA_TRY(cudaMemcpy2DAsync(F.r_ys, (size_t)F.pitch_y * 8, r_ys, (size_t)W * 8, (size_t)W * 8, (size_t)F.rows_y,
+        // the plane part sits at extended column -xk0 (0 unless periodic_z); a periodic plane's wrapped columns come from the same array
+        CUDA_TRY(cudaMemcpy2DAsync(F.r_ys - F.xk0, (size_t)F.pitch_y * 8, r_ys, (size_t)W * 8, (size_t)W * 8, (size_t)F.rows_y,
                                    cudaMemcpyHostToDevice, h->stream));
-        if (M > 0) {
+        if (h->plan.periodic) {
+            if (M > 0) {
+                CUDA_TRY(cudaMemcpy2DAsync(F.r_ys, (size_t)F.pitch_y * 8, r_ys + (W - M), (size_t)W * 8, (size_t)M * 8, (size_t)F.rows_y,
+                                           cudaMemcpyHostToDevice, h->stream));
+                CUDA_TRY(cudaMemcpy2DAsync(F.r_ys + M + W, (size_t)F.pitch_y * 8, r_ys, (size_t)W * 8, (size_t)M * 8, (size_t)F.rows_y,
+                                           cudaMemcpyHostToDevice, h->stream));
+            }
+        } else if (M > 0) {
             if (!left || !right) throw Error{DFB_ERR_ARG, "halo noise missing"};
             CUDA_TRY(cudaMemcpy2DAsync(F.r_zs + F.zoff, (size_t)F.pitch_z * 8, left, halo_pitch, (size_t)M * 8, (size_t)h->D[0].Ny,
                                        cudaMemcpyHostToDevice, h->stream));
@@ -1335,18 +1363,20 @@ int dfb_set_noise(dfb_handle h, int field, const double* r_ys, const double* r_z
 int dfb_set_noise_ref_layout(dfb_handle h, int field, const double* r_ys, const double* r_zs) {
     if (!h || field < 0 || field > 2) return fail(DFB_ERR_ARG, "bad argument");
     const int M = h->D[0].f[field].Nz_max, W = h->D[0].W;
+    if (h->plan.periodic) r_zs = nullptr;                  // periodic_z: nothing of r_zs is noise
     return set_noise_impl(h, field, r_ys, r_zs, r_zs ? r_zs + W + M : nullptr, (size_t)(W + 2 * M) * 8);
 }
 
 int dfb_get_noise(dfb_handle h, int field, double* r_ys, double* r_zs_halo) {
     if (!h || field < 0 || field > 2) return fail(DFB_ERR_ARG, "bad argument");
     if (h->plan.k0 != 0 || h->plan.k1 != h->plan.NzG) return fail(DFB_ERR_STATE, "dfb_get_noise is defined on whole-plane handles");
+    if (h->plan.periodic && r_zs_halo) return fail(DFB_ERR_ARG, "periodic_z: there is no r_zs halo noise, r_zs_halo must be NULL");
     return guarded([&] {
         CUDA_TRY(cudaSetDevice(h->device));
         const FieldDev& F = h->D[h->noise_view].f[field];
         const int W = h->D[0].W, M = F.Nz_max;
         if (r_ys)
-            CUDA_TRY(cudaMemcpy2DAsync(r_ys, (size_t)W * 8, F.r_ys, (size_t)F.pitch_y * 8, (size_t)W * 8, (size_t)F.rows_y,
+            CUDA_TRY(cudaMemcpy2DAsync(r_ys, (size_t)W * 8, F.r_ys - F.xk0, (size_t)F.pitch_y * 8, (size_t)W * 8, (size_t)F.rows_y,
                                        cudaMemcpyDeviceToHost, h->stream));
         if (r_zs_halo && M > 0) {
             CUDA_TRY(cudaMemcpy2DAsync(r_zs_halo, (size_t)2 * M * 8, F.r_zs + F.zoff, (size_t)F.pitch_z * 8, (size_t)M * 8,

@@ -1,12 +1,15 @@
 // csrc/device.cuh -- device-side data layout of one inflow plane (or one spanwise slab of it) in HBM.
 //
 //   r_ys[f]   (Ny + 2*Ny_max[f]) x pitch_y   white noise of the y-sweep (df.cpp:197), columns = the slab's
-//                                            EXTENDED range [xk0, xk1) = [k0-Nz_max, k1+Nz_max) clipped to the plane
+//                                            EXTENDED range [xk0, xk1) = [k0-Nz_max, k1+Nz_max) clipped to the plane;
+//                                            periodic_z: NOT clipped (xk0 may be negative), extended column x holds
+//                                            global column (xk0 + x) mod NzG -- the plane part starts at column -xk0
 //   r_zs[f]   Ny x pitch_z                   logical column c in [0, W+2*Nz_max) lives at zoff + c; c = Nz_max is
 //                                            the slab's first column (df.cpp:157,363).  Columns whose GLOBAL
 //                                            index falls outside [0,NzG) hold raw noise (SURVEY quirk 1),
 //                                            the others are written by the y-sweep (incl. neighbours' columns,
-//                                            recomputed locally instead of exchanged).
+//                                            recomputed locally instead of exchanged).  periodic_z: the y-sweep
+//                                            writes every column (yshift = 0), those beyond an edge wrapped.
 //   filt_old[f], fluc[f], T, rho   dense Ny x W, row-major j*W + k  (df.cpp:106) -> one memcpy to the caller
 //   coefficients: one row per distinct half-width N (CSR keyed by N), plus per-row-group dense band
 //   matrices for the tuned y-sweep; per-row epilogue constants.
@@ -106,10 +109,11 @@ struct StepConsts {
     int first_step;            // constructor semantics (df.cpp:57-62): no blend, T'/rho' untouched
 };
 
-// ---- noise generation work description (one segment = one row of one logical array) ----
+// ---- noise generation work description (one segment = one row of one logical array, or one contiguous piece of a row) ----
 struct NoiseArray {
     const void* seg_jump;      // Jump[n_seg]: jump from `state` to the segment's first pair
-    const int* seg_off;        // r_ys: extended column of a segment's first pair, 2*q0 - (row * NzG + xk0); halo: 0
+    const int* seg_off;        // r_ys: extended column of a segment's first pair, 2*q0 - (row * NzG + xk0) (a piece: + its first column,
+                               // - its first stream element); halo: 0
     const int* seg_np;         // pairs in each segment
     int n_seg;
     int kind;                  // 0 = r_ys rows, 1 = r_zs halo rows
@@ -129,6 +133,12 @@ struct NoiseParams {
     int chunks;                 // ceil(max_np / 128)
     unsigned long long* tl;     // development aid (DFB_TIMELINE): [start, end] globaltimer stamps of this launch, or nullptr
 };
+
+// per array of NoiseParams: r_ys of a periodic plane whose extended rows wrap (periodic_z) -- {padded row, first, end extended column}
+// of each segment, a row being up to three pieces of the stream (wrapped left piece, plane part, wrapped right piece); nullptr:
+// segment = row, columns [0, We).  Only noise_pieces_kernel takes it: the parameters of noise_kernel stay those of a plane that
+// does not wrap.
+struct NoiseWindows { const int4* seg_win[6]; };
 
 struct YParams {
     const YGroup* groups;

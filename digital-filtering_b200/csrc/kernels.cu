@@ -1,6 +1,7 @@
 // csrc/kernels.cu -- the per-timestep hot path DIGITAL_FILTER::filter(dt) (df.cpp:449-468) as sm_100a kernels.
 //
 //   noise_kernel            H1  generate_white_noise   df.cpp:332-349  (replaced: counter-based pcg32, see noise.cuh)
+//   noise_pieces_kernel         the same for a spanwise-periodic plane whose extended rows wrap (periodic_z)
 //   ysweep_tma_kernel       H2y filtering_sweeps, y    df.cpp:360-383  tuned: TMA-staged slabs, dense band matrices
 //   zsweep_epilogue_kernel  H2z filtering_sweeps, z    df.cpp:386-405  tuned: <ZK,1> recursive evaluation of the exponential
 //                                                                      window (default), <ZK,0> direct Toeplitz register window
@@ -52,7 +53,12 @@ __device__ __forceinline__ void tl_stamp(unsigned long long* tl, int end) {
 // One thread = NOISE_PAIRS pairs of one segment (row), NOISE_THREADS pairs apart, so that a warp's stores stay contiguous:
 // ONE position jump per thread (segment jump o slot jump, two table reads), then from pair to pair a constant stride jump
 // of 4*NOISE_THREADS draws -- one 64-bit multiply-add, like a plain LCG step -- instead of two table jumps per pair.
-__device__ __forceinline__ void noise_thread(const NoiseParams& P, const PlaneDev& D, int slot0, int seg, int bz, int pl) {
+// PIECES: the segments of r_ys arrays may be pieces of rows (NoiseWindows; periodic_z, extended rows that wrap around the plane);
+// without, a segment is a whole padded row -- a kernel of its own, so that every other handle keeps the leaner one (48 registers
+// against 50: the noise CTAs run beside the sweeps).
+template <bool PIECES>
+__device__ __forceinline__ void noise_thread(const NoiseParams& P, const PlaneDev& D, const NoiseWindows* Wn, int slot0, int seg, int bz,
+                                             int pl) {
     const NoiseArray& A = P.a[bz];
     if (seg >= A.n_seg) return;
     const uint64_t inc = P.pinc[pl][bz];
@@ -61,14 +67,18 @@ __device__ __forceinline__ void noise_thread(const NoiseParams& P, const PlaneDe
     const Jump sj = reinterpret_cast<const Jump*>(A.seg_jump)[seg];
     const Jump tj = P.slot_jump[min(slot0, P.max_np - 1)];
     const int off = A.seg_off[seg];
+    int4 win = make_int4(seg, 0, 0, 0);                          // PIECES: {padded row, first, end extended column} of the segment
+    if constexpr (PIECES) { if (Wn->seg_win[bz]) win = Wn->seg_win[bz][seg]; else win.z = D.f[A.field].We; }
     if (slot0 >= np) return;
     uint64_t s = sj.A * P.pstate[pl][bz] + inc * sj.C;
     s = tj.A * s + inc * tj.C;
     const uint64_t strideA = P.stride.A, strideC = inc * P.stride.C;
     const FieldDev& F = D.f[A.field];
     if (A.kind == 0) {
-        // r_ys: pair `slot` of padded row `seg` holds the extended columns x0 = 2 slot + off and x0 + 1 (off = 2 q0 - row base)
-        double* dst = F.r_ys + (size_t)pl * F.ps_ys + (size_t)seg * F.pitch_y;
+        // r_ys: pair `slot` of the segment holds the extended columns x0 = 2 slot + off and x0 + 1 of padded row `seg` (PIECES:
+        // win.x); only the columns [0, We) (PIECES: [win.y, win.z)) are the segment's (a pair may straddle two rows of the stream,
+        // or the edge of a wrapped piece)
+        double* dst = F.r_ys + (size_t)pl * F.ps_ys + (size_t)(PIECES ? win.x : seg) * F.pitch_y;
         int x0 = 2 * slot0 + off;
         const bool vec_ok = (x0 & 1) == 0;                       // rows are 128-byte aligned: an even column is 16-byte aligned
         constexpr int NU = NOISE_UNROLL;
@@ -77,7 +87,8 @@ __device__ __forceinline__ void noise_thread(const NoiseParams& P, const PlaneDe
             double z0, z1;
             normal_pair(s, inc, z0, z1);
             s = strideA * s + strideC;
-            const bool in0 = x0 >= 0 && x0 < F.We, in1 = x0 + 1 >= 0 && x0 + 1 < F.We;
+            const bool in0 = PIECES ? x0 >= win.y && x0 < win.z : x0 >= 0 && x0 < F.We;
+            const bool in1 = PIECES ? x0 + 1 >= win.y && x0 + 1 < win.z : x0 + 1 >= 0 && x0 + 1 < F.We;
             if (in0 && in1 && vec_ok) {
                 *reinterpret_cast<double2*>(dst + x0) = make_double2(z0, z1);
             } else {
@@ -111,7 +122,13 @@ __device__ __forceinline__ void noise_thread(const NoiseParams& P, const PlaneDe
 // one CTA per (NOISE_THREADS x NOISE_PAIRS pairs, segment, array x plane of the batch)
 __global__ void __launch_bounds__(NOISE_THREADS) noise_kernel(const NoiseParams P, const PlaneDev D) {
     if (threadIdx.x == 0 && (blockIdx.y & 31) == 0) tl_stamp(P.tl, 0);     // sampled: one row in 32 (same-address atomics)
-    noise_thread(P, D, (int)blockIdx.x * NOISE_PAIRS * NOISE_THREADS + (int)threadIdx.x, blockIdx.y, (int)(blockIdx.z % P.n_arrays), (int)(blockIdx.z / P.n_arrays));
+    noise_thread<false>(P, D, nullptr, (int)blockIdx.x * NOISE_PAIRS * NOISE_THREADS + (int)threadIdx.x, blockIdx.y, (int)(blockIdx.z % P.n_arrays), (int)(blockIdx.z / P.n_arrays));
+    if (threadIdx.x == 0 && (blockIdx.y & 31) == 0) tl_stamp(P.tl, 1);
+}
+// the same for a periodic plane whose extended rows wrap: a segment is one piece of a row (NoiseWindows)
+__global__ void __launch_bounds__(NOISE_THREADS) noise_pieces_kernel(const NoiseParams P, const PlaneDev D, const NoiseWindows Wn) {
+    if (threadIdx.x == 0 && (blockIdx.y & 31) == 0) tl_stamp(P.tl, 0);
+    noise_thread<true>(P, D, &Wn, (int)blockIdx.x * NOISE_PAIRS * NOISE_THREADS + (int)threadIdx.x, blockIdx.y, (int)(blockIdx.z % P.n_arrays), (int)(blockIdx.z / P.n_arrays));
     if (threadIdx.x == 0 && (blockIdx.y & 31) == 0) tl_stamp(P.tl, 1);
 }
 
@@ -123,7 +140,9 @@ __global__ void __launch_bounds__(256) ysweep_simple_kernel(const PlaneDev D, in
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
     const int j = blockIdx.y, pl = blockIdx.z;
     if (x >= F.We) return;
-    const int N = F.Ny_cell ? F.Ny_cell[(size_t)j * D.NzG + F.xk0 + x] : F.Ny_row[j];
+    int g = F.xk0 + x;                                    // global column; periodic_z: wrapped into [0, NzG)
+    if (g < 0) g += D.NzG; else if (g >= D.NzG) g -= D.NzG;
+    const int N = F.Ny_cell ? F.Ny_cell[(size_t)j * D.NzG + g] : F.Ny_row[j];
     const double* b = D.coef_vals + D.coef_ptr[N] + N;
     const double* r = F.r_ys + (size_t)pl * F.ps_ys + (size_t)(j + F.Ny_max) * F.pitch_y + x;
     double sum = 0.0;
@@ -1374,13 +1393,16 @@ __global__ void __launch_bounds__(256) dfma_peak_kernel(double* out, int iters, 
 // =================================================================================================
 // host launchers
 // =================================================================================================
-cudaError_t launch_noise(const NoiseParams& P, const PlaneDev& D, cudaStream_t st) {
+cudaError_t launch_noise(const NoiseParams& P, const NoiseWindows& Wn, const PlaneDev& D, cudaStream_t st) {
     if (P.n_arrays == 0) return cudaSuccess;
     cudaGetLastError();        // the status returned below is this launch's, not a leftover of an unrelated earlier call
     int max_seg = 0;
     for (int a = 0; a < P.n_arrays; ++a) max_seg = P.a[a].n_seg > max_seg ? P.a[a].n_seg : max_seg;
+    bool pieces = false;
+    for (int a = 0; a < P.n_arrays; ++a) pieces = pieces || Wn.seg_win[a] != nullptr;
     dim3 grid((unsigned)P.chunks, (unsigned)max_seg, (unsigned)(P.n_arrays * D.P));
-    noise_kernel<<<grid, NOISE_THREADS, 0, st>>>(P, D);
+    if (pieces) noise_pieces_kernel<<<grid, NOISE_THREADS, 0, st>>>(P, D, Wn);
+    else noise_kernel<<<grid, NOISE_THREADS, 0, st>>>(P, D);
     return cudaGetLastError();
 }
 
@@ -1411,6 +1433,8 @@ cudaError_t ysweep_prepare() {
     // as a process-wide bimodal y-sweep time on small planes: 26 or 43 us on the reference default plane).
     {
         cudaError_t e0 = cudaFuncSetAttribute(noise_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e0 != cudaSuccess) return e0;
+        e0 = cudaFuncSetAttribute(noise_pieces_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
         if (e0 != cudaSuccess) return e0;
         e0 = cudaFuncSetAttribute(stats_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
         if (e0 != cudaSuccess) return e0;

@@ -4,7 +4,7 @@
 
 namespace dfb {
 
-cudaError_t launch_noise(const NoiseParams& P, const PlaneDev& D, cudaStream_t st);
+cudaError_t launch_noise(const NoiseParams& P, const NoiseWindows& Wn, const PlaneDev& D, cudaStream_t st);
 cudaError_t launch_ysweep_simple(const PlaneDev& D, cudaStream_t st);
 cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, cudaStream_t st);
 size_t ysweep_smem_bytes();

@@ -33,6 +33,7 @@ struct FieldPlan {
 struct Plan {
     int Ny = 0, NzG = 0;                         // trimmed rows, global spanwise width
     int k0 = 0, k1 = 0;                          // slab owned by this handle
+    bool periodic = false;                       // dfb_config.periodic_z: the z filter wraps around the plane (Nz_max <= NzG)
     double d_i = 0, d_v = 0, U_e = 0, rho_e = 0, mu = 0, gcon = 287.0;
     double u_tau = 0, tau_w = 0;
     std::vector<double> yc_row, dy_row;          // first column of the geometry (ydline*d_i, df.cpp:115-116)

@@ -326,6 +326,15 @@ void build_plan(const dfb_config& cfg, Plan& P) {
         if (!F.row_uniform) { F.N_y = std::move(Ny_arr); F.N_z = std::move(Nz_arr); }
     }
 
+    // ---- spanwise-periodic plane: a window may wrap at most once around the plane ----
+    if (cfg.periodic_z != 0 && cfg.periodic_z != 1) throw Error{DFB_ERR_ARG, "periodic_z must be 0 or 1"};
+    P.periodic = cfg.periodic_z == 1;
+    if (P.periodic)
+        for (int f = 0; f < 3; ++f)
+            if (P.f[f].Nz_max > NzG)
+                throw Error{DFB_ERR_ARG, std::string("periodic_z: field ") + "uvw"[f] + " has Nz_max = " + std::to_string(P.f[f].Nz_max) +
+                                             " > Nz = " + std::to_string(NzG) + " (a z window may wrap around the plane at most once)"};
+
     // ---- coefficient table keyed by N ----
     int Nmax = 0;
     for (int f = 0; f < 3; ++f) Nmax = std::max({Nmax, P.f[f].Ny_max, P.f[f].Nz_max});

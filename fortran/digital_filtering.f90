@@ -15,6 +15,7 @@
 !   create_digital_filter_batch / filter_batch   BASELINE config 5: P planes of one geometry behind one handle (one launch set per step)
 !   config%k_begin / k_end, comm_unique_id, comm_init, gather_begin / gather_end / gathered_field
 !                                                 BASELINE config 4: this rank's spanwise slab + the NCCL hand-off inside the library
+!   config%periodic_z = 1                         spanwise-periodic plane: the z filter wraps around it
 !   face_map, apply_inflow                        N3: inflow face -> plane cell, ghost cell = mean + fluctuation (us3d_user.f90:85-114)
 !
 ! NOTE: NEVER COMPILED -- no Fortran compiler exists in the build image or on the GPU boxes.  The binding is exercised through
@@ -45,6 +46,7 @@ module DIGITAL_FILTERING
         integer(c_int64_t) :: seed = 0_c_int64_t
         integer :: device = -1, plane_id = 0
         integer :: k_begin = 0, k_end = 0             ! this rank's spanwise slab [k_begin, k_end) (0-based, C convention); 0,0 = the whole plane
+        integer :: periodic_z = 0                     ! 1: spanwise-periodic plane (the z filter wraps around it; needs Nz_max <= Nz)
     end type DFConfig
 
     type :: digital_filter_type
@@ -77,6 +79,7 @@ module DIGITAL_FILTERING
         type(c_ptr) :: yc, dy, dz, rows, scales, N_y, N_z
         integer(c_int64_t) :: seed
         integer(c_int) :: noise_mode, device, plane_id, k_begin, k_end, skip_first_step, kernel_variant
+        integer(c_int) :: periodic_z
     end type dfb_config_c
 
     interface
@@ -189,6 +192,7 @@ contains
         c%line_file = c_loc(config%line_file);          c%line_file_len = len_trim(config%line_file)
         c%seed = config%seed; c%device = config%device; c%plane_id = config%plane_id
         c%k_begin = config%k_begin; c%k_end = config%k_end
+        c%periodic_z = config%periodic_z
     end subroutine fill_config
 
     ! page-lock an array the library copies into every step (failure only costs speed)

@@ -85,9 +85,16 @@ typedef struct dfb_config {
     int plane_id;               /* RNG stream group of this plane (distinct planes -> independent noise) */
     int k_begin, k_end;         /* spanwise slab [k_begin,k_end) of the Nz-wide plane owned by this handle;
                                    0,0 -> the whole plane.  Noise is keyed by the GLOBAL index, so slabs
-                                   reproduce the single-GPU plane bit for bit with no halo exchange. */
+                                   reproduce the single-GPU plane bit for bit with no halo exchange
+                                   (periodic_z included: a wrapped neighbour column is regenerated locally too). */
     int skip_first_step;        /* 1: do not run the constructor's first step (df.cpp:57-62) */
     int kernel_variant;         /* 0 = tuned kernels; 1 = simple cross-check kernels (same maths, one thread per cell) */
+    int periodic_z;             /* 0 (default): the reference's plane, NOT periodic in z -- the z filter reads raw white noise for
+                                   the Nz_max columns beyond each spanwise edge (SURVEY quirk 1);
+                                   1: spanwise-periodic plane -- the z filter wraps, filt[j,k] = sum_i b_i * y_filtered[j, (k+i) mod Nz],
+                                   for spanwise-periodic LES/DNS inflow.  Needs Nz_max <= Nz for every field.  r_ys is drawn exactly
+                                   as with 0 (only columns whose window reaches an edge change); the r_zs halo is not drawn.
+                                   (Occupies what was the struct's tail padding: sizeof(dfb_config) is unchanged.) */
 } dfb_config;
 
 int dfb_config_init(dfb_config* cfg);
@@ -114,7 +121,7 @@ int dfb_dims(dfb_handle h, int* Ny, int* Nz);
  * 10 form of the y-sweep in use: 2 = run-recursive (every row group through the exponential window), 3 = run-recursive on the blocks of
  *    32 rows where it pays + dense band matrices on the rest (e.g. a batch of planes of the reference's default geometry), 1 = chunk-recursive band-matrix
  *    kernel, 0 = dense band matrices (DFB_Y_MODE=0|1|2 forces a form), 11 tiles of the run-recursive kernel, 12 transport of the config-4 hand-off: 2 = peer-to-peer copies (CUDA IPC + copy engines), 1 = NCCL
- *    send/recv, 0 = no communicator */
+ *    send/recv, 0 = no communicator, 13 spanwise-periodic plane (dfb_config.periodic_z) in use (0/1) */
 int dfb_info(dfb_handle h, int what, int field, int64_t* out64);
 /* host copies of the setup tables (for parity tests): which = 0..7 rows R11,R21,R22,R33,Us,Ts,rhos,Ms [Ny];
  * 8 yc row [Ny]; 9 dy row [Ny]; 10 Lt[3]; 11 coefficients of half-width `arg` [2*arg+1];
@@ -194,11 +201,12 @@ int dfb_comm_destroy(dfb_handle h);
 
 /* noise injection ("ingest the reference's own draws", SURVEY quirk 4).  Host arrays in the
  * reference's layouts: r_ys (Ny+2*Ny_max) x Nz (df.cpp:197); halo Ny x (2*Nz_max) = the left and
- * right Nz_max raw-noise columns of r_zs, the only part of it that is read (df.cpp:157,398). */
+ * right Nz_max raw-noise columns of r_zs, the only part of it that is read (df.cpp:157,398).
+ * periodic_z = 1: r_ys alone is the noise (the z filter wraps onto y-filtered columns); r_zs_halo must be NULL. */
 int dfb_set_noise(dfb_handle h, int field, const double* r_ys, const double* r_zs_halo);
-/* same, but r_zs is the reference's full Ny x (Nz+2*Nz_max) array; its interior is ignored */
+/* same, but r_zs is the reference's full Ny x (Nz+2*Nz_max) array; its interior is ignored (all of it with periodic_z = 1; may be NULL) */
 int dfb_set_noise_ref_layout(dfb_handle h, int field, const double* r_ys, const double* r_zs);
-/* read back the noise of the last step in the same layouts (RNG gate) */
+/* read back the noise of the last step in the same layouts (RNG gate); periodic_z = 1: r_zs_halo must be NULL */
 int dfb_get_noise(dfb_handle h, int field, double* r_ys, double* r_zs_halo);
 /* only generate the noise of step `step` (no filtering) -- used by the RNG gate and the benchmarks */
 int dfb_generate_noise(dfb_handle h, int64_t step);

@@ -58,6 +58,7 @@ struct DFConfigEx {
     std::uint64_t seed = 0;
     int noise_mode = DFB_NOISE_GENERATE;
     int device = -1, plane_id = 0, k_begin = 0, k_end = 0;
+    bool periodic_z = false;           // spanwise-periodic plane: the z filter wraps around it (LES/DNS inflow with periodic span)
     bool fetch_every_step = true;      // copy u', v', w', T', rho' into the host vectors after each filter()
 };
 
@@ -155,7 +156,7 @@ class DIGITAL_FILTER {
         k.Ny = c.Ny; k.Nz = c.Nz; k.geom_per_row = c.geom_per_row;
         k.yc = c.yc; k.dy = c.dy; k.dz = c.dz; k.rows = c.rows; k.scales = c.scales; k.N_y = c.N_y; k.N_z = c.N_z;
         k.seed = c.seed; k.noise_mode = c.noise_mode; k.device = c.device; k.plane_id = c.plane_id;
-        k.k_begin = c.k_begin; k.k_end = c.k_end;
+        k.k_begin = c.k_begin; k.k_end = c.k_end; k.periodic_z = c.periodic_z ? 1 : 0;
         fetch_ = c.fetch_every_step;
         check(dfb_create(&k, &h_));
         check(dfb_dims(h_, &Ny, &Nz));
