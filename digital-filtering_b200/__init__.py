@@ -25,6 +25,8 @@ LIB_PATH = os.environ.get("DFB_LIB") or os.path.join(_HERE, "lib", "libdfb200.so
 OK, ERR_ARG, ERR_IO, ERR_CUDA, ERR_STATE, ERR_INTERP = range(6)
 U_FLUC, V_FLUC, W_FLUC, T_FLUC, RHO_FLUC, U_FILT, V_FILT, W_FILT = range(8)
 NOISE_GENERATE, NOISE_INJECT = 0, 1
+CORR_Z, CORR_Y, CORR_T = 0, 1, 2        # correlation directions (dfb_corr_enable)
+DFB_CORR_SUPPORT = CORR_SUPPORT = -1    # lag = the filter's whole support (z and y)
 
 c_dp = C.POINTER(C.c_double)
 c_ip = C.POINTER(C.c_int)
@@ -126,6 +128,10 @@ def lib():
         L.dfb_stats_enable.argtypes = [C.c_void_p, C.c_int]
         L.dfb_stats_get.argtypes = [C.c_void_p, C.c_int, C.c_int, c_dp, C.POINTER(C.c_int64)]
         L.dfb_write_csv.argtypes = [C.c_void_p, C.c_char_p]
+        L.dfb_corr_enable.argtypes = [C.c_void_p, C.c_int, c_ip]
+        L.dfb_corr_get.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, c_dp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+        L.dfb_corr_get_plane.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, c_dp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+        L.dfb_corr_integral_scales.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, c_dp]
         _lib = L
     return _lib
 
@@ -441,6 +447,35 @@ class DIGITAL_FILTER:
         _check(lib().dfb_get_rms(self._h, int(nsteps), float(dt)))
         if path is not None:
             _check(lib().dfb_write_rms_csv(self._h, str(path).encode()))
+
+    # ---- correlation statistics (opt-in; include/dfb200.h, dfb_corr_enable) ----
+    def corr_enable(self, z=DFB_CORR_SUPPORT, y=DFB_CORR_SUPPORT, t=0, on=True):
+        """Accumulate per-row lagged products of u', v', w' after every step: lags z, y (0 = off, DFB_CORR_SUPPORT = the filter's
+        whole support) and t (0..64 steps).  Zeroes the sums; on=False stops accumulating and keeps them readable."""
+        lags = (C.c_int * 3)(int(z), int(y), int(t))
+        _check(lib().dfb_corr_enable(self._h, int(on), lags))
+
+    @property
+    def corr_lags(self):
+        """(L_z, L_y, L_t) of the correlation sums (dfb_info 14); 0 for a direction that is off"""
+        return tuple(self.info(14, d) for d in range(3))
+
+    def corr(self, field, dir, normalized=True, plane=0):
+        """(array [Ny, L+1], pairs [L+1], accumulated steps) of field 0..2 (u', v', w') in direction CORR_Z / CORR_Y / CORR_T:
+        correlation coefficients (normalized=True) or the raw sums"""
+        n = self.corr_lags[dir] + 1
+        out = np.zeros((self.Ny, n))
+        pairs = np.zeros(n, dtype=np.int64)
+        cnt = C.c_int64()
+        _check(lib().dfb_corr_get_plane(self._h, plane, field, dir, int(normalized), _dptr(out),
+                                        pairs.ctypes.data_as(C.POINTER(C.c_int64)), C.byref(cnt)))
+        return out, pairs, cnt.value
+
+    def integral_scales(self, field, dir, plane=0):
+        """per-row integral scale of the normalised correlation up to its first non-positive lag: metres for z and y, steps for t"""
+        out = np.zeros(self.Ny)
+        _check(lib().dfb_corr_integral_scales(self._h, plane, field, dir, _dptr(out)))
+        return out
 
     def write_csv(self, path):
         _check(lib().dfb_write_csv(self._h, str(path).encode()))

@@ -6,6 +6,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <memory>
 #include <string>
 #include <vector>
@@ -95,6 +96,14 @@ struct dfb_filter_s {
     double* stats = nullptr;          // [P][6][Ny*W]: sum u'^2, v'^2, w'^2, T'^2, rho'^2, u'v'
     int64_t stats_count = 0;
     bool stats_on = false;
+    // correlation statistics (opt-in, dfb_corr_enable): lagged products of u', v', w' along z, y and in time, after the z-sweep
+    bool corr_on = false;
+    bool corr_ready = false;          // sums allocated and readable (the first dfb_corr_enable(h, 1, ..) has succeeded)
+    CorrParams corr{};                // lags, sums, scratch, ring
+    int64_t corr_count = 0;           // accumulated steps
+    std::vector<int64_t> corr_tsteps; // [L_t + 1]: accumulated steps that had an accumulated predecessor m steps back in the ring
+    std::vector<void*> corr_mem;      // the sums: freed when the lags change and with the handle
+                                      // (corr.ring and corr.part exist only while accumulating: corr_free_work)
     // config 4: this handle as one spanwise slab of a plane shared with the other ranks of a job (dfb_comm_init)
     ncclComm_t comm = nullptr;
     int comm_rank = -1, comm_world = 0;
@@ -145,6 +154,9 @@ struct dfb_filter_s {
         if (side) cudaStreamSynchronize(side);
         if (stream) cudaStreamSynchronize(stream);
         for (void* p : allocs) cudaFree(p);
+        for (void* p : corr_mem) cudaFree(p);
+        cudaFree(corr.ring);
+        cudaFree(corr.part);
         for (auto& e : ev) if (e) cudaEventDestroy(e);
         for (int b = 0; b < 2; ++b) { if (ev_noise[b]) cudaEventDestroy(ev_noise[b]); if (ev_free[b]) cudaEventDestroy(ev_free[b]); }
         for (int q = 0; q < 2; ++q) { if (ev_staged[q]) cudaEventDestroy(ev_staged[q]); if (ev_copied[q]) cudaEventDestroy(ev_copied[q]); }
@@ -984,6 +996,18 @@ void run_step(dfb_filter_s& H, double dt, bool first) {
         if (accumulate) CUDA_TRY(launch_stats(H.D[0], H.stats, H.stream));
     }
     if (accumulate) H.stats_count += 1;
+    if (H.corr_on && !first) {
+        CorrParams& c = H.corr;
+        if (c.L[0]) CUDA_TRY(launch_corr_z(c, H.stream));
+        if (c.L[1]) CUDA_TRY(launch_corr_y(c, H.stream));
+        if (c.L[2]) {
+            const int M = (int)std::min<long long>(c.L[2], c.ring_count);
+            CUDA_TRY(launch_corr_t(c, M, H.stream));
+            for (int m = 0; m <= M; ++m) H.corr_tsteps[m] += 1;
+            c.ring_count += 1;
+        }
+        H.corr_count += 1;
+    }
     CUDA_TRY(cudaEventRecord(H.ev_free[b], H.stream));
     if (H.timing) CUDA_TRY(cudaEventRecord(H.ev[3], H.stream));
     H.step += 1;
@@ -1149,6 +1173,7 @@ int dfb_info(dfb_handle h, int what, int field, int64_t* out64) {
         case 12: *out64 = h->transport; break;
         case 11: *out64 = h->tuned ? h->yp[0].n_rtiles : 0; break;
         case 13: *out64 = h->plan.periodic ? 1 : 0; break;
+        case 14: *out64 = h->corr_ready ? h->corr.L[field] : 0; break;
         default: return fail(DFB_ERR_ARG, "unknown info selector");
     }
     return DFB_OK;
@@ -1424,6 +1449,7 @@ int dfb_set_state(dfb_handle h, const double* filt_old3, int64_t step) {
         CUDA_TRY(cudaStreamSynchronize(h->side));      // a look-ahead noise launch for the old step counter may still be in flight
         if (step != h->step) { h->buf_step[0] = h->buf_step[1] = -1; h->ybuf_step[0] = h->ybuf_step[1] = -1; }
         h->step = step;
+        h->corr.ring_count = 0;       // the next step follows the restored state: no temporal pair reaches back across it
     });
 }
 
@@ -1498,6 +1524,168 @@ int dfb_stats_get_plane(dfb_handle h, int plane, int which, int as_rms, double* 
     });
 }
 int dfb_stats_get(dfb_handle h, int which, int as_rms, double* dst, int64_t* count) { return dfb_stats_get_plane(h, 0, which, as_rms, dst, count); }
+
+// ---- correlation statistics (dfb_corr_enable / dfb_corr_get / dfb_corr_integral_scales) ----
+int dfb_corr_enable(dfb_handle h, int on, const int lags[3]) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    if (!on) {                                                // the sums stay readable; the ring and the scratch go
+        h->corr_on = false;
+        return guarded([&] {
+            CUDA_TRY(cudaSetDevice(h->device));
+            CUDA_TRY(cudaStreamSynchronize(h->stream));
+            CUDA_TRY(cudaFree(h->corr.ring));
+            CUDA_TRY(cudaFree(h->corr.part));
+            h->corr.ring = h->corr.part = nullptr;
+        });
+    }
+    if (!lags) return fail(DFB_ERR_ARG, "lags is NULL");
+    const Plan& P = h->plan;
+    if (P.k0 != 0 || P.k1 != P.NzG) return fail(DFB_ERR_ARG, "correlation statistics need the whole plane");
+    int L[3];
+    const int extent[2] = {P.NzG, P.Ny};
+    const char* name[3] = {"z", "y", "t"};
+    for (int d = 0; d < 3; ++d) {
+        if (lags[d] == DFB_CORR_SUPPORT) {
+            if (d == DFB_CORR_T) return fail(DFB_ERR_ARG, "lag of direction t must be 0..64: DFB_CORR_SUPPORT is not defined for t");
+            int sup = 0;
+            for (int f = 0; f < 3; ++f) sup = std::max(sup, 2 * (d == DFB_CORR_Z ? P.f[f].Nz_max : P.f[f].Ny_max));
+            L[d] = std::min(sup, extent[d] - 1);
+        } else {
+            const int hi = d == DFB_CORR_T ? 64 : extent[d] - 1;
+            if (lags[d] < 0 || lags[d] > hi)
+                return fail(DFB_ERR_ARG, std::string("lag of direction ") + name[d] + " must be 0.." + std::to_string(hi) +
+                                             (d == DFB_CORR_T ? "" : " or DFB_CORR_SUPPORT") + ", got " + std::to_string(lags[d]));
+            L[d] = lags[d];
+        }
+    }
+    return guarded([&] {
+        CUDA_TRY(cudaSetDevice(h->device));
+        CorrParams& c = h->corr;
+        const int NP = h->nplanes, Ny = P.Ny, W = P.NzG;
+        const size_t rows = (size_t)NP * 3 * Ny;
+        auto alloc = [&](size_t n) {
+            void* q = nullptr;
+            CUDA_TRY(cudaMalloc(&q, std::max<size_t>(n, 1) * sizeof(double)));
+            return static_cast<double*>(q);
+        };
+        if (!h->corr_ready || L[0] != c.L[0] || L[1] != c.L[1] || L[2] != c.L[2]) {
+            CUDA_TRY(cudaStreamSynchronize(h->stream));
+            for (void* q : h->corr_mem) cudaFree(q);
+            h->corr_mem.clear();
+            cudaFree(c.ring);
+            cudaFree(c.part);
+            h->corr_ready = false;
+            h->corr_on = false;
+            c = CorrParams{};
+            for (int f = 0; f < 3; ++f) c.fluc[f] = h->D[0].f[f].fluc;
+            c.P = NP; c.Ny = Ny; c.W = W; c.periodic = P.periodic ? 1 : 0;
+            for (int d = 0; d < 3; ++d) {
+                c.L[d] = L[d];
+                if (L[d]) { c.sum[d] = alloc(rows * (L[d] + 1)); h->corr_mem.push_back(c.sum[d]); }
+            }
+            c.y_nsplit = c.y_split_cols = 1;
+            if (L[1]) corr_y_split(Ny, W, &c.y_nsplit, &c.y_split_cols);
+        }
+        // the ring and the partial-sum scratch exist only while accumulating (on = 0 frees them)
+        const size_t part = corr_part_doubles(NP, Ny, W, c.L[0], c.L[1], c.y_nsplit);
+        if (part && !c.part) c.part = alloc(part);
+        if (c.L[2] && !c.ring) c.ring = alloc((size_t)c.L[2] * rows * W);
+        for (int d = 0; d < 3; ++d)
+            if (c.sum[d]) CUDA_TRY(cudaMemsetAsync(c.sum[d], 0, rows * (c.L[d] + 1) * sizeof(double), h->stream));
+        CUDA_TRY(cudaStreamSynchronize(h->stream));
+        c.ring_count = 0;
+        h->corr_count = 0;
+        h->corr_tsteps.assign(c.L[2] + 1, 0);
+        h->corr_ready = true;
+        h->corr_on = true;
+    });
+}
+
+namespace {
+
+// the sums of one (plane, field, direction) on the host, [Ny][L+1], and the products per row behind each lag
+void corr_fetch(dfb_filter_s& H, int plane, int field, int dir, std::vector<double>& S, std::vector<int64_t>& pairs) {
+    const CorrParams& c = H.corr;
+    const int Ny = c.Ny, nlag = c.L[dir] + 1;
+    S.assign((size_t)Ny * nlag, 0.0);
+    CUDA_TRY(cudaSetDevice(H.device));
+    CUDA_TRY(cudaMemcpyAsync(S.data(), c.sum[dir] + ((size_t)plane * 3 + field) * Ny * nlag, S.size() * sizeof(double), cudaMemcpyDeviceToHost,
+                             H.stream));
+    CUDA_TRY(cudaStreamSynchronize(H.stream));
+    pairs.assign(nlag, 0);
+    for (int d = 0; d < nlag; ++d)
+        pairs[d] = dir == DFB_CORR_Z ? H.corr_count * (c.periodic ? c.W : c.W - d)
+                 : dir == DFB_CORR_Y ? H.corr_count * c.W
+                                     : H.corr_tsteps[d] * c.W;
+}
+
+// correlation coefficients from the sums, in place
+void corr_normalize(const CorrParams& c, int dir, std::vector<double>& S, const std::vector<int64_t>& pairs) {
+    const int Ny = c.Ny, nlag = c.L[dir] + 1;
+    const double nan = std::numeric_limits<double>::quiet_NaN();
+    std::vector<double> var(Ny);
+    for (int j = 0; j < Ny; ++j) var[j] = S[(size_t)j * nlag];
+    for (int j = 0; j < Ny; ++j)
+        for (int d = 0; d < nlag; ++d) {
+            double& r = S[(size_t)j * nlag + d];
+            if (dir == DFB_CORR_Y)
+                r = (j + d >= Ny || var[j] == 0.0 || var[j + d] == 0.0) ? nan : r / std::sqrt(var[j] * var[j + d]);
+            else
+                r = (pairs[d] == 0 || pairs[0] == 0 || var[j] == 0.0) ? nan : (r / (double)pairs[d]) / (var[j] / (double)pairs[0]);
+        }
+}
+
+int corr_check(dfb_handle h, int plane, int field, int dir) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    if (!h->corr_ready) return fail(DFB_ERR_STATE, "correlation statistics are not enabled (dfb_corr_enable)");
+    if (plane < 0 || plane >= h->nplanes) return fail(DFB_ERR_ARG, "plane out of range");
+    if (field < 0 || field > 2) return fail(DFB_ERR_ARG, "field must be 0..2 (u', v', w')");
+    if (dir < 0 || dir > 2) return fail(DFB_ERR_ARG, "direction must be DFB_CORR_Z, DFB_CORR_Y or DFB_CORR_T");
+    if (h->corr.L[dir] == 0) return fail(DFB_ERR_ARG, "that direction was enabled with lag 0 (off)");
+    return DFB_OK;
+}
+
+}  // namespace
+
+int dfb_corr_get_plane(dfb_handle h, int plane, int field, int dir, int normalized, double* dst, int64_t* pairs, int64_t* count) {
+    const int rc = corr_check(h, plane, field, dir);
+    if (rc != DFB_OK) return rc;
+    return guarded([&] {
+        std::vector<double> S;
+        std::vector<int64_t> pr;
+        corr_fetch(*h, plane, field, dir, S, pr);
+        if (normalized) corr_normalize(h->corr, dir, S, pr);
+        if (dst) std::memcpy(dst, S.data(), S.size() * sizeof(double));
+        if (pairs) std::memcpy(pairs, pr.data(), pr.size() * sizeof(int64_t));
+        if (count) *count = h->corr_count;
+    });
+}
+int dfb_corr_get(dfb_handle h, int field, int dir, int normalized, double* dst, int64_t* pairs, int64_t* count) {
+    return dfb_corr_get_plane(h, 0, field, dir, normalized, dst, pairs, count);
+}
+
+int dfb_corr_integral_scales(dfb_handle h, int plane, int field, int dir, double* dst) {
+    const int rc = corr_check(h, plane, field, dir);
+    if (rc != DFB_OK) return rc;
+    if (!dst) return fail(DFB_ERR_ARG, "dst is NULL");
+    return guarded([&] {
+        std::vector<double> R;
+        std::vector<int64_t> pr;
+        corr_fetch(*h, plane, field, dir, R, pr);
+        corr_normalize(h->corr, dir, R, pr);
+        const Plan& P = h->plan;
+        const int Ny = P.Ny, nlag = h->corr.L[dir] + 1;
+        const double wbar = (P.vert_z[P.NzG] - P.vert_z[0]) / P.NzG;
+        for (int j = 0; j < Ny; ++j) {
+            const double* r = R.data() + (size_t)j * nlag;
+            auto x = [&](int d) { return dir == DFB_CORR_Z ? d * wbar : dir == DFB_CORR_Y ? P.yc_row[j + d] - P.yc_row[j] : (double)d; };
+            if (!(r[0] > 0.0)) { dst[j] = std::numeric_limits<double>::quiet_NaN(); continue; }
+            double acc = 0.0;
+            for (int d = 1; d < nlag && r[d] > 0.0; ++d) acc += 0.5 * (r[d - 1] + r[d]) * (x(d) - x(d - 1));
+            dst[j] = acc;
+        }
+    });
+}
 
 // write_csv (df.cpp:764-803), opt-in: header, fixed notation with 15 decimals, one row per cell
 int dfb_write_csv(dfb_handle h, const char* path) {

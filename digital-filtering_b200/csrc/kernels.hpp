@@ -27,4 +27,21 @@ cudaError_t launch_rebuild(double* plane, const double* rowc, int Ny, int NzG, i
 cudaError_t launch_assemble(const double* slab, double* plane, const double* rowc, int Ny, int NzG, int k0, int W, int first_only, cudaStream_t st);
 cudaError_t launch_dfma_peak(double* out, int blocks, int iters, cudaStream_t st);
 
+// correlation statistics (corr.cu, dfb_corr_enable): sums [P][3][Ny][L_d + 1] per direction d = 0 z, 1 y, 2 t
+struct CorrParams {
+    const double* fluc[3];            // u', v', w': dense [P][Ny][W] (W = Nz: whole planes only)
+    int P, Ny, W, periodic;
+    int L[3];                         // lags per direction (0 = off)
+    double* sum[3];
+    double* part;                     // partial sums of the z segments / y column splits (corr_part_doubles)
+    int y_nsplit, y_split_cols;       // corr_y_split
+    double* ring;                     // [L_t][P][3][Ny][W]: the last L_t accumulated fields (allocated while accumulating)
+    long long ring_count;             // fields written into the ring since it was emptied
+};
+void corr_y_split(int Ny, int W, int* nsplit, int* split_cols);
+size_t corr_part_doubles(int P, int Ny, int W, int Lz, int Ly, int nsplit_y);
+cudaError_t launch_corr_z(const CorrParams& p, cudaStream_t st);
+cudaError_t launch_corr_y(const CorrParams& p, cudaStream_t st);
+cudaError_t launch_corr_t(const CorrParams& p, int M, cudaStream_t st);   // lags 0..M (M = min(L_t, ring_count))
+
 }  // namespace dfb

@@ -17,6 +17,7 @@
 !                                                 BASELINE config 4: this rank's spanwise slab + the NCCL hand-off inside the library
 !   config%periodic_z = 1                         spanwise-periodic plane: the z filter wraps around it
 !   face_map, apply_inflow                        N3: inflow face -> plane cell, ghost cell = mean + fluctuation (us3d_user.f90:85-114)
+!   corr_enable, corr_get, integral_scales        correlation statistics along z, y and in time (dfb_corr_*): the delivered scales
 !
 ! NOTE: NEVER COMPILED -- no Fortran compiler exists in the build image or on the GPU boxes.  The binding is exercised through
 ! tests/fortran_abi_mimic.c, a C program that makes exactly these calls with exactly this struct layout and by-reference
@@ -28,6 +29,7 @@ module DIGITAL_FILTERING
     public :: digital_filter_type, create_digital_filter, filter, DFConfig, FilterField, destroy_digital_filter
     public :: digital_filter_batch_type, create_digital_filter_batch, filter_batch
     public :: comm_unique_id, comm_init, gather_begin, gather_end, gathered_field, face_map, apply_inflow
+    public :: corr_enable, corr_get, integral_scales
 
     integer, parameter :: dp = selected_real_kind(15)
 
@@ -155,6 +157,31 @@ module DIGITAL_FILTERING
         integer(c_int) function dfb_destroy_f(handle) bind(C, name='dfb_destroy_f')
             import :: c_int, c_ptr
             type(c_ptr), intent(inout) :: handle
+        end function
+        integer(c_int) function dfb_info(handle, what, field, out64) bind(C, name='dfb_info')
+            import :: c_int, c_ptr, c_int64_t
+            type(c_ptr), value :: handle
+            integer(c_int), value :: what, field
+            integer(c_int64_t), intent(out) :: out64
+        end function
+        integer(c_int) function dfb_corr_enable(handle, on, lags) bind(C, name='dfb_corr_enable')
+            import :: c_int, c_ptr
+            type(c_ptr), value :: handle
+            integer(c_int), value :: on
+            integer(c_int), intent(in) :: lags(3)
+        end function
+        integer(c_int) function dfb_corr_get(handle, field, dir, normalized, dst, pairs, count) bind(C, name='dfb_corr_get')
+            import :: c_int, c_ptr, c_double
+            type(c_ptr), value :: handle
+            integer(c_int), value :: field, dir, normalized
+            real(c_double), intent(inout) :: dst(*)
+            type(c_ptr), value :: pairs, count
+        end function
+        integer(c_int) function dfb_corr_integral_scales(handle, plane, field, dir, dst) bind(C, name='dfb_corr_integral_scales')
+            import :: c_int, c_ptr, c_double
+            type(c_ptr), value :: handle
+            integer(c_int), value :: plane, field, dir
+            real(c_double), intent(inout) :: dst(*)
         end function
         function dfb_last_error() bind(C, name='dfb_last_error') result(msg)
             import :: c_ptr
@@ -314,6 +341,32 @@ contains
             if (cell(i) > 0) q(ghost(i)) = mean(i) + fluc(cell(i))
         end do
     end subroutine apply_inflow
+
+    ! ---- correlation statistics (like the rest of this module, never compiled: see the note at the top) ----
+    subroutine corr_enable(DF, lz, ly, lt)         ! lags along z, y (0 = off, -1 = the filter's whole support) and t (0..64 steps)
+        type(digital_filter_type), intent(inout) :: DF
+        integer, intent(in) :: lz, ly, lt
+        integer(c_int) :: lags(3)
+        lags = [int(lz, c_int), int(ly, c_int), int(lt, c_int)]
+        call check(dfb_corr_enable(DF%handle, 1_c_int, lags), 'corr_enable')
+    end subroutine corr_enable
+
+    subroutine corr_get(DF, field, dir, R)         ! R(0:L, Ny): correlation coefficients of field 0..2 (u', v', w'), dir 0 z, 1 y, 2 t
+        type(digital_filter_type), intent(in) :: DF
+        integer, intent(in) :: field, dir
+        real(kind=dp), allocatable, intent(out) :: R(:, :)
+        integer(c_int64_t) :: L
+        call check(dfb_info(DF%handle, 14_c_int, int(dir, c_int), L), 'corr_get')
+        allocate(R(0:L, DF%Ny))
+        call check(dfb_corr_get(DF%handle, int(field, c_int), int(dir, c_int), 1_c_int, R, c_null_ptr, c_null_ptr), 'corr_get')
+    end subroutine corr_get
+
+    subroutine integral_scales(DF, field, dir, L)  ! L(Ny): per-row integral scale, metres for z and y, steps for t
+        type(digital_filter_type), intent(in) :: DF
+        integer, intent(in) :: field, dir
+        real(kind=dp), intent(inout) :: L(:)
+        call check(dfb_corr_integral_scales(DF%handle, 0_c_int, int(field, c_int), int(dir, c_int), L), 'integral_scales')
+    end subroutine integral_scales
 
     subroutine destroy_digital_filter(DF)
         type(digital_filter_type), intent(inout) :: DF

@@ -121,7 +121,8 @@ int dfb_dims(dfb_handle h, int* Ny, int* Nz);
  * 10 form of the y-sweep in use: 2 = run-recursive (every row group through the exponential window), 3 = run-recursive on the blocks of
  *    32 rows where it pays + dense band matrices on the rest (e.g. a batch of planes of the reference's default geometry), 1 = chunk-recursive band-matrix
  *    kernel, 0 = dense band matrices (DFB_Y_MODE=0|1|2 forces a form), 11 tiles of the run-recursive kernel, 12 transport of the config-4 hand-off: 2 = peer-to-peer copies (CUDA IPC + copy engines), 1 = NCCL
- *    send/recv, 0 = no communicator, 13 spanwise-periodic plane (dfb_config.periodic_z) in use (0/1) */
+ *    send/recv, 0 = no communicator, 13 spanwise-periodic plane (dfb_config.periodic_z) in use (0/1),
+ * 14 lags of correlation direction `field` (0 z, 1 y, 2 t; dfb_corr_enable), 0 when that direction is off or before any enable */
 int dfb_info(dfb_handle h, int what, int field, int64_t* out64);
 /* host copies of the setup tables (for parity tests): which = 0..7 rows R11,R21,R22,R33,Us,Ts,rhos,Ms [Ny];
  * 8 yc row [Ny]; 9 dy row [Ny]; 10 Lt[3]; 11 coefficients of half-width `arg` [2*arg+1];
@@ -226,6 +227,43 @@ int dfb_stats_get_plane(dfb_handle h, int plane, int which, int as_rms, double* 
  * steps (the reference: 500 steps of dt = 1e-5) accumulating on the device.  Results through dfb_stats_get(.., as_rms = 1, ..)
  * and dfb_write_rms_csv. */
 int dfb_get_rms(dfb_handle h, int nsteps, double dt);
+/* Correlation statistics -- does the generated field carry the integral scales it was configured with?  Opt-in: after
+ * dfb_corr_enable(h, 1, lags) every dfb_filter (directly, or through _to_host, _begin, dfb_filter_batch, dfb_get_rms -- the steps N2
+ * accumulates; not the constructor's step, not dfb_first_step) adds, on the handle's stream, per-row sums of lagged products of u', v'
+ * and w' (field = 0, 1, 2; the fluc arrays, after blending and Lund scaling).  With f_s = field `field` of plane `plane` after
+ * accumulated step s, L_d = lags[d], and per row j, summed over the columns k and over the accumulated steps:
+ *   DFB_CORR_Z  S_z[j][d] = sum f(j,k) f(j,k+d),    d = 0..L_z; without periodic_z only k + d < Nz counts, with it the column
+ *                                                    is (k+d) mod Nz and all Nz columns count
+ *   DFB_CORR_Y  S_y[j][d] = sum f(j,k) f(j+d,k),    d = 0..L_y, j + d < Ny (one-sided: (j, j+d) gives the full two-point function)
+ *   DFB_CORR_T  S_t[j][m] = sum f_s(j,k) f_{s-m}(j,k), m = 0..L_t; step s contributes to lag m only if step s-m was accumulated
+ *                                                    too (a device ring holds the last L_t fields: L_t * nplanes * 3 * Ny * Nz doubles)
+ * Lags: 0 turns a direction off; DFB_CORR_SUPPORT = the filter's whole support, where the expected correlation ends: z max over the
+ * fields of 2 Nz_max, capped at Nz-1; y max of 2 Ny_max, capped at Ny-1 (DFB_ERR_ARG for t).  Otherwise 0 <= L_z <= Nz-1,
+ * 0 <= L_y <= Ny-1, 0 <= L_t <= 64, else DFB_ERR_ARG.  Every field uses the same lags: dst is [Ny][L_d+1].
+ * Whole planes only: a slab handle (k_begin/k_end narrower than the plane) gets DFB_ERR_ARG, "correlation statistics need the whole
+ * plane" -- the spanwise sums need the neighbours' columns.  Single planes and batches, every kernel form, both periodic_z modes.
+ * When they are off nothing is launched. */
+enum { DFB_CORR_Z = 0, DFB_CORR_Y = 1, DFB_CORR_T = 2 };
+#define DFB_CORR_SUPPORT (-1)
+/* on = 1: allocates the sums (on the first call, or when the lags change), the ring and a scratch of partial sums (whenever they are
+ * absent; a failed allocation is DFB_ERR_CUDA with a message), zeroes the sums, empties the ring and sets count = 0.  on = 0: stops
+ * accumulating and frees the ring and the scratch; the sums stay readable (lags may be NULL).  Every valid lag fits the kernels'
+ * shared memory: the z kernel stages its lag halo one block of lags at a time.
+ * dfb_set_state empties the ring and keeps the sums: the next step follows the restored state, not the ring.
+ * dfb_info selector 14 gives L_d of direction `field` (0 z, 1 y, 2 t) once enabled, 0 for an off direction and before any enable. */
+int dfb_corr_enable(dfb_handle h, int on, const int lags[3]);
+/* normalized = 0: the raw sums.  normalized = 1: correlation coefficients, z and t (S[j][d]/pairs[d]) / (S[j][0]/pairs[0]),
+ * y S_y[j][d] / sqrt(S_y[j][0] S_y[j+d][0]); NaN where j + d >= Ny, where a variance is 0 (u' on rows with R11 = 0) or where a lag
+ * has no pairs yet.  pairs (optional, [L_d+1]) = products per row behind each lag: z steps*(Nz-d) without periodic_z, steps*Nz with
+ * it; y steps*Nz; t Nz times the number of steps that had a predecessor m steps back.  count (optional) = accumulated steps.
+ * dst may be NULL.  Before any enable: DFB_ERR_STATE.  A field, direction (or one enabled with lag 0) or plane out of range: DFB_ERR_ARG. */
+int dfb_corr_get(dfb_handle h, int field, int dir, int normalized, double* dst, int64_t* pairs, int64_t* count);
+int dfb_corr_get_plane(dfb_handle h, int plane, int field, int dir, int normalized, double* dst, int64_t* pairs, int64_t* count);
+/* Integral scale per row j from the normalised R: with d* the last lag such that R(e) > 0 for every e <= d*,
+ * dst[j] = sum_{d=1..d*} (R(d-1) + R(d))/2 * (x(d) - x(d-1)), where x(d) = d * wbar for z, wbar = (z_v[NzG] - z_v[0]) / NzG of the
+ * vertex table (dfb_get_table 13), metres; x(d) = yc[j+d] - yc[j] for y (dfb_get_table 8), metres, upward; x(m) = m for t, in steps
+ * (multiply by dt).  NaN for a row with zero variance.  Host arithmetic on the copied-back sums, the same for every facade. */
+int dfb_corr_integral_scales(dfb_handle h, int plane, int field, int dir, double* dst /* [Ny] */);
 /* plot_rms (df.cpp:613-675): "z, y, u'_rms, v'_rms, w'_rms, T'_rms, rho'_rms " then one row per cell with the cell's lower-left VERTEX
  * coordinates (z[iidx], y[iidx]), default stream formatting (6 significant digits), ", " separators */
 int dfb_write_rms_csv(dfb_handle h, const char* path);

@@ -122,6 +122,25 @@ class DIGITAL_FILTER {
     }
     void write_csv(const std::string& filename) { check(dfb_write_csv(h_, filename.c_str())); std::printf("CSV written to %s\n", filename.c_str()); }   // df.cpp:764-803
     void write_tecplot(const std::string& filename) { check(dfb_write_tecplot(h_, filename.c_str())); std::printf("Finished plotting.\n"); }           // df.cpp:712-762
+    // correlation statistics (dfb_corr_enable): lags along z, y (0 = off, DFB_CORR_SUPPORT = the filter's support) and t (0..64 steps)
+    void corr_enable(int lz, int ly, int lt) {
+        const int lags[3] = {lz, ly, lt};
+        check(dfb_corr_enable(h_, 1, lags));
+    }
+    // [Ny][L+1] of field 0..2 (u', v', w') in direction DFB_CORR_Z / _Y / _T: correlation coefficients, or the raw sums
+    std::vector<double> corr(int field, int dir, bool normalized = true, int plane = 0) {
+        std::int64_t L = 0;
+        check(dfb_info(h_, 14, dir, &L));
+        std::vector<double> R((size_t)Ny * (size_t)(L + 1));
+        check(dfb_corr_get_plane(h_, plane, field, dir, normalized ? 1 : 0, R.data(), nullptr, nullptr));
+        return R;
+    }
+    // per-row integral scale: metres for z and y, steps for t
+    std::vector<double> integral_scales(int field, int dir, int plane = 0) {
+        std::vector<double> L(Ny);
+        check(dfb_corr_integral_scales(h_, plane, field, dir, L.data()));
+        return L;
+    }
     const Vector& T_rms() const { return T_rms_; }
     const Vector& rho_rms() const { return rho_rms_; }
     int rms_counter = 0;               // df.hpp:63
