@@ -1017,6 +1017,8 @@ void run_step(dfb_filter_s& H, double dt, bool first) {
     if (H.noise_mode == DFB_NOISE_GENERATE && H.overlap && !H.timing) {
         const int nb = (int)(H.step & 1);
         CUDA_TRY(cudaStreamWaitEvent(H.side, H.ev_free[nb], 0));     // readers of that set (step-2... ) are done
+        CUDA_TRY(cudaStreamWaitEvent(H.side, H.ev_noise[nb], 0));    // ... and so is its last writer: a dfb_generate_noise into it
+                                                                       // on the main stream after that step would otherwise race this one
         launch_noise_for(H, H.step, nb, H.side);
         // ... and so does its y-sweep (it reads only that noise and writes only that set's r_zs interior): it
         // becomes resident as this step's z-sweep CTAs retire and keeps the fp64 pipe busy through the tail.
@@ -1048,6 +1050,15 @@ const double* field_ptr0(const dfb_filter_s& H, int which) {
 const double* field_ptr(const dfb_filter_s& H, int which, int plane = 0) {
     const double* p = field_ptr0(H, which);
     return p ? p + (size_t)plane * H.D[0].ps_cells : nullptr;
+}
+
+// dt < 0 gives alpha = exp(-pi dt / Lt) > 1 and sqrt(1 - alpha) = NaN, a NaN dt NaN as well: either would turn every field, filt_old
+// and the statistics into NaN for good.  Checked before a step enqueues anything, so a refused call leaves the handle as it was.
+void check_dt(double dt) {
+    if (std::isfinite(dt) && dt >= 0.0) return;
+    char buf[64];
+    std::snprintf(buf, sizeof(buf), "%g", dt);
+    throw Error{DFB_ERR_ARG, std::string("dt must be finite and >= 0, got ") + buf};
 }
 
 template <class Fn>
@@ -1215,7 +1226,7 @@ int dfb_get_half_widths(dfb_handle h, int field, int dir, int* dst) {
 
 int dfb_filter(dfb_handle h, double dt) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
-    return guarded([&] { run_step(*h, dt, false); });
+    return guarded([&] { check_dt(dt); run_step(*h, dt, false); });
 }
 
 int dfb_first_step(dfb_handle h) {   // constructor semantics on demand (inject mode / after dfb_set_state(.., 0))
@@ -1241,6 +1252,7 @@ int dfb_get_field(dfb_handle h, int which, double* dst, int dst_on_device) { ret
 int dfb_filter_to_host(dfb_handle h, double dt, double* u, double* v, double* w, double* T, double* rho) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     return guarded([&] {
+        check_dt(dt);
         run_step(*h, dt, false);
         const size_t bytes = sizeof(double) * h->D[0].ps_cells * h->nplanes;     // a batch delivers [P][Ny*Nz] per field
         double* dst[5] = {u, v, w, T, rho};
@@ -1253,6 +1265,7 @@ int dfb_filter_to_host(dfb_handle h, double dt, double* u, double* v, double* w,
 int dfb_filter_to_host_begin(dfb_handle h, double dt, double* u, double* v, double* w, double* T, double* rho) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     return guarded([&] {
+        check_dt(dt);
         if (h->pipe_begun - h->pipe_ended >= 2) throw Error{DFB_ERR_STATE, "two dfb_filter_to_host_begin calls are already outstanding: call dfb_filter_to_host_end first"};
         CUDA_TRY(cudaSetDevice(h->device));
         const size_t n = h->D[0].ps_cells * h->nplanes, bytes = n * sizeof(double);
@@ -1293,6 +1306,7 @@ int dfb_filter_to_host_end(dfb_handle h) {
 int dfb_filter_batch(dfb_handle h, int nsteps, const double* dt, double* out) {
     if (!h || !dt || nsteps < 0) return fail(DFB_ERR_ARG, "bad argument");
     return guarded([&] {
+        for (int s = 0; s < nsteps; ++s) check_dt(dt[s]);            // the whole array before the first step
         const size_t n = h->D[0].ps_cells * h->nplanes;
         for (int s = 0; s < nsteps; ++s) {
             run_step(*h, dt[s], false);
@@ -1738,7 +1752,9 @@ int dfb_write_tecplot(dfb_handle h, const char* path) {
 // get_rms (df.cpp:584-611): reset the sums, `nsteps` steps with accumulation (on the device, in the z-sweep's epilogue)
 int dfb_get_rms(dfb_handle h, int nsteps, double dt) {
     if (!h || nsteps < 0) return fail(DFB_ERR_ARG, "bad argument");
-    int rc = dfb_stats_enable(h, 1);
+    int rc = guarded([&] { check_dt(dt); });         // before dfb_stats_enable zeroes the sums
+    if (rc != DFB_OK) return rc;
+    rc = dfb_stats_enable(h, 1);
     if (rc != DFB_OK) return rc;
     return guarded([&] {
         for (int i = 0; i < nsteps; ++i) run_step(*h, dt, false);

@@ -254,7 +254,7 @@ contains
         call check(dfb_get_field(DF%handle, 2_c_int, DF%w%fluc, 0_c_int), 'dfb_get_field')
     end function create_digital_filter
 
-    ! df.f90:621-651
+    ! df.f90:621-651.  dt_input must be finite and >= 0: otherwise the library returns DFB_ERR_ARG (check stops) and changes nothing.
     subroutine filter(DF, dt_input)
         type(digital_filter_type), intent(inout) :: DF
         real(kind=dp), intent(in) :: dt_input

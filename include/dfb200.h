@@ -132,7 +132,12 @@ int dfb_get_table(dfb_handle h, int which, int arg, double* dst, int cap);
 int dfb_get_half_widths(dfb_handle h, int field, int dir, int* dst);
 
 /* DIGITAL_FILTER::filter(double dt_input) df.cpp:449-468 -- enqueues the whole step on the handle's
- * stream and returns; no print, no CSV (SURVEY quirk 8).  Results are read with dfb_get_field. */
+ * stream and returns; no print, no CSV (SURVEY quirk 8).  Results are read with dfb_get_field.
+ * dt must be finite and >= 0 (here and in dfb_filter_to_host, _begin, dfb_get_rms, every entry of dfb_filter_batch's array, and the
+ * _f entry points): otherwise DFB_ERR_ARG and nothing is enqueued -- the step counter, the fields, filt_old, the noise and the N2 and
+ * correlation statistics stay as they were; dfb_filter_batch checks its whole array before the first step.  (A negative dt would give
+ * the blend alpha = exp(-pi dt / Lt) > 1 and sqrt(1 - alpha) = NaN.)  dt = 0 gives alpha = 1: filt = filt_old; dt >> Lt gives
+ * alpha = 0: no blend, the step of dfb_first_step. */
 int dfb_filter(dfb_handle h, double dt);
 /* The constructor's first step on demand (df.cpp:57-62: sweeps + RST scaling, no blend, T'/rho' untouched).
  * dfb_create runs it by itself in generate mode; in inject mode call it after the first dfb_set_noise x3. */

@@ -77,7 +77,7 @@ class DIGITAL_FILTER {
         if (h_) dfb_destroy(h_);
     }
 
-    // df.hpp:100, df.cpp:449-468
+    // df.hpp:100, df.cpp:449-468.  dt_input must be finite and >= 0: otherwise check() throws (DFB_ERR_ARG) and nothing changes.
     void filter(double dt_input) {
         dt = dt_input;
         if (fetch_)
