@@ -197,6 +197,38 @@ class DFConfig:
 dc_config = DFConfig
 
 
+def fill_config(c, config):
+    """Fills the ctypes `dfb_config` c (initialised by dfb_config_init) from a DFConfig.  Returns the arrays c points into: keep
+    them alive as long as c is used."""
+    keep = []
+
+    def arr(a, dtype):
+        if a is None:
+            return None
+        a = np.ascontiguousarray(a, dtype=dtype)
+        keep.append(a)
+        return a
+
+    c.d_i, c.rho_e, c.U_e, c.mu_e = config.d_i, config.rho_e, config.U_e, config.mu_e
+    c.vel_file_offset, c.vel_file_N_values = config.vel_file_offset, config.vel_file_N_values
+    c.grid_file = config.grid_file.encode() if config.grid_file else None
+    c.vel_fluc_file = config.vel_fluc_file.encode() if config.vel_fluc_file else None
+    c.line_file = config.line_file.encode() if config.line_file else None
+    c.honor_flow_config = config.honor_flow_config
+    c.Ny, c.Nz, c.geom_per_row = config.Ny, config.Nz, config.geom_per_row
+    for name in ("yc", "dy", "dz", "rows", "scales"):
+        a = arr(getattr(config, name), np.float64)
+        setattr(c, name, _dptr(a))
+    for name in ("N_y", "N_z"):
+        a = arr(getattr(config, name), np.int32)
+        setattr(c, name, a.ctypes.data_as(c_ip) if a is not None else None)
+    c.seed, c.noise_mode, c.device, c.plane_id = config.seed, config.noise_mode, config.device, config.plane_id
+    c.k_begin, c.k_end = config.k_begin, config.k_end
+    c.skip_first_step, c.kernel_variant = config.skip_first_step, config.kernel_variant
+    c.periodic_z = config.periodic_z
+    return keep
+
+
 class FilterField:
     """Host view of one velocity component (df.hpp:24-34): .fluc and .filt, Ny x Nz, row-major j*Nz+k."""
 
@@ -234,32 +266,7 @@ class DIGITAL_FILTER:
         L = lib()
         c = dfb_config()
         _check(L.dfb_config_init(C.byref(c)))
-        self._keep = []
-
-        def arr(a, dtype):
-            if a is None:
-                return None
-            a = np.ascontiguousarray(a, dtype=dtype)
-            self._keep.append(a)
-            return a
-
-        c.d_i, c.rho_e, c.U_e, c.mu_e = config.d_i, config.rho_e, config.U_e, config.mu_e
-        c.vel_file_offset, c.vel_file_N_values = config.vel_file_offset, config.vel_file_N_values
-        c.grid_file = config.grid_file.encode() if config.grid_file else None
-        c.vel_fluc_file = config.vel_fluc_file.encode() if config.vel_fluc_file else None
-        c.line_file = config.line_file.encode() if config.line_file else None
-        c.honor_flow_config = config.honor_flow_config
-        c.Ny, c.Nz, c.geom_per_row = config.Ny, config.Nz, config.geom_per_row
-        for name in ("yc", "dy", "dz", "rows", "scales"):
-            a = arr(getattr(config, name), np.float64)
-            setattr(c, name, _dptr(a))
-        for name in ("N_y", "N_z"):
-            a = arr(getattr(config, name), np.int32)
-            setattr(c, name, a.ctypes.data_as(c_ip) if a is not None else None)
-        c.seed, c.noise_mode, c.device, c.plane_id = config.seed, config.noise_mode, config.device, config.plane_id
-        c.k_begin, c.k_end = config.k_begin, config.k_end
-        c.skip_first_step, c.kernel_variant = config.skip_first_step, config.kernel_variant
-        c.periodic_z = config.periodic_z
+        self._keep = fill_config(c, config)
         self._h = C.c_void_p()
         self.nplanes = int(nplanes)
         if self.nplanes == 1:

@@ -24,6 +24,16 @@ constexpr int YJ = 8;          // output rows per thread / per row group of the 
 constexpr int Y_G = 4;         // row groups (consumer warps) per y-sweep tile: 32 output rows share one sample stream
 constexpr int Y_TK = 128;      // columns per y-sweep tile (each lane owns 4 of them)
 constexpr int DFB_MAXP = 16;   // planes one handle can advance in one launch set (dfb_create_batch)
+constexpr int Y_RC = 8;        // padded rows per chunk of the band-matrix y-sweep (ysweep_tma_kernel, ysweep_rec_kernel)
+constexpr int Y_NS = 6;        // chunks it keeps in flight
+// pairs per thread of the noise kernel, NOISE_THREADS pairs apart (one position jump per thread, stride jumps between its pairs).  Measured
+// ms/step on 1024x2048 / 4096x8192 profile, pairs and NOISE_UNROLL: 4, 1: 0.1170 / 1.537; 4, 2: 0.1151 / 1.526; 4, 4: 0.1144 / 1.499; 8, 2: 0.1146 / 1.472
+#ifndef NOISE_PAIRS
+#define NOISE_PAIRS 8
+#endif
+#ifndef NOISE_THREADS
+#define NOISE_THREADS 128
+#endif
 
 struct FieldDev {
     int Ny_max, Nz_max;
@@ -103,6 +113,16 @@ struct YRTile {                // row block x 32 columns of one field; its whole
     int wlo, wrows;            // first padded row and row count of the window (union of the groups' windows)
 };
 struct YRMaps { CUtensorMap m[3]; };   // r_ys[f] with box {YR_C columns, YR_BOX rows}
+struct YRSmemCtl {                       // control block in front of the two window buffers
+    uint64_t full[2], empty[2];
+    int next_group[2];
+    YRTile tile[2];
+    int plane[2];
+    int pad[2];
+    alignas(16) YRGroup groups[2][YR_MAXG];      // cp.async.bulk destination
+};
+// dynamic shared memory of ysweep_run_kernel for `nbuf` window buffers of `wrows` rows
+inline size_t ysweep_run_smem(int wrows, int nbuf) { return (sizeof(YRSmemCtl) + 127) / 128 * 128 + (size_t)nbuf * wrows * YR_C * sizeof(double); }
 
 struct StepConsts {
     double sa[3], sb[3];       // sqrt(alpha), sqrt(1-alpha) per field (df.cpp:412-415), from the host's exp/sqrt
@@ -195,7 +215,6 @@ struct ZParams {
     int rc_off, fo_off;          // offsets of the row constants (64 B) and of the staged filt_old strip (32 lines) in a staging buffer
     int nblocks;
     int smem_bytes;
-    int n_sm;
     unsigned long long* tl;      // development aid (DFB_TIMELINE), see NoiseParams
     int zmode;                   // 0: direct Toeplitz tap loop; 1: recursive evaluation of the exponential window
     int debug;                   // development probes only (0 in production)

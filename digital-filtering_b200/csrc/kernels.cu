@@ -14,6 +14,7 @@
 #include <cstdint>
 #include <cstdlib>
 #include <cstdio>
+#include <utility>
 #include "noise.cuh"
 #include "device.cuh"
 #include "kernels.hpp"
@@ -22,19 +23,11 @@
 #ifndef Z_REC_MAXNREG
 #define Z_REC_MAXNREG 168
 #endif
-// pairs per thread of the noise kernel, NOISE_THREADS pairs apart (one position jump per thread, stride jumps between its pairs), two
-// in flight at a time (NOISE_UNROLL: the pair transform is one long dependent chain; with the run-recursive y-sweep and the z-sweep
-// resident beside it the noise kernel gets few warps per scheduler and needs the instruction-level parallelism).
-// Measured ms/step on 1024x2048 profile / 4096x8192 profile: pairs 4 unroll 1: 0.1170 / 1.537; 4, 2: 0.1151 / 1.526; 4, 4: 0.1144 / 1.499;
-// 8, 2: 0.1146 / 1.472
-#ifndef NOISE_PAIRS
-#define NOISE_PAIRS 8
-#endif
+// pair transforms of the noise kernel in flight at a time (NOISE_PAIRS, NOISE_THREADS: device.cuh): the transform is one long
+// dependent chain; with the run-recursive y-sweep and the z-sweep resident beside it the noise kernel gets few warps per scheduler
+// and needs the instruction-level parallelism
 #ifndef NOISE_UNROLL
 #define NOISE_UNROLL 2
-#endif
-#ifndef NOISE_THREADS
-#define NOISE_THREADS 128
 #endif
 
 namespace dfb {
@@ -618,15 +611,6 @@ __global__ void __launch_bounds__(160, 3) ysweep_rec_kernel(const __grid_constan
 // Bound by shared-memory bandwidth (one 8-byte sample per FMA), not by the fp64 pipe.
 // Agreement with the reference's sequential sum: ~1e-15 of the rms (gate 1e-12).
 // =================================================================================================
-struct YRSmemCtl {                       // control block in front of the two window buffers
-    uint64_t full[2], empty[2];
-    int next_group[2];
-    YRTile tile[2];
-    int plane[2];
-    int pad[2];
-    alignas(16) YRGroup groups[2][YR_MAXG];      // cp.async.bulk destination
-};
-
 __global__ void __launch_bounds__(32 * (YR_CONSUMERS + 1), 1) ysweep_run_kernel(const __grid_constant__ YRMaps maps, const YParams P) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     YRSmemCtl& ctl = *reinterpret_cast<YRSmemCtl*>(smem_raw);
@@ -1420,39 +1404,21 @@ cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, cudaStr
     return cudaGetLastError();
 }
 
-constexpr int Y_RC = 8, Y_NS = 6;
-
-size_t ysweep_smem_bytes() { return sizeof(YSmem<Y_RC, Y_NS>); }
-int noise_threads() { return NOISE_THREADS * NOISE_PAIRS; }
-int noise_stride_pairs() { return NOISE_THREADS; }
-int ysweep_rc() { return Y_RC; }
-
 cudaError_t ysweep_prepare() {
     // One shared-memory carve-out for every kernel of the step: an SM only changes its L1 / shared split when it is idle, so a
     // noise CTA running with the default split beside the sweeps could leave an SM unable to take its third y-sweep CTA (observed
-    // as a process-wide bimodal y-sweep time on small planes: 26 or 43 us on the reference default plane).
-    {
-        cudaError_t e0 = cudaFuncSetAttribute(noise_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        if (e0 != cudaSuccess) return e0;
-        e0 = cudaFuncSetAttribute(noise_pieces_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        if (e0 != cudaSuccess) return e0;
-        e0 = cudaFuncSetAttribute(stats_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        if (e0 != cudaSuccess) return e0;
-        e0 = cudaFuncSetAttribute(scatter_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        if (e0 != cudaSuccess) return e0;
+    // as a process-wide bimodal y-sweep time on small planes: 26 or 43 us on the reference default plane).  {kernel, dynamic smem}
+    const std::pair<const void*, int> fns[] = {
+        {(const void*)noise_kernel, 0}, {(const void*)noise_pieces_kernel, 0}, {(const void*)stats_kernel, 0}, {(const void*)scatter_kernel, 0},
+        {(const void*)ysweep_tma_kernel<Y_RC, Y_NS, 128>, (int)sizeof(YSmem<Y_RC, Y_NS, 128>)},
+        {(const void*)ysweep_tma_kernel<Y_RC, Y_NS, 64>, (int)sizeof(YSmem<Y_RC, Y_NS, 64>)},
+        {(const void*)ysweep_rec_kernel<Y_RC, Y_NS>, (int)sizeof(YSmem<Y_RC, Y_NS>)}};
+    for (const auto& [fn, smem] : fns) {
+        cudaError_t e = smem ? cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) : cudaSuccess;
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e != cudaSuccess) return e;
     }
-    cudaError_t e = cudaFuncSetAttribute(ysweep_tma_kernel<Y_RC, Y_NS, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)sizeof(YSmem<Y_RC, Y_NS, 128>));
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(ysweep_tma_kernel<Y_RC, Y_NS, 128>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(ysweep_tma_kernel<Y_RC, Y_NS, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(YSmem<Y_RC, Y_NS, 64>));
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(ysweep_tma_kernel<Y_RC, Y_NS, 64>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(ysweep_rec_kernel<Y_RC, Y_NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(YSmem<Y_RC, Y_NS>));
-    if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(ysweep_rec_kernel<Y_RC, Y_NS>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    return cudaSuccess;
 }
 
 static cudaLaunchConfig_t pdl_config(unsigned grid, unsigned block, size_t smem, cudaStream_t st, cudaLaunchAttribute* attr) {
@@ -1489,8 +1455,6 @@ cudaError_t launch_ysweep_tma(const YMaps& maps, const YParams& P, int n_dense, 
     }
     return cudaSuccess;
 }
-
-size_t ysweep_run_smem(int wrows, int nbuf) { return (sizeof(YRSmemCtl) + 127) / 128 * 128 + (size_t)nbuf * wrows * YR_C * sizeof(double); }
 
 cudaError_t ysweep_run_prepare(size_t smem) {
     cudaError_t e = cudaFuncSetAttribute(ysweep_run_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -7,15 +7,10 @@ namespace dfb {
 cudaError_t launch_noise(const NoiseParams& P, const NoiseWindows& Wn, const PlaneDev& D, cudaStream_t st);
 cudaError_t launch_ysweep_simple(const PlaneDev& D, cudaStream_t st);
 cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, cudaStream_t st);
-size_t ysweep_smem_bytes();
-int noise_stride_pairs();     // pairs between two consecutive pairs of one thread (NoiseParams::stride = jump over 4x that many draws)
-int noise_threads();          // CTA size of noise_kernel (NoiseParams::chunks = ceil(max_np / noise_threads()))
-int ysweep_rc();
 cudaError_t ysweep_prepare();
 // dense band-matrix tiles [0, n_dense) with ysweep_tma_kernel, then recursive tiles [n_dense, n_dense + n_rec) with ysweep_rec_kernel
 cudaError_t launch_ysweep_tma(const YMaps& maps, const YParams& P, int n_dense, int n_rec, cudaStream_t st);
 // run-recursive y-sweep (every row group through the exponential structure; resident window tiles)
-size_t ysweep_run_smem(int wrows, int nbuf);   // dynamic shared memory for `nbuf` window buffers of `wrows` rows
 cudaError_t ysweep_run_prepare(size_t smem);
 cudaError_t launch_ysweep_run(const YRMaps& maps, const YParams& P, cudaStream_t st);
 cudaError_t zsweep_prepare(int zk, int mode, size_t smem, int* blocks_per_sm);

@@ -329,6 +329,7 @@ void build_plan(const dfb_config& cfg, Plan& P) {
     // ---- spanwise-periodic plane: a window may wrap at most once around the plane ----
     if (cfg.periodic_z != 0 && cfg.periodic_z != 1) throw Error{DFB_ERR_ARG, "periodic_z must be 0 or 1"};
     P.periodic = cfg.periodic_z == 1;
+    P.kernel_variant = cfg.kernel_variant;
     if (P.periodic)
         for (int f = 0; f < 3; ++f)
             if (P.f[f].Nz_max > NzG)
