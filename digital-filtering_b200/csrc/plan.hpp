@@ -68,7 +68,7 @@ struct NoiseTable {                              // segments of one logical arra
 // What a handle's step needs that follows from the plan and the device's limits alone, as host values: the layout, the work of
 // the tuned sweeps (tuned only) and the noise tables.  The pointers in D, yp, zp and np are null: the caller uploads.
 struct StepPlan {
-    bool tuned = false;                          // row-uniform half-widths: the tuned sweeps (else the one-thread-per-cell kernels)
+    bool tuned = false;                          // row-uniform half-widths whose z window fits: the tuned sweeps (else the one-thread-per-cell kernels)
     PlaneDev D{};
     std::vector<double> rowc;                    // [Ny][ROWC]
     int y_form = 0;                              // dfb_info 10: 0 dense band matrices, 1 chunk-recursive, 2 run-recursive, 3 run + dense

@@ -387,7 +387,11 @@ void plan_y(const Plan& P, int NP, const DeviceLimits& dev, const Overrides& ovr
     }
 }
 
-void plan_z(const Plan& P, const Overrides& ovr, StepPlan& S) {
+// Plans the tuned z-sweep; false when its staged window does not fit (more than 256 lines, the largest box of a tensor map, or
+// more shared memory than one block may opt in to): the handle then runs the general kernels.  Whether it fits follows from the
+// half-widths and the lane blocking alone, so slabs on 16-column boundaries decide as their plane does.  A window that does not
+// fit under a forced DFB_ZK or DFB_Z_MODE is an error.
+bool plan_z(const Plan& P, const DeviceLimits& dev, const Overrides& ovr, StepPlan& S) {
     ZParams& Z = S.zp;
     const int Ny = P.Ny, W = P.Nz();
     // outputs per lane: 16 (fewest LDS per DFMA) unless the plane is narrower than one 512-column strip
@@ -446,7 +450,12 @@ void plan_z(const Plan& P, const Overrides& ovr, StepPlan& S) {
     Z.unit_bytes = round_up(Z.fo_off + 32 * ZKc * 8, ZKc == 16 ? 1024 : 512);   // the swizzle pattern repeats every 1024 (512) bytes
     // per warp: two staging buffers + the u line buffer (32 lines); then mbarriers, item descriptors (2 x 2 x 8 ints per warp), alignment slack
     Z.smem_bytes = 4 * (2 * Z.unit_bytes + 32 * ZKc * 8) + 64 + 4 * 32 * 4 + 1024;
-    if (maxlines > 256) throw Error{DFB_ERR_ARG, "z half-width too large for the staged window"};
+    if (maxlines > 256 || (size_t)Z.smem_bytes > dev.smem_optin) {
+        if (!ovr.zk && !ovr.z_mode) return false;
+        throw Error{DFB_ERR_ARG, "z half-width too large for the tuned z-sweep under DFB_ZK / DFB_Z_MODE: its staged window needs " +
+                                 std::to_string(maxlines) + " lines (at most 256) and " + std::to_string(Z.smem_bytes) +
+                                 " bytes of shared memory, the device allows " + std::to_string(dev.smem_optin)};
+    }
     // Work items pulled from a counter by the persistent warps: per (row, strip) the pair of units (u, v) -- v' needs u's
     // blended field (df.cpp:437), which the u unit leaves in the warp's shared-memory line buffer for the v unit that
     // follows it -- and the unit w as an item of its own.
@@ -493,6 +502,7 @@ void plan_z(const Plan& P, const Overrides& ovr, StepPlan& S) {
     }
     Z.n_uv = (int)items.size();
     Z.n_items = 2 * (int)items.size();
+    return true;
 }
 
 // ---- noise tables (include/dfb_rng_spec.h) ----
@@ -589,10 +599,11 @@ StepPlan plan_step(const Plan& P, int NP, const DeviceLimits& dev, const Overrid
         F.ps_ys = (size_t)F.rows_y * F.pitch_y;
         F.ps_zs = (size_t)Ny * F.pitch_z;
     }
-    if (S.tuned) {
-        plan_y(P, NP, dev, ovr, S);
-        plan_z(P, ovr, S);
+    if (S.tuned && !plan_z(P, dev, ovr, S)) {
+        S.tuned = false;
+        S.zp = ZParams{}; S.coef_pad.clear(); S.coef_pad_ptr.clear();
     }
+    if (S.tuned) plan_y(P, NP, dev, ovr, S);
     plan_noise(P, S);
     return S;
 }

@@ -88,7 +88,8 @@ typedef struct dfb_config {
                                    reproduce the single-GPU plane bit for bit with no halo exchange
                                    (periodic_z included: a wrapped neighbour column is regenerated locally too). */
     int skip_first_step;        /* 1: do not run the constructor's first step (df.cpp:57-62) */
-    int kernel_variant;         /* 0 = tuned kernels; 1 = simple cross-check kernels (same maths, one thread per cell) */
+    int kernel_variant;         /* 0 = tuned kernels where they apply (row-uniform half-widths whose z window fits in shared memory,
+                                 * dfb_info 3); 1 = simple cross-check kernels (same maths, one thread per cell) */
     int periodic_z;             /* 0 (default): the reference's plane, NOT periodic in z -- the z filter reads raw white noise for
                                    the Nz_max columns beyond each spanwise edge (SURVEY quirk 1);
                                    1: spanwise-periodic plane -- the z filter wraps, filt[j,k] = sum_i b_i * y_filtered[j, (k+i) mod Nz],
@@ -114,7 +115,12 @@ int dfb_num_planes(dfb_handle h, int* nplanes);
 
 /* plane size as the reference ends up with it (Ny trimmed, df.cpp:282-288); Nz is this handle's slab width */
 int dfb_dims(dfb_handle h, int* Ny, int* Nz);
-/* what = 0 Ny_max, 1 Nz_max (per field f), 2 step counter, 3 row-uniform fast path in use (0/1),
+/* what = 0 Ny_max, 1 Nz_max (per field f), 2 step counter, 3 row-uniform fast path in use (0/1): 0 for per-cell half-widths,
+ *    kernel_variant = 1, or a z window too wide for shared memory -- on a B200 (232 448 bytes per block) the tuned z-sweep takes
+ *    N_z <= 1120 in its recursive form and N_z <= 544 in its direct form (a row with N_z = 0, a slab cut off a 16-column boundary)
+ *    with 16 outputs per lane (planes of >= 384 columns), N_z <= 888 / 720 with 8; a wider window runs the whole handle on the
+ *    one-thread-per-cell kernels, which take any half-width (DFB_ZK / DFB_Z_MODE forcing a window that does not fit: DFB_ERR_ARG),
+ *    while any N_y runs on the tuned y-sweep (rows too tall for the run-recursive form go to its band-matrix kernels),
  * 4 algorithmic tap-FMAs per step (as int64 via out64), 5 global Nz, 6 CUDA device ordinal,
  * 7 form of the z-sweep in use: 1 = recursive evaluation of the exponential window, 0 = direct Toeplitz sum,
  * 8 / 9 y-sweep tiles of the band-matrix kernels evaluated recursively / with dense band matrices,

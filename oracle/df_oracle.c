@@ -73,8 +73,11 @@ void orc_half_widths(int Ny, int Nz, const double* yc, const double* dy, const d
     }
 }
 
-/* the 2N+1 coefficients of half-width N, df.cpp:166-177 (identically :202-216): b[N + i], i=-N..N */
+/* the 2N+1 coefficients of half-width N, df.cpp:166-177 (identically :202-216): b[N + i], i=-N..N.
+ * N = 0 only comes from explicit half-width arrays (the reference's geometry gives N >= 2, :148,189), where its expression is
+ * exp(0/0): the one tap of the limit N -> 0+, b_0 = 1, as the library's setup defines it. */
 void orc_coeffs(int N, double* b) {
+    if (N == 0) { b[0] = 1.0; return; }
     double* temp = (double*)malloc(sizeof(double) * (size_t)(N + 1));
     double sum = 0.0;
     for (int i = 0; i <= N; ++i) {

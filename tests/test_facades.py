@@ -15,18 +15,21 @@ BIN = os.path.join(ROOT, "tests", "_bin")
 LIBDIR = os.path.join(ROOT, "digital-filtering_b200", "lib")
 
 
-def _build(dfb):
-    os.makedirs(BIN, exist_ok=True)
+@pytest.fixture(scope="module")
+def facade_bin(dfb, tmp_path_factory):
+    """the C++ example and the Fortran-convention mimic, compiled and linked against libdfb200.so in a temporary directory (the
+    tree may be read-only); returns that directory"""
+    out = str(tmp_path_factory.mktemp("facades"))
     common = ["-I" + os.path.join(ROOT, "include"), "-L" + LIBDIR, "-ldfb200", "-Wl,-rpath," + LIBDIR]
     subprocess.run(["/usr/bin/g++", "-std=c++17", "-Wall", os.path.join(ROOT, "examples", "cpp-main.cpp")] + common +
-                   ["-o", os.path.join(BIN, "cpp-test")], check=True, capture_output=True)
+                   ["-o", os.path.join(out, "cpp-test")], check=True, capture_output=True)
     subprocess.run(["/usr/bin/gcc", "-std=c11", "-Wall", os.path.join(ROOT, "tests", "fortran_abi_mimic.c")] + common +
-                   ["-lm", "-o", os.path.join(BIN, "fortran_abi_mimic")], check=True, capture_output=True)
+                   ["-lm", "-o", os.path.join(out, "fortran_abi_mimic")], check=True, capture_output=True)
+    return out
 
 
-def test_facades_compile_and_link(dfb):
-    _build(dfb)
-    assert os.path.exists(os.path.join(BIN, "cpp-test")) and os.path.exists(os.path.join(BIN, "fortran_abi_mimic"))
+def test_facades_compile_and_link(facade_bin):
+    assert os.path.exists(os.path.join(facade_bin, "cpp-test")) and os.path.exists(os.path.join(facade_bin, "fortran_abi_mimic"))
 
 
 REF_MAIN = "/root/reference/digital-filtering-c++/test/cpp-main.cpp"
@@ -81,9 +84,8 @@ def test_fortran_module_mirrors_the_c_struct():
 
 
 @pytest.mark.gpu
-def test_cpp_facade_runs_the_reference_example(dfb, default_data):
-    _build(dfb)
-    r = subprocess.run([os.path.join(BIN, "cpp-test")], cwd=default_data / "run", capture_output=True, text=True, timeout=300)
+def test_cpp_facade_runs_the_reference_example(facade_bin, default_data):
+    r = subprocess.run([os.path.join(facade_bin, "cpp-test")], cwd=default_data / "run", capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr
     assert "Ny=510 Nz=400" in r.stdout
     rms = float(r.stdout.split("=")[-1].split()[0])
@@ -115,9 +117,8 @@ def test_reference_main_runs_unchanged(dfb, O):
 
 
 @pytest.mark.gpu
-def test_fortran_calling_convention(dfb, default_data):
-    _build(dfb)
-    r = subprocess.run([os.path.join(BIN, "fortran_abi_mimic"), str(default_data / "files" / "RST.dat"), str(default_data / "line.dat")],
+def test_fortran_calling_convention(facade_bin, default_data):
+    r = subprocess.run([os.path.join(facade_bin, "fortran_abi_mimic"), str(default_data / "files" / "RST.dat"), str(default_data / "line.dat")],
                        capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, (r.stdout, r.stderr)
     tok = r.stdout.split()

@@ -482,7 +482,7 @@ def test_G2_both_forms_of_the_y_sweep(dfb, O, W, monkeypatch, ymode):
     through the exponential window -- short groups of <= 8 rows, long lock-step groups of up to min(32, 0.33 N) rows), and the
     band-matrix kernels kept for windows too tall for shared memory -- chunk-recursive (ysweep_rec_kernel) and dense.  Each forced
     in turn, on a boundary-layer profile (N_y changes every few rows: runs of every length, mixed leftovers) and on hand-made runs
-    (lengths 1..40, N from 2 to 200, windows not aligned to the 8-row chunks; the third field one run of N = 128), all must pass
+    (lengths 1..40, N from 2 to 200 and N = 0, windows not aligned to the 8-row chunks; the third field one run of N = 128), all must pass
     the gate."""
     monkeypatch.setenv("DFB_Y_MODE", ymode)
     probe = dfb.DIGITAL_FILTER(dfb.DFConfig.from_plane(W.plane_profile(200, 300, 96, 24), noise_mode=dfb.NOISE_INJECT))
@@ -495,6 +495,7 @@ def test_G2_both_forms_of_the_y_sweep(dfb, O, W, monkeypatch, ymode):
     while sum(runs) < 330:
         runs.append(int(rng.integers(1, 41)))
     row_N = np.concatenate([np.full(r, Ns[int(rng.integers(0, len(Ns)))]) for r in runs])
+    row_N = np.concatenate([row_N[:40], np.zeros(6, dtype=int), row_N[40:], [0]])     # and N = 0: a run of 6 rows, a lone last row
     Ny, Nz = len(row_N), 150
     plane = _explicit_plane(W, Ny, Nz, [row_N, row_N[::-1].copy(), np.full(Ny, 128)], [np.full(Ny, 4)] * 3)
     assert _run_explicit(dfb, O, plane, seed=24, dts=[3e-7])

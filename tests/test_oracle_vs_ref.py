@@ -67,6 +67,7 @@ def test_coefficients_unit_energy_and_symmetry(O):
         b = O.coeffs(N)
         assert len(b) == 2 * N + 1 and np.array_equal(b, b[::-1])
         assert abs(np.sum(b * b) - 1.0) < 1e-14        # df.cpp:168-177: sum b^2 = 1
+    assert np.array_equal(O.coeffs(0), [1.0])          # explicit N = 0: the one tap of the limit N -> 0+, as the library's setup
 
 
 def test_interpolate_clamps_like_reference(O):

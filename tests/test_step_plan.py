@@ -30,14 +30,10 @@ DT = {
 
 @pytest.fixture(scope="module")
 def shim(tmp_path_factory):
-    out_dir = os.path.join(ROOT, "tests", "_bin")
-    os.makedirs(out_dir, exist_ok=True)
-    lib = os.path.join(out_dir, "libstepplan.so")
-    tmp = lib + ".%d.tmp" % os.getpid()
+    lib = str(tmp_path_factory.mktemp("stepplan") / "libstepplan.so")      # a temporary directory: the tree may be read-only
     srcs = [os.path.join(CSRC, "setup.cpp"), os.path.join(CSRC, "stepplan.cpp"), os.path.join(ROOT, "tests", "step_plan_shim.cpp")]
     subprocess.run(["/usr/bin/g++", "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), "-I", "/usr/local/cuda/include",
-                    "-I", CSRC, "-shared", "-fPIC", "-Wl,--no-undefined", *srcs, "-o", tmp], check=True)
-    os.replace(tmp, lib)
+                    "-I", CSRC, "-shared", "-fPIC", "-Wl,--no-undefined", *srcs, "-o", lib], check=True)
     L = C.CDLL(lib)
     L.sp_plan.restype = C.c_void_p
     L.sp_plan.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.POINTER(C.c_int), C.c_int, C.c_char_p, C.c_int]
@@ -125,12 +121,13 @@ def hybrid_plane(W):
 
 
 def ragged_runs_plane(W):
-    """test_G2_both_forms_of_the_y_sweep: runs of length 1..40 of N from 2 to 200"""
+    """test_G2_both_forms_of_the_y_sweep: runs of length 1..40 of N from 2 to 200, and of N = 0"""
     rng = np.random.default_rng(7)
     runs, Ns = [], [2, 8, 15, 16, 17, 18, 31, 40, 64, 66, 100, 128, 200]
     while sum(runs) < 330:
         runs.append(int(rng.integers(1, 41)))
     row_N = np.concatenate([np.full(r, Ns[int(rng.integers(0, len(Ns)))]) for r in runs])
+    row_N = np.concatenate([row_N[:40], np.zeros(6, dtype=int), row_N[40:], [0]])     # and N = 0: a run of 6 rows, a lone last row
     Ny = len(row_N)
     return explicit_plane(W, Ny, 150, [row_N, row_N[::-1].copy(), np.full(Ny, 128)], [np.full(Ny, 4)] * 3)
 
@@ -336,7 +333,7 @@ def test_forced_y_form_on_a_profile(shim, dfbm, W, mode):
     check_y(sp)
 
 
-def test_overrides_and_their_errors(shim, dfbm, W):
+def test_overrides_their_errors_and_the_fallback_beyond_the_z_window_limit(shim, dfbm, W):
     cfg = dfbm.DFConfig.from_plane(W.NAMED["512x512_N32"]())
     assert StepPlan(shim, dfbm, cfg, zk=16).s("zk") == 16
     assert StepPlan(shim, dfbm, cfg, y_mode=0, y_tk=64).s("tk") == 64
@@ -347,9 +344,13 @@ def test_overrides_and_their_errors(shim, dfbm, W):
     slab = dfbm.DFConfig.from_plane(W.NAMED["512x512_N32"](), k_begin=8, k_end=512)
     with pytest.raises(dfbm.DfbError, match="DFB_Z_MODE=1 needs slab boundaries"):
         StepPlan(shim, dfbm, slab, z_mode=1)
-    plane = explicit_plane(W, 4, 64, [np.full(4, 2)] * 3, [np.full(4, 1000)] * 3)    # 8 outputs per lane: a window of 282 lines
-    with pytest.raises(dfbm.DfbError, match="z half-width too large"):
-        StepPlan(shim, dfbm, explicit_config(dfbm, plane))
+    plane = explicit_plane(W, 4, 64, [np.full(4, 2)] * 3, [np.full(4, 1000)] * 3)    # 8 outputs per lane: a window of 283 lines
+    sp = StepPlan(shim, dfbm, explicit_config(dfbm, plane))
+    assert sp.s("tuned") == 0 and sp.info() == (0, 0, 0, 0, 0)                        # the general kernels
+    with pytest.raises(dfbm.DfbError, match=r"z half-width too large for the tuned z-sweep under DFB_ZK / DFB_Z_MODE: its staged window "
+                                            r"needs 283 lines \(at most 256\) and \d+ bytes of shared memory, the device allows 232448") as e:
+        StepPlan(shim, dfbm, explicit_config(dfbm, plane), zk=8)
+    assert e.value.code == dfbm.ERR_ARG
 
 
 def test_periodic_row_count_limit(shim, dfbm, W):
