@@ -27,6 +27,10 @@ U_FLUC, V_FLUC, W_FLUC, T_FLUC, RHO_FLUC, U_FILT, V_FILT, W_FILT = range(8)
 NOISE_GENERATE, NOISE_INJECT = 0, 1
 CORR_Z, CORR_Y, CORR_T = 0, 1, 2        # correlation directions (dfb_corr_enable)
 DFB_CORR_SUPPORT = CORR_SUPPORT = -1    # lag = the filter's whole support (z and y)
+RESTART_STATE, RESTART_STATS, RESTART_CORR = 1, 2, 4   # sections of a restart file (dfb_save_restart)
+RESTART_INFO = ("version", "Ny", "Nz", "plane_id", "nplanes", "seed", "periodic_z", "noise_mode", "step", "sections", "records",
+                "fingerprint", "Ny_max_u", "Ny_max_v", "Ny_max_w", "Nz_max_u", "Nz_max_v", "Nz_max_w", "tuned", "z_form", "y_form",
+                "stats_count", "stats_on", "corr_lag_z", "corr_lag_y", "corr_lag_t", "corr_count", "corr_on", "ring_fields", "bytes")
 
 c_dp = C.POINTER(C.c_double)
 c_ip = C.POINTER(C.c_int)
@@ -132,6 +136,9 @@ def lib():
         L.dfb_corr_get.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, c_dp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.dfb_corr_get_plane.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, c_dp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.dfb_corr_integral_scales.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, c_dp]
+        L.dfb_save_restart.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
+        L.dfb_load_restart.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
+        L.dfb_restart_info.argtypes = [C.c_char_p, C.POINTER(C.c_int64), C.c_int]
         _lib = L
     return _lib
 
@@ -150,6 +157,17 @@ def measure_fp64_peak(device=-1):
     t, m = C.c_double(), C.c_double()
     _check(lib().dfb_measure_fp64_peak(device, C.byref(t), C.byref(m)))
     return t.value, m.value
+
+
+def restart_info(path):
+    """Header of a restart file (dfb_restart_info; no handle, no device): a dict keyed by RESTART_INFO.  seed and fingerprint are
+    unsigned 64-bit values."""
+    out = (C.c_int64 * len(RESTART_INFO))()
+    _check(lib().dfb_restart_info(os.fsencode(path), out, len(out)))
+    d = dict(zip(RESTART_INFO, out))
+    d["seed"] &= (1 << 64) - 1
+    d["fingerprint"] &= (1 << 64) - 1
+    return d
 
 
 class DFConfig:
@@ -436,6 +454,22 @@ class DIGITAL_FILTER:
     def set_state(self, filt_old, step):
         fo = np.ascontiguousarray(filt_old, dtype=np.float64) if filt_old is not None else None
         _check(lib().dfb_set_state(self._h, _dptr(fo), int(step)))
+
+    # ---- restart files (include/dfb200.h, dfb_save_restart) ----
+    @staticmethod
+    def _restart_what(stats, corr):
+        return RESTART_STATE | (RESTART_STATS if stats else 0) | (RESTART_CORR if corr else 0)
+
+    def save_restart(self, path, stats=False, corr=False):
+        """Write this handle's filter state and step counter (and the N2 sums with stats=True, the correlation statistics with
+        corr=True) into the restart file `path`, in the plane's global layout.  Slabs of one plane (or of one batch) may save into one
+        file; it is complete when every writer has returned."""
+        _check(lib().dfb_save_restart(self._h, os.fsencode(path), self._restart_what(stats, corr)))
+
+    def load_restart(self, path, stats=False, corr=False):
+        """Resume from a restart file written by any decomposition of these planes: the next filter() produces the step the saved run
+        would have produced next, bit for bit with the same kernel forms.  A refused load changes nothing."""
+        _check(lib().dfb_load_restart(self._h, os.fsencode(path), self._restart_what(stats, corr)))
 
     # ---- N2 running statistics / N4 CSV (both opt-in; filter() itself never writes or accumulates) ----
     def stats_enable(self, on=True):

@@ -18,6 +18,7 @@
 #include "noise.cuh"
 #include "device.cuh"
 #include "kernels.hpp"
+#include "restart.hpp"
 
 using namespace dfb;
 
@@ -45,6 +46,7 @@ struct dfb_filter_s {
     int noise_mode = DFB_NOISE_GENERATE;
     bool tuned = false;
     uint64_t seed = 0;
+    uint64_t fingerprint = 0;         // of the filter tables (restart.hpp): what a restart file must match
     int plane_id = 0;
     int nplanes = 1;                  // planes advanced together by this handle (dfb_create_batch): plane p draws from stream group plane_id + p
     int64_t step = 0;                 // steps completed (the constructor's first step counts as one)
@@ -444,6 +446,20 @@ void check_dt(double dt) {
     throw Error{DFB_ERR_ARG, std::string("dt must be finite and >= 0, got ") + buf};
 }
 
+// filt_old [3][P][Ny*W] (host; nullptr keeps it) and the step counter (dfb_set_state, dfb_load_restart)
+void restore_state(dfb_filter_s& H, const double* filt_old3, int64_t step) {
+    CUDA_TRY(cudaSetDevice(H.device));
+    const size_t n = H.D[0].ps_cells * H.nplanes;
+    if (filt_old3)
+        for (int f = 0; f < 3; ++f)
+            CUDA_TRY(cudaMemcpyAsync(H.D[0].f[f].filt_old, filt_old3 + f * n, n * 8, cudaMemcpyHostToDevice, H.stream));
+    CUDA_TRY(cudaStreamSynchronize(H.stream));
+    CUDA_TRY(cudaStreamSynchronize(H.side));      // a look-ahead noise launch for the old step counter may still be in flight
+    if (step != H.step) { H.buf_step[0] = H.buf_step[1] = -1; H.ybuf_step[0] = H.ybuf_step[1] = -1; }
+    H.step = step;
+    H.corr.ring_count = 0;       // the next step follows the restored state: no temporal pair reaches back across it
+}
+
 template <class Fn>
 int guarded(Fn&& fn) {
     try {
@@ -501,6 +517,7 @@ static int create_impl(const dfb_config* cfg, int nplanes, dfb_handle* out) {
         H->nplanes = nplanes;
         if (nplanes > 1 && cfg->noise_mode != DFB_NOISE_GENERATE) throw Error{DFB_ERR_ARG, "a batch of planes generates its own noise (noise_mode = DFB_NOISE_GENERATE)"};
         build_plan(*cfg, H->plan);
+        H->fingerprint = rst::fingerprint(H->plan);
         if (H->noise_mode == DFB_NOISE_INJECT && (H->plan.k0 != 0 || H->plan.k1 != H->plan.NzG))
             throw Error{DFB_ERR_ARG, "noise injection is defined on the whole plane (k_begin = k_end = 0)"};
         int prio_lo = 0, prio_hi = 0;
@@ -835,18 +852,7 @@ int dfb_get_state(dfb_handle h, double* filt_old3, int64_t* step) {
 
 int dfb_set_state(dfb_handle h, const double* filt_old3, int64_t step) {
     if (!h || step < 0) return fail(DFB_ERR_ARG, "bad argument");
-    return guarded([&] {
-        CUDA_TRY(cudaSetDevice(h->device));
-        const size_t n = h->D[0].ps_cells * h->nplanes;
-        if (filt_old3)
-            for (int f = 0; f < 3; ++f)
-                CUDA_TRY(cudaMemcpyAsync(h->D[0].f[f].filt_old, filt_old3 + f * n, n * 8, cudaMemcpyHostToDevice, h->stream));
-        CUDA_TRY(cudaStreamSynchronize(h->stream));
-        CUDA_TRY(cudaStreamSynchronize(h->side));      // a look-ahead noise launch for the old step counter may still be in flight
-        if (step != h->step) { h->buf_step[0] = h->buf_step[1] = -1; h->ybuf_step[0] = h->ybuf_step[1] = -1; }
-        h->step = step;
-        h->corr.ring_count = 0;       // the next step follows the restored state: no temporal pair reaches back across it
-    });
+    return guarded([&] { restore_state(*h, filt_old3, step); });
 }
 
 int dfb_set_timing(dfb_handle h, int on) {
@@ -1080,6 +1086,165 @@ int dfb_corr_integral_scales(dfb_handle h, int plane, int field, int dir, double
             for (int d = 1; d < nlag && r[d] > 0.0; ++d) acc += 0.5 * (r[d - 1] + r[d]) * (x(d) - x(d - 1));
             dst[j] = acc;
         }
+    });
+}
+
+// ---- restart files (restart.hpp: format, records and file I/O; here: what moves between the device and the file) ----
+namespace {
+
+int check_restart_call(dfb_handle h, const char* path, int& what) {
+    if (!h || !path) return fail(DFB_ERR_ARG, "handle/path is NULL");
+    if (what & ~(DFB_RESTART_STATE | DFB_RESTART_STATS | DFB_RESTART_CORR)) return fail(DFB_ERR_ARG, "what must be a combination of DFB_RESTART_STATE, _STATS and _CORR");
+    what |= DFB_RESTART_STATE;
+    if (h->pipe_begun != h->pipe_ended || h->g_begun != h->g_ended)
+        return fail(DFB_ERR_STATE, "a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first");
+    const Plan& P = h->plan;
+    if ((what & DFB_RESTART_CORR) && (P.k0 != 0 || P.k1 != P.NzG)) return fail(DFB_ERR_ARG, "correlation statistics need the whole plane");
+    return DFB_OK;
+}
+
+// The handle's sections as blocks of the file: host buffers in the device layout, [3][P][Ny][W], [P][6][Ny][W], [P][3][Ny][L_d+1] per
+// direction, and n_ring ring fields [P][3][Ny][W] oldest first.  plane_ofs = this handle's first plane within the file.
+struct RestartBuffers {
+    std::vector<double> state, stats, sum[3], ring;
+    std::vector<rst::Block> blocks;
+};
+
+void restart_buffers(const dfb_filter_s& H, const rst::Header& hd, int what, int plane_ofs, RestartBuffers& B) {
+    const int NP = H.nplanes, Ny = H.plan.Ny, W = H.plan.Nz(), k0 = H.plan.k0;
+    const size_t n = H.D[0].ps_cells;
+    B.state.assign(3 * NP * n, 0.0);
+    for (int f = 0; f < 3; ++f)
+        for (int p = 0; p < NP; ++p) B.blocks.push_back({rst::SEC_STATE, f, p + plane_ofs, B.state.data() + ((size_t)f * NP + p) * n, Ny, W, k0});
+    if (what & DFB_RESTART_STATS) {
+        B.stats.assign(6 * NP * n, 0.0);
+        for (int p = 0; p < NP; ++p)
+            for (int s = 0; s < 6; ++s) B.blocks.push_back({rst::SEC_STATS, s, p + plane_ofs, B.stats.data() + ((size_t)p * 6 + s) * n, Ny, W, k0});
+    }
+    if (what & DFB_RESTART_CORR) {
+        for (int d = 0; d < 3; ++d) {
+            const int nl = hd.corr_L[d] + 1;
+            if (!hd.corr_L[d]) continue;
+            B.sum[d].assign((size_t)NP * 3 * Ny * nl, 0.0);
+            for (int p = 0; p < NP; ++p)
+                for (int f = 0; f < 3; ++f)
+                    B.blocks.push_back({rst::SEC_CORR_Z + d, f, p + plane_ofs, B.sum[d].data() + ((size_t)p * 3 + f) * Ny * nl, Ny, nl, 0});
+        }
+        B.ring.assign((size_t)hd.n_ring * NP * 3 * n, 0.0);
+        for (int i = 0; i < hd.n_ring; ++i)
+            for (int p = 0; p < NP; ++p)
+                for (int f = 0; f < 3; ++f)
+                    B.blocks.push_back({rst::SEC_RING, i * 3 + f, p + plane_ofs, B.ring.data() + (((size_t)i * NP + p) * 3 + f) * n, Ny, W, 0});
+    }
+}
+
+}  // namespace
+
+int dfb_save_restart(dfb_handle h, const char* path, int what) {
+    int rc = check_restart_call(h, path, what);
+    if (rc != DFB_OK) return rc;
+    if ((what & DFB_RESTART_STATS) && !h->stats) return fail(DFB_ERR_STATE, "DFB_RESTART_STATS: statistics were never enabled (dfb_stats_enable)");
+    if ((what & DFB_RESTART_CORR) && !h->corr_ready) return fail(DFB_ERR_STATE, "DFB_RESTART_CORR: correlation statistics were never enabled (dfb_corr_enable)");
+    return guarded([&] {
+        const Plan& P = h->plan;
+        const CorrParams& c = h->corr;
+        rst::Header hd;
+        hd.lib_version = dfb_version();
+        hd.Ny = P.Ny; hd.NzG = P.NzG; hd.plane0 = h->plane_id; hd.nplanes = h->nplanes; hd.periodic = P.periodic ? 1 : 0;
+        hd.noise_mode = h->noise_mode; hd.seed = h->seed; hd.step = h->step;
+        for (int f = 0; f < 3; ++f) { hd.Ny_max[f] = P.f[f].Ny_max; hd.Nz_max[f] = P.f[f].Nz_max; hd.Lt[f] = P.f[f].Lt; }
+        hd.forms[0] = h->tuned ? 1 : 0; hd.forms[1] = h->tuned ? h->zp[0].zmode : 0; hd.forms[2] = h->tuned ? h->y_form : -1;   // dfb_info 3, 7, 10
+        hd.fingerprint = h->fingerprint;
+        hd.sections = (uint32_t)what;
+        if (what & DFB_RESTART_STATS) { hd.stats_count = h->stats_count; hd.stats_on = h->stats_on ? 1 : 0; }
+        if (what & DFB_RESTART_CORR) {
+            for (int d = 0; d < 3; ++d) hd.corr_L[d] = c.L[d];
+            hd.corr_on = h->corr_on ? 1 : 0;
+            hd.n_ring = (h->corr_on && c.ring) ? (int)std::min<long long>(c.L[2], c.ring_count) : 0;
+            hd.corr_count = h->corr_count;
+            for (int m = 0; m <= c.L[2]; ++m) hd.corr_tsteps[m] = h->corr_tsteps[m];
+        }
+        rst::layout(hd);
+        RestartBuffers B;
+        restart_buffers(*h, hd, what, 0, B);
+        CUDA_TRY(cudaSetDevice(h->device));
+        const size_t n = h->D[0].ps_cells * h->nplanes;
+        for (int f = 0; f < 3; ++f)
+            CUDA_TRY(cudaMemcpyAsync(B.state.data() + f * n, h->D[0].f[f].filt_old, n * 8, cudaMemcpyDeviceToHost, h->stream));
+        if (what & DFB_RESTART_STATS) CUDA_TRY(cudaMemcpyAsync(B.stats.data(), h->stats, 6 * n * 8, cudaMemcpyDeviceToHost, h->stream));
+        if (what & DFB_RESTART_CORR) {
+            for (int d = 0; d < 3; ++d)
+                if (c.L[d]) CUDA_TRY(cudaMemcpyAsync(B.sum[d].data(), c.sum[d], B.sum[d].size() * 8, cudaMemcpyDeviceToHost, h->stream));
+            for (int i = 0; i < hd.n_ring; ++i) {                    // oldest first: slot (ring_count - n_ring + i) mod L_t
+                const long long slot = (c.ring_count - hd.n_ring + i) % c.L[2];
+                CUDA_TRY(cudaMemcpyAsync(B.ring.data() + (size_t)i * 3 * n, c.ring + (size_t)slot * 3 * n, 3 * n * 8, cudaMemcpyDeviceToHost, h->stream));
+            }
+        }
+        CUDA_TRY(cudaStreamSynchronize(h->stream));
+        rst::save(path, hd, rst::Record{h->plane_id, h->nplanes, P.k0, P.k1, h->step, h->fingerprint}, B.blocks);
+    });
+}
+
+int dfb_load_restart(dfb_handle h, const char* path, int what) {
+    int rc = check_restart_call(h, path, what);
+    if (rc != DFB_OK) return rc;
+    return guarded([&] {
+        // ---- everything is checked and read before the device is touched: a refused load leaves the handle as it was ----
+        std::vector<rst::Record> recs;
+        const rst::Header hd = rst::read_header(path, &recs);
+        const Plan& P = h->plan;
+        const int NP = h->nplanes;
+        auto arg = [](const std::string& m) { return Error{DFB_ERR_ARG, m}; };
+        if (hd.Ny != P.Ny || hd.NzG != P.NzG)
+            throw arg("geometry differs: file Ny x Nz = " + std::to_string(hd.Ny) + " x " + std::to_string(hd.NzG) + ", handle " +
+                      std::to_string(P.Ny) + " x " + std::to_string(P.NzG));
+        if (hd.periodic != (P.periodic ? 1 : 0))
+            throw arg("periodic_z differs: file " + std::to_string(hd.periodic) + ", handle " + std::to_string(P.periodic ? 1 : 0));
+        if (hd.fingerprint != h->fingerprint) throw arg("the filter tables differ (half-widths, row tables or time scales)");
+        if (h->noise_mode == DFB_NOISE_GENERATE && hd.seed != h->seed)
+            throw arg("seed differs: file " + std::to_string(hd.seed) + ", handle " + std::to_string(h->seed));
+        if (h->plane_id < hd.plane0 || h->plane_id + NP > hd.plane0 + hd.nplanes)
+            throw arg("planes [" + std::to_string(h->plane_id) + ", " + std::to_string(h->plane_id + NP) + ") of this handle are not in the file's planes [" +
+                      std::to_string(hd.plane0) + ", " + std::to_string(hd.plane0 + hd.nplanes) + ")");
+        if ((what & DFB_RESTART_STATS) && !(hd.sections & DFB_RESTART_STATS)) throw arg("the file has no N2 statistics (saved without DFB_RESTART_STATS)");
+        if ((what & DFB_RESTART_CORR) && !(hd.sections & DFB_RESTART_CORR)) throw arg("the file has no correlation statistics (saved without DFB_RESTART_CORR)");
+        const std::string gap = rst::check_coverage(hd, recs, h->plane_id, h->plane_id + NP, P.k0, P.k1);
+        if (!gap.empty()) throw Error{DFB_ERR_IO, std::string(path) + ": " + gap};
+        RestartBuffers B;
+        restart_buffers(*h, hd, what, h->plane_id - hd.plane0, B);
+        rst::read_blocks(path, hd, B.blocks);
+
+        // ---- the device ----
+        restore_state(*h, B.state.data(), hd.step);
+        const size_t n = h->D[0].ps_cells * NP;
+        if (what & DFB_RESTART_STATS) {
+            if (!h->stats) h->stats = h->dalloc<double>(6 * n, false);
+            CUDA_TRY(cudaMemcpyAsync(h->stats, B.stats.data(), 6 * n * 8, cudaMemcpyHostToDevice, h->stream));
+            h->stats_count = hd.stats_count;
+            h->stats_on = hd.stats_on != 0;
+        }
+        if (what & DFB_RESTART_CORR) {
+            if (dfb_corr_enable(h, 1, hd.corr_L) != DFB_OK) throw Error{DFB_ERR_CUDA, g_last_error};   // allocates, zeroes, empties the ring
+            CorrParams& c = h->corr;
+            for (int d = 0; d < 3; ++d)
+                if (c.L[d]) CUDA_TRY(cudaMemcpyAsync(c.sum[d], B.sum[d].data(), B.sum[d].size() * 8, cudaMemcpyHostToDevice, h->stream));
+            if (hd.n_ring) CUDA_TRY(cudaMemcpyAsync(c.ring, B.ring.data(), B.ring.size() * 8, cudaMemcpyHostToDevice, h->stream));   // slots 0..n_ring-1
+            c.ring_count = hd.n_ring;
+            h->corr_count = hd.corr_count;
+            for (int m = 0; m <= c.L[2]; ++m) h->corr_tsteps[m] = hd.corr_tsteps[m];
+            if (!hd.corr_on && dfb_corr_enable(h, 0, nullptr) != DFB_OK) throw Error{DFB_ERR_CUDA, g_last_error};
+        }
+        CUDA_TRY(cudaStreamSynchronize(h->stream));
+    });
+}
+
+int dfb_restart_info(const char* path, int64_t* out, int cap) {
+    if (!path || cap < 0 || (cap > 0 && !out)) return fail(DFB_ERR_ARG, "bad argument");
+    return guarded([&] {
+        std::vector<rst::Record> recs;
+        const rst::Header hd = rst::read_header(path, &recs);
+        const std::vector<int64_t> v = rst::info_values(hd, (int)recs.size());
+        std::copy(v.begin(), v.begin() + std::min<size_t>(v.size(), (size_t)cap), out);
     });
 }
 
@@ -1592,6 +1757,13 @@ int dfb_gathered_to_host_f(const dfb_handle* h, const int* which, double* dst) {
 }
 int dfb_face_map_f(const dfb_handle* h, const int* n, const double* yf, const double* zf, int* plane_index) {
     return (h && n) ? dfb_face_map(*h, *n, yf, zf, plane_index) : fail(DFB_ERR_ARG, "NULL argument");
+}
+static std::string fortran_path(const char* path, const int* len) { return (len && *len >= 0) ? std::string(path, (size_t)*len) : std::string(path); }
+int dfb_save_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what) {
+    return (h && path && what) ? dfb_save_restart(*h, fortran_path(path, path_len).c_str(), *what) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_load_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what) {
+    return (h && path && what) ? dfb_load_restart(*h, fortran_path(path, path_len).c_str(), *what) : fail(DFB_ERR_ARG, "NULL argument");
 }
 int dfb_destroy_f(dfb_handle* h) {
     if (!h) return DFB_OK;

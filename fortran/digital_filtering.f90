@@ -18,6 +18,7 @@
 !   config%periodic_z = 1                         spanwise-periodic plane: the z filter wraps around it
 !   face_map, apply_inflow                        N3: inflow face -> plane cell, ghost cell = mean + fluctuation (us3d_user.f90:85-114)
 !   corr_enable, corr_get, integral_scales        correlation statistics along z, y and in time (dfb_corr_*): the delivered scales
+!   save_restart, load_restart                    restart files: resume a run across jobs, bit for bit, whatever the slab layout
 !
 ! NOTE: NEVER COMPILED -- no Fortran compiler exists in the build image or on the GPU boxes.  The binding is exercised through
 ! tests/fortran_abi_mimic.c, a C program that makes exactly these calls with exactly this struct layout and by-reference
@@ -30,6 +31,9 @@ module DIGITAL_FILTERING
     public :: digital_filter_batch_type, create_digital_filter_batch, filter_batch
     public :: comm_unique_id, comm_init, gather_begin, gather_end, gathered_field, face_map, apply_inflow
     public :: corr_enable, corr_get, integral_scales
+    public :: save_restart, load_restart, RESTART_STATE, RESTART_STATS, RESTART_CORR
+
+    integer, parameter :: RESTART_STATE = 1, RESTART_STATS = 2, RESTART_CORR = 4   ! DFB_RESTART_* (what to save / load; added together)
 
     integer, parameter :: dp = selected_real_kind(15)
 
@@ -182,6 +186,18 @@ module DIGITAL_FILTERING
             type(c_ptr), value :: handle
             integer(c_int), value :: plane, field, dir
             real(c_double), intent(inout) :: dst(*)
+        end function
+        integer(c_int) function dfb_save_restart_f(handle, path, path_len, what) bind(C, name='dfb_save_restart_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle
+            type(c_ptr), value :: path
+            integer(c_int), intent(in) :: path_len, what
+        end function
+        integer(c_int) function dfb_load_restart_f(handle, path, path_len, what) bind(C, name='dfb_load_restart_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle
+            type(c_ptr), value :: path
+            integer(c_int), intent(in) :: path_len, what
         end function
         function dfb_last_error() bind(C, name='dfb_last_error') result(msg)
             import :: c_ptr
@@ -367,6 +383,29 @@ contains
         real(kind=dp), intent(inout) :: L(:)
         call check(dfb_corr_integral_scales(DF%handle, 0_c_int, int(field, c_int), int(dir, c_int), L), 'integral_scales')
     end subroutine integral_scales
+
+    ! ---- restart files (include/dfb200.h, dfb_save_restart): what = RESTART_STATE (default) [+ RESTART_STATS] [+ RESTART_CORR] ----
+    subroutine save_restart(DF, path, what)         ! every rank of a slab job may save its slab into the same file; MPI_Barrier after
+        type(digital_filter_type), intent(in) :: DF
+        character(len=*), intent(in), target :: path
+        integer, intent(in), optional :: what
+        integer(c_int) :: w, n
+        w = RESTART_STATE
+        if (present(what)) w = what
+        n = len_trim(path)
+        call check(dfb_save_restart_f(DF%handle, c_loc(path), n, w), 'save_restart')
+    end subroutine save_restart
+
+    subroutine load_restart(DF, path, what)         ! after the writers' barrier; the next filter(DF, dt) continues the saved run
+        type(digital_filter_type), intent(in) :: DF
+        character(len=*), intent(in), target :: path
+        integer, intent(in), optional :: what
+        integer(c_int) :: w, n
+        w = RESTART_STATE
+        if (present(what)) w = what
+        n = len_trim(path)
+        call check(dfb_load_restart_f(DF%handle, c_loc(path), n, w), 'load_restart')
+    end subroutine load_restart
 
     subroutine destroy_digital_filter(DF)
         type(digital_filter_type), intent(inout) :: DF

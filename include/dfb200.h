@@ -227,6 +227,42 @@ int dfb_generate_noise(dfb_handle h, int64_t step);
 int dfb_get_state(dfb_handle h, double* filt_old3, int64_t* step);
 int dfb_set_state(dfb_handle h, const double* filt_old3, int64_t step);
 
+/* Restart files -- resume a generator across the jobs of a long run, bit for bit, whatever the decomposition on either side.
+ * A file holds the plane's GLOBAL layout (filt_old [3][P][Ny][Nz_global] and, on request, the N2 sums [P][6][Ny][Nz_global] and the
+ * correlation statistics), the step counter, and a fingerprint of the filter tables (half-widths, row tables, Lt, Ny, Nz, periodic_z).
+ * Noise is keyed by (seed, step, global index), so the continued run equals the uninterrupted one bit for bit when it runs the same
+ * kernel forms (dfb_info 3, 7, 10); a file written under other forms (DFB_Y_MODE, kernel_variant) is accepted and the continuation
+ * then agrees to rounding.  Not saved: the outputs of the last step (u', v', w', T', rho', a gathered plane) -- the first dfb_filter
+ * after a load produces step s+1 exactly as the uninterrupted run would.
+ *
+ * dfb_save_restart writes this handle's planes and columns (DFB_RESTART_STATE is always included).  Several writers may share one
+ * file: the spanwise slabs of one plane or of one batch (one rank each, or several handles of one process).  Each opens the file without
+ * truncating it and, under an open-file-description lock on the header, clears the writer records if they belong to another step (or
+ * another plane range, geometry or set of sections), writes the header and sizes the file; then writes its rows; then adds its writer
+ * record {plane range, k_begin, k_end, step, fingerprint} under the lock (at most 64 per file).  The file is complete when every
+ * writer's call has returned: the caller's barrier (MPI_Barrier, a join) orders the saves before any load.  Saves are synchronous.
+ *   DFB_RESTART_STATS without dfb_stats_enable ever called, DFB_RESTART_CORR without dfb_corr_enable: DFB_ERR_STATE.
+ *   DFB_RESTART_CORR on a slab handle: DFB_ERR_ARG (correlation statistics are whole-plane only).
+ *   A save while a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: DFB_ERR_STATE.
+ * dfb_load_restart restores any handle whose planes [plane_id, plane_id + nplanes) lie in the file's plane range and whose Ny, Nz,
+ * periodic_z and filter tables match (and, in generate mode, its seed); it reads only its own columns, so a file written by 8 slabs
+ * loads into 4, a batch file into single planes or smaller batches, slabs into a whole plane.  It checks everything before it touches
+ * the device: a refused load leaves the handle as it was.  filt_old and the step go through dfb_set_state's path; with
+ * DFB_RESTART_STATS the N2 sums, count and on/off state (the sums are allocated if needed); with DFB_RESTART_CORR (whole-plane handles)
+ * the lags, sums, pair counts, the temporal ring and on/off state, so that the next steps add what the uninterrupted run would add.
+ *   A mismatch (seed, geometry, filter tables, planes outside the file, a section the file lacks): DFB_ERR_ARG, naming it.
+ *   A missing, short or foreign file, another format version, writer records that do not cover the handle's columns or carry another
+ *   step or fingerprint: DFB_ERR_IO, naming the column range.
+ * dfb_restart_info reads a file's header (no handle, no device) into out[0 .. min(cap, 30)):
+ *   0 format version, 1 Ny, 2 Nz_global, 3 first plane id, 4 planes, 5 seed (bits), 6 periodic_z, 7 noise_mode, 8 step counter,
+ *   9 sections (DFB_RESTART_* bits), 10 writer records, 11 fingerprint (bits), 12-14 Ny_max u v w, 15-17 Nz_max u v w,
+ *   18-20 the last writer's dfb_info 3, 7, 10, 21 N2 count, 22 N2 on, 23-25 correlation lags z y t, 26 correlation count,
+ *   27 correlation on, 28 ring fields saved, 29 file size in bytes. */
+enum { DFB_RESTART_STATE = 1, DFB_RESTART_STATS = 2, DFB_RESTART_CORR = 4 };
+int dfb_save_restart(dfb_handle h, const char* path, int what);
+int dfb_load_restart(dfb_handle h, const char* path, int what);
+int dfb_restart_info(const char* path, int64_t* out, int cap);
+
 /* N2 -- running statistics, the reference's only validation tool (rms_add / plot_rms, df.cpp:571-621), on the device
  * and opt-in: after dfb_stats_enable(h, 1) every dfb_filter also accumulates per cell the sums of u'^2, v'^2, w'^2,
  * T'^2, rho'^2 and u'v' (which = 0..5).  dfb_stats_get copies one of them to the host (as_rms != 0: sqrt(sum/count)
@@ -316,6 +352,9 @@ int dfb_gather_end_f(const dfb_handle* h);
 int dfb_gathered_to_host_f(const dfb_handle* h, const int* which, double* dst);
 int dfb_face_map_f(const dfb_handle* h, const int* n, const double* yf, const double* zf, int* plane_index);
 int dfb_destroy_f(dfb_handle* h);
+/* path: Fortran character variable (c_loc) + its len_trim, as the file names of dfb_config (path_len < 0: NUL-terminated) */
+int dfb_save_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);
+int dfb_load_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);
 
 #ifdef __cplusplus
 }

@@ -141,6 +141,11 @@ class DIGITAL_FILTER {
         check(dfb_corr_integral_scales(h_, plane, field, dir, L.data()));
         return L;
     }
+    // restart files (dfb_save_restart / dfb_load_restart): what = DFB_RESTART_STATE [| DFB_RESTART_STATS | DFB_RESTART_CORR].  A load
+    // resumes the saved run: the next filter() produces the step it would have produced next (the host vectors keep the last step's
+    // outputs until then).  Slabs of one plane may save into one file; it is complete when every writer has returned.
+    void save_restart(const std::string& path, int what = DFB_RESTART_STATE) { check(dfb_save_restart(h_, path.c_str(), what)); }
+    void load_restart(const std::string& path, int what = DFB_RESTART_STATE) { check(dfb_load_restart(h_, path.c_str(), what)); }
     const Vector& T_rms() const { return T_rms_; }
     const Vector& rho_rms() const { return rho_rms_; }
     int rms_counter = 0;               // df.hpp:63
