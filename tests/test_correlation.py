@@ -15,6 +15,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, default_plane, normwise_close
+from oracle_harness import np_sums
 
 gpu = pytest.mark.gpu
 TOL = 1e-12
@@ -24,35 +25,6 @@ PI_BLEND = 3.141592654          # the blend's truncated pi (df.cpp:411)
 # ---------------------------------------------------------------------------------------------
 # numpy checker
 # ---------------------------------------------------------------------------------------------
-def np_sums(steps, L, periodic=False):
-    """steps: fields [Ny, Nz] of one (plane, field) after consecutive accumulated steps (the ring never emptied in between).
-    Returns {dir: (S [Ny, L+1], pairs [L+1])} for the directions with L[dir] > 0."""
-    Ny, Nz = steps[0].shape
-    out = {}
-    Lz, Ly, Lt = L
-    if Lz:
-        S = np.zeros((Ny, Lz + 1))
-        for f in steps:
-            for d in range(Lz + 1):
-                S[:, d] += (f * np.roll(f, -d, axis=1)).sum(1) if periodic else (f[:, :Nz - d] * f[:, d:]).sum(1)
-        out[0] = (S, np.array([len(steps) * (Nz if periodic else Nz - d) for d in range(Lz + 1)], dtype=np.int64))
-    if Ly:
-        S = np.zeros((Ny, Ly + 1))
-        for f in steps:
-            for d in range(Ly + 1):
-                S[:Ny - d, d] += (f[:Ny - d] * f[d:]).sum(1)
-        out[1] = (S, np.full(Ly + 1, len(steps) * Nz, dtype=np.int64))
-    if Lt:
-        S = np.zeros((Ny, Lt + 1))
-        pairs = np.zeros(Lt + 1, dtype=np.int64)
-        for s in range(len(steps)):
-            for m in range(min(Lt, s) + 1):
-                S[:, m] += (steps[s] * steps[s - m]).sum(1)
-                pairs[m] += Nz
-        out[2] = (S, pairs)
-    return out
-
-
 def np_normalize(S, pairs, d):
     Ny, n = S.shape
     R = np.full_like(S, np.nan)

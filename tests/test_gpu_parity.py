@@ -15,45 +15,21 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, default_plane, normwise_close
+from oracle_harness import Model, explicit_config, explicit_plane, run
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-12
 
 
-def inject_and_step(dfb, O, plane, variant, seed, dts, check_first=True):
-    """Runs constructor step + len(dts) filter steps in inject mode on the GPU and through the oracle
-    restatement with the same (counter-based) noise; returns worst normwise ratio per output."""
+def inject_and_step(dfb, O, plane, variant, seed, dts):
+    """Runs constructor step + len(dts) filter steps in inject mode on the GPU and in the model (the oracle restatement) with the
+    same (counter-based) noise; returns worst normwise ratio per output."""
     cfg = dfb.DFConfig.from_plane(plane, noise_mode=dfb.NOISE_INJECT, kernel_variant=variant)
     df = dfb.DIGITAL_FILTER(cfg)
     O.half_widths(plane)
-    Ny, Nz = plane["Ny"], plane["Nz"]
     for f in range(3):
         assert np.array_equal(df.half_widths(f, 0), plane["N_y"][f]) and np.array_equal(df.half_widths(f, 1), plane["N_z"][f])
-    fo = np.zeros((3, Ny, Nz))
-    worst = {}
-    for s, dt in enumerate([0.0] + list(dts)):
-        rys = [O.noise_rys(seed, 0, f, s, Ny, plane["Ny_max"][f], Nz) for f in range(3)]
-        hal = [O.noise_halo(seed, 0, f, s, Ny, plane["Nz_max"][f]) for f in range(3)]
-        for f in range(3):
-            df.set_noise(f, rys[f], hal[f])
-        if s == 0:
-            df.first_step()
-        else:
-            df.filter(dt)
-        df.fetch()
-        o = O.step(plane, rys, hal, fo, dt, first_step=(s == 0))
-        fo = o["filt_old"]
-        got = dict(filt=np.stack([df.u.filt, df.v.filt, df.w.filt]), fluc=np.stack([df.u.fluc, df.v.fluc, df.w.fluc]),
-                   T=df.T_fluc, rho=df.rho_fluc)
-        for k in ("filt", "fluc", "T", "rho"):
-            if s == 0 and k in ("T", "rho"):
-                assert not got[k].any()          # SURVEY quirk 3: T', rho' stay 0 after the constructor
-                continue
-            for f in range(3) if k in ("filt", "fluc") else [None]:
-                a, b = (got[k][f], o[k][f]) if f is not None else (got[k], o[k])
-                ok, r = normwise_close(a, b, TOL)
-                worst[k] = max(worst.get(k, 0.0), r)
-                assert ok, (plane["name"], variant, s, k, f, r)
+    worst = run(df, Model(O, plane, seed, 0), dts)
     df.close()
     return worst
 
@@ -194,23 +170,9 @@ def test_G2_default_plane_against_reference_object_code(dfb, O):
 
 def test_G2_generate_mode_equals_oracle_on_the_same_stream(dfb, O, W):
     """generate mode end to end: device noise (G1) + device filter == oracle noise + oracle filter"""
-    plane = W.plane_profile(96, 200, 24, 10)
-    df = dfb.DIGITAL_FILTER(dfb.DFConfig.from_plane(plane, seed=77))
-    O.half_widths(plane)
-    Ny, Nz = 96, 200
-    fo = np.zeros((3, Ny, Nz))
-    for s, dt in enumerate([0.0, 1e-7, 1e-7, 3e-7]):
-        if s > 0:
-            df.filter(dt)
-        else:
-            df.fetch()
-        rys = [O.noise_rys(77, 0, f, s, Ny, plane["Ny_max"][f], Nz) for f in range(3)]
-        hal = [O.noise_halo(77, 0, f, s, Ny, plane["Nz_max"][f]) for f in range(3)]
-        o = O.step(plane, rys, hal, fo, dt, first_step=(s == 0))
-        fo = o["filt_old"]
-        for f, F in enumerate((df.u, df.v, df.w)):
-            ok, r = normwise_close(F.fluc, o["fluc"][f], TOL)
-            assert ok, (s, f, r)
+    plane = O.half_widths(W.plane_profile(96, 200, 24, 10))
+    df = dfb.DIGITAL_FILTER(dfb.DFConfig.from_plane(plane, seed=77), fetch=False)
+    run(df, Model(O, plane, 77, 0), [1e-7, 1e-7, 3e-7])
     assert df.step == 4
     df.close()
 
@@ -417,38 +379,11 @@ def test_N4_csv_matches_reference_writer(dfb, O, tmp_path):
 # ---------------------------------------------------------------------------------------------
 # edge cases: explicit (odd, zero, large) half-widths, awkward shapes, batch call
 # ---------------------------------------------------------------------------------------------
-def _explicit_plane(W, Ny, Nz, Ny_rows, Nz_rows):
-    """row-uniform plane whose half-widths are SUPPLIED (dfb_config.N_y / N_z) instead of derived from geometry"""
-    yc = (np.arange(Ny) + 0.5) * 1e-5
-    N_y = np.stack([np.repeat(np.asarray(Ny_rows[f], dtype=np.int32)[:, None], Nz, axis=1) for f in range(3)])
-    N_z = np.stack([np.repeat(np.asarray(Nz_rows[f], dtype=np.int32)[:, None], Nz, axis=1) for f in range(3)])
-    return dict(name=f"explicit_{Ny}x{Nz}", Ny=Ny, Nz=Nz, d_i=W.D_I, U_e=W.U_E, yc=yc, dy=np.full(Ny, 1e-5), dz=np.full(Ny, 1e-5),
-                rows=W.synthetic_rows(yc + 1e-4), scales=W._scales(W.D_I), explicit_N=True,
-                N_y=N_y, N_z=N_z, Ny_max=[int(N_y[f].max()) for f in range(3)], Nz_max=[int(N_z[f].max()) for f in range(3)])
-
-
-def _run_explicit(dfb, O, plane, seed, dts, variant=0):
-    Ny, Nz = plane["Ny"], plane["Nz"]
-    cfg = dfb.DFConfig.from_plane(plane, noise_mode=dfb.NOISE_INJECT, kernel_variant=variant)
-    cfg.geom_per_row = 0                       # N arrays are per cell
-    cfg.yc = cfg.dy = cfg.dz = None
-    cfg.N_y, cfg.N_z = plane["N_y"], plane["N_z"]
-    df = dfb.DIGITAL_FILTER(cfg)
-    fo = np.zeros((3, Ny, Nz))
-    for s, dt in enumerate([0.0] + list(dts)):
-        rys = [O.noise_rys(seed, 0, f, s, Ny, plane["Ny_max"][f], Nz) for f in range(3)]
-        hal = [O.noise_halo(seed, 0, f, s, Ny, plane["Nz_max"][f]) if plane["Nz_max"][f] else np.zeros((Ny, 0)) for f in range(3)]
-        for f in range(3):
-            df.set_noise(f, rys[f], hal[f] if plane["Nz_max"][f] else None)
-        df.first_step() if s == 0 else df.filter(dt)
-        df.fetch()
-        o = O.step(plane, rys, hal, fo, dt, first_step=(s == 0))
-        fo = o["filt_old"]
-        for f, F in enumerate((df.u, df.v, df.w)):
-            ok, r = normwise_close(F.fluc, o["fluc"][f], TOL)
-            assert ok, (plane["name"], s, f, r)
-        if s:
-            assert normwise_close(df.T_fluc, o["T"], TOL)[0] and normwise_close(df.rho_fluc, o["rho"], TOL)[0]
+def _run_explicit(dfb, O, plane, seed, dts):
+    """constructor step + len(dts) filter steps in inject mode against the model on a plane whose half-widths are supplied; returns
+    whether the tuned kernels ran"""
+    df = dfb.DIGITAL_FILTER(explicit_config(dfb, plane, noise_mode=dfb.NOISE_INJECT))
+    run(df, Model(O, plane, seed, 0), dts)
     tuned = df.tuned
     df.close()
     return tuned
@@ -459,7 +394,7 @@ def test_explicit_odd_and_mixed_half_widths(dfb, O, W):
     Ny, Nz = 37, 530
     Nyr = [rng.integers(1, 40, Ny) for _ in range(3)]            # odd and even, changing every row
     Nzr = [rng.integers(1, 23, Ny) for _ in range(3)]
-    plane = _explicit_plane(W, Ny, Nz, Nyr, Nzr)
+    plane = explicit_plane(W, Ny, Nz, Nyr, Nzr)
     assert _run_explicit(dfb, O, plane, seed=12, dts=[3e-7])     # row-uniform -> tuned kernels, scalar z staging (odd N)
 
 
@@ -472,7 +407,7 @@ def test_large_half_widths_beyond_128(dfb, O, W, monkeypatch, ymode):
     Ny, Nz = 24, 700
     Nyr = [np.full(Ny, 200), np.full(Ny, 96), np.linspace(20, 260, Ny).astype(int) // 2 * 2]
     Nzr = [np.full(Ny, 300), np.full(Ny, 2), np.full(Ny, 130)]
-    plane = _explicit_plane(W, Ny, Nz, Nyr, Nzr)
+    plane = explicit_plane(W, Ny, Nz, Nyr, Nzr)
     assert _run_explicit(dfb, O, plane, seed=13, dts=[3e-7])
 
 
@@ -497,7 +432,7 @@ def test_G2_both_forms_of_the_y_sweep(dfb, O, W, monkeypatch, ymode):
     row_N = np.concatenate([np.full(r, Ns[int(rng.integers(0, len(Ns)))]) for r in runs])
     row_N = np.concatenate([row_N[:40], np.zeros(6, dtype=int), row_N[40:], [0]])     # and N = 0: a run of 6 rows, a lone last row
     Ny, Nz = len(row_N), 150
-    plane = _explicit_plane(W, Ny, Nz, [row_N, row_N[::-1].copy(), np.full(Ny, 128)], [np.full(Ny, 4)] * 3)
+    plane = explicit_plane(W, Ny, Nz, [row_N, row_N[::-1].copy(), np.full(Ny, 128)], [np.full(Ny, 4)] * 3)
     assert _run_explicit(dfb, O, plane, seed=24, dts=[3e-7])
 
 
@@ -511,7 +446,7 @@ def test_recursive_z_sweep_every_window_geometry(dfb, O, W, monkeypatch, zk):
     Ny, Nz = len(Ns), 601                                          # 601: partial last strip, odd width
     Nzr = [np.array(Ns), np.array(Ns[::-1]), np.array(Ns)]
     Nyr = [np.full(Ny, 3), np.full(Ny, 2), np.full(Ny, 5)]
-    plane = _explicit_plane(W, Ny, Nz, Nyr, Nzr)
+    plane = explicit_plane(W, Ny, Nz, Nyr, Nzr)
     assert _run_explicit(dfb, O, plane, seed=19, dts=[2e-7, 5e-7])
 
 
@@ -520,7 +455,7 @@ def test_tiny_and_awkward_shapes(dfb, O, W, shape):
     Ny, Nz = shape
     Nyr = [np.full(Ny, 2), np.full(Ny, 4), np.full(Ny, 2)]
     Nzr = [np.full(Ny, 2), np.full(Ny, 2), np.full(Ny, 4)]
-    plane = _explicit_plane(W, Ny, Nz, Nyr, Nzr)
+    plane = explicit_plane(W, Ny, Nz, Nyr, Nzr)
     _run_explicit(dfb, O, plane, seed=14, dts=[2e-7, 2e-7])
 
 
@@ -968,12 +903,8 @@ def test_G2_hybrid_y_sweep_run_blocks_and_band_matrices(dfb, O, W):
     Ny, Nz = 320, 3400                                                  # wide enough for the run part to be worth a launch of its own
     steep = np.arange(40, 104, 1) * 2                                   # N = 80, 82, ..., 206: a new half-width every row
     row_N = np.concatenate([np.full(96, 40), steep, np.repeat(np.arange(100, 36, -4) * 2, 10)])[:Ny]
-    plane = _explicit_plane(W, Ny, Nz, [row_N, np.full(Ny, 24), row_N[::-1].copy()], [np.full(Ny, 6)] * 3)
-    cfg = dfb.DFConfig.from_plane(plane, noise_mode=dfb.NOISE_INJECT)
-    cfg.geom_per_row = 0
-    cfg.yc = cfg.dy = cfg.dz = None
-    cfg.N_y, cfg.N_z = plane["N_y"], plane["N_z"]
-    probe = dfb.DIGITAL_FILTER(cfg)
+    plane = explicit_plane(W, Ny, Nz, [row_N, np.full(Ny, 24), row_N[::-1].copy()], [np.full(Ny, 6)] * 3)
+    probe = dfb.DIGITAL_FILTER(explicit_config(dfb, plane, noise_mode=dfb.NOISE_INJECT))
     assert probe.tuned and probe.info(10) == 3, probe.info(10)
     probe.close()
     assert _run_explicit(dfb, O, plane, seed=29, dts=[3e-7])

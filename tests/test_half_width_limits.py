@@ -12,25 +12,13 @@ import numpy as np
 import pytest
 
 from conftest import normwise_close
-from test_periodic_z import periodic_step
-from test_step_plan import B200, StepPlan, dfbm, explicit_config, explicit_plane, shim  # noqa: F401  (dfbm, shim: fixtures)
+from oracle_harness import Model, explicit_config, package, run
+from shims import B200, plan, step_plan_shim, y_limits as planner_y_limits, yplane, z_limits as planner_z_limits, zplane
 
-TOL = 1e-12
 SMEM = B200["smem_optin"]
 NZ_SWEEP = 1800                      # beyond the old 256-line limit of both lane blockings
 DTS = [2e-7, 8e-7]
 gpu = pytest.mark.gpu
-
-
-def zplane(W, Nz_rows, Nz=400, Ny_rows=None):
-    """a plane of len(Nz_rows) rows whose three fields all have these N_z (and N_y = 2 unless given), with the oracle's Ny_max /
-    Nz_max; 400 columns take 16 outputs per lane by default (>= 384), 200 take 8"""
-    Ny = len(Nz_rows[0]) if isinstance(Nz_rows[0], (list, np.ndarray)) else len(Nz_rows)
-    zr = Nz_rows if isinstance(Nz_rows[0], (list, np.ndarray)) else [Nz_rows] * 3
-    yr = Ny_rows if Ny_rows is not None else [np.full(Ny, 2)] * 3
-    p = explicit_plane(W, Ny, Nz, [np.asarray(r) for r in yr], [np.asarray(r) for r in zr])
-    p.update(Ny_max=[int(p["N_y"][f].max()) for f in range(3)], Nz_max=[int(p["N_z"][f].max()) for f in range(3)])
-    return p
 
 
 def natural_z(Nz_rows, Nz, k=None):
@@ -40,55 +28,24 @@ def natural_z(Nz_rows, Nz, k=None):
     return zk, 1 if aligned and min(Nz_rows) >= 1 else 0
 
 
-def plan(L, dfbm, plane, k=None, **ovr):
-    kw = {} if k is None else dict(k_begin=k[0], k_end=k[1])
-    return StepPlan(L, dfbm, explicit_config(dfbm, plane, **kw), **ovr)
+@pytest.fixture(scope="module")
+def shim(tmp_path_factory):
+    return step_plan_shim(tmp_path_factory)
 
 
-def forced_fits(L, dfbm, W, N, zk, zmode):
-    """does the planner accept N_z = N under DFB_ZK = zk, DFB_Z_MODE = zmode?  (a refusal must be the over-budget error)"""
-    try:
-        plan(L, dfbm, zplane(W, [N, N]), zk=zk, z_mode=zmode)
-        return True
-    except dfbm.DfbError as e:
-        assert e.code == dfbm.ERR_ARG and "z half-width too large" in str(e), str(e)
-        return False
+@pytest.fixture(scope="module")
+def dfbm():
+    return package()
 
 
 @pytest.fixture(scope="module")
 def z_limits(shim, dfbm, W):
-    """(outputs per lane, z form) -> largest N_z whose tuned z-sweep fits a B200, as the planner decides it"""
-    out = {}
-    for zk in (8, 16):
-        for zmode in (0, 1):
-            N = 1
-            while forced_fits(shim, dfbm, W, N + 1, zk, zmode):
-                N += 1
-            out[(zk, zmode)] = N
-    return out
-
-
-YPLANE = dict(Ny=8, Nz=150)          # the y ladder's limit cases: one 8-row block, partial last column tile
-
-
-def yplane(W, Ny_rows, Ny=YPLANE["Ny"], Nz=YPLANE["Nz"]):
-    yr = Ny_rows if isinstance(Ny_rows[0], (list, np.ndarray)) else [Ny_rows] * 3
-    return zplane(W, [np.full(Ny, 2)] * 3, Nz=Nz, Ny_rows=yr)
+    return planner_z_limits(shim, dfbm, W)
 
 
 @pytest.fixture(scope="module")
 def y_limits(shim, dfbm, W):
-    """largest N_y of the 8-row plane that the run-recursive y-sweep takes: forced (DFB_Y_MODE=2) with two window buffers per CTA,
-    forced with one, and by default (windows of a 128-row block twice in shared memory)"""
-    out = {}
-    for N in range(0, 1000):
-        f2 = plan(shim, dfbm, yplane(W, np.full(8, N)), y_mode=2)
-        fd = plan(shim, dfbm, yplane(W, np.full(8, N)))
-        if f2.s("y_form") == 2:
-            out["forced-2buf" if f2.s("r_nbuf") == 2 else "forced-1buf"] = N
-        if fd.s("y_form") == 2:
-            out["default"] = N
-    return out
+    return planner_y_limits(shim, dfbm, W)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -180,30 +137,11 @@ def forms(df):
 
 
 def against_oracle(dfb, O, plane, seed, periodic=False):
-    """constructor step + two filter(dt) steps in inject mode, every output against O.step (periodic_step for a periodic plane) at
-    the 1e-12 normwise gate.  Returns (dfb_info 3/7/10, worst ratio per output)."""
-    Ny, Nz = plane["Ny"], plane["Nz"]
+    """constructor step + two filter(dt) steps in inject mode, every output against the model (O.step, periodic_step for a periodic
+    plane) at the 1e-12 normwise gate.  Returns (dfb_info 3/7/10, worst ratio per output)."""
     df = handle(dfb, plane, noise_mode=dfb.NOISE_INJECT, periodic_z=int(periodic))
     info = forms(df)
-    fo = np.zeros((3, Ny, Nz))
-    worst = {}
-    for s, dt in enumerate([0.0] + DTS):
-        rys = [O.noise_rys(seed, 0, f, s, Ny, plane["Ny_max"][f], Nz) for f in range(3)]
-        hal = [O.noise_halo(seed, 0, f, s, Ny, plane["Nz_max"][f]) if plane["Nz_max"][f] else np.zeros((Ny, 0)) for f in range(3)]
-        for f in range(3):
-            df.set_noise(f, rys[f], hal[f] if plane["Nz_max"][f] and not periodic else None)
-        df.first_step() if s == 0 else df.filter(dt)
-        df.fetch()
-        o = periodic_step(O, plane, rys, fo, dt, s == 0) if periodic else O.step(plane, rys, hal, fo, dt, first_step=(s == 0))
-        fo = o["filt_old"]
-        got = dict(filt=[df.u.filt, df.v.filt, df.w.filt], fluc=[df.u.fluc, df.v.fluc, df.w.fluc], T=[df.T_fluc], rho=[df.rho_fluc])
-        for key, arrs in got.items():
-            if s == 0 and key in ("T", "rho"):
-                continue
-            for f, a in enumerate(arrs):
-                ok, r = normwise_close(a, o[key][f] if key in ("filt", "fluc") else o[key], TOL)
-                worst[key] = max(worst.get(key, 0.0), r)
-                assert ok, (plane["name"], s, key, f, r)
+    worst = run(df, Model(O, plane, seed, 0, periodic=periodic), DTS)
     df.close()
     return info, worst
 
@@ -358,24 +296,12 @@ def test_slabs_at_the_boundary(dfb, O, W, z_limits, past):
             for i, a in enumerate(part[s][0]):
                 assert np.array_equal(a, whole[s][0][i][:, k[0]:k[1]]), (k, s, i)
     k = (7, 391)
-    info, part = generate(dfb, plane, k=k)
+    df = handle(dfb, plane, k=k, seed=5)
+    info = forms(df)
     assert info[:2] == ((0, 0) if past else (1, 0))
-    Ny, Nz = plane["Ny"], plane["Nz"]
-    fo = np.zeros((3, Ny, Nz))
-    worst = 0.0
-    for s, dt in enumerate([0.0] + DTS):
-        rys = [O.noise_rys(5, 0, f, s, Ny, plane["Ny_max"][f], Nz) for f in range(3)]
-        hal = [O.noise_halo(5, 0, f, s, Ny, plane["Nz_max"][f]) for f in range(3)]
-        o = O.step(plane, rys, hal, fo, dt, first_step=(s == 0))
-        fo = o["filt_old"]
-        want = list(o["fluc"]) + [o["T"], o["rho"]] + list(o["filt"])
-        for i, b in enumerate(want):
-            if s == 0 and i in (3, 4):
-                continue
-            ok, r = normwise_close(part[s][0][i], b[:, k[0]:k[1]], TOL)
-            worst = max(worst, r)
-            assert ok, (s, i, r)
-    note(f"slab {k} at N_z = {N}", info, {"all": worst})
+    worst = run(df, Model(O, plane, 5, 0), DTS, k=k)
+    df.close()
+    note(f"slab {k} at N_z = {N}", info, {"all": max(worst.values())})
 
 
 @gpu

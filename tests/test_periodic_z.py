@@ -1,9 +1,10 @@
 """Spanwise-periodic planes (dfb_config.periodic_z = 1): the z filter wraps around the plane,
 filt[j, k] = sum_i b_i * y_filtered[j, (k + i) mod Nz], for every field, row and column.
 
-CPU: the struct layout, and the periodic restatement (periodic_step below: the oracle's unchanged plain-C stages recomposed with
-the wrap between the sweeps) against a direct circular convolution in numpy.  GPU (-m gpu): the library against that oracle under identical noise, the noise contract (r_ys drawn as
-without periodic_z, no halo), rolled inputs (no seam), interior columns unchanged, slabs, batches, errors, the config-4 gather."""
+CPU: the struct layout, and the periodic restatement (periodic_step in tests/oracle_harness.py: the oracle's unchanged plain-C
+stages recomposed with the wrap between the sweeps) against a direct circular convolution in numpy.  GPU (-m gpu): the library
+against that oracle under identical noise, the noise contract (r_ys drawn as without periodic_z, no halo), rolled inputs (no seam),
+interior columns unchanged, slabs, batches, errors, the config-4 gather."""
 import ctypes
 import os
 import socket
@@ -14,6 +15,7 @@ import numpy as np
 import pytest
 
 from conftest import ROOT, default_plane, normwise_close
+from oracle_harness import Model, explicit_config, explicit_plane, periodic_step, run
 
 TOL = 1e-12
 gpu = pytest.mark.gpu
@@ -22,60 +24,12 @@ gpu = pytest.mark.gpu
 # ---------------------------------------------------------------------------------------------
 # fixtures / helpers local to this file
 # ---------------------------------------------------------------------------------------------
-def _explicit_plane(W, Ny, Nz, Ny_rows, Nz_rows):
-    """row-uniform plane whose half-widths are supplied per row"""
-    yc = (np.arange(Ny) + 0.5) * 1e-5
-    N_y = np.stack([np.repeat(np.asarray(Ny_rows[f], dtype=np.int32)[:, None], Nz, axis=1) for f in range(3)])
-    N_z = np.stack([np.repeat(np.asarray(Nz_rows[f], dtype=np.int32)[:, None], Nz, axis=1) for f in range(3)])
-    return dict(name=f"explicit_{Ny}x{Nz}", Ny=Ny, Nz=Nz, d_i=W.D_I, U_e=W.U_E, yc=yc, dy=np.full(Ny, 1e-5), dz=np.full(Ny, 1e-5),
-                rows=W.synthetic_rows(yc + 1e-4), scales=W._scales(W.D_I), explicit_N=True,
-                N_y=N_y, N_z=N_z, Ny_max=[int(N_y[f].max()) for f in range(3)], Nz_max=[int(N_z[f].max()) for f in range(3)])
-
-
 def _ragged_half_widths(Ny, Nz, Nmax, seed):
     """per-cell half-widths that change from column to column (the general, non row-uniform path)"""
     rng = np.random.default_rng(seed)
     N_y = rng.integers(1, Nmax + 1, (3, Ny, Nz)).astype(np.int32)
     N_z = rng.integers(1, Nmax + 1, (3, Ny, Nz)).astype(np.int32)
     return N_y, N_z
-
-
-def periodic_step(O, plane, rys, fo, dt, first_step=False):
-    """The oracle's step for a spanwise-periodic plane, which the reference does not have: the plain-C restatement's stages
-    (oracle/df_oracle.c, unchanged) recomposed in orc_step's order -- orc_sweep_y per field, then the halo columns of r_zs set to
-    the y-filtered columns of the other edge (r_zs[:, :M] = r_zs[:, Nz:Nz+M], r_zs[:, Nz+M:] = r_zs[:, M:2M]; needs M <= Nz),
-    then the unchanged orc_sweep_z, orc_correlate, orc_rst_scaling and orc_sra.  Returns dict(filt, fluc, filt_old, T, rho, r_zs)
-    like oracle.step."""
-    import ctypes as C
-    L, d, i = O.lib(), O._d, O._i
-    Ny, Nz = plane["Ny"], plane["Nz"]
-    Lt = np.asarray(plane["scales"], dtype=np.float64)[:, 2]
-    rows = np.ascontiguousarray(plane["rows"], dtype=np.float64)
-    fo = [np.array(fo[f], dtype=np.float64).reshape(Ny, Nz).copy() for f in range(3)]
-    filt = [np.zeros((Ny, Nz)) for _ in range(3)]
-    fluc = [np.zeros((Ny, Nz)) for _ in range(3)]
-    T, rho = np.zeros((Ny, Nz)), np.zeros((Ny, Nz))
-    rzs = []
-    for f in range(3):
-        M = int(plane["Nz_max"][f])
-        assert M <= Nz, (f, M, Nz)
-        N_y = np.ascontiguousarray(plane["N_y"][f], dtype=np.int32)
-        N_z = np.ascontiguousarray(plane["N_z"][f], dtype=np.int32)
-        ry = np.ascontiguousarray(rys[f], dtype=np.float64)
-        rz = np.full((Ny, Nz + 2 * M), np.nan)
-        L.orc_sweep_y(C.c_int(Ny), C.c_int(Nz), C.c_int(int(plane["Ny_max"][f])), C.c_int(M), i(N_y), d(ry), d(rz))
-        rz[:, :M] = rz[:, Nz:Nz + M]                       # left of column 0: columns Nz-M .. Nz-1
-        rz[:, Nz + M:] = rz[:, M:2 * M]                    # right of column Nz-1: columns 0 .. M-1
-        L.orc_sweep_z(C.c_int(Ny), C.c_int(Nz), C.c_int(M), i(N_z), d(rz), d(filt[f]))
-        if not first_step:
-            L.orc_correlate(C.c_long(Ny * Nz), d(fo[f]), d(filt[f]), C.c_double(dt), C.c_double(float(Lt[f])))
-        rzs.append(rz)
-    r = [np.ascontiguousarray(rows[k]) for k in range(8)]  # R11, R21, R22, R33, Us, Ts, rhos, Ms
-    L.orc_rst_scaling(C.c_int(Ny), C.c_int(Nz), d(r[0]), d(r[1]), d(r[2]), d(r[3]), d(filt[0]), d(filt[1]), d(filt[2]),
-                      d(fluc[0]), d(fluc[1]), d(fluc[2]), d(fo[0]), d(fo[1]), d(fo[2]))
-    if not first_step:
-        L.orc_sra(C.c_int(Ny), C.c_int(Nz), d(r[7]), d(r[4]), d(r[5]), d(r[6]), d(fluc[0]), d(T), d(rho))
-    return dict(filt=np.stack(filt), fluc=np.stack(fluc), filt_old=np.stack(fo), T=T, rho=rho, r_zs=rzs)
 
 
 def numpy_periodic_step(O, plane, rys, fo, dt, first_step):
@@ -110,38 +64,14 @@ def numpy_periodic_step(O, plane, rys, fo, dt, first_step):
 
 
 def periodic_inject_and_step(dfb, O, plane, variant, seed, dts, explicit=False):
-    """constructor step + len(dts) filter steps of a periodic handle in inject mode against periodic_step on the same
+    """constructor step + len(dts) filter steps of a periodic handle in inject mode against the model (periodic_step) on the same
     counter-based r_ys; returns the worst normwise ratio per output"""
-    cfg = dfb.DFConfig.from_plane(plane, noise_mode=dfb.NOISE_INJECT, kernel_variant=variant, periodic_z=1)
-    if explicit:
-        cfg.geom_per_row = 0
-        cfg.yc = cfg.dy = cfg.dz = None
-        cfg.N_y, cfg.N_z = plane["N_y"], plane["N_z"]
-    else:
+    kw = dict(noise_mode=dfb.NOISE_INJECT, kernel_variant=variant, periodic_z=1)
+    if not explicit:
         O.half_widths(plane)
-    df = dfb.DIGITAL_FILTER(cfg)
+    df = dfb.DIGITAL_FILTER(explicit_config(dfb, plane, **kw) if explicit else dfb.DFConfig.from_plane(plane, **kw))
     assert df.periodic_z
-    Ny, Nz = plane["Ny"], plane["Nz"]
-    fo = np.zeros((3, Ny, Nz))
-    worst = {}
-    for s, dt in enumerate([0.0] + list(dts)):
-        rys = [O.noise_rys(seed, 0, f, s, Ny, plane["Ny_max"][f], Nz) for f in range(3)]
-        for f in range(3):
-            df.set_noise(f, rys[f], None)
-        df.first_step() if s == 0 else df.filter(dt)
-        df.fetch()
-        o = periodic_step(O, plane, rys, fo, dt, first_step=(s == 0))
-        fo = o["filt_old"]
-        got = dict(filt=np.stack([df.u.filt, df.v.filt, df.w.filt]), fluc=np.stack([df.u.fluc, df.v.fluc, df.w.fluc]),
-                   T=df.T_fluc, rho=df.rho_fluc)
-        for k in ("filt", "fluc", "T", "rho"):
-            if s == 0 and k in ("T", "rho"):
-                continue
-            for f in range(3) if k in ("filt", "fluc") else [None]:
-                a, b = (got[k][f], o[k][f]) if f is not None else (got[k], o[k])
-                ok, r = normwise_close(a, b, TOL)
-                worst[k] = max(worst.get(k, 0.0), r)
-                assert ok, (plane.get("name"), variant, s, k, f, r)
+    worst = run(df, Model(O, plane, seed, 0, periodic=True), dts)
     df.close()
     return worst
 
@@ -167,11 +97,11 @@ def test_config_layout(dfb):
 def test_oracle_periodic_restatement_against_numpy(O, W, case):
     """periodic_step == a direct circular convolution over the y-filtered field, within 1e-12"""
     if case == "odd_Nz":
-        plane = _explicit_plane(W, 23, 37, [np.arange(23) % 5 + 1] * 3, [np.arange(23) % 7 + 2, np.full(23, 9), np.arange(23) % 3 + 1])
+        plane = explicit_plane(W, 23, 37, [np.arange(23) % 5 + 1] * 3, [np.arange(23) % 7 + 2, np.full(23, 9), np.arange(23) % 3 + 1])
     elif case == "Nz_max_eq_Nz":
-        plane = _explicit_plane(W, 17, 20, [np.full(17, 3)] * 3, [np.full(17, 20), np.arange(17) % 20 + 1, np.full(17, 7)])
+        plane = explicit_plane(W, 17, 20, [np.full(17, 3)] * 3, [np.full(17, 20), np.arange(17) % 20 + 1, np.full(17, 7)])
     elif case == "ragged":
-        plane = _explicit_plane(W, 19, 31, [np.ones(19, int)] * 3, [np.ones(19, int)] * 3)
+        plane = explicit_plane(W, 19, 31, [np.ones(19, int)] * 3, [np.ones(19, int)] * 3)
         plane["N_y"], plane["N_z"] = _ragged_half_widths(19, 31, 9, seed=4)
         plane["Ny_max"] = [int(plane["N_y"][f].max()) for f in range(3)]
         plane["Nz_max"] = [int(plane["N_z"][f].max()) for f in range(3)]
@@ -252,7 +182,7 @@ def test_G2_periodic_saturated_plane(dfb, O, W, variant):
 def test_G2_periodic_ragged_per_cell_half_widths(dfb, O, W):
     """per-cell half-widths (the one-thread-per-cell path, whose y-sweep looks N_y up at the wrapped global column)"""
     Ny, Nz = 48, 64
-    plane = _explicit_plane(W, Ny, Nz, [np.ones(Ny, int)] * 3, [np.ones(Ny, int)] * 3)
+    plane = explicit_plane(W, Ny, Nz, [np.ones(Ny, int)] * 3, [np.ones(Ny, int)] * 3)
     plane["N_y"], plane["N_z"] = _ragged_half_widths(Ny, Nz, 12, seed=3)
     plane["Ny_max"] = [int(plane["N_y"][f].max()) for f in range(3)]
     plane["Nz_max"] = [int(plane["N_z"][f].max()) for f in range(3)]
@@ -295,22 +225,9 @@ def test_periodic_generate_mode_equals_oracle_on_the_same_stream(dfb, O, W):
     """generate mode end to end: device noise + device filter == oracle noise + periodic oracle, for the whole plane and for
     slabs touching either edge (whose wrapped neighbour columns are regenerated locally)"""
     plane = O.half_widths(W.plane_profile(96, 200, 24, 10))
-    Ny, Nz = 96, 200
-    dts = [0.0, 1e-7, 1e-7, 3e-7]
-    ref, fo = [], np.zeros((3, Ny, Nz))
-    for s, dt in enumerate(dts):
-        rys = [O.noise_rys(77, 0, f, s, Ny, plane["Ny_max"][f], Nz) for f in range(3)]
-        o = periodic_step(O, plane, rys, fo, dt, first_step=(s == 0))
-        fo = o["filt_old"]
-        ref.append(o)
-    for k0, k1 in [(0, 200), (0, 64), (144, 200), (5, 50), (190, 200)]:
-        df = dfb.DIGITAL_FILTER(dfb.DFConfig.from_plane(plane, seed=77, periodic_z=1, k_begin=k0, k_end=k1))
-        for s, dt in enumerate(dts):
-            if s:
-                df.filter(dt)
-            for f, F in enumerate((df.u, df.v, df.w)):
-                ok, r = normwise_close(F.fluc, ref[s]["fluc"][f][:, k0:k1], TOL)
-                assert ok, (k0, k1, s, f, r)
+    for k in [(0, 200), (0, 64), (144, 200), (5, 50), (190, 200)]:
+        df = dfb.DIGITAL_FILTER(dfb.DFConfig.from_plane(plane, seed=77, periodic_z=1, k_begin=k[0], k_end=k[1]), fetch=False)
+        run(df, Model(O, plane, 77, 0, periodic=True), [1e-7, 1e-7, 3e-7], k=k)
         assert df.step == 4
         df.close()
 

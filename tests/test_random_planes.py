@@ -10,7 +10,7 @@ N = 0 rows and fields, per-cell ragged planes, batches, periodic planes, slabs, 
 overrides and the launch knobs that change how work is distributed.
 
 CPU: the committed SEEDS reach every entry of FEATURES (read from each case's plan through tests/step_plan_shim.cpp, B200 limits),
-every plan passes the descriptor invariants of tests/test_step_plan.py, the drawn cases are pinned by a digest, the oracle work is
+every plan passes the descriptor invariants of tests/shims.py, the drawn cases are pinned by a digest, the oracle work is
 bounded, and the per-row gate is checked on hand-made arrays.
 GPU (-m gpu): each case's handle reports the shim's plan (dfb_info 3, 7-11) and its constructor step and three filter(dt) steps
 match the oracle in every output at the field-wide and at a per-row 1e-12 normwise gate; tuned cases match the one-thread-per-cell
@@ -26,10 +26,8 @@ import numpy as np
 import pytest
 
 from conftest import normwise_close
-from test_half_width_limits import y_limits, z_limits  # noqa: F401  (fixtures)
-from test_step_plan import (OVR, StepPlan, check_noise, check_y, check_z, dfbm, explicit_config, explicit_plane,  # noqa: F401
-                            shim, yr_group_cap)
-from test_step_sequences import Model
+from oracle_harness import Model, explicit_config, explicit_plane, package
+from shims import OVR, StepPlan, check_noise, check_y, check_z, step_plan_shim, y_limits, yr_group_cap, z_limits
 
 gpu = pytest.mark.gpu
 TOL = 1e-12
@@ -45,8 +43,18 @@ KNOBS = {"DFB_Z_BLOCKS_PER_SM": ("1", "2", "3"), "DFB_Y_PERSIST": ("1", "2", "7"
 
 
 @pytest.fixture(scope="module")
-def limits(z_limits, y_limits):  # noqa: F811
-    return dict(z={f"{zk}/{zm}": n for (zk, zm), n in z_limits.items()}, y=dict(y_limits))
+def shim(tmp_path_factory):
+    return step_plan_shim(tmp_path_factory)
+
+
+@pytest.fixture(scope="module")
+def dfbm():
+    return package()
+
+
+@pytest.fixture(scope="module")
+def limits(shim, dfbm, W):
+    return dict(z={f"{zk}/{zm}": n for (zk, zm), n in z_limits(shim, dfbm, W).items()}, y=dict(y_limits(shim, dfbm, W)))
 
 
 # ---------------------------------------------------------------------------------------------

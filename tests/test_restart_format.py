@@ -3,13 +3,13 @@ check a loader makes, the offsets of row segments in the global layout, and a sa
 dfb_restart_info then reads.  restart.cpp and csrc/setup.cpp are built with g++ against no CUDA library (tests/restart_shim.cpp)."""
 import ctypes as C
 import os
-import subprocess
 
 import numpy as np
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CSRC = os.path.join(ROOT, "digital-filtering_b200", "csrc")
+from oracle_harness import package
+from shims import build_shim
+
 DATA_AT = 8192
 SEC_STATE, SEC_STATS, SEC_CORR_Z, SEC_CORR_Y, SEC_CORR_T, SEC_RING = range(6)
 I64 = C.POINTER(C.c_int64)
@@ -17,11 +17,7 @@ I64 = C.POINTER(C.c_int64)
 
 @pytest.fixture(scope="module")
 def shim(tmp_path_factory):
-    lib = str(tmp_path_factory.mktemp("restart") / "librestart.so")       # a temporary directory: the tree may be read-only
-    srcs = [os.path.join(CSRC, "setup.cpp"), os.path.join(CSRC, "restart.cpp"), os.path.join(ROOT, "tests", "restart_shim.cpp")]
-    subprocess.run(["/usr/bin/g++", "-std=c++17", "-O2", "-Wall", "-I", os.path.join(ROOT, "include"), "-I", "/usr/local/cuda/include",
-                    "-I", CSRC, "-shared", "-fPIC", "-Wl,--no-undefined", *srcs, "-o", lib], check=True)
-    L = C.CDLL(lib)
+    L = build_shim(tmp_path_factory, "restart", "restart.cpp")
     L.rs_fingerprint.restype = C.c_uint64
     L.rs_fingerprint.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
     L.rs_roundtrip.argtypes = [I64, C.POINTER(C.c_double), I64, C.c_char_p, I64, C.POINTER(C.c_double), I64, C.c_char_p, C.c_char_p, C.c_int]
@@ -37,9 +33,7 @@ def shim(tmp_path_factory):
 
 @pytest.fixture(scope="module")
 def dfbm():
-    import _dfb_import  # noqa: F401
-    import digital_filtering_b200
-    return digital_filtering_b200
+    return package()
 
 
 def i64(a):

@@ -1,11 +1,11 @@
 """Long generate-mode runs against the oracle, step by step, across every way of driving a handle.
 
-A host model of a handle (Model below) is driven in lock step with the library.  Per plane it holds the step counter, filt_old, the
-last u', v', w', T', rho', the N2 sums and the correlation sums and ring; each step is oracle.step (or the periodic restatement of
-tests/test_periodic_z.py) on the oracle's noise for (seed, plane_id + p, field, step).  After every operation the library's fields,
-state, noise and statistics must match the model.  Comparing one handle with another cannot see an error in what run_step decides
-(which noise set a step reads, whether the prefetched set holds this step's noise, when N2 and the correlation sums accumulate),
-because both sides go through the same run_step; the oracle can.
+A host model of a handle (Model, tests/oracle_harness.py) is driven in lock step with the library.  Per plane it holds the step
+counter, filt_old, the last u', v', w', T', rho', the N2 sums and the correlation sums and ring; each step is oracle.step (or the
+periodic restatement, periodic_step in tests/oracle_harness.py) on the oracle's noise for (seed, plane_id + p, field, step).  After
+every operation the library's fields, state, noise and statistics must match the model.  Comparing one handle with another cannot
+see an error in what run_step decides (which noise set a step reads, whether the prefetched set holds this step's noise, when N2
+and the correlation sums accumulate), because both sides go through the same run_step; the oracle can.
 
 CPU: the model against plain oracle.step chains, and the operation generator.  GPU (-m gpu): one scenario per decision of run_step /
 dfb_set_state / dfb_generate_noise, seeded random sequences of ~40 operations, on every y-sweep form, simple kernels, periodic planes,
@@ -16,8 +16,7 @@ import numpy as np
 import pytest
 
 from conftest import normwise_close
-from test_correlation import np_sums
-from test_periodic_z import periodic_step
+from oracle_harness import Model, np_sums, periodic_step
 
 gpu = pytest.mark.gpu
 TOL = 1e-12
@@ -26,124 +25,6 @@ PLANE_ID = 2
 LAGS_A = (9, 7, 3)                   # (L_z, L_y, L_t)
 LAGS_B = (4, 0, 5)                   # changed lags: y off, more time lags than some runs have steps
 DT = (1e-7, 2e-7, 3e-7, 5e-8)        # Lt is 1.2e-6 (u) and 4.5e-7 (v, w): every step blends
-
-
-# ---------------------------------------------------------------------------------------------
-# the host model of a handle
-# ---------------------------------------------------------------------------------------------
-class Model:
-    """What a generate-mode handle holds, per plane p (noise stream group plane_id + p), and what each call does to it.  The
-    semantics are the library's (include/dfb200.h):
-      - a step consumes the noise of (seed, plane_id + p, field, counter), then the counter moves on by one;
-      - a first step (the constructor's, dfb_first_step) does not blend and leaves T' / rho' untouched;
-      - a first step is not accumulated by N2 or by the correlation statistics;
-      - dfb_set_state keeps the N2 sums and empties the correlation ring (the next step follows the restored state, not the ring);
-      - dfb_set_state(NULL, s) moves only the counter; with filt_old it replaces filt_old as well;
-      - dfb_stats_enable(1) zeroes the N2 sums and their count, (0) stops accumulating and keeps them;
-      - dfb_corr_enable(1, lags) zeroes the sums, the pair counts and the step count and empties the ring, (0) stops accumulating
-        and keeps the sums readable;
-      - dfb_generate_noise(k) changes nothing but which noise dfb_get_noise returns."""
-
-    def __init__(self, O, plane, seed=SEED, plane_id=PLANE_ID, nplanes=1, periodic=False):
-        self.O, self.plane, self.seed, self.plane_id, self.P, self.periodic = O, plane, seed, plane_id, nplanes, periodic
-        self.Ny, self.Nz = plane["Ny"], plane["Nz"]
-        self.step = 0
-        self.fo = np.zeros((nplanes, 3, self.Ny, self.Nz))
-        self.out = np.zeros((nplanes, 5, self.Ny, self.Nz))          # u', v', w', T', rho'
-        self.noise_step = None                                      # the step whose noise dfb_get_noise returns
-        self.stats = None                                           # [P][6][Ny][Nz]: u'^2, v'^2, w'^2, T'^2, rho'^2, u'v'
-        self.stats_on, self.stats_count = False, 0
-        self.lags = None                                            # correlation statistics: None before any enable
-        self.corr_on = False
-        self._noise = {}
-
-    def noise(self, p, f, step):
-        key = (p, f, step)
-        if key not in self._noise:
-            pl, O = self.plane, self.O
-            rys = O.noise_rys(self.seed, self.plane_id + p, f, step, self.Ny, pl["Ny_max"][f], self.Nz)
-            hal = None if self.periodic else O.noise_halo(self.seed, self.plane_id + p, f, step, self.Ny, pl["Nz_max"][f])
-            self._noise[key] = (rys, hal)
-        return self._noise[key]
-
-    def filter(self, dt, first=False):
-        for p in range(self.P):
-            rys = [self.noise(p, f, self.step)[0] for f in range(3)]
-            if self.periodic:
-                o = periodic_step(self.O, self.plane, rys, self.fo[p], dt, first_step=first)
-            else:
-                o = self.O.step(self.plane, rys, [self.noise(p, f, self.step)[1] for f in range(3)], self.fo[p], dt, first_step=first)
-            self.fo[p] = o["filt_old"]
-            self.out[p, :3] = o["fluc"]
-            if not first:                                           # a first step leaves T', rho' untouched
-                self.out[p, 3], self.out[p, 4] = o["T"], o["rho"]
-        if not first:                                               # ... and is not accumulated
-            self._accumulate()
-        self.noise_step = self.step
-        self.step += 1
-
-    def first_step(self):
-        self.filter(0.0, first=True)
-
-    def _accumulate(self):
-        if self.stats_on:
-            u, v = self.out[:, 0], self.out[:, 1]
-            self.stats[:, :5] += self.out * self.out
-            self.stats[:, 5] += u * v
-            self.stats_count += 1
-        if self.corr_on:
-            Lz, Ly, Lt = self.lags
-            M = min(Lt, len(self.ring))
-            for p in range(self.P):
-                for f in range(3):
-                    x = self.out[p, f]
-                    s = np_sums([x], (Lz, Ly, 0), self.periodic)
-                    for d in (0, 1):
-                        if d in s:
-                            self.csum[d][p, f] += s[d][0]
-                    if Lt:
-                        for m in range(M + 1):
-                            self.csum[2][p, f][:, m] += (x * (x if m == 0 else self.ring[-m][p, f])).sum(1)
-            if Lt:
-                self.tsteps[:M + 1] += 1
-                self.ring = (self.ring + [self.out[:, :3].copy()])[-Lt:]
-            self.corr_count += 1
-
-    def set_state(self, fo, step):
-        if fo is not None:
-            self.fo = np.array(fo, dtype=np.float64).reshape(3, self.P, self.Ny, self.Nz).transpose(1, 0, 2, 3).copy()
-        self.step = step
-        if self.lags is not None:
-            self.ring = []                                          # the N2 and correlation sums stay
-
-    def stats_enable(self, on):
-        if on:
-            self.stats = np.zeros((self.P, 6, self.Ny, self.Nz))
-            self.stats_count = 0
-        self.stats_on = bool(on)
-
-    def corr_enable(self, on, lags=None):
-        if on:
-            self.lags = tuple(lags)
-            self.csum = {d: np.zeros((self.P, 3, self.Ny, lags[d] + 1)) for d in range(3) if lags[d]}
-            self.corr_count, self.tsteps, self.ring = 0, np.zeros(lags[2] + 1, dtype=np.int64), []
-        self.corr_on = bool(on)
-
-    def generate_noise(self, k):
-        self.noise_step = k
-
-    def state_for_library(self):
-        """filt_old in the layout dfb_set_state takes: [3][P][Ny][Nz] ([3][Ny][Nz] for one plane)"""
-        fo = self.fo.transpose(1, 0, 2, 3)
-        return np.ascontiguousarray(fo[:, 0] if self.P == 1 else fo)
-
-    def pairs(self, d):
-        Lz = self.lags[d]
-        if d == 0:
-            return np.array([self.corr_count * (self.Nz if self.periodic else self.Nz - e) for e in range(Lz + 1)], dtype=np.int64)
-        if d == 1:
-            return np.full(Lz + 1, self.corr_count * self.Nz, dtype=np.int64)
-        return self.tsteps * self.Nz
 
 
 # ---------------------------------------------------------------------------------------------
@@ -187,7 +68,7 @@ class Driver:
         self.dfb, self.O = dfb, O
         cfg = dfb.DFConfig.from_plane(plane, seed=SEED, plane_id=PLANE_ID, periodic_z=int(periodic), **kw)
         self.df = dfb.DIGITAL_FILTER(cfg, fetch=False, nplanes=nplanes)
-        self.m = Model(O, plane, nplanes=nplanes, periodic=periodic)
+        self.m = Model(O, plane, SEED, PLANE_ID, nplanes=nplanes, periodic=periodic)
         self.m.first_step()                                         # the constructor's step
         self.P, self.n = nplanes, plane["Ny"] * plane["Nz"]
         self.pending = []                                           # pipelined copies: (host arrays, expected fields)
@@ -374,7 +255,7 @@ def small(O, W):
 
 def test_model_rewinds_and_counter_moves_follow_oracle_chains(O, small):
     """set_state to an earlier step with that step's filt_old, set_state(None, later) and a first step in the middle of the run"""
-    m = Model(O, small)
+    m = Model(O, small, SEED, PLANE_ID)
     m.first_step()
     m.filter(1e-7)
     saved = m.state_for_library().copy()                          # filt_old after step 1, counter 2
@@ -396,7 +277,7 @@ def test_model_rewinds_and_counter_moves_follow_oracle_chains(O, small):
 def test_model_statistics_across_first_step_and_set_state(O, small):
     """N2: every non-first step since dfb_stats_enable(1), across set_state.  Correlation sums: z and y over the same steps, t only
     between steps with no set_state in between (the ring empties), pairs counted from the steps the ring held"""
-    m = Model(O, small)
+    m = Model(O, small, SEED, PLANE_ID)
     m.first_step()
     m.stats_enable(True)
     L = (5, 4, 3)
@@ -435,12 +316,12 @@ def test_model_statistics_across_first_step_and_set_state(O, small):
 
 def test_model_batch_planes_are_single_planes_and_periodic_uses_the_restatement(O, small):
     """plane p of a batch model is the single-plane model with plane_id + p; a periodic model steps through periodic_step"""
-    b = Model(O, small, nplanes=2)
-    s = Model(O, small, plane_id=PLANE_ID + 1)
+    b = Model(O, small, SEED, PLANE_ID, nplanes=2)
+    s = Model(O, small, SEED, PLANE_ID + 1)
     for m in (b, s):
         m.first_step(); m.filter(1e-7); m.filter(2e-7)
     assert np.array_equal(b.out[1], s.out[0]) and not np.array_equal(b.out[0], b.out[1])
-    pm = Model(O, small, periodic=True)
+    pm = Model(O, small, SEED, PLANE_ID, periodic=True)
     pm.first_step(); pm.filter(1e-7)
     rys = lambda st: [O.noise_rys(SEED, PLANE_ID, f, st, 24, small["Ny_max"][f], 40) for f in range(3)]
     o0 = periodic_step(O, small, rys(0), np.zeros((3, 24, 40)), 0.0, first_step=True)
