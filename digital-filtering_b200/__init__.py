@@ -28,6 +28,9 @@ NOISE_GENERATE, NOISE_INJECT = 0, 1
 CORR_Z, CORR_Y, CORR_T = 0, 1, 2        # correlation directions (dfb_corr_enable)
 DFB_CORR_SUPPORT = CORR_SUPPORT = -1    # lag = the filter's whole support (z and y)
 RESTART_STATE, RESTART_STATS, RESTART_CORR = 1, 2, 4   # sections of a restart file (dfb_save_restart)
+MAP_POINT, MAP_AREA = 0, 1               # face maps (dfb_facemap_create): bilinear at the face centre / average over the face
+MAP_WALL_ZERO = 1                        # point maps: linear to 0 at the wall below the first cell centre
+FLUCS = (U_FLUC, V_FLUC, W_FLUC, T_FLUC, RHO_FLUC)
 RESTART_INFO = ("version", "Ny", "Nz", "plane_id", "nplanes", "seed", "periodic_z", "noise_mode", "step", "sections", "records",
                 "fingerprint", "Ny_max_u", "Ny_max_v", "Ny_max_w", "Nz_max_u", "Nz_max_v", "Nz_max_w", "tuned", "z_form", "y_form",
                 "stats_count", "stats_on", "corr_lag_z", "corr_lag_y", "corr_lag_t", "corr_count", "corr_on", "ring_fields", "bytes")
@@ -139,6 +142,12 @@ def lib():
         L.dfb_save_restart.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
         L.dfb_load_restart.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
         L.dfb_restart_info.argtypes = [C.c_char_p, C.POINTER(C.c_int64), C.c_int]
+        L.dfb_facemap_create.argtypes = [C.c_void_p, C.c_int, C.c_int, c_dp, c_dp, c_dp, c_dp, C.c_int, C.c_int, C.c_int, c_ip]
+        L.dfb_facemap_served.argtypes = [C.c_void_p, C.c_int, c_ip]
+        L.dfb_facemap_destroy.argtypes = [C.c_void_p, C.c_int]
+        L.dfb_interp_to_cells.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_void_p), c_dp,
+                                          C.POINTER(C.c_void_p), C.c_int]
+        L.dfb_interp_to_host.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, c_dp]
         _lib = L
     return _lib
 
@@ -245,6 +254,54 @@ def fill_config(c, config):
     c.skip_first_step, c.kernel_variant = config.skip_first_step, config.kernel_variant
     c.periodic_z = config.periodic_z
     return keep
+
+
+def _mask(fields):
+    m = 0
+    for f in fields:
+        if f not in FLUCS:
+            raise ValueError(f"field {f!r} is not one of U_FLUC .. RHO_FLUC")
+        m |= 1 << f
+    return m
+
+
+class FaceMap:
+    """Interpolation of a handle's outputs onto a CFD code's inflow faces (dfb_facemap_create): made by DIGITAL_FILTER.facemap, alive
+    until close() or the handle's close().  .served: 0/1 per face, 1 where this handle serves the face."""
+
+    def __init__(self, owner, map_id, n):
+        self._o, self.id, self.n = owner, map_id, n
+        self.served = np.zeros(n, dtype=np.int32)
+        _check(lib().dfb_facemap_served(owner._h, map_id, self.served.ctypes.data_as(c_ip)))
+
+    def to_cells(self, dst, dst_index=None, mean=None, scale=None, fields=FLUCS, plane=0, stride=1):
+        """dst[r][dst_index[i] * stride] = (mean[r][i] | dst's own value) + scale[r] * interpolated field fields[r], for each served
+        face i, enqueued on the handle's stream.  dst, mean: sequences aligned with `fields` of CUDA float64 torch tensors on the
+        handle's device (a mean entry may be None), dst_index an int32 CUDA tensor (None: face i -> i), scale a sequence of floats.
+        The handle's stream (stream()) does not wait for other streams: finish writing the arrays first (torch.cuda.synchronize())."""
+        fields = list(fields)
+        d5, m5, s5 = (C.c_void_p * 5)(), (C.c_void_p * 5)(), (C.c_double * 5)(1, 1, 1, 1, 1)
+        for r, f in enumerate(fields):
+            d5[f] = dst[r].data_ptr()
+            if mean is not None and mean[r] is not None:
+                m5[f] = mean[r].data_ptr()
+            if scale is not None:
+                s5[f] = float(scale[r])
+        _check(lib().dfb_interp_to_cells(self._o._h, self.id, plane, _mask(fields),
+                                         C.c_void_p(dst_index.data_ptr()) if dst_index is not None else None, m5, s5, d5, int(stride)))
+
+    def to_host(self, fields=FLUCS, plane=0, out=None):
+        """[len(fields)][n] interpolated fluctuations (rows in increasing field order); only the served faces' entries are written"""
+        fields = sorted(fields)
+        out = np.zeros((len(fields), self.n)) if out is None else out
+        assert out.dtype == np.float64 and out.flags.c_contiguous and out.shape == (len(fields), self.n)
+        _check(lib().dfb_interp_to_host(self._o._h, self.id, plane, _mask(fields), _dptr(out)))
+        return out
+
+    def close(self):
+        if self.id is not None and getattr(self._o, "_h", None):
+            _check(lib().dfb_facemap_destroy(self._o._h, self.id))
+        self.id = None
 
 
 class FilterField:
@@ -531,6 +588,25 @@ class DIGITAL_FILTER:
         out = np.zeros(len(yf), dtype=np.int32)
         _check(lib().dfb_face_map(self._h, len(yf), _dptr(yf), _dptr(zf), out.ctypes.data_as(c_ip)))
         return out
+
+    def facemap(self, yf, zf, hy=None, hz=None, own=None, wall_zero=False):
+        """A face map for the faces centred at (yf, zf): bilinear at the centres, or with the extents hy, hz the average over each face
+        rectangle.  own = (k_begin, k_end): the columns whose faces this handle serves (default its slab); wall_zero: a point map goes
+        linearly to 0 at the wall below the first cell centre."""
+        yf = np.ascontiguousarray(yf, dtype=np.float64)
+        zf = np.ascontiguousarray(zf, dtype=np.float64)
+        if (hy is None) != (hz is None):
+            raise ValueError("give both hy and hz, or neither")
+        kind = MAP_POINT if hy is None else MAP_AREA
+        hy = None if hy is None else np.ascontiguousarray(hy, dtype=np.float64)
+        hz = None if hz is None else np.ascontiguousarray(hz, dtype=np.float64)
+        if any(a is not None and a.shape != yf.shape for a in (zf, hy, hz)) or yf.ndim != 1:
+            raise ValueError("yf, zf (and hy, hz) must be 1-D arrays of one length")
+        own = (0, 0) if own is None else own
+        mid = C.c_int()
+        _check(lib().dfb_facemap_create(self._h, kind, len(yf), _dptr(yf), _dptr(zf), _dptr(hy), _dptr(hz), int(own[0]), int(own[1]),
+                                        MAP_WALL_ZERO if wall_zero else 0, C.byref(mid)))
+        return FaceMap(self, mid.value, len(yf))
 
     # ---- config 4: this handle as one spanwise slab of a plane shared with the other ranks (NCCL inside the library) ----
     @staticmethod

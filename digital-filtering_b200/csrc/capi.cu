@@ -19,6 +19,7 @@
 #include "device.cuh"
 #include "kernels.hpp"
 #include "restart.hpp"
+#include "facemap.hpp"
 
 using namespace dfb;
 
@@ -37,6 +38,21 @@ int fail(int code, const std::string& msg) {
         if (e__ != cudaSuccess)                                                                     \
             throw Error{DFB_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(e__)};         \
     } while (0)
+
+// A face map on the device (dfb_facemap_create): the taps of facemap.hpp, and what dfb_interp_to_host needs to deliver the served faces
+struct FaceMapDev {
+    int kind = DFB_MAP_POINT, n = 0, n_served = 0;
+    std::vector<int> served, faces;   // host: 0/1 per face; the served faces in order
+    int* idx = nullptr;
+    int* ptr = nullptr;               // DFB_MAP_AREA only
+    int* slot = nullptr;              // face -> its row in stage; nullptr when every face is served (face i -> i)
+    double* w = nullptr;
+    double* stage = nullptr;          // [5][n_served], allocated by the first dfb_interp_to_host
+    FaceMapDev() = default;
+    FaceMapDev(const FaceMapDev&) = delete;
+    FaceMapDev& operator=(const FaceMapDev&) = delete;
+    ~FaceMapDev() { cudaFree(idx); cudaFree(ptr); cudaFree(slot); cudaFree(w); cudaFree(stage); }
+};
 
 }  // namespace
 
@@ -119,6 +135,8 @@ struct dfb_filter_s {
     int g_dst = -1;
     int64_t g_begun = 0, g_ended = 0, g_bytes_wire = 0;
     bool g_after_first_only = false;  // the gathered step was the constructor's: T', rho' are zero (df.cpp:57-65)
+    // face maps of the CFD hand-off (dfb_facemap_create): map id = index; a destroyed map leaves nullptr
+    std::vector<std::unique_ptr<FaceMapDev>> facemaps;
     // timing
     bool timing = false;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -143,6 +161,7 @@ struct dfb_filter_s {
         cudaSetDevice(device);
         if (side) cudaStreamSynchronize(side);
         if (stream) cudaStreamSynchronize(stream);
+        facemaps.clear();
         for (void* p : allocs) cudaFree(p);
         for (void* p : corr_mem) cudaFree(p);
         cudaFree(corr.ring);
@@ -1354,6 +1373,147 @@ int dfb_face_map(dfb_handle h, int n, const double* yf, const double* zf, int* p
     return DFB_OK;
 }
 
+}  // extern "C" (reopened below the face maps' helpers)
+
+// ---- face maps: the taps are built on the host (facemap.cpp), summed on the device (interp_kernel) ----
+namespace {
+
+void check_idle(const dfb_filter_s& H) {
+    if (H.pipe_begun != H.pipe_ended || H.g_begun != H.g_ended)
+        throw Error{DFB_ERR_STATE, "a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first"};
+}
+
+FaceMapDev& facemap_of(dfb_filter_s& H, int map_id) {
+    if (map_id < 0 || map_id >= (int)H.facemaps.size() || !H.facemaps[map_id])
+        throw Error{DFB_ERR_ARG, "no face map " + std::to_string(map_id) + " on this handle"};
+    return *H.facemaps[map_id];
+}
+
+template <class T>
+T* upload_now(const std::vector<T>& v, cudaStream_t st) {
+    T* p = nullptr;
+    CUDA_TRY(cudaMalloc(&p, std::max<size_t>(v.size(), 1) * sizeof(T)));
+    if (!v.empty()) {
+        cudaError_t e = cudaMemcpyAsync(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) { cudaFree(p); throw Error{DFB_ERR_CUDA, std::string("face map upload: ") + cudaGetErrorString(e)}; }
+    }
+    return p;
+}
+
+// the checks and arguments dfb_interp_to_cells and dfb_interp_to_host share
+InterpArgs interp_args(dfb_filter_s& H, const FaceMapDev& F, int plane, int fields) {
+    if (plane < 0 || plane >= H.nplanes) throw Error{DFB_ERR_ARG, "plane out of range"};
+    if (fields <= 0 || (fields & ~31)) throw Error{DFB_ERR_ARG, "fields must be a non-empty mask of the bits 1 << DFB_U_FLUC .. 1 << DFB_RHO_FLUC"};
+    InterpArgs a{};
+    for (int f = 0; f < 5; ++f) { a.field[f] = (fields >> f) & 1 ? field_ptr(H, f, plane) : nullptr; a.scale[f] = 1.0; }
+    a.n = F.n; a.fields = fields; a.stride = 1;
+    a.idx = F.idx; a.w = F.w; a.ptr = F.ptr;
+    return a;
+}
+
+}  // namespace
+
+extern "C" {
+
+int dfb_facemap_create(dfb_handle h, int kind, int n, const double* yf, const double* zf, const double* hy, const double* hz, int own_begin,
+                       int own_end, int flags, int* map_id) {
+    if (!h || !map_id) return fail(DFB_ERR_ARG, "handle/map_id is NULL");
+    return guarded([&] {
+        check_idle(*h);
+        const FaceMap M = build_face_map(h->plan, kind, n, yf, zf, hy, hz, own_begin, own_end, flags);
+        CUDA_TRY(cudaSetDevice(h->device));
+        auto F = std::make_unique<FaceMapDev>();
+        F->kind = kind; F->n = n; F->n_served = M.n_served; F->served = M.served;
+        for (int i = 0; i < n; ++i)
+            if (M.served[i]) F->faces.push_back(i);
+        F->idx = upload_now(M.idx, h->stream);
+        F->w = upload_now(M.w, h->stream);
+        if (kind == DFB_MAP_AREA) F->ptr = upload_now(M.ptr, h->stream);
+        if (M.n_served < n) {
+            std::vector<int> slot(n, -1);
+            for (int r = 0; r < M.n_served; ++r) slot[F->faces[r]] = r;
+            F->slot = upload_now(slot, h->stream);
+        }
+        int id = 0;
+        while (id < (int)h->facemaps.size() && h->facemaps[id]) ++id;
+        if (id == (int)h->facemaps.size()) h->facemaps.emplace_back();
+        h->facemaps[id] = std::move(F);
+        *map_id = id;
+    });
+}
+
+int dfb_facemap_served(dfb_handle h, int map_id, int* served) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    return guarded([&] {
+        const FaceMapDev& F = facemap_of(*h, map_id);
+        if (F.n > 0 && !served) throw Error{DFB_ERR_ARG, "served is NULL"};
+        std::copy(F.served.begin(), F.served.end(), served);
+    });
+}
+
+int dfb_facemap_destroy(dfb_handle h, int map_id) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    return guarded([&] {
+        facemap_of(*h, map_id);
+        CUDA_TRY(cudaSetDevice(h->device));
+        CUDA_TRY(cudaStreamSynchronize(h->stream));        // an enqueued dfb_interp_to_cells may still read the taps
+        h->facemaps[map_id].reset();
+    });
+}
+
+int dfb_interp_to_cells(dfb_handle h, int map_id, int plane, int fields, const int* dst_index, const double* const mean[5],
+                        const double scale[5], double* const dst[5], int stride) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    return guarded([&] {
+        check_idle(*h);
+        const FaceMapDev& F = facemap_of(*h, map_id);
+        InterpArgs a = interp_args(*h, F, plane, fields);
+        if (stride < 1) throw Error{DFB_ERR_ARG, "stride must be >= 1"};
+        if (F.n > 0 && !dst) throw Error{DFB_ERR_ARG, "dst is NULL"};
+        for (int f = 0; f < 5; ++f) {
+            if (!((fields >> f) & 1)) continue;
+            if (F.n > 0 && !dst[f]) throw Error{DFB_ERR_ARG, "dst[" + std::to_string(f) + "] is NULL for a requested field"};
+            a.dst[f] = F.n > 0 ? dst[f] : nullptr;
+            a.mean[f] = mean ? mean[f] : nullptr;
+            if (!a.mean[f]) a.add |= 1 << f;                    // dst's own value is the base
+            if (scale) a.scale[f] = scale[f];
+        }
+        a.dst_index = dst_index;
+        a.stride = stride;
+        CUDA_TRY(cudaSetDevice(h->device));
+        CUDA_TRY(launch_interp(a, h->stream));
+    });
+}
+
+int dfb_interp_to_host(dfb_handle h, int map_id, int plane, int fields, double* out) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    return guarded([&] {
+        check_idle(*h);
+        FaceMapDev& F = facemap_of(*h, map_id);
+        InterpArgs a = interp_args(*h, F, plane, fields);
+        if (F.n > 0 && !out) throw Error{DFB_ERR_ARG, "out is NULL"};
+        CUDA_TRY(cudaSetDevice(h->device));
+        const size_t ns = (size_t)F.n_served;
+        if (!F.stage) CUDA_TRY(cudaMalloc(&F.stage, std::max<size_t>(5 * ns, 1) * sizeof(double)));
+        int nf = 0;
+        for (int f = 0; f < 5; ++f)
+            if ((fields >> f) & 1) a.dst[f] = F.stage + ns * nf++;
+        a.dst_index = F.slot;
+        CUDA_TRY(launch_interp(a, h->stream));
+        if (ns == (size_t)F.n) {                                 // every face served: the staged rows are out's rows
+            if (ns) CUDA_TRY(cudaMemcpyAsync(out, F.stage, nf * ns * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+            CUDA_TRY(cudaStreamSynchronize(h->stream));
+        } else {                                                 // only the served faces' entries of out change
+            std::vector<double> buf(nf * ns);
+            if (ns) CUDA_TRY(cudaMemcpyAsync(buf.data(), F.stage, nf * ns * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+            CUDA_TRY(cudaStreamSynchronize(h->stream));
+            for (int r = 0; r < nf; ++r)
+                for (size_t s = 0; s < ns; ++s) out[(size_t)r * F.n + F.faces[s]] = buf[r * ns + s];
+        }
+    });
+}
+
 int dfb_debug_yprof(dfb_handle h, unsigned long long* out8) {
     if (!h || !out8) return fail(DFB_ERR_ARG, "bad argument");
     return guarded([&] {
@@ -1764,6 +1924,26 @@ int dfb_save_restart_f(const dfb_handle* h, const char* path, const int* path_le
 }
 int dfb_load_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what) {
     return (h && path && what) ? dfb_load_restart(*h, fortran_path(path, path_len).c_str(), *what) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_facemap_create_f(const dfb_handle* h, const int* kind, const int* n, const double* yf, const double* zf, const double* hy,
+                         const double* hz, const int* own_begin, const int* own_end, const int* flags, int* map_id) {
+    return (h && kind && n && own_begin && own_end && flags)
+               ? dfb_facemap_create(*h, *kind, *n, yf, zf, hy, hz, *own_begin, *own_end, *flags, map_id)
+               : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_facemap_served_f(const dfb_handle* h, const int* map_id, int* served) {
+    return (h && map_id) ? dfb_facemap_served(*h, *map_id, served) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_facemap_destroy_f(const dfb_handle* h, const int* map_id) {
+    return (h && map_id) ? dfb_facemap_destroy(*h, *map_id) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_interp_to_host_f(const dfb_handle* h, const int* map_id, const int* plane, const int* fields, double* out) {
+    return (h && map_id && plane && fields) ? dfb_interp_to_host(*h, *map_id, *plane, *fields, out) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_interp_to_cells_f(const dfb_handle* h, const int* map_id, const int* plane, const int* fields, const int* dst_index,
+                          const double* const mean[5], const double scale[5], double* const dst[5], const int* stride) {
+    return (h && map_id && plane && fields && stride) ? dfb_interp_to_cells(*h, *map_id, *plane, *fields, dst_index, mean, scale, dst, *stride)
+                                                      : fail(DFB_ERR_ARG, "NULL argument");
 }
 int dfb_destroy_f(dfb_handle* h) {
     if (!h) return DFB_OK;

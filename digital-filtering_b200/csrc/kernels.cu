@@ -1296,6 +1296,46 @@ __global__ void __launch_bounds__(256) scatter_kernel(const double* __restrict__
     dst[d] = __fma_rn(scale, field[c], base);
 }
 
+// Face maps (dfb_interp_to_cells / _to_host): one thread per face reads the face's taps once and feeds every tap to up to five gathers
+// (u', v', w', T', rho').  The taps are summed in the map's order, each field in its own register, so a face's value depends on neither
+// the launch nor the slab nor the batch.  AREA = false: the fixed 4-tap record (idx int4, w 2 x double2); true: CSR.
+template <bool AREA>
+__global__ void __launch_bounds__(256) interp_kernel(const InterpArgs a) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n) return;
+    double acc[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+    if constexpr (!AREA) {
+        const int4 c = __ldg(reinterpret_cast<const int4*>(a.idx) + i);
+        if (c.x < 0) return;                 // not served by this handle
+        const double2 w01 = __ldg(reinterpret_cast<const double2*>(a.w) + 2 * i);
+        const double2 w23 = __ldg(reinterpret_cast<const double2*>(a.w) + 2 * i + 1);
+        const int ct[4] = {c.x, c.y, c.z, c.w};
+        const double wt[4] = {w01.x, w01.y, w23.x, w23.y};
+#pragma unroll
+        for (int t = 0; t < 4; ++t)
+#pragma unroll
+            for (int f = 0; f < 5; ++f)
+                if (a.fields & (1 << f)) acc[f] = __fma_rn(wt[t], __ldg(a.field[f] + ct[t]), acc[f]);
+    } else {
+        const int t0 = __ldg(a.ptr + i), t1 = __ldg(a.ptr + i + 1);
+        if (t0 == t1) return;                // not served by this handle
+        for (int t = t0; t < t1; ++t) {
+            const int c = __ldg(a.idx + t);
+            const double w = __ldg(a.w + t);
+#pragma unroll
+            for (int f = 0; f < 5; ++f)
+                if (a.fields & (1 << f)) acc[f] = __fma_rn(w, __ldg(a.field[f] + c), acc[f]);
+        }
+    }
+    const long long d = (long long)(a.dst_index ? a.dst_index[i] : i) * a.stride;
+#pragma unroll
+    for (int f = 0; f < 5; ++f)
+        if (a.fields & (1 << f)) {
+            const double base = a.mean[f] ? a.mean[f][i] : ((a.add >> f) & 1) ? a.dst[f][d] : 0.0;
+            a.dst[f][d] = __fma_rn(a.scale[f], acc[f], base);
+        }
+}
+
 // config 4, destination rank: ONE rank's staged slab [3][Ny][W] -> its columns [k0, k0+W) of the row-major planes [5][Ny][NzG];
 // T' and rho' are rebuilt from u' with the row constants, with the epilogue's own roundings (df.cpp:474-481), so the assembled
 // plane is bit for bit what the slabs hold.  Launched per source rank as its slab lands (the next rank's transfer runs meanwhile).
@@ -1349,6 +1389,13 @@ cudaError_t launch_scatter(const double* field, int n, const int* plane_index, c
                            double* dst, cudaStream_t st) {
     if (n <= 0) return cudaSuccess;
     scatter_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(field, n, plane_index, dst_index, mean, scale, dst);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_interp(const InterpArgs& a, cudaStream_t st) {
+    if (a.n <= 0) return cudaSuccess;
+    if (a.ptr) interp_kernel<true><<<(unsigned)((a.n + 255) / 256), 256, 0, st>>>(a);
+    else interp_kernel<false><<<(unsigned)((a.n + 255) / 256), 256, 0, st>>>(a);
     return cudaGetLastError();
 }
 
@@ -1410,6 +1457,7 @@ cudaError_t ysweep_prepare() {
     // as a process-wide bimodal y-sweep time on small planes: 26 or 43 us on the reference default plane).  {kernel, dynamic smem}
     const std::pair<const void*, int> fns[] = {
         {(const void*)noise_kernel, 0}, {(const void*)noise_pieces_kernel, 0}, {(const void*)stats_kernel, 0}, {(const void*)scatter_kernel, 0},
+        {(const void*)interp_kernel<false>, 0}, {(const void*)interp_kernel<true>, 0},
         {(const void*)ysweep_tma_kernel<Y_RC, Y_NS, 128>, (int)sizeof(YSmem<Y_RC, Y_NS, 128>)},
         {(const void*)ysweep_tma_kernel<Y_RC, Y_NS, 64>, (int)sizeof(YSmem<Y_RC, Y_NS, 64>)},
         {(const void*)ysweep_rec_kernel<Y_RC, Y_NS>, (int)sizeof(YSmem<Y_RC, Y_NS>)}};

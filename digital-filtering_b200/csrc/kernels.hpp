@@ -18,6 +18,21 @@ cudaError_t launch_zsweep_tuned(const ZMaps& maps, const ZParams& P, cudaStream_
 cudaError_t launch_stats(const PlaneDev& D, double* sums, cudaStream_t st);
 cudaError_t launch_scatter(const double* field, int n, const int* plane_index, const int* dst_index, const double* mean, double scale,
                            double* dst, cudaStream_t st);
+// face maps (facemap.hpp): dst[f][dst_index[i] * stride] = base + scale[f] * sum_t w_t * field[f][idx_t] for the served faces i < n and
+// the fields f in `fields`; base = mean[f][i], else dst's own value where bit f of `add` is set, else 0.  ptr == nullptr: 4 taps per face.
+struct InterpArgs {
+    const double* field[5];
+    const double* mean[5];
+    double scale[5];
+    double* dst[5];
+    const int* dst_index;             // nullptr: face i -> i
+    long long stride;
+    int n, fields, add;
+    const int* idx;
+    const double* w;
+    const int* ptr;
+};
+cudaError_t launch_interp(const InterpArgs& a, cudaStream_t st);
 cudaError_t launch_rebuild(double* plane, const double* rowc, int Ny, int NzG, int k0, int W, int first_only, cudaStream_t st);
 cudaError_t launch_assemble(const double* slab, double* plane, const double* rowc, int Ny, int NzG, int k0, int W, int first_only, cudaStream_t st);
 cudaError_t launch_dfma_peak(double* out, int blocks, int iters, cudaStream_t st);

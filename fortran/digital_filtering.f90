@@ -19,6 +19,8 @@
 !   face_map, apply_inflow                        N3: inflow face -> plane cell, ghost cell = mean + fluctuation (us3d_user.f90:85-114)
 !   corr_enable, corr_get, integral_scales        correlation statistics along z, y and in time (dfb_corr_*): the delivered scales
 !   save_restart, load_restart                    restart files: resume a run across jobs, bit for bit, whatever the slab layout
+!   facemap_create, interp_to_host,               the outputs interpolated onto the CFD code's own faces (bilinear or area-weighted),
+!   interp_to_cells, filter_on_device               all five fields in one pass on the device; only the faces cross PCIe
 !
 ! NOTE: NEVER COMPILED -- no Fortran compiler exists in the build image or on the GPU boxes.  The binding is exercised through
 ! tests/fortran_abi_mimic.c, a C program that makes exactly these calls with exactly this struct layout and by-reference
@@ -32,6 +34,7 @@ module DIGITAL_FILTERING
     public :: comm_unique_id, comm_init, gather_begin, gather_end, gathered_field, face_map, apply_inflow
     public :: corr_enable, corr_get, integral_scales
     public :: save_restart, load_restart, RESTART_STATE, RESTART_STATS, RESTART_CORR
+    public :: facemap_create, interp_to_host, interp_to_cells, facemap_destroy, MAP_POINT, MAP_AREA, MAP_WALL_ZERO, filter_on_device
 
     integer, parameter :: RESTART_STATE = 1, RESTART_STATS = 2, RESTART_CORR = 4   ! DFB_RESTART_* (what to save / load; added together)
 
@@ -71,6 +74,9 @@ module DIGITAL_FILTERING
     end type digital_filter_batch_type
 
     ! image of `struct dfb_config` (include/dfb200.h) -- keep the two in step
+    ! face maps (include/dfb200.h, dfb_facemap_create); fields of interp_*: sum of 2**(0..4) for u', v', w', T', rho'
+    integer, parameter :: MAP_POINT = 0, MAP_AREA = 1, MAP_WALL_ZERO = 1
+
     type, bind(C) :: dfb_config_c
         real(c_double) :: d_i, rho_e, U_e, mu_e
         integer(c_int) :: vel_file_offset, vel_file_N_values
@@ -198,6 +204,46 @@ module DIGITAL_FILTERING
             type(c_ptr), intent(in) :: handle
             type(c_ptr), value :: path
             integer(c_int), intent(in) :: path_len, what
+        end function
+        integer(c_int) function dfb_filter_f(handle, dt) bind(C, name='dfb_filter_f')
+            import :: c_int, c_ptr, c_double
+            type(c_ptr), intent(in) :: handle
+            real(c_double), intent(in) :: dt
+        end function
+        integer(c_int) function dfb_facemap_create_f(handle, kind, n, yf, zf, hy, hz, own_begin, own_end, flags, map_id) &
+                bind(C, name='dfb_facemap_create_f')
+            import :: c_int, c_ptr, c_double
+            type(c_ptr), intent(in) :: handle
+            integer(c_int), intent(in) :: kind, n, own_begin, own_end, flags
+            real(c_double), intent(in) :: yf(*), zf(*)
+            type(c_ptr), value :: hy, hz
+            integer(c_int), intent(out) :: map_id
+        end function
+        integer(c_int) function dfb_facemap_destroy_f(handle, map_id) bind(C, name='dfb_facemap_destroy_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle
+            integer(c_int), intent(in) :: map_id
+        end function
+        integer(c_int) function dfb_facemap_served_f(handle, map_id, served) bind(C, name='dfb_facemap_served_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle
+            integer(c_int), intent(in) :: map_id
+            integer(c_int), intent(inout) :: served(*)
+        end function
+        integer(c_int) function dfb_interp_to_host_f(handle, map_id, plane, fields, out) bind(C, name='dfb_interp_to_host_f')
+            import :: c_int, c_ptr, c_double
+            type(c_ptr), intent(in) :: handle
+            integer(c_int), intent(in) :: map_id, plane, fields
+            real(c_double), intent(inout) :: out(*)
+        end function
+        integer(c_int) function dfb_interp_to_cells_f(handle, map_id, plane, fields, dst_index, mean, scale, dst, stride) &
+                bind(C, name='dfb_interp_to_cells_f')
+            import :: c_int, c_ptr, c_double
+            type(c_ptr), intent(in) :: handle
+            integer(c_int), intent(in) :: map_id, plane, fields, stride
+            type(c_ptr), value :: dst_index
+            type(c_ptr), intent(in) :: mean(5), dst(5)
+            real(c_double), intent(in) :: scale(5)
         end function
         function dfb_last_error() bind(C, name='dfb_last_error') result(msg)
             import :: c_ptr
@@ -357,6 +403,76 @@ contains
             if (cell(i) > 0) q(ghost(i)) = mean(i) + fluc(cell(i))
         end do
     end subroutine apply_inflow
+
+    ! ---- face maps: the outputs interpolated onto this rank's own faces (include/dfb200.h, dfb_facemap_create) ----
+    subroutine filter_on_device(DF, dt_input)     ! filter(DF, dt) without the copy of the five fields to DF%u%fluc ... (face maps read them)
+        type(digital_filter_type), intent(inout) :: DF
+        real(kind=dp), intent(in) :: dt_input
+        real(c_double) :: dt
+        dt = dt_input
+        call check(dfb_filter_f(DF%handle, dt), 'filter_on_device')
+    end subroutine filter_on_device
+
+    subroutine facemap_create(DF, n, yf, zf, map_id, hy, hz, own_begin, own_end, wall_zero, served)
+        ! bilinear at the face centres, or with hy, hz the average over each face; own_begin/own_end: 0-based columns [own_begin,
+        ! own_end) whose faces this rank serves (default: its slab); served(i) = 1 where it serves face i
+        type(digital_filter_type), intent(in) :: DF
+        integer, intent(in) :: n
+        real(kind=dp), intent(in) :: yf(n), zf(n)
+        integer, intent(out) :: map_id
+        real(kind=dp), intent(in), target, optional :: hy(n), hz(n)
+        integer, intent(in), optional :: own_begin, own_end
+        logical, intent(in), optional :: wall_zero
+        integer, intent(out), optional :: served(n)
+        integer(c_int) :: nn, kind, o0, o1, flags, id
+        type(c_ptr) :: phy, phz
+        nn = n; kind = MAP_POINT; o0 = 0; o1 = 0; flags = 0
+        phy = c_null_ptr; phz = c_null_ptr
+        if (present(hy) .and. present(hz)) then
+            kind = MAP_AREA; phy = c_loc(hy); phz = c_loc(hz)
+        end if
+        if (present(own_begin)) o0 = own_begin
+        if (present(own_end)) o1 = own_end
+        if (present(wall_zero)) then
+            if (wall_zero) flags = MAP_WALL_ZERO
+        end if
+        call check(dfb_facemap_create_f(DF%handle, kind, nn, yf, zf, phy, phz, o0, o1, flags, id), 'facemap_create')
+        map_id = id
+        if (present(served)) call check(dfb_facemap_served_f(DF%handle, id, served), 'facemap_create')
+    end subroutine facemap_create
+
+    subroutine interp_to_host(DF, map_id, fields, out, plane)   ! out(n, nfields): the served faces' entries, fields in increasing order
+        type(digital_filter_type), intent(in) :: DF
+        integer, intent(in) :: map_id, fields
+        real(kind=dp), intent(inout) :: out(:, :)
+        integer, intent(in), optional :: plane
+        integer(c_int) :: id, f, p
+        id = map_id; f = fields; p = 0
+        if (present(plane)) p = plane
+        call check(dfb_interp_to_host_f(DF%handle, id, p, f, out), 'interp_to_host')
+    end subroutine interp_to_host
+
+    subroutine interp_to_cells(DF, map_id, fields, dst_index, mean, scale, dst, stride, plane)
+        ! device arrays (CUDA Fortran / OpenACC host_data): dst(f)[dst_index(i) * stride] = mean(f)[i] (or dst's own value where
+        ! mean(f) is c_null_ptr) + scale(f) * interpolated field f; 0-based dst_index, c_null_ptr for face i -> i
+        type(digital_filter_type), intent(in) :: DF
+        integer, intent(in) :: map_id, fields, stride
+        type(c_ptr), intent(in) :: dst_index, mean(5), dst(5)
+        real(kind=dp), intent(in) :: scale(5)
+        integer, intent(in), optional :: plane
+        integer(c_int) :: id, f, s, p
+        id = map_id; f = fields; s = stride; p = 0
+        if (present(plane)) p = plane
+        call check(dfb_interp_to_cells_f(DF%handle, id, p, f, dst_index, mean, scale, dst, s), 'interp_to_cells')
+    end subroutine interp_to_cells
+
+    subroutine facemap_destroy(DF, map_id)
+        type(digital_filter_type), intent(in) :: DF
+        integer, intent(in) :: map_id
+        integer(c_int) :: id
+        id = map_id
+        call check(dfb_facemap_destroy_f(DF%handle, id), 'facemap_destroy')
+    end subroutine facemap_destroy
 
     ! ---- correlation statistics (like the rest of this module, never compiled: see the note at the top) ----
     subroutine corr_enable(DF, lz, ly, lt)         ! lags along z, y (0 = off, -1 = the filter's whole support) and t (0..64 steps)

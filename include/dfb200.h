@@ -327,6 +327,46 @@ int dfb_write_tecplot(dfb_handle h, const char* path);
  * the result is what dfb_scatter_to_cells takes as plane_index (after a copy to the device). */
 int dfb_face_map(dfb_handle h, int n, const double* yf, const double* zf, int* plane_index);
 
+/* Face maps -- interpolate the outputs onto a CFD code's own inflow faces, on the device, all five fields in one pass.
+ * A map is built once from the plane's global geometry: per face a fixed list of (plane cell, weight) taps.
+ *   DFB_MAP_POINT  bilinear at the face centre (yf, zf) between the cell centres dfb_write_csv prints (at most 4 taps).  Beyond the
+ *                  last centre z wraps with periodic_z (column Nz-1 with column 0) and clamps to the edge column without it; y clamps
+ *                  to the top row above it and to the first row below csv_yc[0] -- with DFB_MAP_WALL_ZERO it goes linearly to 0 at the
+ *                  wall vert_y[0] (dfb_get_table 12) instead and is 0 below it (no-slip fluctuations).  Needs increasing yc.
+ *   DFB_MAP_AREA   the average over the face rectangle [yf -+ hy/2] x [zf -+ hz/2] of the cells [vert_y[j], vert_y[j+1]) x
+ *                  [vert_z[k], vert_z[k+1]) (the cells dfb_face_map uses), weight = overlap area / face area, for finite-volume ghost
+ *                  cells.  A part of a face outside the plane counts toward the nearest edge cell (wraps in z with periodic_z).  The
+ *                  weights sum to 1; a face equal to a cell is that cell.
+ * Serving: face i is served by the handle whose columns [own_begin, own_end) (0,0: its slab) contain the column of the cell holding the
+ * face centre (dfb_face_map's clamped rule); every other face is not served (dfb_facemap_served).  A served face whose taps need a
+ * column the handle does not compute (a bilinear tap across a slab cut, a wide area face) fails the creation with DFB_ERR_ARG naming
+ * the face and the columns.  Remedy: create each slab 16 columns wider on each side (k_begin - 16, k_end + 16, within the plane) and
+ * pass the unwidened columns as own_begin, own_end.  Slabs cut on multiples of 16 compute the whole plane's bits, so the overlap columns
+ * hold the same values on both ranks and the faces of all ranks together are exactly the whole-plane result, with no communication.
+ * (On a periodic plane, faces within half a cell of the seam -- bilinear between columns Nz-1 and 0 -- need a whole-plane handle.)
+ * Errors: DFB_ERR_ARG for a bad kind, flag, mask, plane or map id, NULL arrays where n > 0, a non-finite coordinate, an extent <= 0
+ * in an AREA map or extents given for a POINT map; DFB_ERR_STATE while a dfb_filter_to_host_begin or dfb_gather_begin is outstanding.
+ * Maps are geometry only: they stay valid across dfb_set_state and dfb_load_restart, are not saved, and launch nothing per step.
+ * dfb_destroy frees the maps still alive. */
+enum { DFB_MAP_POINT = 0, DFB_MAP_AREA = 1 };
+enum { DFB_MAP_WALL_ZERO = 1 };
+int dfb_facemap_create(dfb_handle h, int kind, int n, const double* yf, const double* zf,
+                       const double* hy, const double* hz,      /* face extents, AREA only (NULL for POINT) */
+                       int own_begin, int own_end, int flags, int* map_id);
+int dfb_facemap_served(dfb_handle h, int map_id, int* served /* [n] 0/1, host */);
+int dfb_facemap_destroy(dfb_handle h, int map_id);
+/* dst_f[dst_index[i] * stride] = mean_f[i] (dst's own value when mean or mean[f] is NULL) + scale_f * sum_t w_t * field_f[cell_t]
+ * for every served face i and every field f in `fields` (bit 1 << DFB_U_FLUC .. 1 << DFB_RHO_FLUC) of plane `plane` of the handle.
+ * Taps are summed in the map's fixed order (no atomics, no reduction across threads): a result depends on neither the launch, the
+ * slab nor the batch.  dst_index, mean[f] ([n]) and dst[f] are DEVICE arrays; dst_index NULL means face i -> i; scale NULL means 1;
+ * stride >= 1 lets dst be an array-of-structs state vector q(nvar, ncell) (dst[f] = &q(f, 0)).  Entries of unserved faces are not read
+ * or written.  Enqueued on the handle's stream after the last enqueued step, like dfb_scatter_to_cells. */
+int dfb_interp_to_cells(dfb_handle h, int map_id, int plane, int fields, const int* dst_index, const double* const mean[5],
+                        const double scale[5], double* const dst[5], int stride);
+/* The plain interpolated fluctuations of the served faces into host out[nfields][n] (the fields of the mask in increasing order):
+ * sampled into a device staging buffer, then only those doubles cross PCIe.  Synchronous.  Entries of unserved faces are untouched. */
+int dfb_interp_to_host(dfb_handle h, int map_id, int plane, int fields, double* out);
+
 /* CUDA-event time of the last dfb_filter, ms: stage 0 noise, 1 y-sweep, 2 z-sweep+epilogue, 3 whole step.
  * Only recorded when enabled with dfb_set_timing(h, 1). */
 int dfb_set_timing(dfb_handle h, int on);
@@ -355,6 +395,14 @@ int dfb_destroy_f(dfb_handle* h);
 /* path: Fortran character variable (c_loc) + its len_trim, as the file names of dfb_config (path_len < 0: NUL-terminated) */
 int dfb_save_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);
 int dfb_load_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);
+/* face maps: hy, hz by address (NULL for a POINT map); mean, dst: five addresses (type(c_ptr) mean(5), dst(5)), mean may be NULL */
+int dfb_facemap_create_f(const dfb_handle* h, const int* kind, const int* n, const double* yf, const double* zf, const double* hy,
+                         const double* hz, const int* own_begin, const int* own_end, const int* flags, int* map_id);
+int dfb_facemap_served_f(const dfb_handle* h, const int* map_id, int* served);
+int dfb_facemap_destroy_f(const dfb_handle* h, const int* map_id);
+int dfb_interp_to_host_f(const dfb_handle* h, const int* map_id, const int* plane, const int* fields, double* out);
+int dfb_interp_to_cells_f(const dfb_handle* h, const int* map_id, const int* plane, const int* fields, const int* dst_index,
+                          const double* const mean[5], const double scale[5], double* const dst[5], const int* stride);
 
 #ifdef __cplusplus
 }

@@ -62,6 +62,41 @@ struct DFConfigEx {
     bool fetch_every_step = true;      // copy u', v', w', T', rho' into the host vectors after each filter()
 };
 
+// A face map of the CFD hand-off (dfb_facemap_create), from DIGITAL_FILTER::face_map_interp; destroyed with this object, which must
+// not outlive its DIGITAL_FILTER.  fields: mask of 1 << DFB_U_FLUC .. 1 << DFB_RHO_FLUC.
+class FaceMap {
+  public:
+    FaceMap(dfb_handle h, int id, int n) : h_(h), id_(id), n_(n), served_(n) {
+        if (n > 0 && dfb_facemap_served(h_, id_, served_.data()) != DFB_OK) throw std::runtime_error(std::string("FaceMap: ") + dfb_last_error());
+    }
+    FaceMap(FaceMap&& o) noexcept : h_(o.h_), id_(o.id_), n_(o.n_), served_(std::move(o.served_)) { o.h_ = nullptr; }
+    FaceMap(const FaceMap&) = delete;
+    FaceMap& operator=(const FaceMap&) = delete;
+    ~FaceMap() { if (h_) dfb_facemap_destroy(h_, id_); }
+    const std::vector<int>& served() const { return served_; }   // 1 where this handle serves the face
+    // device arrays: dst[f][dst_index[i] * stride] = (mean[f][i] | dst's own value) + scale[f] * interpolated field f
+    void to_cells(int fields, const int* dst_index, const double* const mean[5], const double scale[5], double* const dst[5], int stride = 1,
+                  int plane = 0) {
+        check(dfb_interp_to_cells(h_, id_, plane, fields, dst_index, mean, scale, dst, stride));
+    }
+    // [nfields][n] interpolated fluctuations on the host (rows in increasing field order; unserved faces 0)
+    std::vector<double> to_host(int fields = 31, int plane = 0) {
+        int nf = 0;
+        for (int f = 0; f < 5; ++f) nf += (fields >> f) & 1;
+        std::vector<double> out((size_t)nf * n_, 0.0);
+        check(dfb_interp_to_host(h_, id_, plane, fields, out.data()));
+        return out;
+    }
+
+  private:
+    dfb_handle h_;
+    int id_, n_;
+    std::vector<int> served_;
+    static void check(int rc) {
+        if (rc != DFB_OK) throw std::runtime_error(std::string("FaceMap: ") + dfb_last_error());
+    }
+};
+
 class DIGITAL_FILTER {
   public:
     FilterField u, v, w;               // df.hpp:87
@@ -146,6 +181,18 @@ class DIGITAL_FILTER {
     // outputs until then).  Slabs of one plane may save into one file; it is complete when every writer has returned.
     void save_restart(const std::string& path, int what = DFB_RESTART_STATE) { check(dfb_save_restart(h_, path.c_str(), what)); }
     void load_restart(const std::string& path, int what = DFB_RESTART_STATE) { check(dfb_load_restart(h_, path.c_str(), what)); }
+    // face map at the face centres (yf, zf): bilinear (hy, hz empty) or the average over each face (extents hy, hz); own_begin,
+    // own_end: the columns whose faces this handle serves (0, 0: its slab); flags: DFB_MAP_WALL_ZERO
+    FaceMap face_map_interp(const std::vector<double>& yf, const std::vector<double>& zf, const std::vector<double>& hy = {},
+                            const std::vector<double>& hz = {}, int own_begin = 0, int own_end = 0, int flags = 0) {
+        const bool area = !hy.empty() || !hz.empty();
+        if (zf.size() != yf.size() || (area && (hy.size() != yf.size() || hz.size() != yf.size())))
+            throw std::runtime_error("DIGITAL_FILTER: yf, zf (and hy, hz) must have one length");
+        int id = -1;
+        check(dfb_facemap_create(h_, area ? DFB_MAP_AREA : DFB_MAP_POINT, (int)yf.size(), yf.data(), zf.data(), area ? hy.data() : nullptr,
+                                 area ? hz.data() : nullptr, own_begin, own_end, flags, &id));
+        return FaceMap(h_, id, (int)yf.size());
+    }
     const Vector& T_rms() const { return T_rms_; }
     const Vector& rho_rms() const { return rho_rms_; }
     int rms_counter = 0;               // df.hpp:63
