@@ -148,6 +148,8 @@ def lib():
         L.dfb_interp_to_cells.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_void_p), c_dp,
                                           C.POINTER(C.c_void_p), C.c_int]
         L.dfb_interp_to_host.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, c_dp]
+        L.dfb_attach_stream.argtypes = [C.c_void_p, C.c_void_p]
+        L.dfb_filter_dev.argtypes = [C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -387,6 +389,23 @@ class DIGITAL_FILTER:
 
     def first_step(self):
         _check(lib().dfb_first_step(self._h))
+
+    # ---- GPU-resident callers: steps on the caller's stream, dt in device memory, capturable (include/dfb200.h, dfb_attach_stream) ----
+    def attach_stream(self, stream):
+        """Every later call of this handle that enqueues device work goes on `stream` (a torch.cuda.Stream, or a raw cudaStream_t as an
+        int), with the step's state in device memory, so that filter_dev() can be captured by torch.cuda.graph on that stream.  None
+        detaches (synchronises, reads the step state back)."""
+        if stream is not None and not isinstance(stream, int):
+            stream = stream.cuda_stream
+        _check(lib().dfb_attach_stream(self._h, C.c_void_p(stream) if stream else None))
+
+    def filter_dev(self, dt):
+        """One step with dt read from device memory when the step runs: dt is a 1-element CUDA float64 tensor on this handle's device,
+        which must stay alive until the step has run (for a captured graph: as long as the graph is replayed).  The handle must be
+        attached (attach_stream).  A dt that is not finite or < 0 voids the step; the next synchronising call raises DfbError(ERR_ARG)."""
+        if not dt.is_cuda or dt.dtype.itemsize != 8 or not dt.dtype.is_floating_point or dt.numel() != 1:
+            raise ValueError("dt must be a 1-element CUDA float64 tensor")
+        _check(lib().dfb_filter_dev(self._h, C.c_void_p(dt.data_ptr())))
 
     def filter_batch(self, dts, out=None):
         dts = np.ascontiguousarray(dts, dtype=np.float64)

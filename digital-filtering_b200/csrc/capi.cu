@@ -70,6 +70,12 @@ struct dfb_filter_s {
     cudaStream_t stream = nullptr;    // main stream (high priority): sweeps + epilogue
     cudaStream_t side = nullptr;      // low-priority stream: next step's noise, generated while this step filters
     cudaStream_t copy = nullptr;      // dfb_filter_to_host_begin/end: device-to-host copies of step t under the compute of step t+1
+    // dfb_attach_stream: while attached, `stream` IS the caller's stream (every call that enqueues or synchronises uses it) and the
+    // handle's own main stream waits in own_stream; the step's host state lives in the device record `rec`
+    bool attached = false;
+    cudaStream_t own_stream = nullptr;
+    StepRecord* rec = nullptr;
+    AdvanceParams adv{};              // what every attached step's advance launch takes (rec, time scales, seed, streams, pairs)
     double* stage[2] = {nullptr, nullptr};                 // staged copies of the five output fields
     cudaEvent_t ev_staged[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
     long long pipe_begun = 0, pipe_ended = 0;
@@ -159,6 +165,7 @@ struct dfb_filter_s {
     }
     ~dfb_filter_s() {
         cudaSetDevice(device);
+        if (attached) { cudaStreamSynchronize(stream); stream = own_stream; }
         if (side) cudaStreamSynchronize(side);
         if (stream) cudaStreamSynchronize(stream);
         facemaps.clear();
@@ -333,20 +340,7 @@ void build_device(dfb_filter_s& H) {
     CUDA_TRY(cudaStreamSynchronize(H.stream));
 }
 
-void fill_noise_params(dfb_filter_s& H, int64_t step) {
-    for (int n = 0; n < H.np.n_arrays; ++n) {
-        const NoiseArray& a = H.np.a[n];
-        for (int p = 0; p < H.nplanes; ++p) {
-            // stream ((plane*3 + field)*2 + array) of include/dfb_rng_spec.h; plane p of a batch is plane_id + p
-            const uint64_t stream = (uint64_t)((((int64_t)H.plane_id + p) * 3 + a.field) * 2 + a.kind);
-            const uint64_t inc = (stream << 1) | 1u;
-            const uint64_t state0 = pcg_lcg(H.seed + inc, inc);
-            const Jump j = pcg_jump(4u * ((uint64_t)step * H.npairs[n]), inc);
-            H.np.pstate[p][n] = j.A * state0 + j.C;
-            H.np.pinc[p][n] = inc;
-        }
-    }
-}
+void fill_noise_params(dfb_filter_s& H, int64_t step) { fill_noise_states(H.np, H.npairs, H.seed, H.plane_id, H.nplanes, step); }
 
 void launch_noise_for(dfb_filter_s& H, int64_t step, int b, cudaStream_t st) {
     H.ybuf_step[b] = -1;                 // new noise invalidates whatever y-sweep result the set held
@@ -357,7 +351,50 @@ void launch_noise_for(dfb_filter_s& H, int64_t step, int b, cudaStream_t st) {
     H.buf_step[b] = step;
 }
 
+// A step of a handle attached to a caller's stream (dfb_attach_stream): advance -> noise -> y-sweep(s) -> z-sweep (-> N2 for the
+// one-thread-per-cell kernels), all on that stream, buffer set 0 only, the host's decisions taken on the device from the step record.
+// No side stream, no event, no synchronisation, no allocation: the step can be captured into a CUDA graph, and each replay advances
+// the generator by one step.  dt_dev == nullptr: dt and its blend constants are the host's (dfb_filter), bit for bit a host-driven step.
+void run_step_attached(dfb_filter_s& H, double dt, const double* dt_dev, bool first) {
+    CUDA_TRY(cudaSetDevice(H.device));
+    const bool accumulate = H.stats_on && !first;
+    AdvanceParams A = H.adv;
+    A.dt_dev = dt_dev;
+    A.dt = dt;
+    if (!dt_dev)
+        for (int f = 0; f < 3; ++f) blend_consts(dt, H.plan.f[f].Lt, A.sa[f], A.sb[f]);
+    A.stats = accumulate ? 1 : 0;
+    CUDA_TRY(launch_advance(A, H.stream));
+    NoiseParams np = H.np;
+    np.rec = H.rec;
+    np.tl = nullptr;
+    CUDA_TRY(launch_noise(np, H.nwin, H.D[0], H.stream));
+    H.buf_step[0] = H.buf_step[1] = -1;            // the sets hold no step the host knows of: host-driven steps after a detach draw anew
+    H.ybuf_step[0] = H.ybuf_step[1] = -1;
+    H.noise_view = 0;
+    StepConsts S{};
+    S.first_step = first ? 1 : 0;
+    if (H.tuned) {
+        YParams Y = H.yp[0];
+        Y.tl = nullptr;
+        Y.zcounter_init = 8 * H.zp[0].nblocks;
+        if (H.y_form != 2) CUDA_TRY(launch_ysweep_tma(H.maps[0], Y, H.n_tiles_dense, H.n_tiles_rec, H.stream));
+        if (H.y_form >= 2) CUDA_TRY(launch_ysweep_run(H.rmaps[0], Y, H.stream));
+        ZParams Z = H.zp[0];
+        Z.S = S;
+        Z.rec = H.rec;
+        Z.tl = nullptr;
+        Z.stats = accumulate ? H.stats : nullptr;
+        CUDA_TRY(launch_zsweep_tuned(H.zmaps[0], Z, H.stream));
+    } else {
+        CUDA_TRY(launch_ysweep_simple(H.D[0], H.stream));
+        CUDA_TRY(launch_zsweep_simple(H.D[0], S, H.rec, H.stream));
+        if (accumulate) CUDA_TRY(launch_stats(H.D[0], H.stats, H.rec, H.stream));
+    }
+}
+
 void run_step(dfb_filter_s& H, double dt, bool first) {
+    if (H.attached) { run_step_attached(H, dt, nullptr, first); return; }
     CUDA_TRY(cudaSetDevice(H.device));
     const int b = (int)(H.step & 1);
     if (H.timing) CUDA_TRY(cudaEventRecord(H.ev[0], H.stream));
@@ -384,20 +421,15 @@ void run_step(dfb_filter_s& H, double dt, bool first) {
     if (H.timing) CUDA_TRY(cudaEventRecord(H.ev[2], H.stream));
     StepConsts S{};
     S.first_step = first ? 1 : 0;
-    for (int f = 0; f < 3; ++f) {
-        const double pi = 3.141592654;                             // df.cpp:411 (SURVEY quirk 2)
-        const double alpha = std::exp(-pi * dt / H.plan.f[f].Lt);  // df.cpp:412
-        S.sa[f] = std::sqrt(alpha);                                // df.cpp:415
-        S.sb[f] = std::sqrt(1.0 - alpha);
-    }
+    for (int f = 0; f < 3; ++f) blend_consts(dt, H.plan.f[f].Lt, S.sa[f], S.sb[f]);
     const bool accumulate = H.stats_on && !first;                  // rms_add, df.cpp:606
     if (H.tuned) {
         H.zp[b].S = S;
         H.zp[b].stats = accumulate ? H.stats : nullptr;            // N2 fused into the epilogue
         CUDA_TRY(launch_zsweep_tuned(H.zmaps[b], H.zp[b], H.stream));
     } else {
-        CUDA_TRY(launch_zsweep_simple(H.D[b], S, H.stream));
-        if (accumulate) CUDA_TRY(launch_stats(H.D[0], H.stats, H.stream));
+        CUDA_TRY(launch_zsweep_simple(H.D[b], S, nullptr, H.stream));
+        if (accumulate) CUDA_TRY(launch_stats(H.D[0], H.stats, nullptr, H.stream));
     }
     if (accumulate) H.stats_count += 1;
     if (H.corr_on && !first) {
@@ -463,6 +495,43 @@ void check_dt(double dt) {
     char buf[64];
     std::snprintf(buf, sizeof(buf), "%g", dt);
     throw Error{DFB_ERR_ARG, std::string("dt must be finite and >= 0, got ") + buf};
+}
+
+const char* const VOID_STEP_MSG = "dt must be finite and >= 0: an attached step (dfb_filter_dev) read such a dt from device memory and was void";
+
+std::string attached_msg(const char* call) { return std::string(call) + " is not available while the handle is attached to a stream (dfb_attach_stream)"; }
+void refuse_attached(const dfb_filter_s& H, const char* call) { if (H.attached) throw Error{DFB_ERR_STATE, attached_msg(call)}; }
+
+// Attached: waits for the caller's stream and reads the device step record back into the host's step counter and N2 count.  A void
+// step since the last read is reported once, as DFB_ERR_ARG, and forgotten.  Host-driven: nothing.
+void sync_record(dfb_filter_s& H) {
+    if (!H.attached) return;
+    CUDA_TRY(cudaSetDevice(H.device));
+    StepRecord R;
+    CUDA_TRY(cudaMemcpyAsync(&R, H.rec, sizeof(R), cudaMemcpyDeviceToHost, H.stream));
+    CUDA_TRY(cudaStreamSynchronize(H.stream));
+    H.step = R.step;
+    H.stats_count = R.stats_count;
+    if (R.void_seen) {
+        static const int zero = 0;
+        CUDA_TRY(cudaMemcpyAsync(&H.rec->void_seen, &zero, sizeof(zero), cudaMemcpyHostToDevice, H.stream));
+        CUDA_TRY(cudaStreamSynchronize(H.stream));
+        throw Error{DFB_ERR_ARG, VOID_STEP_MSG};
+    }
+}
+
+// Writes the host's step counter and N2 count into the device step record (dfb_attach_stream, and dfb_set_state / dfb_load_restart
+// while attached).  Its noise positions are those of the last step taken, which a void step's noise launch reproduces.
+void push_record(dfb_filter_s& H) {
+    StepRecord R{};
+    R.step = H.step;
+    R.stats_count = H.stats_count;
+    NoiseParams np = H.np;
+    fill_noise_states(np, H.npairs, H.seed, H.plane_id, H.nplanes, std::max<int64_t>(H.step - 1, 0));
+    std::memcpy(R.pstate, np.pstate, sizeof(R.pstate));
+    CUDA_TRY(cudaSetDevice(H.device));
+    CUDA_TRY(cudaMemcpyAsync(H.rec, &R, sizeof(R), cudaMemcpyHostToDevice, H.stream));
+    CUDA_TRY(cudaStreamSynchronize(H.stream));
 }
 
 // filt_old [3][P][Ny*W] (host; nullptr keeps it) and the step counter (dfb_set_state, dfb_load_restart)
@@ -587,6 +656,10 @@ int dfb_dims(dfb_handle h, int* Ny, int* Nz) {
 int dfb_info(dfb_handle h, int what, int field, int64_t* out64) {
     if (!h || !out64) return fail(DFB_ERR_ARG, "handle/out is NULL");
     if (field < 0 || field > 2) return fail(DFB_ERR_ARG, "field must be 0..2");
+    if (h->attached) {
+        const int rc = guarded([&] { sync_record(*h); });
+        if (rc != DFB_OK) return rc;
+    }
     switch (what) {
         case 0: *out64 = h->plan.f[field].Ny_max; break;
         case 1: *out64 = h->plan.f[field].Nz_max; break;
@@ -658,6 +731,7 @@ int dfb_get_field_plane(dfb_handle h, int plane, int which, double* dst, int dst
     const double* src = field_ptr(*h, which, plane);
     if (!src) return fail(DFB_ERR_ARG, "unknown field selector");
     return guarded([&] {
+        sync_record(*h);
         CUDA_TRY(cudaSetDevice(h->device));
         const size_t bytes = sizeof(double) * h->D[0].ps_cells;
         CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, dst_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, h->stream));
@@ -671,6 +745,7 @@ int dfb_filter_to_host(dfb_handle h, double dt, double* u, double* v, double* w,
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     return guarded([&] {
         check_dt(dt);
+        sync_record(*h);
         run_step(*h, dt, false);
         const size_t bytes = sizeof(double) * h->D[0].ps_cells * h->nplanes;     // a batch delivers [P][Ny*Nz] per field
         double* dst[5] = {u, v, w, T, rho};
@@ -683,6 +758,7 @@ int dfb_filter_to_host(dfb_handle h, double dt, double* u, double* v, double* w,
 int dfb_filter_to_host_begin(dfb_handle h, double dt, double* u, double* v, double* w, double* T, double* rho) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     return guarded([&] {
+        refuse_attached(*h, "dfb_filter_to_host_begin");
         check_dt(dt);
         if (h->pipe_begun - h->pipe_ended >= 2) throw Error{DFB_ERR_STATE, "two dfb_filter_to_host_begin calls are already outstanding: call dfb_filter_to_host_end first"};
         CUDA_TRY(cudaSetDevice(h->device));
@@ -715,6 +791,7 @@ int dfb_filter_to_host_begin(dfb_handle h, double dt, double* u, double* v, doub
 int dfb_filter_to_host_end(dfb_handle h) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     return guarded([&] {
+        refuse_attached(*h, "dfb_filter_to_host_end");
         if (h->pipe_ended >= h->pipe_begun) throw Error{DFB_ERR_STATE, "no dfb_filter_to_host_begin is outstanding"};
         CUDA_TRY(cudaEventSynchronize(h->ev_copied[(int)(h->pipe_ended & 1)]));
         h->pipe_ended += 1;
@@ -724,6 +801,7 @@ int dfb_filter_to_host_end(dfb_handle h) {
 int dfb_filter_batch(dfb_handle h, int nsteps, const double* dt, double* out) {
     if (!h || !dt || nsteps < 0) return fail(DFB_ERR_ARG, "bad argument");
     return guarded([&] {
+        refuse_attached(*h, "dfb_filter_batch");
         for (int s = 0; s < nsteps; ++s) check_dt(dt[s]);            // the whole array before the first step
         const size_t n = h->D[0].ps_cells * h->nplanes;
         for (int s = 0; s < nsteps; ++s) {
@@ -777,7 +855,59 @@ int dfb_host_unregister(void* ptr) {
 
 int dfb_sync(dfb_handle h) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
-    return guarded([&] { CUDA_TRY(cudaSetDevice(h->device)); CUDA_TRY(cudaStreamSynchronize(h->stream)); });
+    return guarded([&] { CUDA_TRY(cudaSetDevice(h->device)); CUDA_TRY(cudaStreamSynchronize(h->stream)); sync_record(*h); });
+}
+
+int dfb_attach_stream(dfb_handle h, void* stream) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    return guarded([&] {
+        if (!stream) {                                   // detach: the record back to the host, the handle's own stream again
+            if (!h->attached) return;
+            std::string void_msg;
+            try { sync_record(*h); } catch (const Error& e) { if (e.code != DFB_ERR_ARG) throw; void_msg = e.msg; }
+            h->stream = h->own_stream;
+            h->own_stream = nullptr;
+            h->attached = false;
+            if (!void_msg.empty()) throw Error{DFB_ERR_ARG, void_msg};
+            return;
+        }
+        if (h->attached) throw Error{DFB_ERR_STATE, "dfb_attach_stream: the handle is attached already (detach with stream = NULL first)"};
+        if (h->noise_mode != DFB_NOISE_GENERATE) throw Error{DFB_ERR_STATE, "dfb_attach_stream: a handle in inject mode cannot be attached"};
+        if (h->corr_on) throw Error{DFB_ERR_STATE, "dfb_attach_stream: correlation statistics are on (dfb_corr_enable(h, 0, NULL) first)"};
+        if (h->timing) throw Error{DFB_ERR_STATE, "dfb_attach_stream: timing is on (dfb_set_timing(h, 0) first)"};
+        if (h->pipe_begun != h->pipe_ended || h->g_begun != h->g_ended)
+            throw Error{DFB_ERR_STATE, "dfb_attach_stream: a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first"};
+        int dev = -1;
+        CUDA_TRY(cudaStreamGetDevice(static_cast<cudaStream_t>(stream), &dev));
+        if (dev != h->device)
+            throw Error{DFB_ERR_ARG, "dfb_attach_stream: the stream belongs to device " + std::to_string(dev) + ", the handle to device " +
+                                         std::to_string(h->device)};
+        CUDA_TRY(cudaSetDevice(h->device));
+        CUDA_TRY(attach_prepare());
+        if (!h->rec) h->rec = h->dalloc<StepRecord>(1);
+        CUDA_TRY(cudaStreamSynchronize(h->side));        // the look-ahead noise of the next host-driven step is not used
+        AdvanceParams& A = h->adv;
+        A = AdvanceParams{};
+        A.rec = h->rec;
+        for (int f = 0; f < 3; ++f) A.Lt[f] = h->plan.f[f].Lt;
+        A.seed = h->seed;
+        NoiseParams np = h->np;
+        fill_noise_states(np, h->npairs, h->seed, h->plane_id, h->nplanes, 0);
+        std::memcpy(A.pinc, np.pinc, sizeof(A.pinc));
+        for (int n = 0; n < 6; ++n) A.npairs[n] = h->npairs[n];
+        A.n_arrays = h->np.n_arrays;
+        A.P = h->nplanes;
+        push_record(*h);                                 // on the handle's own stream, which it also drains
+        h->own_stream = h->stream;
+        h->stream = static_cast<cudaStream_t>(stream);
+        h->attached = true;
+    });
+}
+
+int dfb_filter_dev(dfb_handle h, const double* dt_dev) {
+    if (!h || !dt_dev) return fail(DFB_ERR_ARG, "handle/dt_dev is NULL");
+    if (!h->attached) return fail(DFB_ERR_STATE, "dfb_filter_dev needs a stream attached with dfb_attach_stream");
+    return guarded([&] { run_step_attached(*h, 0.0, dt_dev, false); });
 }
 
 static int set_noise_impl(dfb_handle h, int field, const double* r_ys, const double* left, const double* right, size_t halo_pitch) {
@@ -829,6 +959,7 @@ int dfb_get_noise(dfb_handle h, int field, double* r_ys, double* r_zs_halo) {
     if (h->plan.k0 != 0 || h->plan.k1 != h->plan.NzG) return fail(DFB_ERR_STATE, "dfb_get_noise is defined on whole-plane handles");
     if (h->plan.periodic && r_zs_halo) return fail(DFB_ERR_ARG, "periodic_z: there is no r_zs halo noise, r_zs_halo must be NULL");
     return guarded([&] {
+        sync_record(*h);
         CUDA_TRY(cudaSetDevice(h->device));
         const FieldDev& F = h->D[h->noise_view].f[field];
         const int W = h->D[0].W, M = F.Nz_max;
@@ -848,6 +979,7 @@ int dfb_get_noise(dfb_handle h, int field, double* r_ys, double* r_zs_halo) {
 int dfb_generate_noise(dfb_handle h, int64_t step) {
     if (!h || step < 0) return fail(DFB_ERR_ARG, "bad argument");
     return guarded([&] {
+        refuse_attached(*h, "dfb_generate_noise");
         CUDA_TRY(cudaSetDevice(h->device));
         const int b = (int)(step & 1);
         CUDA_TRY(cudaStreamWaitEvent(h->stream, h->ev_noise[b], 0));   // order after any prefetch into that set
@@ -859,6 +991,7 @@ int dfb_generate_noise(dfb_handle h, int64_t step) {
 int dfb_get_state(dfb_handle h, double* filt_old3, int64_t* step) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     return guarded([&] {
+        sync_record(*h);
         CUDA_TRY(cudaSetDevice(h->device));
         const size_t n = h->D[0].ps_cells * h->nplanes;                 // [3][P][Ny*Nz]
         if (filt_old3)
@@ -871,11 +1004,16 @@ int dfb_get_state(dfb_handle h, double* filt_old3, int64_t* step) {
 
 int dfb_set_state(dfb_handle h, const double* filt_old3, int64_t step) {
     if (!h || step < 0) return fail(DFB_ERR_ARG, "bad argument");
-    return guarded([&] { restore_state(*h, filt_old3, step); });
+    return guarded([&] {
+        sync_record(*h);
+        restore_state(*h, filt_old3, step);
+        if (h->attached) push_record(*h);
+    });
 }
 
 int dfb_set_timing(dfb_handle h, int on) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    if (on && h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_set_timing(h, 1)"));
     h->timing = on != 0;
     return DFB_OK;
 }
@@ -919,6 +1057,7 @@ int dfb_measure_fp64_peak(int device, double* tflops, double* sm_mhz_est) {
 
 int dfb_stats_enable(dfb_handle h, int on) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_stats_enable") + ": set N2 on or off before attaching");
     return guarded([&] {
         CUDA_TRY(cudaSetDevice(h->device));
         const size_t n = h->D[0].ps_cells * h->nplanes;
@@ -933,6 +1072,7 @@ int dfb_stats_get_plane(dfb_handle h, int plane, int which, int as_rms, double* 
     if (plane < 0 || plane >= h->nplanes) return fail(DFB_ERR_ARG, "plane out of range");
     if (!h->stats) return fail(DFB_ERR_STATE, "statistics are not enabled (dfb_stats_enable)");
     return guarded([&] {
+        sync_record(*h);
         CUDA_TRY(cudaSetDevice(h->device));
         const size_t n = h->D[0].ps_cells;
         if (dst) {
@@ -949,6 +1089,7 @@ int dfb_stats_get(dfb_handle h, int which, int as_rms, double* dst, int64_t* cou
 // ---- correlation statistics (dfb_corr_enable / dfb_corr_get / dfb_corr_integral_scales) ----
 int dfb_corr_enable(dfb_handle h, int on, const int lags[3]) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_corr_enable"));
     if (!on) {                                                // the sums stay readable; the ring and the scratch go
         h->corr_on = false;
         return guarded([&] {
@@ -1165,6 +1306,7 @@ int dfb_save_restart(dfb_handle h, const char* path, int what) {
     if ((what & DFB_RESTART_STATS) && !h->stats) return fail(DFB_ERR_STATE, "DFB_RESTART_STATS: statistics were never enabled (dfb_stats_enable)");
     if ((what & DFB_RESTART_CORR) && !h->corr_ready) return fail(DFB_ERR_STATE, "DFB_RESTART_CORR: correlation statistics were never enabled (dfb_corr_enable)");
     return guarded([&] {
+        sync_record(*h);
         const Plan& P = h->plan;
         const CorrParams& c = h->corr;
         rst::Header hd;
@@ -1208,6 +1350,7 @@ int dfb_load_restart(dfb_handle h, const char* path, int what) {
     int rc = check_restart_call(h, path, what);
     if (rc != DFB_OK) return rc;
     return guarded([&] {
+        sync_record(*h);
         // ---- everything is checked and read before the device is touched: a refused load leaves the handle as it was ----
         std::vector<rst::Record> recs;
         const rst::Header hd = rst::read_header(path, &recs);
@@ -1254,6 +1397,7 @@ int dfb_load_restart(dfb_handle h, const char* path, int what) {
             if (!hd.corr_on && dfb_corr_enable(h, 0, nullptr) != DFB_OK) throw Error{DFB_ERR_CUDA, g_last_error};
         }
         CUDA_TRY(cudaStreamSynchronize(h->stream));
+        if (h->attached) push_record(*h);
     });
 }
 
@@ -1318,6 +1462,7 @@ int dfb_write_tecplot(dfb_handle h, const char* path) {
 // get_rms (df.cpp:584-611): reset the sums, `nsteps` steps with accumulation (on the device, in the z-sweep's epilogue)
 int dfb_get_rms(dfb_handle h, int nsteps, double dt) {
     if (!h || nsteps < 0) return fail(DFB_ERR_ARG, "bad argument");
+    if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_get_rms"));
     int rc = guarded([&] { check_dt(dt); });         // before dfb_stats_enable zeroes the sums
     if (rc != DFB_OK) return rc;
     rc = dfb_stats_enable(h, 1);
@@ -1334,6 +1479,7 @@ int dfb_write_rms_csv(dfb_handle h, const char* path) {
     if (!h || !path) return fail(DFB_ERR_ARG, "bad argument");
     if (!h->stats) return fail(DFB_ERR_STATE, "statistics are not enabled (dfb_stats_enable / dfb_get_rms)");
     return guarded([&] {
+        sync_record(*h);
         CUDA_TRY(cudaSetDevice(h->device));
         const int Ny = h->D[0].Ny, W = h->D[0].W, k0 = h->plan.k0;
         const size_t n = (size_t)Ny * W;
@@ -1490,6 +1636,7 @@ int dfb_interp_to_host(dfb_handle h, int map_id, int plane, int fields, double* 
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     return guarded([&] {
         check_idle(*h);
+        sync_record(*h);
         FaceMapDev& F = facemap_of(*h, map_id);
         InterpArgs a = interp_args(*h, F, plane, fields);
         if (F.n > 0 && !out) throw Error{DFB_ERR_ARG, "out is NULL"};
@@ -1660,6 +1807,7 @@ int dfb_comm_unique_id(void* id128) {
 int dfb_comm_init(dfb_handle h, const void* id128, int rank, int world) {
     if (!h || !id128 || world < 1 || rank < 0 || rank >= world) return fail(DFB_ERR_ARG, "bad argument");
     if (h->comm) return fail(DFB_ERR_STATE, "dfb_comm_init was already called on this handle");
+    if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_comm_init"));
     if (h->nplanes != 1) return fail(DFB_ERR_STATE, "slab communication is defined for single-plane handles");
     return guarded([&] {
         CUDA_TRY(cudaSetDevice(h->device));
@@ -1767,6 +1915,7 @@ int dfb_gather_begin(dfb_handle h, int dst_rank) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     if (!h->comm) return fail(DFB_ERR_STATE, "dfb_comm_init has not been called");
     if (dst_rank < 0 || dst_rank >= h->comm_world) return fail(DFB_ERR_ARG, "dst_rank out of range");
+    if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_gather_begin"));
     if (h->g_begun != h->g_ended) return fail(DFB_ERR_STATE, "a gather is already outstanding: call dfb_gather_end first");
     return guarded([&] {
         CUDA_TRY(cudaSetDevice(h->device));
@@ -1830,6 +1979,7 @@ int dfb_gather_end(dfb_handle h) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     if (!h->comm) return fail(DFB_ERR_STATE, "dfb_comm_init has not been called");
     if (h->g_begun == h->g_ended) return fail(DFB_ERR_STATE, "no dfb_gather_begin is outstanding");
+    if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_gather_end"));
     return guarded([&] {
         CUDA_TRY(cudaSetDevice(h->device));
         // bounded wait: a rank that died would otherwise leave this one blocked for ever on a flag that never comes
@@ -1944,6 +2094,12 @@ int dfb_interp_to_cells_f(const dfb_handle* h, const int* map_id, const int* pla
                           const double* const mean[5], const double scale[5], double* const dst[5], const int* stride) {
     return (h && map_id && plane && fields && stride) ? dfb_interp_to_cells(*h, *map_id, *plane, *fields, dst_index, mean, scale, dst, *stride)
                                                       : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_attach_stream_f(const dfb_handle* h, void* const* stream) {
+    return (h && stream) ? dfb_attach_stream(*h, *stream) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_filter_dev_f(const dfb_handle* h, const double* const* dt_dev) {
+    return (h && dt_dev) ? dfb_filter_dev(*h, *dt_dev) : fail(DFB_ERR_ARG, "NULL argument");
 }
 int dfb_destroy_f(dfb_handle* h) {
     if (!h) return DFB_OK;

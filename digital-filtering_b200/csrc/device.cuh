@@ -14,6 +14,7 @@
 //   coefficients: one row per distinct half-width N (CSR keyed by N), plus per-row-group dense band
 //   matrices for the tuned y-sweep; per-row epilogue constants.
 #pragma once
+#include <cmath>
 #include <cstdint>
 #include <cuda_runtime.h>
 #include <cuda.h>
@@ -124,9 +125,44 @@ struct YRSmemCtl {                       // control block in front of the two wi
 // dynamic shared memory of ysweep_run_kernel for `nbuf` window buffers of `wrows` rows
 inline size_t ysweep_run_smem(int wrows, int nbuf) { return (sizeof(YRSmemCtl) + 127) / 128 * 128 + (size_t)nbuf * wrows * YR_C * sizeof(double); }
 
+// Blend constants of one field (df.cpp:411-415): sa = sqrt(alpha), sb = sqrt(1 - alpha), alpha = exp(-pi dt / Lt).  The host evaluates
+// them with its libm's exp (dfb_filter), step_advance_kernel with CUDA's (dfb_filter_dev); both are within one ulp of the exact value,
+// so the two agree to rounding.  Multiply, divide and sqrt are correctly rounded on both sides.
+__host__ __device__ inline void blend_consts(double dt, double Lt, double& sa, double& sb) {
+    const double pi = 3.141592654;                             // df.cpp:411 (SURVEY quirk 2)
+    const double alpha = exp(-pi * dt / Lt);                   // df.cpp:412
+    sa = sqrt(alpha);                                          // df.cpp:415
+    sb = sqrt(1.0 - alpha);
+}
+
 struct StepConsts {
     double sa[3], sb[3];       // sqrt(alpha), sqrt(1-alpha) per field (df.cpp:412-415), from the host's exp/sqrt
     int first_step;            // constructor semantics (df.cpp:57-62): no blend, T'/rho' untouched
+};
+
+// Step record of a handle attached to a caller's stream (dfb_attach_stream): what the host holds for a host-driven step, in device
+// memory, so that a step needs no host decision and replays of a captured graph advance the generator.  Written by step_advance_kernel,
+// the first launch of every attached step; read by the step's noise and z-sweep launches through their `rec` pointer.
+struct StepRecord {
+    long long step;            // steps completed (the host's dfb_filter_s::step)
+    long long stats_count;     // N2: accumulated steps
+    double dt;                 // dt of the current step
+    double sa[3], sb[3];       // blend constants of the current step
+    uint64_t pstate[DFB_MAXP][6];   // per plane and noise array: pcg32 state at the first draw of the current step (NoiseParams::pstate)
+    int void_step;             // the current step is void (dt not finite or < 0): the z-sweep writes nothing
+    int void_seen;             // sticky: a step was void since the host last read the record
+};
+
+struct AdvanceParams {
+    StepRecord* rec;
+    const double* dt_dev;      // dfb_filter_dev: dt in device memory; nullptr: dt, sa, sb below come from the host
+    double dt, sa[3], sb[3];
+    double Lt[3];              // time scales of u, v, w (df.cpp:412)
+    uint64_t seed;
+    uint64_t pinc[DFB_MAXP][6];     // stream increments, as NoiseParams::pinc
+    uint64_t npairs[6];        // pairs one step draws from each array's stream
+    int n_arrays, P;
+    int stats;                 // this step accumulates N2: count it
 };
 
 // ---- noise generation work description (one segment = one row of one logical array, or one contiguous piece of a row) ----
@@ -152,6 +188,7 @@ struct NoiseParams {
     int max_np;                 // largest segment (pairs)
     int chunks;                 // ceil(max_np / 128)
     unsigned long long* tl;     // development aid (DFB_TIMELINE): [start, end] globaltimer stamps of this launch, or nullptr
+    const StepRecord* rec;      // attached step: the states come from rec->pstate instead of pstate; nullptr host-driven
 };
 
 // per array of NoiseParams: r_ys of a periodic plane whose extended rows wrap (periodic_z) -- {padded row, first, end extended column}
@@ -219,6 +256,7 @@ struct ZParams {
     int zmode;                   // 0: direct Toeplitz tap loop; 1: recursive evaluation of the exponential window
     int debug;                   // development probes only (0 in production)
     unsigned long long* prof;    // [8] cycle counters filled when debug & 16
+    const StepRecord* rec;       // attached step: sa, sb come from the record, and a void step writes nothing; nullptr host-driven
 };
 
 }  // namespace dfb

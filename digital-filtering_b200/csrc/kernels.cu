@@ -48,8 +48,9 @@ __device__ __forceinline__ void tl_stamp(unsigned long long* tl, int end) {
 // of 4*NOISE_THREADS draws -- one 64-bit multiply-add, like a plain LCG step -- instead of two table jumps per pair.
 // PIECES: the segments of r_ys arrays may be pieces of rows (NoiseWindows; periodic_z, extended rows that wrap around the plane);
 // without, a segment is a whole padded row -- a kernel of its own, so that every other handle keeps the leaner one (48 registers
-// against 50: the noise CTAs run beside the sweeps).
-template <bool PIECES>
+// against 50: the noise CTAs run beside the sweeps).  REC: an attached step (dfb_attach_stream) reads the states from the step record;
+// host-driven steps keep the kernel that takes them as parameters.
+template <bool PIECES, bool REC>
 __device__ __forceinline__ void noise_thread(const NoiseParams& P, const PlaneDev& D, const NoiseWindows* Wn, int slot0, int seg, int bz,
                                              int pl) {
     const NoiseArray& A = P.a[bz];
@@ -63,7 +64,7 @@ __device__ __forceinline__ void noise_thread(const NoiseParams& P, const PlaneDe
     int4 win = make_int4(seg, 0, 0, 0);                          // PIECES: {padded row, first, end extended column} of the segment
     if constexpr (PIECES) { if (Wn->seg_win[bz]) win = Wn->seg_win[bz][seg]; else win.z = D.f[A.field].We; }
     if (slot0 >= np) return;
-    uint64_t s = sj.A * P.pstate[pl][bz] + inc * sj.C;
+    uint64_t s = sj.A * (REC ? P.rec->pstate[pl][bz] : P.pstate[pl][bz]) + inc * sj.C;
     s = tj.A * s + inc * tj.C;
     const uint64_t strideA = P.stride.A, strideC = inc * P.stride.C;
     const FieldDev& F = D.f[A.field];
@@ -113,15 +114,17 @@ __device__ __forceinline__ void noise_thread(const NoiseParams& P, const PlaneDe
 }
 
 // one CTA per (NOISE_THREADS x NOISE_PAIRS pairs, segment, array x plane of the batch)
+template <bool REC>
 __global__ void __launch_bounds__(NOISE_THREADS) noise_kernel(const NoiseParams P, const PlaneDev D) {
     if (threadIdx.x == 0 && (blockIdx.y & 31) == 0) tl_stamp(P.tl, 0);     // sampled: one row in 32 (same-address atomics)
-    noise_thread<false>(P, D, nullptr, (int)blockIdx.x * NOISE_PAIRS * NOISE_THREADS + (int)threadIdx.x, blockIdx.y, (int)(blockIdx.z % P.n_arrays), (int)(blockIdx.z / P.n_arrays));
+    noise_thread<false, REC>(P, D, nullptr, (int)blockIdx.x * NOISE_PAIRS * NOISE_THREADS + (int)threadIdx.x, blockIdx.y, (int)(blockIdx.z % P.n_arrays), (int)(blockIdx.z / P.n_arrays));
     if (threadIdx.x == 0 && (blockIdx.y & 31) == 0) tl_stamp(P.tl, 1);
 }
 // the same for a periodic plane whose extended rows wrap: a segment is one piece of a row (NoiseWindows)
+template <bool REC>
 __global__ void __launch_bounds__(NOISE_THREADS) noise_pieces_kernel(const NoiseParams P, const PlaneDev D, const NoiseWindows Wn) {
     if (threadIdx.x == 0 && (blockIdx.y & 31) == 0) tl_stamp(P.tl, 0);
-    noise_thread<true>(P, D, &Wn, (int)blockIdx.x * NOISE_PAIRS * NOISE_THREADS + (int)threadIdx.x, blockIdx.y, (int)(blockIdx.z % P.n_arrays), (int)(blockIdx.z / P.n_arrays));
+    noise_thread<true, REC>(P, D, &Wn, (int)blockIdx.x * NOISE_PAIRS * NOISE_THREADS + (int)threadIdx.x, blockIdx.y, (int)(blockIdx.z % P.n_arrays), (int)(blockIdx.z / P.n_arrays));
     if (threadIdx.x == 0 && (blockIdx.y & 31) == 0) tl_stamp(P.tl, 1);
 }
 
@@ -163,10 +166,14 @@ __device__ __forceinline__ void epilogue_cell(const double* __restrict__ rc, con
     o.rho = -t2 * rc[6];                                  // df.cpp:481
 }
 
-__global__ void __launch_bounds__(256) zsweep_epilogue_simple_kernel(const PlaneDev D, const StepConsts S) {
+__global__ void __launch_bounds__(256) zsweep_epilogue_simple_kernel(const PlaneDev D, StepConsts S, const StepRecord* rec) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     const int j = blockIdx.y, pl = blockIdx.z;
     if (k >= D.W) return;
+    if (rec) {                                            // attached step (dfb_attach_stream): a void step writes nothing
+        if (rec->void_step) return;
+        for (int f = 0; f < 3; ++f) { S.sa[f] = rec->sa[f]; S.sb[f] = rec->sb[f]; }
+    }
     double z[3];
 #pragma unroll
     for (int f = 0; f < 3; ++f) {
@@ -857,7 +864,9 @@ __device__ __forceinline__ void z_issue_unit(const ZParams& P, const ZMaps& maps
     if (fo) tma_load_1d(b + P.fo_off, P.D.f[f].filt_old + (size_t)plane * P.D.ps_cells + (size_t)j * P.D.W + c0, strip_bytes, bar);
 }
 
-template <int ZK, int MODE, bool STATS>
+// REC: an attached step (dfb_attach_stream) reads sa, sb from the step record and writes nothing when the step is void; host-driven
+// steps keep the kernel that takes them as parameters
+template <int ZK, int MODE, bool STATS, bool REC>
 __global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_kernel(const __grid_constant__ ZMaps maps, const ZParams P) {
     constexpr int LB = ZK * 8;               // bytes per staged line (= one lane's ZK samples): 128 -> SWIZZLE_128B, 64 -> SWIZZLE_64B
     constexpr int PPL = ZK / 2;              // 16-byte pieces per line
@@ -881,6 +890,9 @@ __global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_ker
     // Programmatic dependent launch: this CTA became resident while the y-sweep's last tiles were still running;
     // wait for that grid to complete (and its writes to r_zs to be visible) before the first item is claimed/staged.
     asm volatile("griddepcontrol.wait;" ::: "memory");
+    // attached step (dfb_attach_stream): a void step ends here.  The y-sweep before it has already reset the work counter, and this is
+    // the only kernel of the step that writes state which outlives it, so the handle is left as the previous step left it.
+    if (REC && P.rec->void_step) return;
 
     if (lane == 0) tl_stamp(P.tl, 0);
     const long long tstart = (P.debug & 16) ? clock64() : 0;
@@ -1123,7 +1135,7 @@ __global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_ker
             const double* rc = reinterpret_cast<const double*>(cbuf + P.rc_off);        // the row's constants, staged with the window
             const double rc_own = rc[f == 0 ? 0 : (f == 1 ? 2 : 3)];
             const double rc0 = rc[0], rc1 = rc[1], rc4 = rc[4], rc5 = rc[5], rc6 = rc[6];
-            const double sa = P.S.sa[f], sb = P.S.sb[f];
+            const double sa = REC ? P.rec->sa[f] : P.S.sa[f], sb = REC ? P.rec->sb[f] : P.S.sb[f];
             double* stats = (STATS && blend) ? P.stats + (size_t)plA * 6 * D.ps_cells + ((size_t)j * D.W) : nullptr;
             if (coalesced) {
                 // One transpose per unit: lane l owns line l (its ZK cells) of a 32-line tile; global memory wants 16-byte piece
@@ -1266,12 +1278,49 @@ __global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_ker
 }
 
 // =================================================================================================
+// attached steps (dfb_attach_stream): the step's host decisions, made on the device
+// =================================================================================================
+// One CTA, the first launch of every attached step.  Reads dt (device memory, or the host's immediate with the host's blend
+// constants), validates it, computes the blend constants and the pcg32 positions of the record's step with the host's own functions
+// (blend_consts, noise_step_state), and advances the step counter and the N2 count -- only when the step is not void.  A void step
+// leaves the positions as they were, so its noise launch rewrites the previous step's noise unchanged.
+__global__ void __launch_bounds__(128) step_advance_kernel(const AdvanceParams A) {
+    __shared__ int ok;
+    StepRecord* R = A.rec;
+    const long long step = R->step;
+    if (threadIdx.x == 0) {
+        const double dt = A.dt_dev ? *A.dt_dev : A.dt;
+        ok = isfinite(dt) && dt >= 0.0;
+        R->void_step = ok ? 0 : 1;
+        if (ok) {
+            R->dt = dt;
+            for (int f = 0; f < 3; ++f) {
+                if (A.dt_dev) blend_consts(dt, A.Lt[f], R->sa[f], R->sb[f]);
+                else { R->sa[f] = A.sa[f]; R->sb[f] = A.sb[f]; }
+            }
+        } else {
+            R->void_seen = 1;
+        }
+    }
+    __syncthreads();
+    if (!ok) return;
+    for (int i = threadIdx.x; i < A.P * A.n_arrays; i += blockDim.x) {
+        const int p = i / A.n_arrays, n = i % A.n_arrays;
+        R->pstate[p][n] = noise_step_state(A.seed, A.pinc[p][n], step, A.npairs[n]);
+    }
+    if (threadIdx.x == 0) {
+        R->step = step + 1;
+        if (A.stats) R->stats_count += 1;
+    }
+}
+
+// =================================================================================================
 // N2: running sums of squares (rms_add, df.cpp:571-582) + u'v', opt-in.  mul then add, like the reference.
 // Separate kernel for the general (one-thread-per-cell) path only; the tuned z-sweep accumulates in its epilogue.
 // =================================================================================================
-__global__ void __launch_bounds__(256) stats_kernel(const PlaneDev D, double* __restrict__ sums, size_t n) {
+__global__ void __launch_bounds__(256) stats_kernel(const PlaneDev D, double* __restrict__ sums, size_t n, const StepRecord* rec) {
     const size_t c = (size_t)blockIdx.x * blockDim.x + threadIdx.x;       // cell within the plane
-    if (c >= n) return;
+    if (c >= n || (rec && rec->void_step)) return;
     const size_t i = (size_t)blockIdx.y * n + c;                          // cell within the batch's dense arrays
     double* s = sums + (size_t)blockIdx.y * 6 * n + c;                    // [P][6][n]
     const double u = D.f[0].fluc[i], v = D.f[1].fluc[i], w = D.f[2].fluc[i], T = D.T_fluc[i], r = D.rho_fluc[i];
@@ -1399,9 +1448,9 @@ cudaError_t launch_interp(const InterpArgs& a, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-cudaError_t launch_stats(const PlaneDev& D, double* sums, cudaStream_t st) {
+cudaError_t launch_stats(const PlaneDev& D, double* sums, const StepRecord* rec, cudaStream_t st) {
     const size_t n = (size_t)D.Ny * D.W;
-    stats_kernel<<<dim3((unsigned)((n + 255) / 256), (unsigned)D.P), 256, 0, st>>>(D, sums, n);
+    stats_kernel<<<dim3((unsigned)((n + 255) / 256), (unsigned)D.P), 256, 0, st>>>(D, sums, n, rec);
     return cudaGetLastError();
 }
 
@@ -1432,8 +1481,13 @@ cudaError_t launch_noise(const NoiseParams& P, const NoiseWindows& Wn, const Pla
     bool pieces = false;
     for (int a = 0; a < P.n_arrays; ++a) pieces = pieces || Wn.seg_win[a] != nullptr;
     dim3 grid((unsigned)P.chunks, (unsigned)max_seg, (unsigned)(P.n_arrays * D.P));
-    if (pieces) noise_pieces_kernel<<<grid, NOISE_THREADS, 0, st>>>(P, D, Wn);
-    else noise_kernel<<<grid, NOISE_THREADS, 0, st>>>(P, D);
+    if (P.rec) {
+        if (pieces) noise_pieces_kernel<true><<<grid, NOISE_THREADS, 0, st>>>(P, D, Wn);
+        else noise_kernel<true><<<grid, NOISE_THREADS, 0, st>>>(P, D);
+    } else {
+        if (pieces) noise_pieces_kernel<false><<<grid, NOISE_THREADS, 0, st>>>(P, D, Wn);
+        else noise_kernel<false><<<grid, NOISE_THREADS, 0, st>>>(P, D);
+    }
     return cudaGetLastError();
 }
 
@@ -1445,9 +1499,9 @@ cudaError_t launch_ysweep_simple(const PlaneDev& D, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, cudaStream_t st) {
+cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, const StepRecord* rec, cudaStream_t st) {
     dim3 grid((unsigned)((D.W + 255) / 256), (unsigned)D.Ny, (unsigned)D.P);
-    zsweep_epilogue_simple_kernel<<<grid, 256, 0, st>>>(D, S);
+    zsweep_epilogue_simple_kernel<<<grid, 256, 0, st>>>(D, S, rec);
     return cudaGetLastError();
 }
 
@@ -1456,7 +1510,8 @@ cudaError_t ysweep_prepare() {
     // noise CTA running with the default split beside the sweeps could leave an SM unable to take its third y-sweep CTA (observed
     // as a process-wide bimodal y-sweep time on small planes: 26 or 43 us on the reference default plane).  {kernel, dynamic smem}
     const std::pair<const void*, int> fns[] = {
-        {(const void*)noise_kernel, 0}, {(const void*)noise_pieces_kernel, 0}, {(const void*)stats_kernel, 0}, {(const void*)scatter_kernel, 0},
+        {(const void*)noise_kernel<false>, 0}, {(const void*)noise_pieces_kernel<false>, 0}, {(const void*)noise_kernel<true>, 0},
+        {(const void*)noise_pieces_kernel<true>, 0}, {(const void*)stats_kernel, 0}, {(const void*)scatter_kernel, 0},
         {(const void*)interp_kernel<false>, 0}, {(const void*)interp_kernel<true>, 0},
         {(const void*)ysweep_tma_kernel<Y_RC, Y_NS, 128>, (int)sizeof(YSmem<Y_RC, Y_NS, 128>)},
         {(const void*)ysweep_tma_kernel<Y_RC, Y_NS, 64>, (int)sizeof(YSmem<Y_RC, Y_NS, 64>)},
@@ -1517,18 +1572,22 @@ cudaError_t launch_ysweep_run(const YRMaps& maps, const YParams& P, cudaStream_t
     return cudaLaunchKernelEx(&cfg, ysweep_run_kernel, maps, P);
 }
 
-static const void* zsweep_fn(int zk, int mode, bool stats) {
+template <bool REC>
+static const void* zsweep_fn_rec(int zk, int mode, bool stats) {
     if (stats) {
-        if (zk == 16) return mode == 1 ? (const void*)zsweep_epilogue_kernel<16, 1, true> : (const void*)zsweep_epilogue_kernel<16, 0, true>;
-        return mode == 1 ? (const void*)zsweep_epilogue_kernel<8, 1, true> : (const void*)zsweep_epilogue_kernel<8, 0, true>;
+        if (zk == 16) return mode == 1 ? (const void*)zsweep_epilogue_kernel<16, 1, true, REC> : (const void*)zsweep_epilogue_kernel<16, 0, true, REC>;
+        return mode == 1 ? (const void*)zsweep_epilogue_kernel<8, 1, true, REC> : (const void*)zsweep_epilogue_kernel<8, 0, true, REC>;
     }
-    if (zk == 16) return mode == 1 ? (const void*)zsweep_epilogue_kernel<16, 1, false> : (const void*)zsweep_epilogue_kernel<16, 0, false>;
-    return mode == 1 ? (const void*)zsweep_epilogue_kernel<8, 1, false> : (const void*)zsweep_epilogue_kernel<8, 0, false>;
+    if (zk == 16) return mode == 1 ? (const void*)zsweep_epilogue_kernel<16, 1, false, REC> : (const void*)zsweep_epilogue_kernel<16, 0, false, REC>;
+    return mode == 1 ? (const void*)zsweep_epilogue_kernel<8, 1, false, REC> : (const void*)zsweep_epilogue_kernel<8, 0, false, REC>;
+}
+static const void* zsweep_fn(int zk, int mode, bool stats, bool rec = false) {
+    return rec ? zsweep_fn_rec<true>(zk, mode, stats) : zsweep_fn_rec<false>(zk, mode, stats);
 }
 
 cudaError_t zsweep_prepare(int zk, int mode, size_t smem, int* blocks_per_sm) {
-    for (int st = 1; st >= 0; --st) {
-        const void* fn = zsweep_fn(zk, mode, st != 0);
+    for (int v = 3; v >= 0; --v) {                      // bit 0: N2 accumulation, bit 1: attached step
+        const void* fn = zsweep_fn(zk, mode, (v & 1) != 0, (v & 2) != 0);
         cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -1543,7 +1602,24 @@ cudaError_t launch_zsweep_tuned(const ZMaps& maps, const ZParams& P, cudaStream_
     static const int pdl = std::getenv("DFB_Z_PDL") ? std::atoi(std::getenv("DFB_Z_PDL")) : 1;
     if (!pdl) cfg.numAttrs = 0;
     void* args[2] = {const_cast<ZMaps*>(&maps), const_cast<ZParams*>(&P)};
-    return cudaLaunchKernelExC(&cfg, zsweep_fn(P.zk, P.zmode, P.stats != nullptr), args);
+    return cudaLaunchKernelExC(&cfg, zsweep_fn(P.zk, P.zmode, P.stats != nullptr, P.rec != nullptr), args);
+}
+
+cudaError_t launch_advance(const AdvanceParams& A, cudaStream_t st) {
+    step_advance_kernel<<<1, 128, 0, st>>>(A);
+    return cudaGetLastError();
+}
+
+cudaError_t attach_prepare() {
+    // load the kernels an attached step may launch for the first time now, not while the caller's stream is being captured
+    const void* fns[] = {(const void*)step_advance_kernel, (const void*)ysweep_simple_kernel, (const void*)zsweep_epilogue_simple_kernel,
+                         (const void*)stats_kernel, (const void*)noise_kernel<true>, (const void*)noise_pieces_kernel<true>};
+    for (const void* fn : fns) {
+        cudaFuncAttributes a;
+        const cudaError_t e = cudaFuncGetAttributes(&a, fn);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
 }
 
 cudaError_t launch_dfma_peak(double* out, int blocks, int iters, cudaStream_t st) {

@@ -6,7 +6,10 @@ namespace dfb {
 
 cudaError_t launch_noise(const NoiseParams& P, const NoiseWindows& Wn, const PlaneDev& D, cudaStream_t st);
 cudaError_t launch_ysweep_simple(const PlaneDev& D, cudaStream_t st);
-cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, cudaStream_t st);
+cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, const StepRecord* rec, cudaStream_t st);
+// attached steps (dfb_attach_stream): the step's first launch, and loading every kernel such a step may launch
+cudaError_t launch_advance(const AdvanceParams& A, cudaStream_t st);
+cudaError_t attach_prepare();
 cudaError_t ysweep_prepare();
 // dense band-matrix tiles [0, n_dense) with ysweep_tma_kernel, then recursive tiles [n_dense, n_dense + n_rec) with ysweep_rec_kernel
 cudaError_t launch_ysweep_tma(const YMaps& maps, const YParams& P, int n_dense, int n_rec, cudaStream_t st);
@@ -15,7 +18,7 @@ cudaError_t ysweep_run_prepare(size_t smem);
 cudaError_t launch_ysweep_run(const YRMaps& maps, const YParams& P, cudaStream_t st);
 cudaError_t zsweep_prepare(int zk, int mode, size_t smem, int* blocks_per_sm);
 cudaError_t launch_zsweep_tuned(const ZMaps& maps, const ZParams& P, cudaStream_t st);
-cudaError_t launch_stats(const PlaneDev& D, double* sums, cudaStream_t st);
+cudaError_t launch_stats(const PlaneDev& D, double* sums, const StepRecord* rec, cudaStream_t st);
 cudaError_t launch_scatter(const double* field, int n, const int* plane_index, const int* dst_index, const double* mean, double scale,
                            double* dst, cudaStream_t st);
 // face maps (facemap.hpp): dst[f][dst_index[i] * stride] = base + scale[f] * sum_t w_t * field[f][idx_t] for the served faces i < n and

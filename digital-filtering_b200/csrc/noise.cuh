@@ -25,7 +25,7 @@ __host__ __device__ inline uint32_t pcg_xsh_rr(uint64_t s) {
 }
 
 // Brown's arbitrary-stride jump (pcg_random.hpp:640-669) as a composable affine map
-inline Jump pcg_jump(uint64_t delta, uint64_t inc) {
+__host__ __device__ inline Jump pcg_jump(uint64_t delta, uint64_t inc) {
     uint64_t acc_mult = 1u, acc_plus = 0u, cur_mult = DFB_PCG32_MULT, cur_plus = inc;
     while (delta > 0) {
         if (delta & 1u) { acc_mult *= cur_mult; acc_plus = acc_plus * cur_mult + cur_plus; }
@@ -34,6 +34,20 @@ inline Jump pcg_jump(uint64_t delta, uint64_t inc) {
         delta >>= 1;
     }
     return Jump{acc_mult, acc_plus};
+}
+
+// increment of stream ((plane*3 + field)*2 + kind) of include/dfb_rng_spec.h, kind 0 = r_ys, 1 = r_zs halo
+__host__ __device__ inline uint64_t noise_inc(int64_t plane, int field, int kind) {
+    const uint64_t stream = (uint64_t)((plane * 3 + field) * 2 + kind);
+    return (stream << 1) | 1u;
+}
+
+// pcg32 state at the first draw of step `step` of an array that draws `npairs` pairs per step: the host (fill_noise_states) and the
+// step's advance kernel (dfb_attach_stream) both position the noise through this one function
+__host__ __device__ inline uint64_t noise_step_state(uint64_t seed, uint64_t inc, int64_t step, uint64_t npairs) {
+    const uint64_t state0 = pcg_lcg(seed + inc, inc);
+    const Jump j = pcg_jump(4u * ((uint64_t)step * npairs), inc);
+    return j.A * state0 + j.C;
 }
 
 #ifdef __CUDACC__

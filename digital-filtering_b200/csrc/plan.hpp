@@ -87,6 +87,10 @@ struct StepPlan {
 // No CUDA call, no environment; throws dfb::Error.
 StepPlan plan_step(const Plan& plan, int nplanes, const DeviceLimits& dev, const Overrides& ovr);
 
+// np.pstate / np.pinc of every array np draws and every plane of the handle: pcg32 state at the first draw of step `step` (plane p of a
+// batch draws from stream group plane_id + p).  The advance kernel of attached steps computes the same states with noise_step_state.
+void fill_noise_states(NoiseParams& np, const uint64_t* npairs, uint64_t seed, int plane_id, int nplanes, int64_t step);
+
 // pieces, exposed for unit tests through the C ABI
 void coefficients(int N, double* b /* 2N+1 */);
 std::vector<double> linear_interpolate(const std::vector<double>& y_data, const std::vector<double>& f_data,

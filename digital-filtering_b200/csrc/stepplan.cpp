@@ -608,4 +608,13 @@ StepPlan plan_step(const Plan& P, int NP, const DeviceLimits& dev, const Overrid
     return S;
 }
 
+void fill_noise_states(NoiseParams& np, const uint64_t* npairs, uint64_t seed, int plane_id, int nplanes, int64_t step) {
+    for (int n = 0; n < np.n_arrays; ++n)
+        for (int p = 0; p < nplanes; ++p) {
+            const uint64_t inc = noise_inc((int64_t)plane_id + p, np.a[n].field, np.a[n].kind);
+            np.pstate[p][n] = noise_step_state(seed, inc, step, npairs[n]);
+            np.pinc[p][n] = inc;
+        }
+}
+
 }  // namespace dfb

@@ -21,6 +21,8 @@
 !   save_restart, load_restart                    restart files: resume a run across jobs, bit for bit, whatever the slab layout
 !   facemap_create, interp_to_host,               the outputs interpolated onto the CFD code's own faces (bilinear or area-weighted),
 !   interp_to_cells, filter_on_device               all five fields in one pass on the device; only the faces cross PCIe
+!   attach_stream, filter_dev                     GPU-resident CFD codes: steps on the code's own CUDA stream with dt in device memory,
+!                                                 capturable into its CUDA graph (include/dfb200.h, dfb_attach_stream)
 !
 ! NOTE: NEVER COMPILED -- no Fortran compiler exists in the build image or on the GPU boxes.  The binding is exercised through
 ! tests/fortran_abi_mimic.c, a C program that makes exactly these calls with exactly this struct layout and by-reference
@@ -35,6 +37,7 @@ module DIGITAL_FILTERING
     public :: corr_enable, corr_get, integral_scales
     public :: save_restart, load_restart, RESTART_STATE, RESTART_STATS, RESTART_CORR
     public :: facemap_create, interp_to_host, interp_to_cells, facemap_destroy, MAP_POINT, MAP_AREA, MAP_WALL_ZERO, filter_on_device
+    public :: attach_stream, filter_dev
 
     integer, parameter :: RESTART_STATE = 1, RESTART_STATS = 2, RESTART_CORR = 4   ! DFB_RESTART_* (what to save / load; added together)
 
@@ -245,6 +248,14 @@ module DIGITAL_FILTERING
             type(c_ptr), intent(in) :: mean(5), dst(5)
             real(c_double), intent(in) :: scale(5)
         end function
+        integer(c_int) function dfb_attach_stream_f(handle, stream) bind(C, name='dfb_attach_stream_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle, stream
+        end function
+        integer(c_int) function dfb_filter_dev_f(handle, dt_dev) bind(C, name='dfb_filter_dev_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle, dt_dev
+        end function
         function dfb_last_error() bind(C, name='dfb_last_error') result(msg)
             import :: c_ptr
             type(c_ptr) :: msg
@@ -412,6 +423,21 @@ contains
         dt = dt_input
         call check(dfb_filter_f(DF%handle, dt), 'filter_on_device')
     end subroutine filter_on_device
+
+    ! every later step, interp_to_cells and copy of DF goes on `stream` (a cudaStream_t, e.g. from CUDA Fortran or the CFD code's own
+    ! C layer; c_null_ptr detaches), with the step's state in device memory, so that filter_dev can be captured into a CUDA graph
+    subroutine attach_stream(DF, stream)
+        type(digital_filter_type), intent(in) :: DF
+        type(c_ptr), intent(in) :: stream
+        call check(dfb_attach_stream_f(DF%handle, stream), 'attach_stream')
+    end subroutine attach_stream
+
+    ! one step with dt read from device memory (dt_dev: the device address of one real(c_double)) when it runs; DF must be attached
+    subroutine filter_dev(DF, dt_dev)
+        type(digital_filter_type), intent(in) :: DF
+        type(c_ptr), intent(in) :: dt_dev
+        call check(dfb_filter_dev_f(DF%handle, dt_dev), 'filter_dev')
+    end subroutine filter_dev
 
     subroutine facemap_create(DF, n, yf, zf, map_id, hy, hz, own_begin, own_end, wall_zero, served)
         ! bilinear at the face centres, or with hy, hz the average over each face; own_begin/own_end: 0-based columns [own_begin,

@@ -176,6 +176,35 @@ int dfb_stream(dfb_handle h, void** stream);
 int dfb_scatter_to_cells(dfb_handle h, int which, int n, const int* plane_index, const int* dst_index,
                          const double* mean, double scale, double* dst);
 int dfb_sync(dfb_handle h);
+
+/* GPU-resident CFD codes: run the steps on the caller's stream, with dt in device memory, capturable into a CUDA graph.
+ * dfb_attach_stream(h, stream): from now on every call of this handle that enqueues device work goes on `stream` (a cudaStream_t of
+ * the handle's device): steps, dfb_interp_to_cells, dfb_scatter_to_cells, and the copies of dfb_get_field / dfb_filter_to_host
+ * (dfb_stream returns it).  The step's host state moves into device memory: step counter, pcg32 positions, blend constants, N2 count.
+ * A step then needs no host decision: it is advance -> noise -> y-sweep -> z-sweep on `stream` alone, with no second stream, event,
+ * synchronisation or allocation, so it can be captured with cudaStreamBeginCapture (cudaStreamCaptureModeGlobal included), and each
+ * replay of the graph advances the generator by one step.  stream == NULL detaches: synchronises the attached stream, copies the device
+ * step state back and continues host-driven.  An attached step does not overlap the next step's noise with this step's sweeps.
+ * dfb_filter(h, dt) with a host dt still works while attached: the same device-driven step, with the blend constants computed on the
+ * host as always, so a host-dt step is bit for bit the same attached or not.
+ * dfb_filter_dev(h, dt_dev): one step whose dt is read from DEVICE memory (one double) when the step executes; the handle must be
+ * attached (else DFB_ERR_STATE).  Nothing is read back and nothing synchronises.  The blend constants sqrt(exp(-3.141592654 dt / Lt))
+ * are then computed on the device: CUDA's exp and the host's libm are each within one ulp, so they agree with dfb_filter's to rounding
+ * (the fields to ~1e-15 of their rms), not bit for bit.  A dt that is not finite, or is < 0, voids the step: the fields, filt_old, the
+ * N2 sums and the step counter stay as they were (the noise read back is the previous step's), and a sticky flag is set.  The next call
+ * that synchronises (dfb_sync, dfb_info, dfb_get_state, dfb_set_state, dfb_get_field, dfb_filter_to_host, dfb_get_noise,
+ * dfb_stats_get, dfb_save_restart, dfb_load_restart, dfb_interp_to_host, dfb_attach_stream(h, NULL)) returns DFB_ERR_ARG "dt must be
+ * finite and >= 0 ..." once, does nothing else (a detach still detaches), and clears the flag.
+ * While attached these return DFB_ERR_STATE, naming the call: dfb_comm_init and the gathers, dfb_corr_enable, dfb_stats_enable (set N2
+ * on or off before attaching), dfb_set_timing(h, 1), dfb_filter_to_host_begin / _end, dfb_filter_batch, dfb_generate_noise,
+ * dfb_get_rms.  Attaching an inject-mode handle, a handle with correlation statistics on or timing on, or while a _begin call is
+ * outstanding is DFB_ERR_STATE; a stream of another device is DFB_ERR_ARG.  dfb_get_state / dfb_set_state, restart files, dfb_info,
+ * dfb_stats_get, dfb_get_noise and face maps work: each synchronises the attached stream and reads or writes the device step record.
+ * Load the kernels before capturing: dfb_attach_stream does it.  A captured graph references the handle's memory: it must not be
+ * launched after a detach, a dfb_set_state / dfb_load_restart, or dfb_destroy; and the stream must outlive the attachment (dfb_destroy
+ * of an attached handle synchronises it). */
+int dfb_attach_stream(dfb_handle h, void* stream);
+int dfb_filter_dev(dfb_handle h, const double* dt_dev);
 /* page-lock (cudaHostRegister) / release a caller-owned host array: dfb_filter_to_host into registered arrays runs at the PCIe
  * rate; pageable arrays cost an extra staging pass inside the driver.  The C++ facade does this for its std::vectors. */
 int dfb_host_register(void* ptr, size_t bytes);
@@ -392,6 +421,9 @@ int dfb_gather_end_f(const dfb_handle* h);
 int dfb_gathered_to_host_f(const dfb_handle* h, const int* which, double* dst);
 int dfb_face_map_f(const dfb_handle* h, const int* n, const double* yf, const double* zf, int* plane_index);
 int dfb_destroy_f(dfb_handle* h);
+/* stream and dt_dev by reference: Fortran type(c_ptr) arguments (the stream as a cudaStream_t, dt_dev = the device address of dt) */
+int dfb_attach_stream_f(const dfb_handle* h, void* const* stream);
+int dfb_filter_dev_f(const dfb_handle* h, const double* const* dt_dev);
 /* path: Fortran character variable (c_loc) + its len_trim, as the file names of dfb_config (path_len < 0: NUL-terminated) */
 int dfb_save_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);
 int dfb_load_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);

@@ -120,6 +120,11 @@ class DIGITAL_FILTER {
         else
             check(dfb_filter(h_, dt));
     }
+    // GPU-resident callers (dfb_attach_stream): every later step, dfb_interp_to_cells and copy goes on `stream` (a cudaStream_t;
+    // nullptr detaches), with the step's state in device memory, so that filter_dev can be captured into the caller's CUDA graph
+    void attach_stream(struct CUstream_st* stream) { check(dfb_attach_stream(h_, stream)); }
+    // one step with dt read from device memory when it runs (the handle must be attached); the host vectors are not refreshed
+    void filter_dev(const double* dt_dev) { check(dfb_filter_dev(h_, dt_dev)); }
     // explicit fetch for fetch_every_step = false (also refreshes .filt)
     void fetch() {
         FilterField* F[3] = {&u, &v, &w};
