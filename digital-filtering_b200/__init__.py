@@ -150,6 +150,8 @@ def lib():
         L.dfb_interp_to_host.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, c_dp]
         L.dfb_attach_stream.argtypes = [C.c_void_p, C.c_void_p]
         L.dfb_filter_dev.argtypes = [C.c_void_p, C.c_void_p]
+        L.dfb_set_time_scales.argtypes = [C.c_void_p, c_dp]
+        L.dfb_time_scales_from_lengths.argtypes = [C.c_void_p, c_dp, C.c_double, c_dp]
         _lib = L
     return _lib
 
@@ -407,6 +409,33 @@ class DIGITAL_FILTER:
             raise ValueError("dt must be a 1-element CUDA float64 tensor")
         _check(lib().dfb_filter_dev(self._h, C.c_void_p(dt.data_ptr())))
 
+    # ---- per-row temporal scales (include/dfb200.h, dfb_set_time_scales) ----
+    def set_time_scales(self, rows):
+        """Lt per field and row for the temporal blend from the next step on: rows = [3][Ny] (u, v, w), finite and > 0; None returns to
+        the config's scalar Lt.  Refused (DfbError) while attached or while a filter_to_host_begin / gather_begin is outstanding."""
+        if rows is None:
+            _check(lib().dfb_set_time_scales(self._h, None))
+            return
+        a = np.ascontiguousarray(rows, dtype=np.float64)
+        if a.shape != (3, self.Ny):
+            raise ValueError("time scales must be [3][Ny] = [3][%d], got %s" % (self.Ny, a.shape))
+        _check(lib().dfb_set_time_scales(self._h, _dptr(a)))
+
+    @property
+    def time_scales(self):
+        """the [3][Ny] time scales in use: the rows of set_time_scales, or the scalar Lt of each field repeated (dfb_get_table 14)"""
+        return np.stack([self.table(14, f) for f in range(3)])
+
+    def time_scales_from_lengths(self, Ix, u_min):
+        """[3][Ny] time scales Ix_f(y_j) / max(Us_j, u_min) from streamwise lengths Ix = (inn_u, out_u, inn_v, out_v, inn_w, out_w),
+        blended across the boundary layer like Iz (dfb_time_scales_from_lengths); host only, sets nothing"""
+        ix = np.ascontiguousarray(Ix, dtype=np.float64)
+        if ix.shape != (6,):
+            raise ValueError("Ix must hold 6 lengths")
+        out = np.zeros((3, self.Ny))
+        _check(lib().dfb_time_scales_from_lengths(self._h, _dptr(ix), float(u_min), _dptr(out)))
+        return out
+
     def filter_batch(self, dts, out=None):
         dts = np.ascontiguousarray(dts, dtype=np.float64)
         _check(lib().dfb_filter_batch(self._h, len(dts), _dptr(dts), out.ctypes.data if out is not None else None))
@@ -484,7 +513,7 @@ class DIGITAL_FILTER:
         return self.info(4)
 
     def table(self, which, arg=0, n=None):
-        n = n if n is not None else (3 if which == 10 else (2 * arg + 1 if which == 11 else self.Ny))
+        n = n if n is not None else (3 if which == 10 else (2 * arg + 1 if which == 11 else self.Ny))   # 14: [Ny]
         out = np.zeros(n)
         _check(lib().dfb_get_table(self._h, which, arg, _dptr(out), n))
         return out

@@ -143,6 +143,20 @@ struct dfb_filter_s {
     bool g_after_first_only = false;  // the gathered step was the constructor's: T', rho' are zero (df.cpp:57-65)
     // face maps of the CFD hand-off (dfb_facemap_create): map id = index; a destroyed map leaves nullptr
     std::vector<std::unique_ptr<FaceMapDev>> facemaps;
+    // per-row time scales (dfb_set_time_scales; the rows themselves are plan.Lt_rows): the blend constants {sa, sb} of every (field,
+    // row) in device memory.  Host-driven steps: rows_tab holds those of dt = rows_dt, computed on the host and uploaded on the main
+    // stream before a step whose dt differs (the z-sweeps that read the table are on that stream too, so one table serves both buffer
+    // sets).  The uploads come from a ring of ROWS_SLOTS pinned slots: a slot is rewritten only after the event recorded behind its
+    // last copy, so the host may run that many uploads ahead of the device.  Attached steps: step_advance_rows_kernel writes rows_att
+    // from Lt_rows_dev.
+    static constexpr int ROWS_SLOTS = 4;
+    double* Lt_rows_dev = nullptr;    // [3][Ny]
+    double2* rows_tab = nullptr;      // [3][Ny]
+    double2* rows_att = nullptr;      // [3][Ny]
+    double2* rows_host = nullptr;     // pinned, [ROWS_SLOTS][3][Ny]
+    cudaEvent_t ev_rows[ROWS_SLOTS] = {};
+    int rows_next = 0;
+    double rows_dt = std::numeric_limits<double>::quiet_NaN();   // dt of rows_tab (NaN: none)
     // timing
     bool timing = false;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -182,6 +196,8 @@ struct dfb_filter_s {
         for (auto& pf : peer_flags) if (pf) cudaIpcCloseMemHandle(pf);
         if (peer_plane) cudaIpcCloseMemHandle(peer_plane);
         if (seq_ring) cudaFreeHost(seq_ring);
+        if (rows_host) cudaFreeHost(rows_host);
+        for (auto& e : ev_rows) if (e) cudaEventDestroy(e);
         if (ev_gstaged) cudaEventDestroy(ev_gstaged);
         if (ev_gdone) cudaEventDestroy(ev_gdone);
         comm_release();
@@ -340,6 +356,22 @@ void build_device(dfb_filter_s& H) {
     CUDA_TRY(cudaStreamSynchronize(H.stream));
 }
 
+// Host-driven step with per-row time scales: the device table of blend constants for dt, uploaded on the main stream when it holds
+// another dt (see dfb_filter_s::rows_tab).  Called before the step's first launch: nothing goes between its y- and z-sweep.
+const double2* rows_for_step(dfb_filter_s& H, double dt) {
+    if (H.rows_dt == dt) return H.rows_tab;
+    const size_t n = H.plan.Lt_rows.size();
+    const int slot = H.rows_next;
+    H.rows_next = (H.rows_next + 1) % dfb_filter_s::ROWS_SLOTS;
+    CUDA_TRY(cudaEventSynchronize(H.ev_rows[slot]));            // the copy that last read this slot has completed
+    double2* src = H.rows_host + (size_t)slot * n;
+    for (size_t i = 0; i < n; ++i) blend_consts(dt, H.plan.Lt_rows[i], src[i].x, src[i].y);
+    CUDA_TRY(cudaMemcpyAsync(H.rows_tab, src, n * sizeof(double2), cudaMemcpyHostToDevice, H.stream));
+    CUDA_TRY(cudaEventRecord(H.ev_rows[slot], H.stream));
+    H.rows_dt = dt;
+    return H.rows_tab;
+}
+
 void fill_noise_params(dfb_filter_s& H, int64_t step) { fill_noise_states(H.np, H.npairs, H.seed, H.plane_id, H.nplanes, step); }
 
 void launch_noise_for(dfb_filter_s& H, int64_t step, int b, cudaStream_t st) {
@@ -364,6 +396,8 @@ void run_step_attached(dfb_filter_s& H, double dt, const double* dt_dev, bool fi
     if (!dt_dev)
         for (int f = 0; f < 3; ++f) blend_consts(dt, H.plan.f[f].Lt, A.sa[f], A.sb[f]);
     A.stats = accumulate ? 1 : 0;
+    const double2* rows = (!first && !H.plan.Lt_rows.empty()) ? H.rows_att : nullptr;
+    if (rows) { A.Lt_rows = H.Lt_rows_dev; A.rows = H.rows_att; A.n_rows = (int)H.plan.Lt_rows.size(); }
     CUDA_TRY(launch_advance(A, H.stream));
     NoiseParams np = H.np;
     np.rec = H.rec;
@@ -383,12 +417,13 @@ void run_step_attached(dfb_filter_s& H, double dt, const double* dt_dev, bool fi
         ZParams Z = H.zp[0];
         Z.S = S;
         Z.rec = H.rec;
+        Z.rows = rows;
         Z.tl = nullptr;
         Z.stats = accumulate ? H.stats : nullptr;
         CUDA_TRY(launch_zsweep_tuned(H.zmaps[0], Z, H.stream));
     } else {
         CUDA_TRY(launch_ysweep_simple(H.D[0], H.stream));
-        CUDA_TRY(launch_zsweep_simple(H.D[0], S, H.rec, H.stream));
+        CUDA_TRY(launch_zsweep_simple(H.D[0], S, H.rec, rows, H.stream));
         if (accumulate) CUDA_TRY(launch_stats(H.D[0], H.stats, H.rec, H.stream));
     }
 }
@@ -398,6 +433,7 @@ void run_step(dfb_filter_s& H, double dt, bool first) {
     CUDA_TRY(cudaSetDevice(H.device));
     const int b = (int)(H.step & 1);
     if (H.timing) CUDA_TRY(cudaEventRecord(H.ev[0], H.stream));
+    const double2* rows = (!first && !H.plan.Lt_rows.empty()) ? rows_for_step(H, dt) : nullptr;
     if (H.noise_mode == DFB_NOISE_GENERATE) {
         // ev_noise[b] = the last noise launch into set b on EITHER stream: wait for it whether its result is the one this step
         // wants (prefetched) or not (after a dfb_set_state rewind the side stream's prefetch may still be writing set b)
@@ -425,10 +461,11 @@ void run_step(dfb_filter_s& H, double dt, bool first) {
     const bool accumulate = H.stats_on && !first;                  // rms_add, df.cpp:606
     if (H.tuned) {
         H.zp[b].S = S;
+        H.zp[b].rows = rows;
         H.zp[b].stats = accumulate ? H.stats : nullptr;            // N2 fused into the epilogue
         CUDA_TRY(launch_zsweep_tuned(H.zmaps[b], H.zp[b], H.stream));
     } else {
-        CUDA_TRY(launch_zsweep_simple(H.D[b], S, nullptr, H.stream));
+        CUDA_TRY(launch_zsweep_simple(H.D[b], S, nullptr, rows, H.stream));
         if (accumulate) CUDA_TRY(launch_stats(H.D[0], H.stats, nullptr, H.stream));
     }
     if (accumulate) H.stats_count += 1;
@@ -676,6 +713,7 @@ int dfb_info(dfb_handle h, int what, int field, int64_t* out64) {
         case 11: *out64 = h->tuned ? h->yp[0].n_rtiles : 0; break;
         case 13: *out64 = h->plan.periodic ? 1 : 0; break;
         case 14: *out64 = h->corr_ready ? h->corr.L[field] : 0; break;
+        case 15: *out64 = h->plan.Lt_rows.empty() ? 0 : 1; break;
         default: return fail(DFB_ERR_ARG, "unknown info selector");
     }
     return DFB_OK;
@@ -696,6 +734,12 @@ int dfb_get_table(dfb_handle h, int which, int arg, double* dst, int cap) {
         src = P.coef.vals.data() + P.coef.ptr[arg]; n = 2 * arg + 1;
     } else if (which == 12) { src = P.vert_y.data(); n = P.Ny + 1; }
     else if (which == 13) { src = P.vert_z.data(); n = P.NzG + 1; }
+    else if (which == 14) {
+        if (arg < 0 || arg > 2) return fail(DFB_ERR_ARG, "table 14: field must be 0..2");
+        if (P.Lt_rows.empty()) { tmp.assign(P.Ny, P.f[arg].Lt); src = tmp.data(); }
+        else src = P.Lt_rows.data() + (size_t)arg * P.Ny;
+        n = P.Ny;
+    }
     else return fail(DFB_ERR_ARG, "unknown table selector");
     if (cap < n) return fail(DFB_ERR_ARG, "dst too small");
     std::memcpy(dst, src, sizeof(double) * n);
@@ -908,6 +952,42 @@ int dfb_filter_dev(dfb_handle h, const double* dt_dev) {
     if (!h || !dt_dev) return fail(DFB_ERR_ARG, "handle/dt_dev is NULL");
     if (!h->attached) return fail(DFB_ERR_STATE, "dfb_filter_dev needs a stream attached with dfb_attach_stream");
     return guarded([&] { run_step_attached(*h, 0.0, dt_dev, false); });
+}
+
+int dfb_set_time_scales(dfb_handle h, const double* Lt_rows) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_set_time_scales") + ": set the rows before attaching");
+    if (h->pipe_begun != h->pipe_ended || h->g_begun != h->g_ended)
+        return fail(DFB_ERR_STATE, "dfb_set_time_scales: a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first");
+    return guarded([&] {
+        Plan& P = h->plan;
+        if (!Lt_rows) {
+            P.Lt_rows.clear();
+            h->fingerprint = rst::fingerprint(P);
+            return;
+        }
+        check_time_scales(P, Lt_rows);
+        const size_t n = (size_t)3 * P.Ny;
+        CUDA_TRY(cudaSetDevice(h->device));
+        if (!h->rows_host) {
+            h->Lt_rows_dev = h->dalloc<double>(n, false);
+            h->rows_tab = h->dalloc<double2>(n, false);
+            h->rows_att = h->dalloc<double2>(n, false);
+            for (auto& e : h->ev_rows) CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            CUDA_TRY(cudaHostAlloc(&h->rows_host, dfb_filter_s::ROWS_SLOTS * n * sizeof(double2), cudaHostAllocDefault));
+        }
+        // the attached steps' copy of the rows; the handle is not attached, so no step reads it now
+        CUDA_TRY(cudaMemcpyAsync(h->Lt_rows_dev, Lt_rows, n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        CUDA_TRY(cudaStreamSynchronize(h->stream));
+        P.Lt_rows.assign(Lt_rows, Lt_rows + n);
+        h->rows_dt = std::numeric_limits<double>::quiet_NaN();    // the next step uploads the new rows' constants
+        h->fingerprint = rst::fingerprint(P);
+    });
+}
+
+int dfb_time_scales_from_lengths(dfb_handle h, const double Ix[6], double u_min, double* Lt_rows) {
+    if (!h || !Ix || !Lt_rows) return fail(DFB_ERR_ARG, "handle/Ix/Lt_rows is NULL");
+    return guarded([&] { time_scales_from_lengths(h->plan, Ix, u_min, Lt_rows); });
 }
 
 static int set_noise_impl(dfb_handle h, int field, const double* r_ys, const double* left, const double* right, size_t halo_pitch) {
@@ -2100,6 +2180,12 @@ int dfb_attach_stream_f(const dfb_handle* h, void* const* stream) {
 }
 int dfb_filter_dev_f(const dfb_handle* h, const double* const* dt_dev) {
     return (h && dt_dev) ? dfb_filter_dev(*h, *dt_dev) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_set_time_scales_f(const dfb_handle* h, const double* const* Lt_rows) {
+    return (h && Lt_rows) ? dfb_set_time_scales(*h, *Lt_rows) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_time_scales_from_lengths_f(const dfb_handle* h, const double* Ix, const double* u_min, double* Lt_rows) {
+    return (h && u_min) ? dfb_time_scales_from_lengths(*h, Ix, *u_min, Lt_rows) : fail(DFB_ERR_ARG, "NULL argument");
 }
 int dfb_destroy_f(dfb_handle* h) {
     if (!h) return DFB_OK;

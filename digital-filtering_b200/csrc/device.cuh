@@ -163,6 +163,10 @@ struct AdvanceParams {
     uint64_t npairs[6];        // pairs one step draws from each array's stream
     int n_arrays, P;
     int stats;                 // this step accumulates N2: count it
+    // per-row time scales (dfb_set_time_scales): step_advance_rows_kernel writes rows[i] = {sa, sb} of Lt_rows[i], i < n_rows = 3 Ny
+    const double* Lt_rows;
+    double2* rows;
+    int n_rows;
 };
 
 // ---- noise generation work description (one segment = one row of one logical array, or one contiguous piece of a row) ----
@@ -257,6 +261,8 @@ struct ZParams {
     int debug;                   // development probes only (0 in production)
     unsigned long long* prof;    // [8] cycle counters filled when debug & 16
     const StepRecord* rec;       // attached step: sa, sb come from the record, and a void step writes nothing; nullptr host-driven
+    const double2* rows;         // per-row time scales (dfb_set_time_scales): {sa, sb} of field f, row j at [f * Ny + j]; read by
+                                 // zsweep_epilogue_rows_kernel only (sa, sb of S and rec are then unused)
 };
 
 }  // namespace dfb

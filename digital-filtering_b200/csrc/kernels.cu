@@ -166,13 +166,20 @@ __device__ __forceinline__ void epilogue_cell(const double* __restrict__ rc, con
     o.rho = -t2 * rc[6];                                  // df.cpp:481
 }
 
-__global__ void __launch_bounds__(256) zsweep_epilogue_simple_kernel(const PlaneDev D, StepConsts S, const StepRecord* rec) {
+// ROWS: per-row time scales (dfb_set_time_scales), sa, sb of row j from rows[f * Ny + j]
+template <bool ROWS>
+__device__ __forceinline__ void zsweep_epilogue_simple(const PlaneDev& D, StepConsts& S, const StepRecord* rec, const double2* rows) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     const int j = blockIdx.y, pl = blockIdx.z;
     if (k >= D.W) return;
     if (rec) {                                            // attached step (dfb_attach_stream): a void step writes nothing
         if (rec->void_step) return;
-        for (int f = 0; f < 3; ++f) { S.sa[f] = rec->sa[f]; S.sb[f] = rec->sb[f]; }
+        if (!ROWS)
+            for (int f = 0; f < 3; ++f) { S.sa[f] = rec->sa[f]; S.sb[f] = rec->sb[f]; }
+    }
+    if (ROWS) {
+        const double2 pu = rows[j], pv = rows[D.Ny + j], pw = rows[2 * D.Ny + j];
+        S.sa[0] = pu.x; S.sb[0] = pu.y; S.sa[1] = pv.x; S.sb[1] = pv.y; S.sa[2] = pw.x; S.sb[2] = pw.y;
     }
     double z[3];
 #pragma unroll
@@ -188,11 +195,32 @@ __global__ void __launch_bounds__(256) zsweep_epilogue_simple_kernel(const Plane
     const size_t idx = (size_t)pl * D.ps_cells + (size_t)j * D.W + k;
     EpiOut o;
     double ou, ov, ow;
-    epilogue_cell(D.rowc + (size_t)j * ROWC, S, z[0], z[1], z[2],
-                  D.f[0].filt_old[idx], D.f[1].filt_old[idx], D.f[2].filt_old[idx], ou, ov, ow, o);
+    if constexpr (ROWS) {
+        // the blend of epilogue_cell written out with the contraction the compiler gives it in zsweep_epilogue_simple_kernel
+        // (fu * sa fused, zu * sb rounded): with sa, sb loaded instead of kernel parameters it would fuse the other product
+        if (!S.first_step)
+#pragma unroll
+            for (int f = 0; f < 3; ++f) z[f] = __fma_rn(D.f[f].filt_old[idx], S.sa[f], __dmul_rn(z[f], S.sb[f]));
+        StepConsts E = S;
+        E.first_step = 1;
+        epilogue_cell(D.rowc + (size_t)j * ROWC, E, z[0], z[1], z[2], 0.0, 0.0, 0.0, ou, ov, ow, o);
+    } else {
+        epilogue_cell(D.rowc + (size_t)j * ROWC, S, z[0], z[1], z[2],
+                      D.f[0].filt_old[idx], D.f[1].filt_old[idx], D.f[2].filt_old[idx], ou, ov, ow, o);
+    }
     D.f[0].filt_old[idx] = ou; D.f[1].filt_old[idx] = ov; D.f[2].filt_old[idx] = ow;
     D.f[0].fluc[idx] = o.u; D.f[1].fluc[idx] = o.v; D.f[2].fluc[idx] = o.w;
     if (!S.first_step) { D.T_fluc[idx] = o.T; D.rho_fluc[idx] = o.rho; }                 // df.cpp:65 (quirk 3)
+}
+
+__global__ void __launch_bounds__(256) zsweep_epilogue_simple_kernel(const PlaneDev D, StepConsts S, const StepRecord* rec) {
+    zsweep_epilogue_simple<false>(D, S, rec, nullptr);
+}
+
+// launched with 256 threads like the kernel above; under __launch_bounds__(256) ptxas held it to 32 registers and spilled
+__global__ void __maxnreg__(64) zsweep_epilogue_simple_rows_kernel(const PlaneDev D, StepConsts S, const StepRecord* rec,
+                                                                          const double2* rows) {
+    zsweep_epilogue_simple<true>(D, S, rec, rows);
 }
 
 // =================================================================================================
@@ -865,9 +893,10 @@ __device__ __forceinline__ void z_issue_unit(const ZParams& P, const ZMaps& maps
 }
 
 // REC: an attached step (dfb_attach_stream) reads sa, sb from the step record and writes nothing when the step is void; host-driven
-// steps keep the kernel that takes them as parameters
-template <int ZK, int MODE, bool STATS, bool REC>
-__global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_kernel(const __grid_constant__ ZMaps maps, const ZParams P) {
+// steps keep the kernel that takes them as parameters.  ROWS: per-row time scales (dfb_set_time_scales), sa, sb of each unit's row
+// from P.rows (zsweep_epilogue_rows_kernel); handles without them keep zsweep_epilogue_kernel.
+template <int ZK, int MODE, bool STATS, bool REC, bool ROWS>
+__device__ __forceinline__ void zsweep_epilogue(const ZMaps& maps, const ZParams& P) {
     constexpr int LB = ZK * 8;               // bytes per staged line (= one lane's ZK samples): 128 -> SWIZZLE_128B, 64 -> SWIZZLE_64B
     constexpr int PPL = ZK / 2;              // 16-byte pieces per line
     constexpr int UB = 32 * LB;              // bytes of the per-warp u line buffer
@@ -948,6 +977,8 @@ __global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_ker
         if (P.debug & 16) pa_stage += clock64() - ttop;                                           // staging the next unit (lane 0)
 
         const int j = dcur[0], c0 = dcur[1], f = dcur[2];
+        double2 row_sab;
+        if (ROWS) row_sab = __ldg(P.rows + f * D.Ny + j);    // issued before the tap loop, used in the epilogue: its latency hides behind the loop
         const int nchunk = __shfl_sync(0xffffffffu, dcur[3], 0);
         const int k0 = c0 + lane * ZK;
         const bool active = k0 < D.W;
@@ -1135,7 +1166,7 @@ __global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_ker
             const double* rc = reinterpret_cast<const double*>(cbuf + P.rc_off);        // the row's constants, staged with the window
             const double rc_own = rc[f == 0 ? 0 : (f == 1 ? 2 : 3)];
             const double rc0 = rc[0], rc1 = rc[1], rc4 = rc[4], rc5 = rc[5], rc6 = rc[6];
-            const double sa = REC ? P.rec->sa[f] : P.S.sa[f], sb = REC ? P.rec->sb[f] : P.S.sb[f];
+            const double sa = ROWS ? row_sab.x : REC ? P.rec->sa[f] : P.S.sa[f], sb = ROWS ? row_sab.y : REC ? P.rec->sb[f] : P.S.sb[f];
             double* stats = (STATS && blend) ? P.stats + (size_t)plA * 6 * D.ps_cells + ((size_t)j * D.W) : nullptr;
             if (coalesced) {
                 // One transpose per unit: lane l owns line l (its ZK cells) of a 32-line tile; global memory wants 16-byte piece
@@ -1277,6 +1308,18 @@ __global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_ker
     }
 }
 
+template <int ZK, int MODE, bool STATS, bool REC>
+__global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_kernel(const __grid_constant__ ZMaps maps, const ZParams P) {
+    zsweep_epilogue<ZK, MODE, STATS, REC, false>(maps, P);
+}
+
+// The row's {sa, sb} is held in registers across the tap loop: the recursive form at 16 outputs per lane would spill them at
+// Z_REC_MAXNREG, so it gets 8 more registers (it runs at most two CTAs per SM, which 176 registers per thread still allow).
+template <int ZK, int MODE, bool STATS, bool REC>
+__global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG + (ZK == 16 ? 8 : 0) : 168) zsweep_epilogue_rows_kernel(const __grid_constant__ ZMaps maps, const ZParams P) {
+    zsweep_epilogue<ZK, MODE, STATS, REC, true>(maps, P);
+}
+
 // =================================================================================================
 // attached steps (dfb_attach_stream): the step's host decisions, made on the device
 // =================================================================================================
@@ -1284,7 +1327,7 @@ __global__ void __maxnreg__(MODE == 1 ? Z_REC_MAXNREG : 168) zsweep_epilogue_ker
 // constants), validates it, computes the blend constants and the pcg32 positions of the record's step with the host's own functions
 // (blend_consts, noise_step_state), and advances the step counter and the N2 count -- only when the step is not void.  A void step
 // leaves the positions as they were, so its noise launch rewrites the previous step's noise unchanged.
-__global__ void __launch_bounds__(128) step_advance_kernel(const AdvanceParams A) {
+__device__ __forceinline__ void step_advance(const AdvanceParams& A) {
     __shared__ int ok;
     StepRecord* R = A.rec;
     const long long step = R->step;
@@ -1311,6 +1354,22 @@ __global__ void __launch_bounds__(128) step_advance_kernel(const AdvanceParams A
     if (threadIdx.x == 0) {
         R->step = step + 1;
         if (A.stats) R->stats_count += 1;
+    }
+}
+
+__global__ void __launch_bounds__(128) step_advance_kernel(const AdvanceParams A) { step_advance(A); }
+
+// A handle with per-row time scales (dfb_set_time_scales): block 0 is step_advance_kernel, and every block writes its share of the
+// step's per-row blend constants, {sa, sb} of Lt_rows[i], with the same blend_consts -- only when dt is valid (a void step's z-sweep
+// writes nothing, so it reads no table).  No block reads what another writes.
+__global__ void __launch_bounds__(128) step_advance_rows_kernel(const AdvanceParams A) {
+    if (blockIdx.x == 0) step_advance(A);
+    const double dt = A.dt_dev ? *A.dt_dev : A.dt;
+    if (!(isfinite(dt) && dt >= 0.0)) return;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A.n_rows; i += gridDim.x * blockDim.x) {
+        double sa, sb;
+        blend_consts(dt, A.Lt_rows[i], sa, sb);
+        A.rows[i] = make_double2(sa, sb);
     }
 }
 
@@ -1499,9 +1558,10 @@ cudaError_t launch_ysweep_simple(const PlaneDev& D, cudaStream_t st) {
     return cudaGetLastError();
 }
 
-cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, const StepRecord* rec, cudaStream_t st) {
+cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, const StepRecord* rec, const double2* rows, cudaStream_t st) {
     dim3 grid((unsigned)((D.W + 255) / 256), (unsigned)D.Ny, (unsigned)D.P);
-    zsweep_epilogue_simple_kernel<<<grid, 256, 0, st>>>(D, S, rec);
+    if (rows) zsweep_epilogue_simple_rows_kernel<<<grid, 256, 0, st>>>(D, S, rec, rows);
+    else zsweep_epilogue_simple_kernel<<<grid, 256, 0, st>>>(D, S, rec);
     return cudaGetLastError();
 }
 
@@ -1581,13 +1641,23 @@ static const void* zsweep_fn_rec(int zk, int mode, bool stats) {
     if (zk == 16) return mode == 1 ? (const void*)zsweep_epilogue_kernel<16, 1, false, REC> : (const void*)zsweep_epilogue_kernel<16, 0, false, REC>;
     return mode == 1 ? (const void*)zsweep_epilogue_kernel<8, 1, false, REC> : (const void*)zsweep_epilogue_kernel<8, 0, false, REC>;
 }
-static const void* zsweep_fn(int zk, int mode, bool stats, bool rec = false) {
+template <bool REC>
+static const void* zsweep_rows_fn_rec(int zk, int mode, bool stats) {
+    if (stats) {
+        if (zk == 16) return mode == 1 ? (const void*)zsweep_epilogue_rows_kernel<16, 1, true, REC> : (const void*)zsweep_epilogue_rows_kernel<16, 0, true, REC>;
+        return mode == 1 ? (const void*)zsweep_epilogue_rows_kernel<8, 1, true, REC> : (const void*)zsweep_epilogue_rows_kernel<8, 0, true, REC>;
+    }
+    if (zk == 16) return mode == 1 ? (const void*)zsweep_epilogue_rows_kernel<16, 1, false, REC> : (const void*)zsweep_epilogue_rows_kernel<16, 0, false, REC>;
+    return mode == 1 ? (const void*)zsweep_epilogue_rows_kernel<8, 1, false, REC> : (const void*)zsweep_epilogue_rows_kernel<8, 0, false, REC>;
+}
+static const void* zsweep_fn(int zk, int mode, bool stats, bool rec = false, bool rows = false) {
+    if (rows) return rec ? zsweep_rows_fn_rec<true>(zk, mode, stats) : zsweep_rows_fn_rec<false>(zk, mode, stats);
     return rec ? zsweep_fn_rec<true>(zk, mode, stats) : zsweep_fn_rec<false>(zk, mode, stats);
 }
 
 cudaError_t zsweep_prepare(int zk, int mode, size_t smem, int* blocks_per_sm) {
-    for (int v = 3; v >= 0; --v) {                      // bit 0: N2 accumulation, bit 1: attached step
-        const void* fn = zsweep_fn(zk, mode, (v & 1) != 0, (v & 2) != 0);
+    for (int v = 7; v >= 0; --v) {                      // bit 0: N2 accumulation, bit 1: attached step, bit 2: per-row time scales
+        const void* fn = zsweep_fn(zk, mode, (v & 1) != 0, (v & 2) != 0, (v & 4) != 0);
         cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -1602,17 +1672,19 @@ cudaError_t launch_zsweep_tuned(const ZMaps& maps, const ZParams& P, cudaStream_
     static const int pdl = std::getenv("DFB_Z_PDL") ? std::atoi(std::getenv("DFB_Z_PDL")) : 1;
     if (!pdl) cfg.numAttrs = 0;
     void* args[2] = {const_cast<ZMaps*>(&maps), const_cast<ZParams*>(&P)};
-    return cudaLaunchKernelExC(&cfg, zsweep_fn(P.zk, P.zmode, P.stats != nullptr, P.rec != nullptr), args);
+    return cudaLaunchKernelExC(&cfg, zsweep_fn(P.zk, P.zmode, P.stats != nullptr, P.rec != nullptr, P.rows != nullptr), args);
 }
 
 cudaError_t launch_advance(const AdvanceParams& A, cudaStream_t st) {
-    step_advance_kernel<<<1, 128, 0, st>>>(A);
+    if (A.rows) step_advance_rows_kernel<<<(unsigned)(A.n_rows > 128 ? (A.n_rows + 127) / 128 : 1), 128, 0, st>>>(A);
+    else step_advance_kernel<<<1, 128, 0, st>>>(A);
     return cudaGetLastError();
 }
 
 cudaError_t attach_prepare() {
     // load the kernels an attached step may launch for the first time now, not while the caller's stream is being captured
-    const void* fns[] = {(const void*)step_advance_kernel, (const void*)ysweep_simple_kernel, (const void*)zsweep_epilogue_simple_kernel,
+    const void* fns[] = {(const void*)step_advance_kernel, (const void*)step_advance_rows_kernel, (const void*)ysweep_simple_kernel,
+                         (const void*)zsweep_epilogue_simple_kernel, (const void*)zsweep_epilogue_simple_rows_kernel,
                          (const void*)stats_kernel, (const void*)noise_kernel<true>, (const void*)noise_pieces_kernel<true>};
     for (const void* fn : fns) {
         cudaFuncAttributes a;

@@ -6,8 +6,9 @@ namespace dfb {
 
 cudaError_t launch_noise(const NoiseParams& P, const NoiseWindows& Wn, const PlaneDev& D, cudaStream_t st);
 cudaError_t launch_ysweep_simple(const PlaneDev& D, cudaStream_t st);
-cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, const StepRecord* rec, cudaStream_t st);
-// attached steps (dfb_attach_stream): the step's first launch, and loading every kernel such a step may launch
+cudaError_t launch_zsweep_simple(const PlaneDev& D, const StepConsts& S, const StepRecord* rec, const double2* rows, cudaStream_t st);
+// attached steps (dfb_attach_stream): the step's first launch (with the per-row blend constants when A.rows is set), and loading
+// every kernel such a step may launch
 cudaError_t launch_advance(const AdvanceParams& A, cudaStream_t st);
 cudaError_t attach_prepare();
 cudaError_t ysweep_prepare();

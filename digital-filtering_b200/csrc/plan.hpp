@@ -46,6 +46,7 @@ struct Plan {
     FieldPlan f[3];
     CoefTable coef;
     int64_t taps_per_step = 0;                   // sum over fields and LOCAL cells of (2Ny+1)+(2Nz+1)
+    std::vector<double> Lt_rows;                 // [3][Ny] per-row time scales (dfb_set_time_scales); empty: f[].Lt for every row
     int Nz() const { return k1 - k0; }
 };
 
@@ -90,6 +91,11 @@ StepPlan plan_step(const Plan& plan, int nplanes, const DeviceLimits& dev, const
 // np.pstate / np.pinc of every array np draws and every plane of the handle: pcg32 state at the first draw of step `step` (plane p of a
 // batch draws from stream group plane_id + p).  The advance kernel of attached steps computes the same states with noise_step_state.
 void fill_noise_states(NoiseParams& np, const uint64_t* npairs, uint64_t seed, int plane_id, int nplanes, int64_t step);
+
+// Per-row time scales [3][Ny]: throws DFB_ERR_ARG naming the first entry that is not finite or not > 0.
+void check_time_scales(const Plan& plan, const double* Lt_rows);
+// dfb_time_scales_from_lengths: Lt_f(j) = Ix_f(y_j) / max(Us_j, u_min), Ix_f blended from Ix[2f] to Ix[2f+1] like Iz.  Throws dfb::Error.
+void time_scales_from_lengths(const Plan& plan, const double Ix[6], double u_min, double* Lt_rows);
 
 // pieces, exposed for unit tests through the C ABI
 void coefficients(int N, double* b /* 2N+1 */);

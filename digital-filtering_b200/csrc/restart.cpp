@@ -144,6 +144,11 @@ uint64_t fingerprint(const Plan& P) {
     }
     H.word(P.rows.size());
     for (double v : P.rows) H.f64(v);
+    if (!P.Lt_rows.empty()) {                    // per-row time scales: hashed only when set, so a handle without them keeps its fingerprint
+        H.word(0x4c745f726f7773ull);             // "Lt_rows"
+        H.word(P.Lt_rows.size());
+        for (double v : P.Lt_rows) H.f64(v);
+    }
     return H.h;
 }
 

@@ -6,6 +6,7 @@
 // test_G2_default_plane_against_reference_object_code compares rows, half-widths, coefficients and Lt
 // with the running reference object; tests/test_oracle_vs_ref.py pins the restatement they are checked with).
 #include <cmath>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
@@ -363,6 +364,32 @@ void build_plan(const dfb_config& cfg, Plan& P) {
             if (F.row_uniform) P.taps_per_step += (int64_t)(P.k1 - P.k0) * ((2 * F.N_y_row[j] + 1) + (2 * F.N_z_row[j] + 1));
             else for (int k = P.k0; k < P.k1; ++k)
                 P.taps_per_step += (2 * F.N_y[(size_t)j * NzG + k] + 1) + (2 * F.N_z[(size_t)j * NzG + k] + 1);
+        }
+    }
+}
+
+void check_time_scales(const Plan& P, const double* Lt_rows) {
+    static const char* const name[3] = {"u", "v", "w"};
+    for (int f = 0; f < 3; ++f)
+        for (int j = 0; j < P.Ny; ++j) {
+            const double v = Lt_rows[(size_t)f * P.Ny + j];
+            if (std::isfinite(v) && v > 0.0) continue;
+            char buf[160];
+            std::snprintf(buf, sizeof(buf), "time scale of field %d (%s), row %d is %g: every entry must be finite and > 0", f, name[f], j, v);
+            throw Error{DFB_ERR_ARG, buf};
+        }
+}
+
+void time_scales_from_lengths(const Plan& P, const double Ix[6], double u_min, double* Lt_rows) {
+    if (!(std::isfinite(u_min) && u_min > 0.0)) throw Error{DFB_ERR_ARG, "u_min must be finite and > 0"};
+    for (int i = 0; i < 6; ++i)
+        if (!(std::isfinite(Ix[i]) && Ix[i] > 0.0)) throw Error{DFB_ERR_ARG, "the lengths Ix must be finite and > 0"};
+    const double* Us = P.rows.data() + (size_t)4 * P.Ny;
+    for (int f = 0; f < 3; ++f) {
+        const double inn = Ix[2 * f], out = Ix[2 * f + 1];
+        for (int j = 0; j < P.Ny; ++j) {
+            const double Ixj = inn + (out - inn) * 0.5 * (1 + std::tanh((P.yc_row[j] / P.d_i - 0.2) / 0.03));   // the Iz blend, df.cpp:146
+            Lt_rows[(size_t)f * P.Ny + j] = Ixj / std::max(Us[j], u_min);
         }
     }
 }

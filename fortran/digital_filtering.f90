@@ -23,6 +23,8 @@
 !   interp_to_cells, filter_on_device               all five fields in one pass on the device; only the faces cross PCIe
 !   attach_stream, filter_dev                     GPU-resident CFD codes: steps on the code's own CUDA stream with dt in device memory,
 !                                                 capturable into its CUDA graph (include/dfb200.h, dfb_attach_stream)
+!   set_time_scales, clear_time_scales,           per-row temporal scales Lt(y) for the temporal blend, e.g. from a prescribed
+!   time_scales_from_lengths                        streamwise length: Lt = Ix(y) / U(y) (include/dfb200.h, dfb_set_time_scales)
 !
 ! NOTE: NEVER COMPILED -- no Fortran compiler exists in the build image or on the GPU boxes.  The binding is exercised through
 ! tests/fortran_abi_mimic.c, a C program that makes exactly these calls with exactly this struct layout and by-reference
@@ -38,6 +40,7 @@ module DIGITAL_FILTERING
     public :: save_restart, load_restart, RESTART_STATE, RESTART_STATS, RESTART_CORR
     public :: facemap_create, interp_to_host, interp_to_cells, facemap_destroy, MAP_POINT, MAP_AREA, MAP_WALL_ZERO, filter_on_device
     public :: attach_stream, filter_dev
+    public :: set_time_scales, clear_time_scales, time_scales_from_lengths
 
     integer, parameter :: RESTART_STATE = 1, RESTART_STATS = 2, RESTART_CORR = 4   ! DFB_RESTART_* (what to save / load; added together)
 
@@ -256,6 +259,16 @@ module DIGITAL_FILTERING
             import :: c_int, c_ptr
             type(c_ptr), intent(in) :: handle, dt_dev
         end function
+        integer(c_int) function dfb_set_time_scales_f(handle, Lt_rows) bind(C, name='dfb_set_time_scales_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle, Lt_rows
+        end function
+        integer(c_int) function dfb_time_scales_from_lengths_f(handle, Ix, u_min, Lt_rows) bind(C, name='dfb_time_scales_from_lengths_f')
+            import :: c_int, c_ptr, c_double
+            type(c_ptr), intent(in) :: handle
+            real(c_double), intent(in) :: Ix(6), u_min
+            real(c_double), intent(out) :: Lt_rows(*)
+        end function
         function dfb_last_error() bind(C, name='dfb_last_error') result(msg)
             import :: c_ptr
             type(c_ptr) :: msg
@@ -438,6 +451,29 @@ contains
         type(c_ptr), intent(in) :: dt_dev
         call check(dfb_filter_dev_f(DF%handle, dt_dev), 'filter_dev')
     end subroutine filter_dev
+
+    ! per-row time scales of the temporal blend from the next step on: Lt_rows(j, f), j = 1..Ny (after the trim), f = 1..3 (u, v, w),
+    ! finite and > 0; set them before attach_stream and before load_restart of a file saved with them
+    subroutine set_time_scales(DF, Lt_rows)
+        type(digital_filter_type), intent(in) :: DF
+        real(c_double), intent(in), target, contiguous :: Lt_rows(:, :)
+        call check(dfb_set_time_scales_f(DF%handle, c_loc(Lt_rows)), 'set_time_scales')
+    end subroutine set_time_scales
+
+    ! back to the scalar Lt of the configuration
+    subroutine clear_time_scales(DF)
+        type(digital_filter_type), intent(in) :: DF
+        call check(dfb_set_time_scales_f(DF%handle, c_null_ptr), 'clear_time_scales')
+    end subroutine clear_time_scales
+
+    ! Lt_rows(j, f) = Ix_f(y_j) / max(U(y_j), u_min): Ix = (inn_u, out_u, inn_v, out_v, inn_w, out_w) blended across the boundary layer
+    ! like Iz; host only, sets nothing (pass the result to set_time_scales)
+    subroutine time_scales_from_lengths(DF, Ix, u_min, Lt_rows)
+        type(digital_filter_type), intent(in) :: DF
+        real(c_double), intent(in) :: Ix(6), u_min
+        real(c_double), intent(out) :: Lt_rows(:, :)
+        call check(dfb_time_scales_from_lengths_f(DF%handle, Ix, u_min, Lt_rows), 'time_scales_from_lengths')
+    end subroutine time_scales_from_lengths
 
     subroutine facemap_create(DF, n, yf, zf, map_id, hy, hz, own_begin, own_end, wall_zero, served)
         ! bilinear at the face centres, or with hy, hz the average over each face; own_begin/own_end: 0-based columns [own_begin,

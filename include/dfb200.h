@@ -128,11 +128,13 @@ int dfb_dims(dfb_handle h, int* Ny, int* Nz);
  *    32 rows where it pays + dense band matrices on the rest (e.g. a batch of planes of the reference's default geometry), 1 = chunk-recursive band-matrix
  *    kernel, 0 = dense band matrices (DFB_Y_MODE=0|1|2 forces a form), 11 tiles of the run-recursive kernel, 12 transport of the config-4 hand-off: 2 = peer-to-peer copies (CUDA IPC + copy engines), 1 = NCCL
  *    send/recv, 0 = no communicator, 13 spanwise-periodic plane (dfb_config.periodic_z) in use (0/1),
- * 14 lags of correlation direction `field` (0 z, 1 y, 2 t; dfb_corr_enable), 0 when that direction is off or before any enable */
+ * 14 lags of correlation direction `field` (0 z, 1 y, 2 t; dfb_corr_enable), 0 when that direction is off or before any enable,
+ * 15 per-row time scales in use (dfb_set_time_scales, 0/1) */
 int dfb_info(dfb_handle h, int what, int field, int64_t* out64);
 /* host copies of the setup tables (for parity tests): which = 0..7 rows R11,R21,R22,R33,Us,Ts,rhos,Ms [Ny];
  * 8 yc row [Ny]; 9 dy row [Ny]; 10 Lt[3]; 11 coefficients of half-width `arg` [2*arg+1];
- * 12 y of the vertex rows [Ny+1]; 13 z of the vertex columns [Nz_global+1] (df.cpp:99-100: the y / z the writers print) */
+ * 12 y of the vertex rows [Ny+1]; 13 z of the vertex columns [Nz_global+1] (df.cpp:99-100: the y / z the writers print);
+ * 14 time scales Lt of field `arg` (0..2) per row in use [Ny]: the rows of dfb_set_time_scales, or the scalar Lt repeated */
 int dfb_get_table(dfb_handle h, int which, int arg, double* dst, int cap);
 /* N_y / N_z of field f (dir 0 = y, 1 = z) for the local slab, [Ny*Nz] */
 int dfb_get_half_widths(dfb_handle h, int field, int dir, int* dst);
@@ -205,6 +207,26 @@ int dfb_sync(dfb_handle h);
  * of an attached handle synchronises it). */
 int dfb_attach_stream(dfb_handle h, void* stream);
 int dfb_filter_dev(dfb_handle h, const double* dt_dev);
+
+/* Per-row temporal scales (opt-in).  The temporal blend of field f uses alpha = exp(-pi dt / Lt_f) with one Lt per field for the
+ * whole plane (dfb_config.scales); under Taylor's hypothesis that fixes the streamwise length at row j to U(y_j) Lt_f, a small fraction
+ * of its freestream value near the wall.  dfb_set_time_scales gives each field one Lt per row instead, e.g. Lt(y) = Ix(y) / U(y) for a
+ * prescribed streamwise length Ix(y).
+ * dfb_set_time_scales(h, Lt_rows): Lt_rows = [3][Ny] (u, v, w; Ny = dfb_dims, i.e. after the trim), every entry finite and > 0; NULL
+ * returns to the config's scalar Lt.  Takes effect from the next step; the noise, filt_old and the step counter are untouched.  Rows
+ * are global rows: every slab of a plane and every plane of a batch uses them, and slabs cut on multiples of 16 columns stay bit for
+ * bit the whole plane.  Rows equal to the scalar Lt give the scalar path's results bit for bit.  Host-driven steps compute each row's
+ * blend constants on the host with the scalar path's expressions and upload them when dt changes; attached steps (dfb_attach_stream)
+ * compute them on the device, so with rows set an attached step agrees with a host-driven one to rounding (CUDA's exp against libm's),
+ * also for a host dt.  Refused, leaving the handle as it was: an entry not finite or <= 0 (DFB_ERR_ARG, naming the field and row);
+ * an attached handle (DFB_ERR_STATE: set the rows before attaching); an outstanding dfb_filter_to_host_begin or dfb_gather_begin
+ * (DFB_ERR_STATE).  The rows are part of the restart fingerprint: a file saved with rows loads only into a handle with the same rows
+ * (set them before dfb_load_restart); without rows the fingerprint is the one a handle without this feature has.
+ * dfb_time_scales_from_lengths(h, Ix, u_min, Lt_rows): host only, fills Lt_rows[3][Ny] with Lt_f(j) = Ix_f(y_j) / max(Us_j, u_min),
+ * Ix_f(y) = Ix_inn + (Ix_out - Ix_inn) * 0.5 * (1 + tanh((y / d_i - 0.2) / 0.03)) (the blend of Iz, df.cpp:146),
+ * Ix = {inn_u, out_u, inn_v, out_v, inn_w, out_w} (metres, finite, > 0), y_j = dfb_get_table 8, Us = dfb_get_table 4, u_min > 0 (m/s). */
+int dfb_set_time_scales(dfb_handle h, const double* Lt_rows);
+int dfb_time_scales_from_lengths(dfb_handle h, const double Ix[6], double u_min, double* Lt_rows);
 /* page-lock (cudaHostRegister) / release a caller-owned host array: dfb_filter_to_host into registered arrays runs at the PCIe
  * rate; pageable arrays cost an extra staging pass inside the driver.  The C++ facade does this for its std::vectors. */
 int dfb_host_register(void* ptr, size_t bytes);
@@ -424,6 +446,9 @@ int dfb_destroy_f(dfb_handle* h);
 /* stream and dt_dev by reference: Fortran type(c_ptr) arguments (the stream as a cudaStream_t, dt_dev = the device address of dt) */
 int dfb_attach_stream_f(const dfb_handle* h, void* const* stream);
 int dfb_filter_dev_f(const dfb_handle* h, const double* const* dt_dev);
+/* Lt_rows by reference as a Fortran type(c_ptr) (c_loc of a [Ny,3] array); c_null_ptr clears the rows */
+int dfb_set_time_scales_f(const dfb_handle* h, const double* const* Lt_rows);
+int dfb_time_scales_from_lengths_f(const dfb_handle* h, const double* Ix, const double* u_min, double* Lt_rows);
 /* path: Fortran character variable (c_loc) + its len_trim, as the file names of dfb_config (path_len < 0: NUL-terminated) */
 int dfb_save_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);
 int dfb_load_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);

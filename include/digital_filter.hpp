@@ -125,6 +125,19 @@ class DIGITAL_FILTER {
     void attach_stream(struct CUstream_st* stream) { check(dfb_attach_stream(h_, stream)); }
     // one step with dt read from device memory when it runs (the handle must be attached); the host vectors are not refreshed
     void filter_dev(const double* dt_dev) { check(dfb_filter_dev(h_, dt_dev)); }
+    // per-row temporal scales (dfb_set_time_scales): Lt_rows = [3][Ny] (u, v, w rows), from the next step on; clear_time_scales
+    // returns to the config's scalar Lt.  time_scales_from_lengths converts streamwise lengths Ix = {inn_u, out_u, inn_v, out_v,
+    // inn_w, out_w}, blended across the boundary layer like Iz, with the plane's mean velocity: Lt = Ix(y) / max(U(y), u_min)
+    void set_time_scales(const std::vector<double>& Lt_rows) {
+        if (Lt_rows.size() != (size_t)3 * Ny) throw std::invalid_argument("set_time_scales: Lt_rows must hold 3 * Ny values");
+        check(dfb_set_time_scales(h_, Lt_rows.data()));
+    }
+    void clear_time_scales() { check(dfb_set_time_scales(h_, nullptr)); }
+    std::vector<double> time_scales_from_lengths(const double Ix[6], double u_min) const {
+        std::vector<double> Lt_rows((size_t)3 * Ny);
+        check(dfb_time_scales_from_lengths(h_, Ix, u_min, Lt_rows.data()));
+        return Lt_rows;
+    }
     // explicit fetch for fetch_every_step = false (also refreshes .filt)
     void fetch() {
         FilterField* F[3] = {&u, &v, &w};
