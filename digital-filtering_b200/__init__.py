@@ -25,6 +25,7 @@ LIB_PATH = os.environ.get("DFB_LIB") or os.path.join(_HERE, "lib", "libdfb200.so
 OK, ERR_ARG, ERR_IO, ERR_CUDA, ERR_STATE, ERR_INTERP = range(6)
 U_FLUC, V_FLUC, W_FLUC, T_FLUC, RHO_FLUC, U_FILT, V_FILT, W_FILT = range(8)
 NOISE_GENERATE, NOISE_INJECT = 0, 1
+FILTER_EXPONENTIAL, FILTER_GAUSSIAN = 0, 1    # filter shapes (dfb_set_filter_shape)
 CORR_Z, CORR_Y, CORR_T = 0, 1, 2        # correlation directions (dfb_corr_enable)
 DFB_CORR_SUPPORT = CORR_SUPPORT = -1    # lag = the filter's whole support (z and y)
 RESTART_STATE, RESTART_STATS, RESTART_CORR = 1, 2, 4   # sections of a restart file (dfb_save_restart)
@@ -152,6 +153,7 @@ def lib():
         L.dfb_filter_dev.argtypes = [C.c_void_p, C.c_void_p]
         L.dfb_set_time_scales.argtypes = [C.c_void_p, c_dp]
         L.dfb_time_scales_from_lengths.argtypes = [C.c_void_p, c_dp, C.c_double, c_dp]
+        L.dfb_set_filter_shape.argtypes = [C.c_void_p, C.c_int]
         _lib = L
     return _lib
 
@@ -206,6 +208,7 @@ class DFConfig:
         self.skip_first_step = 0
         self.kernel_variant = 0
         self.periodic_z = 0              # 1: spanwise-periodic plane (the z filter wraps around it; include/dfb200.h)
+        self.filter_shape = FILTER_EXPONENTIAL   # FILTER_GAUSSIAN: Klein et al.'s kernel, which delivers the configured Iz / Iy
         for k, v in kw.items():
             if not hasattr(self, k):
                 raise TypeError(f"DFConfig has no field {k!r}")
@@ -348,11 +351,22 @@ class DIGITAL_FILTER:
         self._keep = fill_config(c, config)
         self._h = C.c_void_p()
         self.nplanes = int(nplanes)
+        shaped = config.filter_shape != FILTER_EXPONENTIAL
+        if shaped:
+            c.skip_first_step = 1        # the shape is set before any step; the constructor's step follows below
         if self.nplanes == 1:
             _check(L.dfb_create(C.byref(c), C.byref(self._h)))
         else:
             _check(L.dfb_create_batch(C.byref(c), self.nplanes, C.byref(self._h)))
             fetch = False
+        if shaped:
+            try:
+                self.set_filter_shape(config.filter_shape)
+                if config.noise_mode == NOISE_GENERATE and not config.skip_first_step:
+                    self.first_step()
+            except Exception:
+                self.close()
+                raise
         ny, nz = C.c_int(), C.c_int()
         _check(L.dfb_dims(self._h, C.byref(ny), C.byref(nz)))
         self.Ny, self.Nz, self.n_cells = ny.value, nz.value, ny.value * nz.value
@@ -408,6 +422,16 @@ class DIGITAL_FILTER:
         if not dt.is_cuda or dt.dtype.itemsize != 8 or not dt.dtype.is_floating_point or dt.numel() != 1:
             raise ValueError("dt must be a 1-element CUDA float64 tensor")
         _check(lib().dfb_filter_dev(self._h, C.c_void_p(dt.data_ptr())))
+
+    # ---- filter shape (include/dfb200.h, dfb_set_filter_shape) ----
+    def set_filter_shape(self, shape):
+        """FILTER_EXPONENTIAL or FILTER_GAUSSIAN, on a handle that has not stepped (DFConfig(filter_shape=...) does this for you)"""
+        _check(lib().dfb_set_filter_shape(self._h, int(shape)))
+
+    @property
+    def filter_shape(self):
+        """FILTER_EXPONENTIAL or FILTER_GAUSSIAN (dfb_info 17)"""
+        return self.info(17)
 
     # ---- per-row temporal scales (include/dfb200.h, dfb_set_time_scales) ----
     def set_time_scales(self, rows):

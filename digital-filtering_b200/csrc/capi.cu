@@ -80,6 +80,7 @@ struct dfb_filter_s {
     cudaEvent_t ev_staged[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
     long long pipe_begun = 0, pipe_ended = 0;
     std::vector<void*> allocs;
+    std::vector<void*> sweep_allocs;  // what build_sweeps allocated: freed when dfb_set_filter_shape rebuilds the sweeps
     // Two noise buffer sets (r_ys, r_zs): step s uses set s&1, so noise(s+1) can be written while
     // y(s)/z(s) still read set s&1.  D[b] differs from D[1-b] only in the r_ys / r_zs pointers.
     PlaneDev D[2]{};
@@ -184,6 +185,7 @@ struct dfb_filter_s {
         if (stream) cudaStreamSynchronize(stream);
         facemaps.clear();
         for (void* p : allocs) cudaFree(p);
+        for (void* p : sweep_allocs) cudaFree(p);
         for (void* p : corr_mem) cudaFree(p);
         cudaFree(corr.ring);
         cudaFree(corr.part);
@@ -257,20 +259,23 @@ void encode_map(CUtensorMap& m, double* base, cuuint32_t rank, const cuuint64_t*
 
 std::optional<int> env_int(const char* name) { const char* e = std::getenv(name); return e ? std::optional<int>(std::atoi(e)) : std::nullopt; }
 
+StepPlan plan_for_device(const dfb_filter_s& H, const Plan& P) {
+    cudaDeviceProp prop;
+    CUDA_TRY(cudaGetDeviceProperties(&prop, H.device));
+    return plan_step(P, H.nplanes, DeviceLimits{prop.multiProcessorCount, prop.sharedMemPerBlockOptin},
+                     Overrides{env_int("DFB_Y_MODE"), env_int("DFB_Y_TK"), env_int("DFB_Y_COLGROUP"), env_int("DFB_ZK"), env_int("DFB_Z_MODE")});
+}
+
+void build_sweeps(dfb_filter_s& H, const StepPlan& S);
+
 // Carries out the step's plan (stepplan.cpp) on the device: allocations, uploads, tensor maps, kernel attributes, occupancy.
 void build_device(dfb_filter_s& H) {
     const Plan& P = H.plan;
     const int NP = H.nplanes, Ny = P.Ny, W = P.Nz();
-    cudaDeviceProp prop;
-    CUDA_TRY(cudaGetDeviceProperties(&prop, H.device));
-    const StepPlan S = plan_step(P, NP, DeviceLimits{prop.multiProcessorCount, prop.sharedMemPerBlockOptin},
-                                 Overrides{env_int("DFB_Y_MODE"), env_int("DFB_Y_TK"), env_int("DFB_Y_COLGROUP"), env_int("DFB_ZK"), env_int("DFB_Z_MODE")});
-    H.tuned = S.tuned;
+    const StepPlan S = plan_for_device(H, P);
     PlaneDev& D = H.D[0];
     D = S.D;
     D.rowc = H.upload(S.rowc);
-    D.coef_ptr = H.upload(P.coef.ptr);
-    D.coef_vals = H.upload(P.coef.vals);
     D.T_fluc = H.dalloc<double>((size_t)NP * Ny * W);
     D.rho_fluc = H.dalloc<double>((size_t)NP * Ny * W);
     for (int f = 0; f < 3; ++f) {
@@ -290,6 +295,33 @@ void build_device(dfb_filter_s& H) {
         H.D[1].f[f].r_ys = H.dalloc<double>(NP * D.f[f].ps_ys);
         H.D[1].f[f].r_zs = H.dalloc<double>(NP * D.f[f].ps_zs);
     }
+    build_sweeps(H, S);
+
+    H.np = S.np;
+    for (int n = 0; n < H.np.n_arrays; ++n) {
+        const NoiseTable& A = S.noise[n];
+        H.np.a[n].seg_jump = H.upload(A.jump); H.np.a[n].seg_off = H.upload(A.off); H.np.a[n].seg_np = H.upload(A.np);
+        H.nwin.seg_win[n] = A.win.empty() ? nullptr : H.upload(A.win);
+        H.npairs[n] = A.npairs;
+    }
+    H.np.slot_jump = H.upload(S.slot_jump);
+    CUDA_TRY(cudaStreamSynchronize(H.stream));
+}
+
+// What of the step's plan follows from the coefficients: their table, and the forms, work descriptions, tensor maps and grids of the
+// sweeps.  The layout, the plane's buffers and the noise tables follow from the half-widths alone (build_device).  Its allocations are
+// kept in sweep_allocs, so that dfb_set_filter_shape can build it anew.
+void build_sweeps(dfb_filter_s& H, const StepPlan& S) {
+    const Plan& P = H.plan;
+    const int NP = H.nplanes, Ny = P.Ny;
+    cudaDeviceProp prop;
+    CUDA_TRY(cudaGetDeviceProperties(&prop, H.device));
+    const size_t first_alloc = H.allocs.size();
+    H.tuned = S.tuned;
+    H.D[0].coef_ptr = H.upload(P.coef.ptr);
+    H.D[0].coef_vals = H.upload(P.coef.vals);
+    H.D[1].coef_ptr = H.D[0].coef_ptr;
+    H.D[1].coef_vals = H.D[0].coef_vals;
 
     if (H.tuned) {
         YParams& Y = H.yp[0];
@@ -344,16 +376,8 @@ void build_device(dfb_filter_s& H) {
                 encode_map(H.zmaps[b].m[f], F.r_zs, 3, zdims, zstrides, zbox, Z.zk == 16 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, " (z)");
             }
     }
-
-    H.np = S.np;
-    for (int n = 0; n < H.np.n_arrays; ++n) {
-        const NoiseTable& A = S.noise[n];
-        H.np.a[n].seg_jump = H.upload(A.jump); H.np.a[n].seg_off = H.upload(A.off); H.np.a[n].seg_np = H.upload(A.np);
-        H.nwin.seg_win[n] = A.win.empty() ? nullptr : H.upload(A.win);
-        H.npairs[n] = A.npairs;
-    }
-    H.np.slot_jump = H.upload(S.slot_jump);
-    CUDA_TRY(cudaStreamSynchronize(H.stream));
+    H.sweep_allocs.insert(H.sweep_allocs.end(), H.allocs.begin() + first_alloc, H.allocs.end());
+    H.allocs.resize(first_alloc);
 }
 
 // Host-driven step with per-row time scales: the device table of blend constants for dt, uploaded on the main stream when it holds
@@ -714,6 +738,7 @@ int dfb_info(dfb_handle h, int what, int field, int64_t* out64) {
         case 13: *out64 = h->plan.periodic ? 1 : 0; break;
         case 14: *out64 = h->corr_ready ? h->corr.L[field] : 0; break;
         case 15: *out64 = h->plan.Lt_rows.empty() ? 0 : 1; break;
+        case 17: *out64 = h->plan.filter_shape; break;
         default: return fail(DFB_ERR_ARG, "unknown info selector");
     }
     return DFB_OK;
@@ -988,6 +1013,41 @@ int dfb_set_time_scales(dfb_handle h, const double* Lt_rows) {
 int dfb_time_scales_from_lengths(dfb_handle h, const double Ix[6], double u_min, double* Lt_rows) {
     if (!h || !Ix || !Lt_rows) return fail(DFB_ERR_ARG, "handle/Ix/Lt_rows is NULL");
     return guarded([&] { time_scales_from_lengths(h->plan, Ix, u_min, Lt_rows); });
+}
+
+int dfb_set_filter_shape(dfb_handle h, int shape) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    if (shape != DFB_FILTER_EXPONENTIAL && shape != DFB_FILTER_GAUSSIAN)
+        return fail(DFB_ERR_ARG, "unknown filter shape " + std::to_string(shape) + " (DFB_FILTER_EXPONENTIAL = 0, DFB_FILTER_GAUSSIAN = 1)");
+    const char* why = nullptr;
+    if (h->attached) why = "the handle is attached to a stream (dfb_attach_stream)";
+    else if (h->step != 0) why = "the handle has stepped (create it with skip_first_step = 1, set the shape, then call dfb_first_step)";
+    else if (h->comm) why = "the handle has a communicator (dfb_comm_init)";
+    else if (h->stats_on) why = "N2 statistics are enabled (dfb_stats_enable)";
+    else if (h->corr_on) why = "correlation statistics are enabled (dfb_corr_enable)";
+    else if (!h->plan.Lt_rows.empty()) why = "per-row time scales are set (dfb_set_time_scales)";
+    else if (std::any_of(h->facemaps.begin(), h->facemaps.end(), [](const auto& m) { return m != nullptr; }))
+        why = "the handle has face maps (dfb_facemap_create)";
+    else if (h->pipe_begun != h->pipe_ended) why = "a dfb_filter_to_host_begin is outstanding";
+    if (why) return fail(DFB_ERR_STATE, std::string("dfb_set_filter_shape: ") + why);
+    return guarded([&] {
+        if (shape == h->plan.filter_shape) return;
+        Plan P = h->plan;
+        P.filter_shape = shape;
+        build_coef_table(P);
+        const StepPlan S = plan_for_device(*h, P);        // refusals (DFB_Y_MODE / DFB_Z_MODE against the shape) throw here
+        CUDA_TRY(cudaSetDevice(h->device));
+        CUDA_TRY(cudaStreamSynchronize(h->stream));
+        CUDA_TRY(cudaStreamSynchronize(h->side));
+        for (void* p : h->sweep_allocs) CUDA_TRY(cudaFree(p));
+        h->sweep_allocs.clear();
+        for (int b = 0; b < 2; ++b) { h->yp[b] = YParams{}; h->zp[b] = ZParams{}; h->maps[b] = YMaps{}; h->rmaps[b] = YRMaps{}; h->zmaps[b] = ZMaps{}; }
+        h->y_form = 0; h->n_tiles_dense = h->n_tiles_rec = 0; h->tl = nullptr;
+        h->plan = std::move(P);
+        build_sweeps(*h, S);
+        h->fingerprint = rst::fingerprint(h->plan);
+        CUDA_TRY(cudaStreamSynchronize(h->stream));
+    });
 }
 
 static int set_noise_impl(dfb_handle h, int field, const double* r_ys, const double* left, const double* right, size_t halo_pitch) {
@@ -1396,6 +1456,7 @@ int dfb_save_restart(dfb_handle h, const char* path, int what) {
         for (int f = 0; f < 3; ++f) { hd.Ny_max[f] = P.f[f].Ny_max; hd.Nz_max[f] = P.f[f].Nz_max; hd.Lt[f] = P.f[f].Lt; }
         hd.forms[0] = h->tuned ? 1 : 0; hd.forms[1] = h->tuned ? h->zp[0].zmode : 0; hd.forms[2] = h->tuned ? h->y_form : -1;   // dfb_info 3, 7, 10
         hd.fingerprint = h->fingerprint;
+        hd.filter_shape = P.filter_shape;
         hd.sections = (uint32_t)what;
         if (what & DFB_RESTART_STATS) { hd.stats_count = h->stats_count; hd.stats_on = h->stats_on ? 1 : 0; }
         if (what & DFB_RESTART_CORR) {
@@ -1442,6 +1503,11 @@ int dfb_load_restart(dfb_handle h, const char* path, int what) {
                       std::to_string(P.Ny) + " x " + std::to_string(P.NzG));
         if (hd.periodic != (P.periodic ? 1 : 0))
             throw arg("periodic_z differs: file " + std::to_string(hd.periodic) + ", handle " + std::to_string(P.periodic ? 1 : 0));
+        if (hd.filter_shape != P.filter_shape) {
+            static const char* const shape_name[2] = {"exponential", "Gaussian"};
+            throw arg(std::string("filter shape differs: file ") + shape_name[hd.filter_shape] + ", handle " + shape_name[P.filter_shape] +
+                      " (dfb_set_filter_shape)");
+        }
         if (hd.fingerprint != h->fingerprint) throw arg("the filter tables differ (half-widths, row tables or time scales)");
         if (h->noise_mode == DFB_NOISE_GENERATE && hd.seed != h->seed)
             throw arg("seed differs: file " + std::to_string(hd.seed) + ", handle " + std::to_string(h->seed));
@@ -2186,6 +2252,9 @@ int dfb_set_time_scales_f(const dfb_handle* h, const double* const* Lt_rows) {
 }
 int dfb_time_scales_from_lengths_f(const dfb_handle* h, const double* Ix, const double* u_min, double* Lt_rows) {
     return (h && u_min) ? dfb_time_scales_from_lengths(*h, Ix, *u_min, Lt_rows) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_set_filter_shape_f(const dfb_handle* h, const int* shape) {
+    return (h && shape) ? dfb_set_filter_shape(*h, *shape) : fail(DFB_ERR_ARG, "NULL argument");
 }
 int dfb_destroy_f(dfb_handle* h) {
     if (!h) return DFB_OK;

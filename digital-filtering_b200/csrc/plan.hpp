@@ -37,6 +37,7 @@ struct Plan {
     int k0 = 0, k1 = 0;                          // slab owned by this handle
     bool periodic = false;                       // dfb_config.periodic_z: the z filter wraps around the plane (Nz_max <= NzG)
     int kernel_variant = 0;                      // dfb_config.kernel_variant: != 0 forces the one-thread-per-cell kernels
+    int filter_shape = DFB_FILTER_EXPONENTIAL;   // dfb_set_filter_shape: the kernel of the spatial filters (coef)
     double d_i = 0, d_v = 0, U_e = 0, rho_e = 0, mu = 0, gcon = 287.0;
     double u_tau = 0, tau_w = 0;
     std::vector<double> yc_row, dy_row;          // first column of the geometry (ydline*d_i, df.cpp:115-116)
@@ -50,8 +51,10 @@ struct Plan {
     int Nz() const { return k1 - k0; }
 };
 
-// Builds the plan from the config; throws dfb::Error.
+// Builds the plan from the config (exponential filter shape); throws dfb::Error.
 void build_plan(const dfb_config& cfg, Plan& plan);
+// (Re)builds plan.coef for plan.filter_shape: one row per half-width that occurs in the plane.
+void build_coef_table(Plan& plan);
 
 struct DeviceLimits { int sms; size_t smem_optin; };   // multiprocessors, shared memory one block may opt in to (bytes)
 
@@ -98,7 +101,7 @@ void check_time_scales(const Plan& plan, const double* Lt_rows);
 void time_scales_from_lengths(const Plan& plan, const double Ix[6], double u_min, double* Lt_rows);
 
 // pieces, exposed for unit tests through the C ABI
-void coefficients(int N, double* b /* 2N+1 */);
+void coefficients(int N, int shape /* DFB_FILTER_* */, double* b /* 2N+1 */);
 std::vector<double> linear_interpolate(const std::vector<double>& y_data, const std::vector<double>& f_data,
                                        const std::vector<double>& y_new);
 

@@ -149,6 +149,10 @@ uint64_t fingerprint(const Plan& P) {
         H.word(P.Lt_rows.size());
         for (double v : P.Lt_rows) H.f64(v);
     }
+    if (P.filter_shape != DFB_FILTER_EXPONENTIAL) {   // hashed only when Gaussian, so an exponential handle keeps its fingerprint
+        H.word(0x67617573736961ull);             // "gaussia"
+        H.word((uint64_t)P.filter_shape);
+    }
     return H.h;
 }
 
@@ -185,6 +189,7 @@ void encode_header(const Header& h, unsigned char* out) {
     for (int m = 0; m <= MAX_LT; ++m) o.i64(h.corr_tsteps[m]);
     for (int s = 0; s < N_SECTIONS; ++s) o.i64(h.off[s]);
     o.i64(h.file_bytes);
+    o.i32(h.filter_shape);
 }
 
 Header decode_header(const unsigned char* in_) {
@@ -210,8 +215,9 @@ Header decode_header(const unsigned char* in_) {
     int64_t off[N_SECTIONS];
     for (int s = 0; s < N_SECTIONS; ++s) off[s] = in.i64();
     const int64_t bytes = in.i64();
+    h.filter_shape = in.i32();
     if (h.Ny <= 0 || h.NzG <= 0 || h.nplanes <= 0 || h.nplanes > DFB_MAXP || h.corr_L[2] < 0 || h.corr_L[2] > MAX_LT || h.n_ring < 0 ||
-        h.n_ring > h.corr_L[2] || h.corr_L[0] < 0 || h.corr_L[0] >= h.NzG || h.corr_L[1] < 0 || h.corr_L[1] >= h.Ny)
+        h.n_ring > h.corr_L[2] || h.filter_shape < 0 || h.filter_shape > DFB_FILTER_GAUSSIAN || h.corr_L[0] < 0 || h.corr_L[0] >= h.NzG || h.corr_L[1] < 0 || h.corr_L[1] >= h.Ny)
         throw io("corrupt restart header (sizes)");
     layout(h);
     if (bytes != h.file_bytes || std::memcmp(off, h.off, sizeof(off)) != 0) throw io("corrupt restart header (section offsets)");

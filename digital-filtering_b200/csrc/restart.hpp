@@ -46,6 +46,7 @@ struct Header {
     int32_t corr_on = 0, n_ring = 0;              // n_ring: fields in the ring section (min(L_t, ring_count) while accumulating, else 0)
     int64_t corr_count = 0;
     int64_t corr_tsteps[MAX_LT + 1] = {};
+    int32_t filter_shape = 0;                     // DFB_FILTER_*; stored after file_bytes, so files written before it read 0 (exponential)
     // derived by layout(): byte offset of each section (0 when absent) and the file's size
     int64_t off[N_SECTIONS] = {};
     int64_t file_bytes = 0;
@@ -58,7 +59,8 @@ struct Record {
 };
 
 // Everything that decides the numbers of the next steps besides the seed and the plane range: Ny, NzG, periodic_z, the whole-plane
-// half-width tables of each field (per row when row-uniform, per cell otherwise), Lt of each field and the [8][Ny] row tables.
+// half-width tables of each field (per row when row-uniform, per cell otherwise), Lt of each field and the [8][Ny] row tables,
+// the per-row time scales when set, and the filter shape when it is Gaussian.
 uint64_t fingerprint(const Plan& P);
 
 void layout(Header& h);                                       // fills off[] and file_bytes from the sizes and sections

@@ -84,20 +84,41 @@ std::vector<double> linear_interpolate(const std::vector<double>& xs, const std:
     return out;
 }
 
-// Filter coefficients of half-width N (df.cpp:166-177 == 202-216): a two-sided exponential exp(-2 pi |i| / N)
-// normalised to unit energy.  One side is evaluated and mirrored; the energy is accumulated from the centre
-// outwards in the reference's order (t_0^2, then 2 t_i^2) so that the table is bit-identical to its by / bz.
-void coefficients(int N, double* b) {
+// Filter coefficients of half-width N (df.cpp:166-177 == 202-216), normalised to unit energy.  DFB_FILTER_EXPONENTIAL: the
+// reference's two-sided exponential exp(-2 pi |i| / N).  DFB_FILTER_GAUSSIAN: Klein, Sadiki & Janicka's exp(-pi i^2 / (2 n^2)) with
+// n = N / 2, i.e. exp(-2 pi i^2 / N^2), whose correlation exp(-pi d^2 / (4 n^2)) has an integral scale of n cells.  One side is
+// evaluated and mirrored; the energy is accumulated from the centre outwards in the reference's order (t_0^2, then 2 t_i^2) so that
+// the exponential table is bit-identical to its by / bz.  N = 0: [1] in either shape.
+void coefficients(int N, int shape, double* b) {
+    if (N == 0) { b[0] = 1.0; return; }
     double* mid = b + N;
     double energy = 0.0;
     for (int i = 0; i <= N; ++i) {
-        const double t = std::exp(pi_c * i / N);
+        const double t = shape == DFB_FILTER_GAUSSIAN ? std::exp(pi_c * ((double)i * i) / ((double)N * N)) : std::exp(pi_c * i / N);
         mid[i] = t;
         energy += (i ? 2.0 : 1.0) * t * t;
     }
     const double norm = std::sqrt(energy);
     for (int i = 0; i <= N; ++i) mid[i] /= norm;
     for (int i = 1; i <= N; ++i) mid[-i] = mid[i];
+}
+
+void build_coef_table(Plan& P) {
+    int Nmax = 0;
+    for (int f = 0; f < 3; ++f) Nmax = std::max({Nmax, P.f[f].Ny_max, P.f[f].Nz_max});
+    std::vector<char> present(Nmax + 1, 0);
+    for (int f = 0; f < 3; ++f) {
+        const FieldPlan& F = P.f[f];
+        if (F.row_uniform) { for (int j = 0; j < P.Ny; ++j) { present[F.N_y_row[j]] = 1; present[F.N_z_row[j]] = 1; } }
+        else { for (int v : F.N_y) present[v] = 1; for (int v : F.N_z) present[v] = 1; }
+    }
+    P.coef.Nmax = Nmax;
+    P.coef.ptr.assign(Nmax + 1, -1);
+    int64_t total = 0;
+    for (int N = 0; N <= Nmax; ++N) if (present[N]) { P.coef.ptr[N] = total; total += 2 * N + 1; }
+    P.coef.vals.assign(total, 0.0);
+    for (int N = 0; N <= Nmax; ++N)
+        if (present[N]) coefficients(N, P.filter_shape, P.coef.vals.data() + P.coef.ptr[N]);   // N = 0 only through explicit N arrays
 }
 
 void build_plan(const dfb_config& cfg, Plan& P) {
@@ -338,23 +359,8 @@ void build_plan(const dfb_config& cfg, Plan& P) {
                                              " > Nz = " + std::to_string(NzG) + " (a z window may wrap around the plane at most once)"};
 
     // ---- coefficient table keyed by N ----
-    int Nmax = 0;
-    for (int f = 0; f < 3; ++f) Nmax = std::max({Nmax, P.f[f].Ny_max, P.f[f].Nz_max});
-    std::vector<char> present(Nmax + 1, 0);
-    for (int f = 0; f < 3; ++f) {
-        const FieldPlan& F = P.f[f];
-        if (F.row_uniform) { for (int j = 0; j < Ny; ++j) { present[F.N_y_row[j]] = 1; present[F.N_z_row[j]] = 1; } }
-        else { for (int v : F.N_y) present[v] = 1; for (int v : F.N_z) present[v] = 1; }
-    }
-    P.coef.Nmax = Nmax;
-    P.coef.ptr.assign(Nmax + 1, -1);
-    int64_t total = 0;
-    for (int N = 0; N <= Nmax; ++N) if (present[N]) { P.coef.ptr[N] = total; total += 2 * N + 1; }
-    P.coef.vals.resize(total);
-    for (int N = 0; N <= Nmax; ++N) if (present[N]) {
-        if (N == 0) P.coef.vals[P.coef.ptr[0]] = 1.0;   // only reachable through explicit N arrays
-        else coefficients(N, P.coef.vals.data() + P.coef.ptr[N]);
-    }
+    P.filter_shape = DFB_FILTER_EXPONENTIAL;
+    build_coef_table(P);
 
     // ---- algorithmic work of one step on the local slab (SURVEY 8d: F_alg = 2 * taps) ----
     P.taps_per_step = 0;

@@ -11,6 +11,13 @@ namespace {
 
 inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 
+// The run-recursive and chunk-recursive y forms and the recursive z form evaluate the two-sided exponential by its sliding recursion;
+// a Gaussian has none, so a Gaussian plane runs the direct forms, which read the coefficient table and nothing else.
+Error shape_refusal(const char* what) {
+    return Error{DFB_ERR_ARG, std::string(what) + " evaluates the exponential filter recursively: the filter shape is Gaussian "
+                                                  "(DFB_FILTER_GAUSSIAN), which runs the direct forms only"};
+}
+
 // ratio of neighbouring coefficients, b_i = a^|i| / s (df.cpp:168-177)
 inline long double exp_ratio(int N) { return (long double)std::exp(-2.0 * 3.14159265358979323846 * 1.0 / N); }
 
@@ -32,7 +39,10 @@ void plan_y(const Plan& P, int NP, const DeviceLimits& dev, const Overrides& ovr
     // its window has to be staged whole).  Decided per block of 32 rows: run form where it executes less than half of the
     // direct sum's multiply-adds (and two of the block's windows fit in shared memory); the other rows keep the band matrices.
     // DFB_Y_MODE=2 forces the run form wherever a window fits at all, 0 / 1 force the band-matrix kernels (dense / chunk-recursive).
-    const int ymode_env = ovr.y_mode.value_or(-1);
+    // a Gaussian plane: dense band matrices on every block (as DFB_Y_MODE=0)
+    if (P.filter_shape == DFB_FILTER_GAUSSIAN && (ovr.y_mode == 1 || ovr.y_mode == 2))
+        throw shape_refusal(ovr.y_mode == 1 ? "DFB_Y_MODE=1 (chunk-recursive y-sweep)" : "DFB_Y_MODE=2 (run-recursive y-sweep)");
+    const int ymode_env = P.filter_shape == DFB_FILTER_GAUSSIAN ? 0 : ovr.y_mode.value_or(-1);
     std::vector<char> run_row[3];
     std::vector<YRGroup>& rg = S.rgroups;
     std::vector<YRTile>& rt = S.rtiles;
@@ -417,7 +427,7 @@ bool plan_z(const Plan& P, const DeviceLimits& dev, const Overrides& ovr, StepPl
         double* B = pvals.data() + pptr[N];
         const double* b = P.coef.vals.data() + P.coef.ptr[N];
         for (int t = 0; t <= 2 * N; ++t) B[t + ZKc + zp.d] = b[t];
-        if (N >= 1) {
+        if (N >= 1 && P.filter_shape == DFB_FILTER_EXPONENTIAL) {
             // b_i = a^|i| / s with a = exp(-2 pi / N) (df.cpp:168-177): the header carries what the recursive
             // evaluation needs: a, a^(N+1), 1/s, N, d.  a is the reference's own i = 1 weight: b_1 / b_0.
             double* hdr = B + zp.clen - 16;
@@ -436,9 +446,10 @@ bool plan_z(const Plan& P, const DeviceLimits& dev, const Overrides& ovr, StepPl
     Z.box_bytes = maxlines * ZKc * 8;
     // Recursive evaluation of the truncated two-sided exponential (see the kernel) unless the slab starts or ends off a
     // 16-column boundary of the plane (its lane blocks would differ from the whole plane's: results would agree to
-    // ~1e-14 but not bit for bit) or a row has N = 0.  DFB_Z_MODE=0 forces the direct Toeplitz form.
+    // ~1e-14 but not bit for bit), a row has N = 0, or the filter shape is Gaussian.  DFB_Z_MODE=0 forces the direct Toeplitz form.
     {
-        bool rec = (P.k0 % 16) == 0 && (P.k1 % 16 == 0 || P.k1 == P.NzG);
+        if (P.filter_shape == DFB_FILTER_GAUSSIAN && ovr.z_mode == 1) throw shape_refusal("DFB_Z_MODE=1 (recursive z-sweep)");
+        bool rec = P.filter_shape == DFB_FILTER_EXPONENTIAL && (P.k0 % 16) == 0 && (P.k1 % 16 == 0 || P.k1 == P.NzG);
         for (int f = 0; f < 3; ++f) for (int v : P.f[f].N_z_row) rec = rec && v >= 1;
         Z.zmode = ovr.z_mode ? *ovr.z_mode : (rec ? 1 : 0);
         if (Z.zmode == 1 && !rec) throw Error{DFB_ERR_ARG, "DFB_Z_MODE=1 needs slab boundaries on multiples of 16 columns and N_z >= 1"};

@@ -25,6 +25,8 @@
 !                                                 capturable into its CUDA graph (include/dfb200.h, dfb_attach_stream)
 !   set_time_scales, clear_time_scales,           per-row temporal scales Lt(y) for the temporal blend, e.g. from a prescribed
 !   time_scales_from_lengths                        streamwise length: Lt = Ix(y) / U(y) (include/dfb200.h, dfb_set_time_scales)
+!   config%filter_shape = FILTER_GAUSSIAN,        Klein et al.'s Gaussian filter kernel, which delivers the configured integral
+!   set_filter_shape                                scales Iz / Iy (include/dfb200.h, dfb_set_filter_shape)
 !
 ! NOTE: NEVER COMPILED -- no Fortran compiler exists in the build image or on the GPU boxes.  The binding is exercised through
 ! tests/fortran_abi_mimic.c, a C program that makes exactly these calls with exactly this struct layout and by-reference
@@ -41,8 +43,10 @@ module DIGITAL_FILTERING
     public :: facemap_create, interp_to_host, interp_to_cells, facemap_destroy, MAP_POINT, MAP_AREA, MAP_WALL_ZERO, filter_on_device
     public :: attach_stream, filter_dev
     public :: set_time_scales, clear_time_scales, time_scales_from_lengths
+    public :: set_filter_shape, FILTER_EXPONENTIAL, FILTER_GAUSSIAN
 
     integer, parameter :: RESTART_STATE = 1, RESTART_STATS = 2, RESTART_CORR = 4   ! DFB_RESTART_* (what to save / load; added together)
+    integer, parameter :: FILTER_EXPONENTIAL = 0, FILTER_GAUSSIAN = 1                ! DFB_FILTER_* (DFConfig%filter_shape)
 
     integer, parameter :: dp = selected_real_kind(15)
 
@@ -62,6 +66,7 @@ module DIGITAL_FILTERING
         integer :: device = -1, plane_id = 0
         integer :: k_begin = 0, k_end = 0             ! this rank's spanwise slab [k_begin, k_end) (0-based, C convention); 0,0 = the whole plane
         integer :: periodic_z = 0                     ! 1: spanwise-periodic plane (the z filter wraps around it; needs Nz_max <= Nz)
+        integer :: filter_shape = 0                   ! FILTER_EXPONENTIAL (the reference's) or FILTER_GAUSSIAN
     end type DFConfig
 
     type :: digital_filter_type
@@ -263,6 +268,15 @@ module DIGITAL_FILTERING
             import :: c_int, c_ptr
             type(c_ptr), intent(in) :: handle, Lt_rows
         end function
+        integer(c_int) function dfb_set_filter_shape_f(handle, shape) bind(C, name='dfb_set_filter_shape_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle
+            integer(c_int), intent(in) :: shape
+        end function
+        integer(c_int) function dfb_first_step(handle) bind(C, name='dfb_first_step')
+            import :: c_int, c_ptr
+            type(c_ptr), value :: handle
+        end function
         integer(c_int) function dfb_time_scales_from_lengths_f(handle, Ix, u_min, Lt_rows) bind(C, name='dfb_time_scales_from_lengths_f')
             import :: c_int, c_ptr, c_double
             type(c_ptr), intent(in) :: handle
@@ -306,7 +320,19 @@ contains
         c%seed = config%seed; c%device = config%device; c%plane_id = config%plane_id
         c%k_begin = config%k_begin; c%k_end = config%k_end
         c%periodic_z = config%periodic_z
+        if (config%filter_shape /= FILTER_EXPONENTIAL) c%skip_first_step = 1   ! shaped_start sets the shape, then takes the first step
     end subroutine fill_config
+
+    ! a handle of another filter shape is created without its first step: set the shape, then take the constructor's step
+    subroutine shaped_start(config, handle)
+        type(DFConfig), intent(in) :: config
+        type(c_ptr), intent(in) :: handle
+        integer(c_int) :: shape
+        if (config%filter_shape == FILTER_EXPONENTIAL) return
+        shape = config%filter_shape
+        call check(dfb_set_filter_shape_f(handle, shape), 'dfb_set_filter_shape')
+        call check(dfb_first_step(handle), 'dfb_first_step')
+    end subroutine shaped_start
 
     ! page-lock an array the library copies into every step (failure only costs speed)
     ! page-lock an array the library copies into every step (a failure only costs speed)
@@ -326,6 +352,7 @@ contains
 
         call fill_config(config, c)
         call check(dfb_create_f(c, DF%handle), 'create_digital_filter')
+        call shaped_start(config, DF%handle)
         call check(dfb_dims_f(DF%handle, Ny, Nz), 'dfb_dims')
         DF%Ny = Ny; DF%Nz = Nz; DF%n_cells = Ny * Nz
         allocate(DF%u%fluc(DF%n_cells), DF%v%fluc(DF%n_cells), DF%w%fluc(DF%n_cells))
@@ -358,6 +385,7 @@ contains
         call fill_config(config, c)
         np = nplanes
         call check(dfb_create_batch_f(c, np, B%handle), 'create_digital_filter_batch')
+        call shaped_start(config, B%handle)
         call check(dfb_dims_f(B%handle, Ny, Nz), 'dfb_dims')
         B%Ny = Ny; B%Nz = Nz; B%n_cells = Ny * Nz; B%nplanes = nplanes
         allocate(B%u(B%n_cells, nplanes), B%v(B%n_cells, nplanes), B%w(B%n_cells, nplanes), B%T(B%n_cells, nplanes), B%rho(B%n_cells, nplanes))
@@ -459,6 +487,15 @@ contains
         real(c_double), intent(in), target, contiguous :: Lt_rows(:, :)
         call check(dfb_set_time_scales_f(DF%handle, c_loc(Lt_rows)), 'set_time_scales')
     end subroutine set_time_scales
+
+    ! FILTER_EXPONENTIAL or FILTER_GAUSSIAN on a handle that has not stepped (config%filter_shape does this in create_digital_filter)
+    subroutine set_filter_shape(DF, shape)
+        type(digital_filter_type), intent(in) :: DF
+        integer, intent(in) :: shape
+        integer(c_int) :: s
+        s = shape
+        call check(dfb_set_filter_shape_f(DF%handle, s), 'set_filter_shape')
+    end subroutine set_filter_shape
 
     ! back to the scalar Lt of the configuration
     subroutine clear_time_scales(DF)

@@ -117,7 +117,8 @@ int dfb_num_planes(dfb_handle h, int* nplanes);
 int dfb_dims(dfb_handle h, int* Ny, int* Nz);
 /* what = 0 Ny_max, 1 Nz_max (per field f), 2 step counter, 3 row-uniform fast path in use (0/1): 0 for per-cell half-widths,
  *    kernel_variant = 1, or a z window too wide for shared memory -- on a B200 (232 448 bytes per block) the tuned z-sweep takes
- *    N_z <= 1120 in its recursive form and N_z <= 544 in its direct form (a row with N_z = 0, a slab cut off a 16-column boundary)
+ *    N_z <= 1120 in its recursive form and N_z <= 544 in its direct form (a row with N_z = 0, a slab cut off a 16-column boundary,
+ *    the Gaussian filter shape)
  *    with 16 outputs per lane (planes of >= 384 columns), N_z <= 888 / 720 with 8; a wider window runs the whole handle on the
  *    one-thread-per-cell kernels, which take any half-width (DFB_ZK / DFB_Z_MODE forcing a window that does not fit: DFB_ERR_ARG),
  *    while any N_y runs on the tuned y-sweep (rows too tall for the run-recursive form go to its band-matrix kernels),
@@ -129,10 +130,11 @@ int dfb_dims(dfb_handle h, int* Ny, int* Nz);
  *    kernel, 0 = dense band matrices (DFB_Y_MODE=0|1|2 forces a form), 11 tiles of the run-recursive kernel, 12 transport of the config-4 hand-off: 2 = peer-to-peer copies (CUDA IPC + copy engines), 1 = NCCL
  *    send/recv, 0 = no communicator, 13 spanwise-periodic plane (dfb_config.periodic_z) in use (0/1),
  * 14 lags of correlation direction `field` (0 z, 1 y, 2 t; dfb_corr_enable), 0 when that direction is off or before any enable,
- * 15 per-row time scales in use (dfb_set_time_scales, 0/1) */
+ * 15 per-row time scales in use (dfb_set_time_scales, 0/1), 17 filter shape (dfb_set_filter_shape: DFB_FILTER_EXPONENTIAL /
+ *    DFB_FILTER_GAUSSIAN) */
 int dfb_info(dfb_handle h, int what, int field, int64_t* out64);
 /* host copies of the setup tables (for parity tests): which = 0..7 rows R11,R21,R22,R33,Us,Ts,rhos,Ms [Ny];
- * 8 yc row [Ny]; 9 dy row [Ny]; 10 Lt[3]; 11 coefficients of half-width `arg` [2*arg+1];
+ * 8 yc row [Ny]; 9 dy row [Ny]; 10 Lt[3]; 11 coefficients of half-width `arg` [2*arg+1], in the handle's filter shape;
  * 12 y of the vertex rows [Ny+1]; 13 z of the vertex columns [Nz_global+1] (df.cpp:99-100: the y / z the writers print);
  * 14 time scales Lt of field `arg` (0..2) per row in use [Ny]: the rows of dfb_set_time_scales, or the scalar Lt repeated */
 int dfb_get_table(dfb_handle h, int which, int arg, double* dst, int cap);
@@ -227,6 +229,26 @@ int dfb_filter_dev(dfb_handle h, const double* dt_dev);
  * Ix = {inn_u, out_u, inn_v, out_v, inn_w, out_w} (metres, finite, > 0), y_j = dfb_get_table 8, Us = dfb_get_table 4, u_min > 0 (m/s). */
 int dfb_set_time_scales(dfb_handle h, const double* Lt_rows);
 int dfb_time_scales_from_lengths(dfb_handle h, const double Ix[6], double u_min, double* Lt_rows);
+/* Filter shape (opt-in).  The spatial filters of every handle start as the reference's two-sided exponential (Xie & Castro),
+ * b_i = exp(-2 pi |i| / N) / s: its correlation falls off as exp(-pi d / n) times a polynomial, and the integral scale it delivers is
+ * about 0.64 of the configured Iz / Iy (N = 2 int(I / delta) = 2n).  DFB_FILTER_GAUSSIAN is the kernel of Klein, Sadiki & Janicka
+ * (2003), b_i = exp(-2 pi i^2 / N^2) / s = exp(-pi i^2 / (2 n^2)) / s, whose correlation exp(-pi d^2 / (4 n^2)) has an integral scale of
+ * n cells: the configured length to within one cell.  Both are normalised to sum b_i^2 = 1 over the same half-widths N (computed or
+ * given in N_y / N_z); N = 0 is [1] in either shape.  The temporal blend is the exponential one in both: the temporal scale stays
+ * 2 Lt / pi.
+ * dfb_set_filter_shape(h, shape) sets the shape of a handle that has not stepped yet: in generate mode one created with
+ * skip_first_step = 1 (call dfb_first_step afterwards for the constructor's step), in inject mode one whose step counter is still 0.  It
+ * rebuilds the coefficient table and the step's whole plan (kernel forms, band matrices, z pads, tensor maps, grid sizes) and the
+ * restart fingerprint; the noise, filt_old and the step counter are untouched.  A Gaussian has no exact sliding recursion, so a Gaussian
+ * handle runs the direct forms: dense band matrices in y (dfb_info 10 = 0) and the direct z-sweep (dfb_info 7 = 0); a z window too
+ * wide for the direct form runs the handle on the one-thread-per-cell kernels (dfb_info 3 = 0); DFB_Y_MODE=1|2 and DFB_Z_MODE=1 are
+ * DFB_ERR_ARG.  Refused, leaving the handle as it was: an unknown shape (DFB_ERR_ARG); DFB_ERR_STATE, naming the reason, for a handle
+ * that has stepped, is attached, has a communicator, has N2 or correlation statistics enabled, has per-row time scales or face maps,
+ * or has a dfb_filter_to_host_begin outstanding.  The shape is part of the restart fingerprint when it is Gaussian (exponential
+ * fingerprints are the ones handles without this call have) and is recorded in the file's header: a file written under the other
+ * shape is DFB_ERR_ARG, naming both.  dfb_info 17 returns the shape. */
+enum { DFB_FILTER_EXPONENTIAL = 0, DFB_FILTER_GAUSSIAN = 1 };
+int dfb_set_filter_shape(dfb_handle h, int shape);
 /* page-lock (cudaHostRegister) / release a caller-owned host array: dfb_filter_to_host into registered arrays runs at the PCIe
  * rate; pageable arrays cost an extra staging pass inside the driver.  The C++ facade does this for its std::vectors. */
 int dfb_host_register(void* ptr, size_t bytes);
@@ -449,6 +471,7 @@ int dfb_filter_dev_f(const dfb_handle* h, const double* const* dt_dev);
 /* Lt_rows by reference as a Fortran type(c_ptr) (c_loc of a [Ny,3] array); c_null_ptr clears the rows */
 int dfb_set_time_scales_f(const dfb_handle* h, const double* const* Lt_rows);
 int dfb_time_scales_from_lengths_f(const dfb_handle* h, const double* Ix, const double* u_min, double* Lt_rows);
+int dfb_set_filter_shape_f(const dfb_handle* h, const int* shape);
 /* path: Fortran character variable (c_loc) + its len_trim, as the file names of dfb_config (path_len < 0: NUL-terminated) */
 int dfb_save_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);
 int dfb_load_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);

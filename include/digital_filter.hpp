@@ -59,6 +59,7 @@ struct DFConfigEx {
     int noise_mode = DFB_NOISE_GENERATE;
     int device = -1, plane_id = 0, k_begin = 0, k_end = 0;
     bool periodic_z = false;           // spanwise-periodic plane: the z filter wraps around it (LES/DNS inflow with periodic span)
+    int filter_shape = DFB_FILTER_EXPONENTIAL;   // DFB_FILTER_GAUSSIAN: Klein et al.'s kernel, which delivers the configured Iz / Iy
     bool fetch_every_step = true;      // copy u', v', w', T', rho' into the host vectors after each filter()
 };
 
@@ -137,6 +138,12 @@ class DIGITAL_FILTER {
         std::vector<double> Lt_rows((size_t)3 * Ny);
         check(dfb_time_scales_from_lengths(h_, Ix, u_min, Lt_rows.data()));
         return Lt_rows;
+    }
+    // DFB_FILTER_EXPONENTIAL or DFB_FILTER_GAUSSIAN (DFConfigEx::filter_shape; dfb_info 17)
+    int filter_shape() const {
+        std::int64_t v = 0;
+        check(dfb_info(h_, 17, 0, &v));
+        return (int)v;
     }
     // explicit fetch for fetch_every_step = false (also refreshes .filt)
     void fetch() {
@@ -247,7 +254,18 @@ class DIGITAL_FILTER {
         k.seed = c.seed; k.noise_mode = c.noise_mode; k.device = c.device; k.plane_id = c.plane_id;
         k.k_begin = c.k_begin; k.k_end = c.k_end; k.periodic_z = c.periodic_z ? 1 : 0;
         fetch_ = c.fetch_every_step;
+        const bool shaped = c.filter_shape != DFB_FILTER_EXPONENTIAL;
+        if (shaped) k.skip_first_step = 1;   // the shape is set before any step; the constructor's step follows
         check(dfb_create(&k, &h_));
+        if (shaped) {
+            if (dfb_set_filter_shape(h_, c.filter_shape) != DFB_OK ||
+                (c.noise_mode == DFB_NOISE_GENERATE && dfb_first_step(h_) != DFB_OK)) {
+                const std::string msg = std::string("DIGITAL_FILTER: ") + dfb_last_error();
+                dfb_destroy(h_);
+                h_ = nullptr;
+                throw std::runtime_error(msg);
+            }
+        }
         check(dfb_dims(h_, &Ny, &Nz));
         n_cells = Ny * Nz;
         rho_fluc_.assign(n_cells, 0.0); T_fluc_.assign(n_cells, 0.0);
