@@ -26,6 +26,7 @@ OK, ERR_ARG, ERR_IO, ERR_CUDA, ERR_STATE, ERR_INTERP = range(6)
 U_FLUC, V_FLUC, W_FLUC, T_FLUC, RHO_FLUC, U_FILT, V_FILT, W_FILT = range(8)
 NOISE_GENERATE, NOISE_INJECT = 0, 1
 FILTER_EXPONENTIAL, FILTER_GAUSSIAN = 0, 1    # filter shapes (dfb_set_filter_shape)
+FLUX_OFF, FLUX_MASS, FLUX_VOLUME = 0, 1, 2    # inflow flux correction modes (dfb_set_flux_correction)
 CORR_Z, CORR_Y, CORR_T = 0, 1, 2        # correlation directions (dfb_corr_enable)
 DFB_CORR_SUPPORT = CORR_SUPPORT = -1    # lag = the filter's whole support (z and y)
 RESTART_STATE, RESTART_STATS, RESTART_CORR = 1, 2, 4   # sections of a restart file (dfb_save_restart)
@@ -154,6 +155,8 @@ def lib():
         L.dfb_set_time_scales.argtypes = [C.c_void_p, c_dp]
         L.dfb_time_scales_from_lengths.argtypes = [C.c_void_p, c_dp, C.c_double, c_dp]
         L.dfb_set_filter_shape.argtypes = [C.c_void_p, C.c_int]
+        L.dfb_set_flux_correction.argtypes = [C.c_void_p, C.c_int]
+        L.dfb_flux_info.argtypes = [C.c_void_p, C.c_int, c_dp]
         _lib = L
     return _lib
 
@@ -432,6 +435,24 @@ class DIGITAL_FILTER:
     def filter_shape(self):
         """FILTER_EXPONENTIAL or FILTER_GAUSSIAN (dfb_info 17)"""
         return self.info(17)
+
+    # ---- inflow mass-flux correction (include/dfb200.h, dfb_set_flux_correction) ----
+    def set_flux_correction(self, mode):
+        """FLUX_OFF, FLUX_MASS or FLUX_VOLUME from the next step on: each step's plane-integrated first-order mass (or volume) flux of
+        u' (and T', rho') is held at its mean; filt_old, v' and w' are untouched.  Whole planes and batches only (DfbError otherwise)."""
+        _check(lib().dfb_set_flux_correction(self._h, int(mode)))
+
+    @property
+    def flux_correction(self):
+        """FLUX_OFF, FLUX_MASS or FLUX_VOLUME (dfb_info 18)"""
+        return self.info(18)
+
+    def flux_info(self, plane=0):
+        """(c, m', mean flux) of the last corrected step of `plane`: the subtracted multiple of sqrt(R11), the plane's first-order flux
+        fluctuation before the correction, and sum A rhos Us (mass) or sum A Us (volume)"""
+        out = np.zeros(3)
+        _check(lib().dfb_flux_info(self._h, int(plane), _dptr(out)))
+        return float(out[0]), float(out[1]), float(out[2])
 
     # ---- per-row temporal scales (include/dfb200.h, dfb_set_time_scales) ----
     def set_time_scales(self, rows):

@@ -158,6 +158,11 @@ struct dfb_filter_s {
     cudaEvent_t ev_rows[ROWS_SLOTS] = {};
     int rows_next = 0;
     double rows_dt = std::numeric_limits<double>::quiet_NaN();   // dt of rows_tab (NaN: none)
+    // inflow mass-flux correction (dfb_set_flux_correction): the mode, the host tables of the mode last enabled (mode 0: never
+    // enabled) and the device buffers, allocated by the first enable
+    int flux_mode = DFB_FLUX_OFF;
+    FluxTables flux_tab;
+    FluxParams fx{};
     // timing
     bool timing = false;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -414,6 +419,7 @@ void launch_noise_for(dfb_filter_s& H, int64_t step, int b, cudaStream_t st) {
 void run_step_attached(dfb_filter_s& H, double dt, const double* dt_dev, bool first) {
     CUDA_TRY(cudaSetDevice(H.device));
     const bool accumulate = H.stats_on && !first;
+    const bool flux = H.flux_mode != DFB_FLUX_OFF && !first;      // the sums of N2 then describe the corrected fields: stats_kernel after it
     AdvanceParams A = H.adv;
     A.dt_dev = dt_dev;
     A.dt = dt;
@@ -443,13 +449,14 @@ void run_step_attached(dfb_filter_s& H, double dt, const double* dt_dev, bool fi
         Z.rec = H.rec;
         Z.rows = rows;
         Z.tl = nullptr;
-        Z.stats = accumulate ? H.stats : nullptr;
+        Z.stats = (accumulate && !flux) ? H.stats : nullptr;
         CUDA_TRY(launch_zsweep_tuned(H.zmaps[0], Z, H.stream));
     } else {
         CUDA_TRY(launch_ysweep_simple(H.D[0], H.stream));
         CUDA_TRY(launch_zsweep_simple(H.D[0], S, H.rec, rows, H.stream));
-        if (accumulate) CUDA_TRY(launch_stats(H.D[0], H.stats, H.rec, H.stream));
     }
+    if (flux) CUDA_TRY(launch_flux(H.fx, H.rec, H.stream));
+    if (accumulate && (!H.tuned || flux)) CUDA_TRY(launch_stats(H.D[0], H.stats, H.rec, H.stream));
 }
 
 void run_step(dfb_filter_s& H, double dt, bool first) {
@@ -483,15 +490,17 @@ void run_step(dfb_filter_s& H, double dt, bool first) {
     S.first_step = first ? 1 : 0;
     for (int f = 0; f < 3; ++f) blend_consts(dt, H.plan.f[f].Lt, S.sa[f], S.sb[f]);
     const bool accumulate = H.stats_on && !first;                  // rms_add, df.cpp:606
+    const bool flux = H.flux_mode != DFB_FLUX_OFF && !first;      // the constructor's step is never corrected
     if (H.tuned) {
         H.zp[b].S = S;
         H.zp[b].rows = rows;
-        H.zp[b].stats = accumulate ? H.stats : nullptr;            // N2 fused into the epilogue
+        H.zp[b].stats = (accumulate && !flux) ? H.stats : nullptr; // N2 fused into the epilogue, unless the correction changes u', T', rho' after it
         CUDA_TRY(launch_zsweep_tuned(H.zmaps[b], H.zp[b], H.stream));
     } else {
         CUDA_TRY(launch_zsweep_simple(H.D[b], S, nullptr, rows, H.stream));
-        if (accumulate) CUDA_TRY(launch_stats(H.D[0], H.stats, nullptr, H.stream));
     }
+    if (flux) CUDA_TRY(launch_flux(H.fx, nullptr, H.stream));
+    if (accumulate && (!H.tuned || flux)) CUDA_TRY(launch_stats(H.D[0], H.stats, nullptr, H.stream));
     if (accumulate) H.stats_count += 1;
     if (H.corr_on && !first) {
         CorrParams& c = H.corr;
@@ -739,6 +748,7 @@ int dfb_info(dfb_handle h, int what, int field, int64_t* out64) {
         case 14: *out64 = h->corr_ready ? h->corr.L[field] : 0; break;
         case 15: *out64 = h->plan.Lt_rows.empty() ? 0 : 1; break;
         case 17: *out64 = h->plan.filter_shape; break;
+        case 18: *out64 = h->flux_mode; break;
         default: return fail(DFB_ERR_ARG, "unknown info selector");
     }
     return DFB_OK;
@@ -1047,6 +1057,54 @@ int dfb_set_filter_shape(dfb_handle h, int shape) {
         build_sweeps(*h, S);
         h->fingerprint = rst::fingerprint(h->plan);
         CUDA_TRY(cudaStreamSynchronize(h->stream));
+    });
+}
+
+int dfb_set_flux_correction(dfb_handle h, int mode) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    if (mode != DFB_FLUX_OFF && mode != DFB_FLUX_MASS && mode != DFB_FLUX_VOLUME)
+        return fail(DFB_ERR_ARG, "unknown flux correction mode " + std::to_string(mode) + " (DFB_FLUX_OFF = 0, DFB_FLUX_MASS = 1, DFB_FLUX_VOLUME = 2)");
+    if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_set_flux_correction") + ": set the mode before attaching");
+    if (h->pipe_begun != h->pipe_ended || h->g_begun != h->g_ended)
+        return fail(DFB_ERR_STATE, "dfb_set_flux_correction: a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first");
+    if (mode == DFB_FLUX_OFF) { h->flux_mode = DFB_FLUX_OFF; return DFB_OK; }
+    return guarded([&] {
+        FluxTables T = flux_tables(h->plan, mode);          // refusals (slab, R11 = 0 everywhere) throw before anything changes
+        CUDA_TRY(cudaSetDevice(h->device));
+        FluxParams& F = h->fx;
+        const int NP = h->nplanes, Ny = h->plan.Ny, W = h->plan.NzG;
+        if (!F.out) {
+            CUDA_TRY(flux_prepare());
+            F.u = h->D[0].f[0].fluc; F.T = h->D[0].T_fluc; F.rho = h->D[0].rho_fluc; F.rowc = h->D[0].rowc;
+            F.Ny = Ny; F.W = W; F.P = NP; F.ps_cells = h->D[0].ps_cells;
+            F.wy = h->dalloc<double>(Ny, false);
+            F.hz = h->upload(T.hz);
+            F.part = h->dalloc<double>((size_t)NP * Ny, false);
+            F.counter = h->dalloc<unsigned>(NP);
+            F.out = h->dalloc<double2>(NP);
+        }
+        if (h->flux_tab.mode != mode) {
+            // steps enqueued before read the previous table on this stream
+            CUDA_TRY(cudaMemcpyAsync(const_cast<double*>(F.wy), T.wy.data(), Ny * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+            CUDA_TRY(cudaStreamSynchronize(h->stream));
+        }
+        F.D = T.D;
+        h->flux_tab = std::move(T);
+        h->flux_mode = mode;
+    });
+}
+
+int dfb_flux_info(dfb_handle h, int plane, double out[3]) {
+    if (!h || !out) return fail(DFB_ERR_ARG, "handle/out is NULL");
+    if (plane < 0 || plane >= h->nplanes) return fail(DFB_ERR_ARG, "plane out of range");
+    if (!h->fx.out) return fail(DFB_ERR_STATE, "the flux correction was never enabled (dfb_set_flux_correction)");
+    return guarded([&] {
+        sync_record(*h);
+        CUDA_TRY(cudaSetDevice(h->device));
+        double2 r;
+        CUDA_TRY(cudaMemcpyAsync(&r, h->fx.out + plane, sizeof(r), cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(cudaStreamSynchronize(h->stream));
+        out[0] = r.x; out[1] = r.y; out[2] = h->flux_tab.mean;
     });
 }
 
@@ -2255,6 +2313,12 @@ int dfb_time_scales_from_lengths_f(const dfb_handle* h, const double* Ix, const 
 }
 int dfb_set_filter_shape_f(const dfb_handle* h, const int* shape) {
     return (h && shape) ? dfb_set_filter_shape(*h, *shape) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_set_flux_correction_f(const dfb_handle* h, const int* mode) {
+    return (h && mode) ? dfb_set_flux_correction(*h, *mode) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_flux_info_f(const dfb_handle* h, const int* plane, double* out) {
+    return (h && plane) ? dfb_flux_info(*h, *plane, out) : fail(DFB_ERR_ARG, "NULL argument");
 }
 int dfb_destroy_f(dfb_handle* h) {
     if (!h) return DFB_OK;

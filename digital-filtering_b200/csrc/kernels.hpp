@@ -41,6 +41,24 @@ cudaError_t launch_rebuild(double* plane, const double* rowc, int Ny, int NzG, i
 cudaError_t launch_assemble(const double* slab, double* plane, const double* rowc, int Ny, int NzG, int k0, int W, int first_only, cudaStream_t st);
 cudaError_t launch_dfma_peak(double* out, int blocks, int iters, cudaStream_t st);
 
+// inflow mass-flux correction (flux.cu, dfb_set_flux_correction): u', T', rho' dense [P][Ny][W] (whole planes, W = Nz)
+struct FluxParams {
+    double* u;
+    double* T;
+    double* rho;
+    const double* rowc;               // [Ny][ROWC]: rc0 = sqrt(R11), rc4, Ts, rhos of the epilogue
+    const double* wy;                 // [Ny] g_j hy_j
+    const double* hz;                 // [W]
+    double* part;                     // [P][Ny] row partials
+    unsigned* counter;                // [P] tickets of the row CTAs; 0 between launches
+    double2* out;                     // [P] {c, m'} of the last corrected step
+    double D;
+    int Ny, W, P;
+    size_t ps_cells;
+};
+cudaError_t flux_prepare();
+cudaError_t launch_flux(const FluxParams& F, const StepRecord* rec, cudaStream_t st);   // a void attached step (rec) changes nothing
+
 // correlation statistics (corr.cu, dfb_corr_enable): sums [P][3][Ny][L_d + 1] per direction d = 0 z, 1 y, 2 t
 struct CorrParams {
     const double* fluc[3];            // u', v', w': dense [P][Ny][W] (W = Nz: whole planes only)

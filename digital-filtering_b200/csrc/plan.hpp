@@ -100,6 +100,18 @@ void check_time_scales(const Plan& plan, const double* Lt_rows);
 // dfb_time_scales_from_lengths: Lt_f(j) = Ix_f(y_j) / max(Us_j, u_min), Ix_f blended from Ix[2f] to Ix[2f+1] like Iz.  Throws dfb::Error.
 void time_scales_from_lengths(const Plan& plan, const double Ix[6], double u_min, double* Lt_rows);
 
+// Inflow mass-flux correction (dfb_set_flux_correction, fluxtables.cpp): per plane and step c = m' / D with m' = sum_j wy_j sum_k hz_k u'_jk,
+// and u' <- u' - c rc0_j.  wy_j = g_j hy_j, g_j = rhos_j (1 + 0.2 Ms_j^2) (DFB_FLUX_MASS) or 1 (DFB_FLUX_VOLUME); rc0_j = sqrt(R11_j);
+// D = sum_jk hy_j hz_k g_j rc0_j; mean = sum_jk hy_j hz_k rhos_j Us_j (mass) or hy_j hz_k Us_j (volume).
+struct FluxTables {
+    int mode = 0;
+    std::vector<double> wy, rc0;                 // [Ny]
+    std::vector<double> hz;                      // [NzG]
+    double D = 0, mean = 0;
+};
+// Throws DFB_ERR_ARG for a mode other than DFB_FLUX_MASS / DFB_FLUX_VOLUME, a slab plan, or D = 0.
+FluxTables flux_tables(const Plan& plan, int mode);
+
 // pieces, exposed for unit tests through the C ABI
 void coefficients(int N, int shape /* DFB_FILTER_* */, double* b /* 2N+1 */);
 std::vector<double> linear_interpolate(const std::vector<double>& y_data, const std::vector<double>& f_data,

@@ -27,6 +27,8 @@
 !   time_scales_from_lengths                        streamwise length: Lt = Ix(y) / U(y) (include/dfb200.h, dfb_set_time_scales)
 !   config%filter_shape = FILTER_GAUSSIAN,        Klein et al.'s Gaussian filter kernel, which delivers the configured integral
 !   set_filter_shape                                scales Iz / Iy (include/dfb200.h, dfb_set_filter_shape)
+!   set_flux_correction, flux_info                each step's plane-integrated mass (or volume) flux of the inflow held at its mean
+!                                                   (include/dfb200.h, dfb_set_flux_correction)
 !
 ! NOTE: NEVER COMPILED -- no Fortran compiler exists in the build image or on the GPU boxes.  The binding is exercised through
 ! tests/fortran_abi_mimic.c, a C program that makes exactly these calls with exactly this struct layout and by-reference
@@ -44,9 +46,11 @@ module DIGITAL_FILTERING
     public :: attach_stream, filter_dev
     public :: set_time_scales, clear_time_scales, time_scales_from_lengths
     public :: set_filter_shape, FILTER_EXPONENTIAL, FILTER_GAUSSIAN
+    public :: set_flux_correction, flux_info, FLUX_OFF, FLUX_MASS, FLUX_VOLUME
 
     integer, parameter :: RESTART_STATE = 1, RESTART_STATS = 2, RESTART_CORR = 4   ! DFB_RESTART_* (what to save / load; added together)
     integer, parameter :: FILTER_EXPONENTIAL = 0, FILTER_GAUSSIAN = 1                ! DFB_FILTER_* (DFConfig%filter_shape)
+    integer, parameter :: FLUX_OFF = 0, FLUX_MASS = 1, FLUX_VOLUME = 2               ! DFB_FLUX_* (set_flux_correction)
 
     integer, parameter :: dp = selected_real_kind(15)
 
@@ -273,6 +277,17 @@ module DIGITAL_FILTERING
             type(c_ptr), intent(in) :: handle
             integer(c_int), intent(in) :: shape
         end function
+        integer(c_int) function dfb_set_flux_correction_f(handle, mode) bind(C, name='dfb_set_flux_correction_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle
+            integer(c_int), intent(in) :: mode
+        end function
+        integer(c_int) function dfb_flux_info_f(handle, plane, out) bind(C, name='dfb_flux_info_f')
+            import :: c_int, c_ptr, c_double
+            type(c_ptr), intent(in) :: handle
+            integer(c_int), intent(in) :: plane
+            real(c_double), intent(out) :: out(3)
+        end function
         integer(c_int) function dfb_first_step(handle) bind(C, name='dfb_first_step')
             import :: c_int, c_ptr
             type(c_ptr), value :: handle
@@ -496,6 +511,25 @@ contains
         s = shape
         call check(dfb_set_filter_shape_f(DF%handle, s), 'set_filter_shape')
     end subroutine set_filter_shape
+
+    ! FLUX_OFF, FLUX_MASS or FLUX_VOLUME from the next step on (whole planes only; not while attached)
+    subroutine set_flux_correction(DF, mode)
+        type(digital_filter_type), intent(in) :: DF
+        integer, intent(in) :: mode
+        integer(c_int) :: m
+        m = mode
+        call check(dfb_set_flux_correction_f(DF%handle, m), 'set_flux_correction')
+    end subroutine set_flux_correction
+
+    ! out = (c, m', mean flux) of the last corrected step of the (0-based) plane
+    subroutine flux_info(DF, plane, out)
+        type(digital_filter_type), intent(in) :: DF
+        integer, intent(in) :: plane
+        real(c_double), intent(out) :: out(3)
+        integer(c_int) :: p
+        p = plane
+        call check(dfb_flux_info_f(DF%handle, p, out), 'flux_info')
+    end subroutine flux_info
 
     ! back to the scalar Lt of the configuration
     subroutine clear_time_scales(DF)

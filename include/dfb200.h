@@ -131,7 +131,7 @@ int dfb_dims(dfb_handle h, int* Ny, int* Nz);
  *    send/recv, 0 = no communicator, 13 spanwise-periodic plane (dfb_config.periodic_z) in use (0/1),
  * 14 lags of correlation direction `field` (0 z, 1 y, 2 t; dfb_corr_enable), 0 when that direction is off or before any enable,
  * 15 per-row time scales in use (dfb_set_time_scales, 0/1), 17 filter shape (dfb_set_filter_shape: DFB_FILTER_EXPONENTIAL /
- *    DFB_FILTER_GAUSSIAN) */
+ *    DFB_FILTER_GAUSSIAN), 18 flux correction mode (dfb_set_flux_correction: DFB_FLUX_OFF / _MASS / _VOLUME) */
 int dfb_info(dfb_handle h, int what, int field, int64_t* out64);
 /* host copies of the setup tables (for parity tests): which = 0..7 rows R11,R21,R22,R33,Us,Ts,rhos,Ms [Ny];
  * 8 yc row [Ny]; 9 dy row [Ny]; 10 Lt[3]; 11 coefficients of half-width `arg` [2*arg+1], in the handle's filter shape;
@@ -249,6 +249,30 @@ int dfb_time_scales_from_lengths(dfb_handle h, const double Ix[6], double u_min,
  * shape is DFB_ERR_ARG, naming both.  dfb_info 17 returns the shape. */
 enum { DFB_FILTER_EXPONENTIAL = 0, DFB_FILTER_GAUSSIAN = 1 };
 int dfb_set_filter_shape(dfb_handle h, int shape);
+/* Inflow mass-flux correction (opt-in).  Every step's u' has a nonzero area-weighted plane mean, correlated over Lt: a low-frequency
+ * pulsation of the inflow mass flow, which a compressible calculation receives as an acoustic disturbance.  With the correction on,
+ * each plane p of each step (after the z-sweep) delivers
+ *     u' <- fma(-c_p, sqrt(R11_j), u'),   c_p = m'_p / D,   m'_p = sum_jk A_jk g_j u'_jk,   D = sum_jk A_jk g_j sqrt(R11_j),
+ * and T', rho' rebuilt from that u' with the epilogue's roundings (t2 = rc4 u'; T' = t2 Ts; rho' = -t2 rhos).  A_jk = hy_j hz_k are the
+ * cells of the area face maps ([vert_y[j], vert_y[j+1]) x [vert_z[k], vert_z[k+1]), dfb_get_table 12, 13).  DFB_FLUX_MASS weighs with
+ * g_j = rhos_j (1 + 0.2 Ms_j^2), the first-order mass flux rhos u' + Us rho' of the strong Reynolds analogy in use; DFB_FLUX_VOLUME with
+ * g_j = 1.  The delivered first-order flux sum A g u' is then zero to rounding.  Rows with R11 = 0 are unchanged.
+ * Only the delivered u', T', rho' change: filt_old (DFB_*_FILT), v' and w' are the same as with the correction off, so the generator
+ * evolves the same way whatever the mode, and a restart file (its header and fingerprint) does not depend on it.  The second-order
+ * flux rho' u' is not balanced (it has a nonzero mean of its own, fixed by the Reynolds stresses rather than by the filter's
+ * sampling).  The constructor's step and dfb_first_step are never corrected.  N2 statistics, correlation statistics, face maps,
+ * dfb_scatter_to_cells and every copy of the fields see the corrected fields.  Batches are corrected plane by plane, each plane bit for
+ * bit as a single-plane handle of its plane_id.
+ * dfb_set_flux_correction(h, mode): DFB_FLUX_OFF (default), DFB_FLUX_MASS or DFB_FLUX_VOLUME, from the next step on.  Refused,
+ * leaving the handle as it was: an unknown mode or, for a mode other than DFB_FLUX_OFF, a slab handle (k_begin, k_end), or a plane with
+ * R11 = 0 on every row (DFB_ERR_ARG); an attached handle or an outstanding dfb_filter_to_host_begin (DFB_ERR_STATE).  Attached steps and
+ * graph replays take the correction; a void step changes nothing.  dfb_info 18 returns the mode.
+ * dfb_flux_info(h, plane, out[3]): c_p and m'_p of the last corrected step of `plane`, and the mean flux sum A rhos Us (mass) or
+ * sum A Us (volume) of the mode last enabled; before the first corrected step c_p = m'_p = 0.  DFB_ERR_STATE if the correction was
+ * never enabled.  Synchronises the handle's stream (and an attached handle's step record). */
+enum { DFB_FLUX_OFF = 0, DFB_FLUX_MASS = 1, DFB_FLUX_VOLUME = 2 };
+int dfb_set_flux_correction(dfb_handle h, int mode);
+int dfb_flux_info(dfb_handle h, int plane, double out[3]);
 /* page-lock (cudaHostRegister) / release a caller-owned host array: dfb_filter_to_host into registered arrays runs at the PCIe
  * rate; pageable arrays cost an extra staging pass inside the driver.  The C++ facade does this for its std::vectors. */
 int dfb_host_register(void* ptr, size_t bytes);
@@ -472,6 +496,8 @@ int dfb_filter_dev_f(const dfb_handle* h, const double* const* dt_dev);
 int dfb_set_time_scales_f(const dfb_handle* h, const double* const* Lt_rows);
 int dfb_time_scales_from_lengths_f(const dfb_handle* h, const double* Ix, const double* u_min, double* Lt_rows);
 int dfb_set_filter_shape_f(const dfb_handle* h, const int* shape);
+int dfb_set_flux_correction_f(const dfb_handle* h, const int* mode);
+int dfb_flux_info_f(const dfb_handle* h, const int* plane, double* out);
 /* path: Fortran character variable (c_loc) + its len_trim, as the file names of dfb_config (path_len < 0: NUL-terminated) */
 int dfb_save_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);
 int dfb_load_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);

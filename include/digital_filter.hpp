@@ -22,6 +22,7 @@
 //   * the noise is the counter-based pcg32 stream of include/dfb_rng_spec.h (seedable, reproducible)
 //     instead of a random_device-seeded process-wide static (df.cpp:334).
 #pragma once
+#include <array>
 #include <cstdint>
 #include <cstdio>
 #include <stdexcept>
@@ -144,6 +145,19 @@ class DIGITAL_FILTER {
         std::int64_t v = 0;
         check(dfb_info(h_, 17, 0, &v));
         return (int)v;
+    }
+    // inflow mass-flux correction (dfb_set_flux_correction): DFB_FLUX_OFF, DFB_FLUX_MASS or DFB_FLUX_VOLUME from the next step on;
+    // flux_info(plane) = {c, m', mean flux} of the last corrected step of that plane
+    void set_flux_correction(int mode) { check(dfb_set_flux_correction(h_, mode)); }
+    int flux_correction() const {
+        std::int64_t v = 0;
+        check(dfb_info(h_, 18, 0, &v));
+        return (int)v;
+    }
+    std::array<double, 3> flux_info(int plane = 0) const {
+        std::array<double, 3> out{};
+        check(dfb_flux_info(h_, plane, out.data()));
+        return out;
     }
     // explicit fetch for fetch_every_step = false (also refreshes .filt)
     void fetch() {

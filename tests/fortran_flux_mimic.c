@@ -1,0 +1,61 @@
+/* tests/fortran_flux_mimic.c -- the flux correction of fortran/digital_filtering.f90 (set_flux_correction, flux_info) made the way a
+ * Fortran compiler makes the calls, as tests/fortran_abi_mimic.c does for the rest of the module: every scalar by reference through
+ * dfb_set_flux_correction_f and dfb_flux_info_f (plane 0-based, out(3) by address).  Handle A is made that way, handle B through the C
+ * ABI; both take the same steps through dfb_filter_to_host_f and must agree bit for bit, with the same {c, m', mean}.
+ *   usage: fortran_flux_mimic <RST.dat> <line.dat>      prints "FLUX_OK Ny" or exits non-zero */
+#include <stdio.h>
+#include <stdlib.h>
+#include <string.h>
+#include "dfb200.h"
+
+static void blank_pad(char* dst, const char* src, int n) {
+    int l = (int)strlen(src);
+    memset(dst, ' ', (size_t)n);
+    memcpy(dst, src, (size_t)(l < n ? l : n));
+}
+static int len_trim(const char* s, int n) {
+    while (n > 0 && s[n - 1] == ' ') --n;
+    return n;
+}
+
+int main(int argc, char** argv) {
+    if (argc < 3) { fprintf(stderr, "usage: %s RST.dat line.dat\n", argv[0]); return 2; }
+    char vel_fluc_file[256], line_file[256];
+    blank_pad(vel_fluc_file, argv[1], 256);
+    blank_pad(line_file, argv[2], 256);
+    dfb_config c;
+    if (dfb_config_init(&c) != DFB_OK) return 3;
+    c.d_i = 0.0013; c.rho_e = 0.044; c.U_e = 869.1; c.mu_e = 7.1212e-6;
+    c.vel_file_offset = 0; c.vel_file_N_values = 330;
+    c.honor_flow_config = 1;
+    c.vel_fluc_file = vel_fluc_file; c.vel_fluc_file_len = len_trim(vel_fluc_file, 256);
+    c.line_file = line_file;         c.line_file_len = len_trim(line_file, 256);
+    c.seed = 4243; c.device = -1;
+
+    dfb_handle a = NULL, b = NULL;
+    const int mode = DFB_FLUX_VOLUME, bad = 5, plane = 0;
+    if (dfb_create_f(&c, &a) != DFB_OK || dfb_set_flux_correction_f(&a, &mode) != DFB_OK) { fprintf(stderr, "module path: %s\n", dfb_last_error()); return 4; }
+    if (dfb_set_flux_correction_f(&a, &bad) != DFB_ERR_ARG) return 5;
+    if (dfb_create(&c, &b) != DFB_OK || dfb_set_flux_correction(b, DFB_FLUX_VOLUME) != DFB_OK) { fprintf(stderr, "C ABI: %s\n", dfb_last_error()); return 6; }
+    int Ny = 0, Nz = 0;
+    if (dfb_dims_f(&a, &Ny, &Nz) != DFB_OK) return 7;
+    const size_t n = (size_t)Ny * Nz;
+    double* x = malloc(5 * n * sizeof(double));
+    double* y = malloc(5 * n * sizeof(double));
+    for (int s = 0; s < 3; ++s) {
+        const double dt = 2e-6 * (s + 1);
+        if (dfb_filter_to_host_f(&a, &dt, x, x + n, x + 2 * n, x + 3 * n, x + 4 * n) != DFB_OK) return 8;
+        if (dfb_filter_to_host(b, dt, y, y + n, y + 2 * n, y + 3 * n, y + 4 * n) != DFB_OK) return 9;
+        if (memcmp(x, y, 5 * n * sizeof(double)) != 0) { fprintf(stderr, "step %d differs\n", s); return 10; }
+    }
+    double fa[3], fb[3];
+    int64_t m = -1;
+    if (dfb_flux_info_f(&a, &plane, fa) != DFB_OK || dfb_flux_info(b, 0, fb) != DFB_OK || memcmp(fa, fb, sizeof(fa)) != 0) return 11;
+    if (fa[0] == 0.0 || !(fa[2] > 0.0)) return 12;
+    if (dfb_info(a, 18, 0, &m) != DFB_OK || m != DFB_FLUX_VOLUME) return 13;
+    free(x); free(y);
+    dfb_destroy_f(&a);
+    dfb_destroy(b);
+    printf("FLUX_OK %d\n", Ny);
+    return 0;
+}
