@@ -2,6 +2,7 @@
 // Mirrors DIGITAL_FILTER's constructor (df.cpp:4-66) and filter(dt) (df.cpp:449-468).
 // There is no CPU fallback: without an sm_100 device dfb_create fails with DFB_ERR_CUDA.
 #include <algorithm>
+#include <array>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -39,6 +40,50 @@ int fail(int code, const std::string& msg) {
             throw Error{DFB_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(e__)};         \
     } while (0)
 
+// Device memory with one owner: everything allocated through it is freed when it is reset, destroyed or assigned over.
+class DeviceMem {
+public:
+    DeviceMem() = default;
+    DeviceMem(DeviceMem&& o) noexcept : ptrs_(std::move(o.ptrs_)) { o.ptrs_.clear(); }
+    DeviceMem& operator=(DeviceMem&& o) noexcept {
+        if (this != &o) { reset(); ptrs_ = std::move(o.ptrs_); o.ptrs_.clear(); }
+        return *this;
+    }
+    ~DeviceMem() { reset(); }
+    // frees everything; the first error of the frees
+    cudaError_t reset() {
+        cudaError_t first = cudaSuccess;
+        for (void* p : ptrs_) {
+            const cudaError_t e = cudaFree(p);
+            if (first == cudaSuccess) first = e;
+        }
+        ptrs_.clear();
+        return first;
+    }
+    template <class T>
+    T* alloc(size_t n) {
+        void* p = nullptr;
+        CUDA_TRY(cudaMalloc(&p, std::max<size_t>(n, 1) * sizeof(T)));
+        ptrs_.push_back(p);
+        return static_cast<T*>(p);
+    }
+    template <class T>
+    T* zeroed(size_t n, cudaStream_t st) {
+        T* p = alloc<T>(n);
+        CUDA_TRY(cudaMemsetAsync(p, 0, std::max<size_t>(n, 1) * sizeof(T), st));
+        return p;
+    }
+    template <class T>
+    T* upload(const std::vector<T>& v, cudaStream_t st) {
+        T* p = alloc<T>(v.size());
+        if (!v.empty()) CUDA_TRY(cudaMemcpyAsync(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, st));
+        return p;
+    }
+
+private:
+    std::vector<void*> ptrs_;
+};
+
 // A face map on the device (dfb_facemap_create): the taps of facemap.hpp, and what dfb_interp_to_host needs to deliver the served faces
 struct FaceMapDev {
     int kind = DFB_MAP_POINT, n = 0, n_served = 0;
@@ -48,10 +93,28 @@ struct FaceMapDev {
     int* slot = nullptr;              // face -> its row in stage; nullptr when every face is served (face i -> i)
     double* w = nullptr;
     double* stage = nullptr;          // [5][n_served], allocated by the first dfb_interp_to_host
-    FaceMapDev() = default;
-    FaceMapDev(const FaceMapDev&) = delete;
-    FaceMapDev& operator=(const FaceMapDev&) = delete;
-    ~FaceMapDev() { cudaFree(idx); cudaFree(ptr); cudaFree(slot); cudaFree(w); cudaFree(stage); }
+    DeviceMem mem;
+};
+
+// What of the step's plan follows from the coefficients (build_sweeps): their device table, and the forms, work descriptions, tensor
+// maps and grids of the sweeps for each buffer set b.  The plane's buffers and the noise tables follow from the half-widths alone and
+// belong to the handle.
+struct Sweeps {
+    bool tuned = false;
+    int y_form = 0;                           // 0 dense band matrices, 1 chunk-recursive, 2 run-recursive, 3 run + dense
+    int n_tiles_dense = 0, n_tiles_rec = 0;   // y-sweep tiles: dense band-matrix tiles first, then recursive tiles
+    YParams y[2]{};
+    ZParams z[2]{};
+    YMaps ymaps[2]{};
+    YRMaps rmaps[2]{};                        // run-recursive y-sweep (the default form): tensor maps of r_ys with its box
+    ZMaps zmaps[2]{};
+    const int64_t* coef_ptr = nullptr;        // the coefficient table that PlaneDev::coef_ptr / coef_vals of both sets point at
+    const double* coef_vals = nullptr;
+    unsigned long long* tl = nullptr;         // development aid (DFB_TIMELINE): 64 steps x {noise, y, z} x {start, end}
+    DeviceMem mem;
+
+    // dfb_info 3, 7 and 10; the kernel forms a restart file records
+    std::array<int, 3> forms() const { return {tuned ? 1 : 0, tuned ? z[0].zmode : 0, tuned ? y_form : -1}; }
 };
 
 }  // namespace
@@ -60,7 +123,6 @@ struct dfb_filter_s {
     Plan plan;
     int device = 0;
     int noise_mode = DFB_NOISE_GENERATE;
-    bool tuned = false;
     uint64_t seed = 0;
     uint64_t fingerprint = 0;         // of the filter tables (restart.hpp): what a restart file must match
     int plane_id = 0;
@@ -79,32 +141,19 @@ struct dfb_filter_s {
     double* stage[2] = {nullptr, nullptr};                 // staged copies of the five output fields
     cudaEvent_t ev_staged[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
     long long pipe_begun = 0, pipe_ended = 0;
-    std::vector<void*> allocs;
-    std::vector<void*> sweep_allocs;  // what build_sweeps allocated: freed when dfb_set_filter_shape rebuilds the sweeps
+    DeviceMem mem;                    // device memory that lives as long as the handle (dalloc, upload)
     // Two noise buffer sets (r_ys, r_zs): step s uses set s&1, so noise(s+1) can be written while
     // y(s)/z(s) still read set s&1.  D[b] differs from D[1-b] only in the r_ys / r_zs pointers.
     PlaneDev D[2]{};
     int64_t buf_step[2] = {-1, -1};   // which step's noise set b currently holds (or -1)
-    int64_t ybuf_step[2] = {-1, -1};  // which step's y-sweep result the r_zs interior of set b holds (or -1)
-    bool y_ahead = false;             // optionally run the next step's y-sweep on the side stream too (measured: contention
-                                      // with the z-sweep costs more than the filled tail gains; off by default)
     int noise_view = 0;               // set holding the most recently consumed / generated noise
     cudaEvent_t ev_noise[2] = {nullptr, nullptr};   // noise into set b complete (either stream)
     cudaEvent_t ev_free[2] = {nullptr, nullptr};    // last readers of set b complete (main stream)
-    // tuned y-sweep
-    YMaps maps[2]{};
-    YParams yp[2]{};
-    int n_tiles_dense = 0, n_tiles_rec = 0;   // y-sweep tiles: dense band-matrix tiles first, then recursive tiles
-    YRMaps rmaps[2]{};                        // run-recursive y-sweep (the default form): tensor maps of r_ys with its box
-    int y_form = 0;                           // 0 dense band matrices, 1 chunk-recursive (ysweep_rec_kernel), 2 run-recursive (ysweep_run_kernel)
-    // tuned z-sweep
-    ZParams zp[2]{};
-    ZMaps zmaps[2]{};
+    Sweeps sw;                        // the sweeps of both sets and the coefficient table (build_sweeps)
     // noise
     NoiseParams np{};                 // geometry of the drawn arrays (fixed), their states (per step: fill_noise_params)
     uint64_t npairs[6] = {};          // pairs one step draws from each array's stream
     NoiseWindows nwin{};              // periodic_z: segment windows of the r_ys arrays whose extended rows wrap (else all nullptr)
-    unsigned long long* tl = nullptr; // development aid (DFB_TIMELINE): 64 steps x {noise, y, z} x {start, end}
     // N2: running statistics (opt-in)
     double* stats = nullptr;          // [P][6][Ny*W]: sum u'^2, v'^2, w'^2, T'^2, rho'^2, u'v'
     int64_t stats_count = 0;
@@ -115,8 +164,8 @@ struct dfb_filter_s {
     CorrParams corr{};                // lags, sums, scratch, ring
     int64_t corr_count = 0;           // accumulated steps
     std::vector<int64_t> corr_tsteps; // [L_t + 1]: accumulated steps that had an accumulated predecessor m steps back in the ring
-    std::vector<void*> corr_mem;      // the sums: freed when the lags change and with the handle
-                                      // (corr.ring and corr.part exist only while accumulating: corr_free_work)
+    DeviceMem corr_sums;              // corr.sum: replaced when the lags change
+    DeviceMem corr_work;              // corr.ring and corr.part: they exist only while accumulating
     // config 4: this handle as one spanwise slab of a plane shared with the other ranks of a job (dfb_comm_init)
     ncclComm_t comm = nullptr;
     int comm_rank = -1, comm_world = 0;
@@ -170,30 +219,19 @@ struct dfb_filter_s {
 
     void comm_release();              // ncclCommDestroy through the lazily loaded library (below)
     template <class T>
-    T* dalloc(size_t n, bool zero = true) {
-        void* p = nullptr;
-        CUDA_TRY(cudaMalloc(&p, std::max<size_t>(n, 1) * sizeof(T)));
-        allocs.push_back(p);
-        if (zero) CUDA_TRY(cudaMemsetAsync(p, 0, std::max<size_t>(n, 1) * sizeof(T), stream));
-        return static_cast<T*>(p);
-    }
+    T* dalloc(size_t n, bool zero = true) { return zero ? mem.zeroed<T>(n, stream) : mem.alloc<T>(n); }
     template <class T>
-    T* upload(const std::vector<T>& v) {
-        T* p = dalloc<T>(v.size(), false);
-        if (!v.empty()) CUDA_TRY(cudaMemcpyAsync(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, stream));
-        return p;
-    }
+    T* upload(const std::vector<T>& v) { return mem.upload(v, stream); }
     ~dfb_filter_s() {
         cudaSetDevice(device);
         if (attached) { cudaStreamSynchronize(stream); stream = own_stream; }
         if (side) cudaStreamSynchronize(side);
         if (stream) cudaStreamSynchronize(stream);
-        facemaps.clear();
-        for (void* p : allocs) cudaFree(p);
-        for (void* p : sweep_allocs) cudaFree(p);
-        for (void* p : corr_mem) cudaFree(p);
-        cudaFree(corr.ring);
-        cudaFree(corr.part);
+        facemaps.clear();             // the device memory goes here, not after the last cudaGetLastError below
+        sw = Sweeps{};
+        corr_sums.reset();
+        corr_work.reset();
+        mem.reset();
         for (auto& e : ev) if (e) cudaEventDestroy(e);
         for (int b = 0; b < 2; ++b) { if (ev_noise[b]) cudaEventDestroy(ev_noise[b]); if (ev_free[b]) cudaEventDestroy(ev_free[b]); }
         for (int q = 0; q < 2; ++q) { if (ev_staged[q]) cudaEventDestroy(ev_staged[q]); if (ev_copied[q]) cudaEventDestroy(ev_copied[q]); }
@@ -232,23 +270,23 @@ Fn driver_fn(const char* name) {
 typedef CUresult (*StreamWaitValue64Fn)(CUstream, CUdeviceptr, cuuint64_t, unsigned int);
 StreamWaitValue64Fn stream_wait_value64() { static const auto fn = driver_fn<StreamWaitValue64Fn>("cuStreamWaitValue64"); return fn; }
 
-void timeline_reset(dfb_filter_s& H) {
+void timeline_reset(unsigned long long* tl) {
     std::vector<unsigned long long> init(512, 0ull);
     for (int i = 0; i < 512; i += 2) init[i] = ~0ull;                  // starts: atomicMin
-    CUDA_TRY(cudaMemcpy(H.tl, init.data(), 512 * sizeof(unsigned long long), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(tl, init.data(), 512 * sizeof(unsigned long long), cudaMemcpyHostToDevice));
 }
 
 // Tile queues of the run-recursive y-sweep (one per buffer set: {next tile, producers done}): at rest they hold the size of the
-// persistent grid -- CTA b starts on tile b, the kernel puts the value back when its last producer has finished.  Written here
-// when the plan is built and again whenever the grid changes (dfb_comm_init leaving SMs free for NCCL); the stream is idle then.
-void reset_run_queues(dfb_filter_s& H) {
-    if (!H.yp[0].rcounter) return;
+// persistent grid -- CTA b starts on tile b, the kernel puts the value back when its last producer has finished.  Written when the
+// sweeps are built and again whenever the grid changes (dfb_comm_init leaving SMs free for NCCL); the stream is idle then.
+void reset_run_queues(const dfb_filter_s& H, const Sweeps& sw) {
+    if (!sw.y[0].rcounter) return;
     CUDA_TRY(cudaStreamSynchronize(H.stream));
     if (H.side) CUDA_TRY(cudaStreamSynchronize(H.side));
     for (int b = 0; b < 2; ++b) {
-        const int grid = (int)std::min<long long>((long long)H.yp[b].n_rtiles * H.nplanes, (long long)H.yp[b].r_grid);
+        const int grid = (int)std::min<long long>((long long)sw.y[b].n_rtiles * H.nplanes, (long long)sw.y[b].r_grid);
         const int init[2] = {grid, 0};
-        CUDA_TRY(cudaMemcpy(H.yp[b].rcounter, init, sizeof(init), cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(sw.y[b].rcounter, init, sizeof(init), cudaMemcpyHostToDevice));
     }
 }
 
@@ -271,7 +309,13 @@ StepPlan plan_for_device(const dfb_filter_s& H, const Plan& P) {
                      Overrides{env_int("DFB_Y_MODE"), env_int("DFB_Y_TK"), env_int("DFB_Y_COLGROUP"), env_int("DFB_ZK"), env_int("DFB_Z_MODE")});
 }
 
-void build_sweeps(dfb_filter_s& H, const StepPlan& S);
+Sweeps build_sweeps(const dfb_filter_s& H, const Plan& P, const StepPlan& S);
+
+// Makes sw the handle's sweeps: both buffer sets read its coefficient table, and the memory of the sweeps it replaces is freed.
+void install_sweeps(dfb_filter_s& H, Sweeps&& sw) {
+    H.sw = std::move(sw);
+    for (PlaneDev& D : H.D) { D.coef_ptr = H.sw.coef_ptr; D.coef_vals = H.sw.coef_vals; }
+}
 
 // Carries out the step's plan (stepplan.cpp) on the device: allocations, uploads, tensor maps, kernel attributes, occupancy.
 void build_device(dfb_filter_s& H) {
@@ -300,7 +344,7 @@ void build_device(dfb_filter_s& H) {
         H.D[1].f[f].r_ys = H.dalloc<double>(NP * D.f[f].ps_ys);
         H.D[1].f[f].r_zs = H.dalloc<double>(NP * D.f[f].ps_zs);
     }
-    build_sweeps(H, S);
+    install_sweeps(H, build_sweeps(H, P, S));
 
     H.np = S.np;
     for (int n = 0; n < H.np.n_arrays; ++n) {
@@ -313,50 +357,50 @@ void build_device(dfb_filter_s& H) {
     CUDA_TRY(cudaStreamSynchronize(H.stream));
 }
 
-// What of the step's plan follows from the coefficients: their table, and the forms, work descriptions, tensor maps and grids of the
-// sweeps.  The layout, the plane's buffers and the noise tables follow from the half-widths alone (build_device).  Its allocations are
-// kept in sweep_allocs, so that dfb_set_filter_shape can build it anew.
-void build_sweeps(dfb_filter_s& H, const StepPlan& S) {
-    const Plan& P = H.plan;
+// What of the step's plan follows from the coefficients of P: their table, and the forms, work descriptions, tensor maps and grids of
+// the sweeps.  The layout, the plane's buffers and the noise tables follow from the half-widths alone (build_device).  The handle is
+// not changed, so that dfb_set_filter_shape can build new sweeps beside the old ones and install them only when this has succeeded.
+Sweeps build_sweeps(const dfb_filter_s& H, const Plan& P, const StepPlan& S) {
     const int NP = H.nplanes, Ny = P.Ny;
     cudaDeviceProp prop;
     CUDA_TRY(cudaGetDeviceProperties(&prop, H.device));
-    const size_t first_alloc = H.allocs.size();
-    H.tuned = S.tuned;
-    H.D[0].coef_ptr = H.upload(P.coef.ptr);
-    H.D[0].coef_vals = H.upload(P.coef.vals);
-    H.D[1].coef_ptr = H.D[0].coef_ptr;
-    H.D[1].coef_vals = H.D[0].coef_vals;
+    Sweeps sw;
+    DeviceMem& mem = sw.mem;
+    sw.tuned = S.tuned;
+    sw.coef_ptr = mem.upload(P.coef.ptr, H.stream);
+    sw.coef_vals = mem.upload(P.coef.vals, H.stream);
+    PlaneDev D[2] = {H.D[0], H.D[1]};                    // the buffer sets as the sweeps see them: with the new table
+    for (PlaneDev& d : D) { d.coef_ptr = sw.coef_ptr; d.coef_vals = sw.coef_vals; }
 
-    if (H.tuned) {
-        YParams& Y = H.yp[0];
+    if (sw.tuned) {
+        YParams& Y = sw.y[0];
         Y = S.yp;
-        Y.yrec = H.upload(S.yrec); Y.ygc = H.upload(S.ygc);
+        Y.yrec = mem.upload(S.yrec, H.stream); Y.ygc = mem.upload(S.ygc, H.stream);
         Y.resident_grid = env_int("DFB_Y_PERSIST").value_or(0);
-        Y.groups = H.upload(S.groups); Y.tiles = H.upload(S.tiles); Y.cmat = H.upload(S.cmat);
-        Y.D = H.D[0];
-        Y.prof = H.dalloc<unsigned long long>(8);
-        if (std::getenv("DFB_TIMELINE")) { H.tl = H.dalloc<unsigned long long>(512); timeline_reset(H); }
+        Y.groups = mem.upload(S.groups, H.stream); Y.tiles = mem.upload(S.tiles, H.stream); Y.cmat = mem.upload(S.cmat, H.stream);
+        Y.D = D[0];
+        Y.prof = mem.zeroed<unsigned long long>(8, H.stream);
+        if (std::getenv("DFB_TIMELINE")) { sw.tl = mem.zeroed<unsigned long long>(512, H.stream); timeline_reset(sw.tl); }
         Y.debug = env_int("DFB_DEBUG_Y").value_or(0);
-        H.y_form = S.y_form; H.n_tiles_dense = S.n_tiles_dense; H.n_tiles_rec = S.n_tiles_rec;
-        if (H.y_form >= 2) {
-            Y.rgroups = H.upload(S.rgroups); Y.rtiles = H.upload(S.rtiles);
-            Y.rcounter = H.dalloc<int>(4, false);          // tile queues, filled by reset_run_queues() below
+        sw.y_form = S.y_form; sw.n_tiles_dense = S.n_tiles_dense; sw.n_tiles_rec = S.n_tiles_rec;
+        if (sw.y_form >= 2) {
+            Y.rgroups = mem.upload(S.rgroups, H.stream); Y.rtiles = mem.upload(S.rtiles, H.stream);
+            Y.rcounter = mem.alloc<int>(4);                 // tile queues, filled by reset_run_queues() below
             CUDA_TRY(ysweep_run_prepare((size_t)Y.r_smem));
         }
-        H.yp[1] = Y; H.yp[1].D = H.D[1];
-        if (H.yp[1].rcounter) H.yp[1].rcounter += 2;
-        reset_run_queues(H);
+        sw.y[1] = Y; sw.y[1].D = D[1];
+        if (sw.y[1].rcounter) sw.y[1].rcounter += 2;
+        reset_run_queues(H, sw);
         CUDA_TRY(ysweep_prepare());
-        ZParams& Z = H.zp[0];
+        ZParams& Z = sw.z[0];
         Z = S.zp;
-        Z.D = H.D[0];
-        Z.coef_pad = H.upload(S.coef_pad); Z.coef_pad_ptr = H.upload(S.coef_pad_ptr);
-        Z.units = H.upload(S.units);
-        Z.unit_par = S.unit_par.empty() ? nullptr : H.upload(S.unit_par);
-        Z.counter = H.dalloc<int>(2);        // one work counter per buffer set: y(s+1) resets its own while z(s) still pulls from the other
+        Z.D = D[0];
+        Z.coef_pad = mem.upload(S.coef_pad, H.stream); Z.coef_pad_ptr = mem.upload(S.coef_pad_ptr, H.stream);
+        Z.units = mem.upload(S.units, H.stream);
+        Z.unit_par = S.unit_par.empty() ? nullptr : mem.upload(S.unit_par, H.stream);
+        Z.counter = mem.zeroed<int>(2, H.stream);   // one work counter per buffer set: y(s+1) resets its own while z(s) still pulls from the other
         Z.debug = env_int("DFB_DEBUG_Z").value_or(0);
-        Z.prof = H.dalloc<unsigned long long>(4096);
+        Z.prof = mem.zeroed<unsigned long long>(4096, H.stream);
         int zb = 1;
         CUDA_TRY(zsweep_prepare(Z.zk, Z.zmode, (size_t)Z.smem_bytes, &zb));
         // The recursive form is bound by shared-memory traffic and latency, not by the fp64 pipe: two CTAs per SM run it as
@@ -365,24 +409,23 @@ void build_sweeps(dfb_filter_s& H, const StepPlan& S) {
         if (Z.zmode == 1 && Z.zk == 16) zb = std::min(zb, 2);
         if (std::getenv("DFB_Z_BLOCKS_PER_SM")) zb = std::min(std::max(zb, 3), std::atoi(std::getenv("DFB_Z_BLOCKS_PER_SM")));
         Z.nblocks = std::max(1, std::min(std::max(zb, 1) * prop.multiProcessorCount, (Z.n_items * NP + 3) / 4));
-        H.yp[0].zcounter = Z.counter; H.yp[1].zcounter = Z.counter + 1;
-        H.zp[1] = Z; H.zp[1].D = H.D[1]; H.zp[1].counter = Z.counter + 1;
+        sw.y[0].zcounter = Z.counter; sw.y[1].zcounter = Z.counter + 1;
+        sw.z[1] = Z; sw.z[1].D = D[1]; sw.z[1].counter = Z.counter + 1;
         for (int b = 0; b < 2; ++b)
             for (int f = 0; f < 3; ++f) {
-                const FieldDev& F = H.D[b].f[f];
+                const FieldDev& F = D[b].f[f];
                 const cuuint64_t ydims[2] = {(cuuint64_t)F.We, (cuuint64_t)F.rows_y * (cuuint64_t)NP};   // planes of a batch stacked along the rows
                 const cuuint64_t ystrides[1] = {(cuuint64_t)F.pitch_y * sizeof(double)};
                 const cuuint32_t ybox[2] = {(cuuint32_t)Y.tk, (cuuint32_t)Y_RC}, rbox[2] = {(cuuint32_t)YR_C, (cuuint32_t)YR_BOX};
-                encode_map(H.maps[b].m[f], F.r_ys, 2, ydims, ystrides, ybox, CU_TENSOR_MAP_SWIZZLE_NONE, "");
-                if (H.y_form >= 2) encode_map(H.rmaps[b].m[f], F.r_ys, 2, ydims, ystrides, rbox, CU_TENSOR_MAP_SWIZZLE_NONE, " (y, run form)");
+                encode_map(sw.ymaps[b].m[f], F.r_ys, 2, ydims, ystrides, ybox, CU_TENSOR_MAP_SWIZZLE_NONE, "");
+                if (sw.y_form >= 2) encode_map(sw.rmaps[b].m[f], F.r_ys, 2, ydims, ystrides, rbox, CU_TENSOR_MAP_SWIZZLE_NONE, " (y, run form)");
                 const cuuint64_t zdims[3] = {(cuuint64_t)Z.zk, (cuuint64_t)(F.pitch_z / Z.zk), (cuuint64_t)Ny * (cuuint64_t)NP};
                 const cuuint64_t zstrides[2] = {(cuuint64_t)Z.zk * 8, (cuuint64_t)F.pitch_z * sizeof(double)};
                 const cuuint32_t zbox[3] = {(cuuint32_t)Z.zk, (cuuint32_t)Z.box_lines, 1u};
-                encode_map(H.zmaps[b].m[f], F.r_zs, 3, zdims, zstrides, zbox, Z.zk == 16 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, " (z)");
+                encode_map(sw.zmaps[b].m[f], F.r_zs, 3, zdims, zstrides, zbox, Z.zk == 16 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, " (z)");
             }
     }
-    H.sweep_allocs.insert(H.sweep_allocs.end(), H.allocs.begin() + first_alloc, H.allocs.end());
-    H.allocs.resize(first_alloc);
+    return sw;
 }
 
 // Host-driven step with per-row time scales: the device table of blend constants for dt, uploaded on the main stream when it holds
@@ -404,12 +447,44 @@ const double2* rows_for_step(dfb_filter_s& H, double dt) {
 void fill_noise_params(dfb_filter_s& H, int64_t step) { fill_noise_states(H.np, H.npairs, H.seed, H.plane_id, H.nplanes, step); }
 
 void launch_noise_for(dfb_filter_s& H, int64_t step, int b, cudaStream_t st) {
-    H.ybuf_step[b] = -1;                 // new noise invalidates whatever y-sweep result the set held
     fill_noise_params(H, step);
-    H.np.tl = H.tl ? H.tl + (step % 64) * 8 : nullptr;
+    H.np.tl = H.sw.tl ? H.sw.tl + (step % 64) * 8 : nullptr;
     CUDA_TRY(launch_noise(H.np, H.nwin, H.D[b], st));
     CUDA_TRY(cudaEventRecord(H.ev_noise[b], st));
     H.buf_step[b] = step;
+}
+
+// The sweeps of one step on the main stream, after its noise: the y-sweep (band-matrix tiles, if any, first, then the run-recursive
+// tiles: disjoint rows of r_zs), the z-sweep, the flux correction and N2 where the z-sweep's epilogue does not accumulate it.  Buffer set
+// b; rec: the step record of an attached step (nullptr host-driven); tl: the step's timeline slot (DFB_TIMELINE) or nullptr.
+void enqueue_sweeps(dfb_filter_s& H, int b, const StepConsts& S, const double2* rows, const StepRecord* rec, unsigned long long* tl) {
+    const Sweeps& sw = H.sw;
+    const bool first = S.first_step != 0;
+    const bool accumulate = H.stats_on && !first;                  // rms_add, df.cpp:606
+    const bool flux = H.flux_mode != DFB_FLUX_OFF && !first;      // the constructor's step is never corrected
+    if (sw.tuned) {
+        YParams Y = sw.y[b];
+        Y.tl = tl ? tl + 2 : nullptr;
+        Y.zcounter_init = 8 * sw.z[b].nblocks;                     // the z-sweep's warps (4 per CTA) start on two fixed items each
+        if (sw.y_form != 2) CUDA_TRY(launch_ysweep_tma(sw.ymaps[b], Y, sw.n_tiles_dense, sw.n_tiles_rec, H.stream));
+        if (sw.y_form >= 2) CUDA_TRY(launch_ysweep_run(sw.rmaps[b], Y, H.stream));
+    } else {
+        CUDA_TRY(launch_ysweep_simple(H.D[b], H.stream));
+    }
+    if (H.timing) CUDA_TRY(cudaEventRecord(H.ev[2], H.stream));
+    if (sw.tuned) {
+        ZParams Z = sw.z[b];
+        Z.S = S;
+        Z.rec = rec;
+        Z.rows = rows;
+        Z.tl = tl ? tl + 4 : nullptr;
+        Z.stats = (accumulate && !flux) ? H.stats : nullptr;       // N2 fused into the epilogue, unless the correction changes u', T', rho' after it
+        CUDA_TRY(launch_zsweep_tuned(sw.zmaps[b], Z, H.stream));
+    } else {
+        CUDA_TRY(launch_zsweep_simple(H.D[b], S, rec, rows, H.stream));
+    }
+    if (flux) CUDA_TRY(launch_flux(H.fx, rec, H.stream));
+    if (accumulate && (!sw.tuned || flux)) CUDA_TRY(launch_stats(H.D[0], H.stats, rec, H.stream));
 }
 
 // A step of a handle attached to a caller's stream (dfb_attach_stream): advance -> noise -> y-sweep(s) -> z-sweep (-> N2 for the
@@ -419,7 +494,6 @@ void launch_noise_for(dfb_filter_s& H, int64_t step, int b, cudaStream_t st) {
 void run_step_attached(dfb_filter_s& H, double dt, const double* dt_dev, bool first) {
     CUDA_TRY(cudaSetDevice(H.device));
     const bool accumulate = H.stats_on && !first;
-    const bool flux = H.flux_mode != DFB_FLUX_OFF && !first;      // the sums of N2 then describe the corrected fields: stats_kernel after it
     AdvanceParams A = H.adv;
     A.dt_dev = dt_dev;
     A.dt = dt;
@@ -434,29 +508,10 @@ void run_step_attached(dfb_filter_s& H, double dt, const double* dt_dev, bool fi
     np.tl = nullptr;
     CUDA_TRY(launch_noise(np, H.nwin, H.D[0], H.stream));
     H.buf_step[0] = H.buf_step[1] = -1;            // the sets hold no step the host knows of: host-driven steps after a detach draw anew
-    H.ybuf_step[0] = H.ybuf_step[1] = -1;
     H.noise_view = 0;
     StepConsts S{};
     S.first_step = first ? 1 : 0;
-    if (H.tuned) {
-        YParams Y = H.yp[0];
-        Y.tl = nullptr;
-        Y.zcounter_init = 8 * H.zp[0].nblocks;
-        if (H.y_form != 2) CUDA_TRY(launch_ysweep_tma(H.maps[0], Y, H.n_tiles_dense, H.n_tiles_rec, H.stream));
-        if (H.y_form >= 2) CUDA_TRY(launch_ysweep_run(H.rmaps[0], Y, H.stream));
-        ZParams Z = H.zp[0];
-        Z.S = S;
-        Z.rec = H.rec;
-        Z.rows = rows;
-        Z.tl = nullptr;
-        Z.stats = (accumulate && !flux) ? H.stats : nullptr;
-        CUDA_TRY(launch_zsweep_tuned(H.zmaps[0], Z, H.stream));
-    } else {
-        CUDA_TRY(launch_ysweep_simple(H.D[0], H.stream));
-        CUDA_TRY(launch_zsweep_simple(H.D[0], S, H.rec, rows, H.stream));
-    }
-    if (flux) CUDA_TRY(launch_flux(H.fx, H.rec, H.stream));
-    if (accumulate && (!H.tuned || flux)) CUDA_TRY(launch_stats(H.D[0], H.stats, H.rec, H.stream));
+    enqueue_sweeps(H, 0, S, rows, H.rec, nullptr);
 }
 
 void run_step(dfb_filter_s& H, double dt, bool first) {
@@ -474,34 +529,12 @@ void run_step(dfb_filter_s& H, double dt, bool first) {
         throw Error{DFB_ERR_STATE, "noise_mode = inject: dfb_set_noise must be called for u, v and w before every step"};
     }
     H.noise_view = b;
-    if (H.tl) { H.yp[b].tl = H.tl + (H.step % 64) * 8 + 2; H.zp[b].tl = H.tl + (H.step % 64) * 8 + 4; }
     if (H.timing) CUDA_TRY(cudaEventRecord(H.ev[1], H.stream));
-    if (H.noise_mode == DFB_NOISE_GENERATE && H.ybuf_step[b] == H.step) {
-        // this step's y-sweep already ran (or is running) on the side stream; ev_noise[b] above covers it
-    } else if (H.tuned) {
-        // band-matrix tiles (if any) first, then the run-recursive tiles: disjoint rows of r_zs
-        H.yp[b].zcounter_init = 8 * H.zp[b].nblocks;               // the z-sweep's warps (4 per CTA) start on two fixed items each
-        if (H.y_form != 2) CUDA_TRY(launch_ysweep_tma(H.maps[b], H.yp[b], H.n_tiles_dense, H.n_tiles_rec, H.stream));
-        if (H.y_form >= 2) CUDA_TRY(launch_ysweep_run(H.rmaps[b], H.yp[b], H.stream));
-    }
-    else CUDA_TRY(launch_ysweep_simple(H.D[b], H.stream));
-    if (H.timing) CUDA_TRY(cudaEventRecord(H.ev[2], H.stream));
     StepConsts S{};
     S.first_step = first ? 1 : 0;
     for (int f = 0; f < 3; ++f) blend_consts(dt, H.plan.f[f].Lt, S.sa[f], S.sb[f]);
-    const bool accumulate = H.stats_on && !first;                  // rms_add, df.cpp:606
-    const bool flux = H.flux_mode != DFB_FLUX_OFF && !first;      // the constructor's step is never corrected
-    if (H.tuned) {
-        H.zp[b].S = S;
-        H.zp[b].rows = rows;
-        H.zp[b].stats = (accumulate && !flux) ? H.stats : nullptr; // N2 fused into the epilogue, unless the correction changes u', T', rho' after it
-        CUDA_TRY(launch_zsweep_tuned(H.zmaps[b], H.zp[b], H.stream));
-    } else {
-        CUDA_TRY(launch_zsweep_simple(H.D[b], S, nullptr, rows, H.stream));
-    }
-    if (flux) CUDA_TRY(launch_flux(H.fx, nullptr, H.stream));
-    if (accumulate && (!H.tuned || flux)) CUDA_TRY(launch_stats(H.D[0], H.stats, nullptr, H.stream));
-    if (accumulate) H.stats_count += 1;
+    enqueue_sweeps(H, b, S, rows, nullptr, H.sw.tl ? H.sw.tl + (H.step % 64) * 8 : nullptr);
+    if (H.stats_on && !first) H.stats_count += 1;
     if (H.corr_on && !first) {
         CorrParams& c = H.corr;
         if (c.L[0]) CUDA_TRY(launch_corr_z(c, H.stream));
@@ -526,15 +559,6 @@ void run_step(dfb_filter_s& H, double dt, bool first) {
         CUDA_TRY(cudaStreamWaitEvent(H.side, H.ev_noise[nb], 0));    // ... and so is its last writer: a dfb_generate_noise into it
                                                                        // on the main stream after that step would otherwise race this one
         launch_noise_for(H, H.step, nb, H.side);
-        // ... and so does its y-sweep (it reads only that noise and writes only that set's r_zs interior): it
-        // becomes resident as this step's z-sweep CTAs retire and keeps the fp64 pipe busy through the tail.
-        if (H.tuned && H.y_ahead) {
-            H.yp[nb].zcounter_init = 8 * H.zp[nb].nblocks;
-            if (H.y_form != 2) CUDA_TRY(launch_ysweep_tma(H.maps[nb], H.yp[nb], H.n_tiles_dense, H.n_tiles_rec, H.side));
-            if (H.y_form >= 2) CUDA_TRY(launch_ysweep_run(H.rmaps[nb], H.yp[nb], H.side));
-            CUDA_TRY(cudaEventRecord(H.ev_noise[nb], H.side));      // "set nb is ready" now means noise + y-sweep
-            H.ybuf_step[nb] = H.step;
-        }
     }
     if (H.timing) {
         CUDA_TRY(cudaEventSynchronize(H.ev[3]));
@@ -571,6 +595,13 @@ const char* const VOID_STEP_MSG = "dt must be finite and >= 0: an attached step 
 
 std::string attached_msg(const char* call) { return std::string(call) + " is not available while the handle is attached to a stream (dfb_attach_stream)"; }
 void refuse_attached(const dfb_filter_s& H, const char* call) { if (H.attached) throw Error{DFB_ERR_STATE, attached_msg(call)}; }
+
+// Calls that change what a staged copy or a hand-off reads wait until neither is outstanding.  call: the message's prefix, or nullptr.
+void refuse_outstanding(const dfb_filter_s& H, const char* call) {
+    if (H.pipe_begun == H.pipe_ended && H.g_begun == H.g_ended) return;
+    const std::string prefix = call ? std::string(call) + ": " : "";
+    throw Error{DFB_ERR_STATE, prefix + "a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first"};
+}
 
 // Attached: waits for the caller's stream and reads the device step record back into the host's step counter and N2 count.  A void
 // step since the last read is reported once, as DFB_ERR_ARG, and forgotten.  Host-driven: nothing.
@@ -613,7 +644,7 @@ void restore_state(dfb_filter_s& H, const double* filt_old3, int64_t step) {
             CUDA_TRY(cudaMemcpyAsync(H.D[0].f[f].filt_old, filt_old3 + f * n, n * 8, cudaMemcpyHostToDevice, H.stream));
     CUDA_TRY(cudaStreamSynchronize(H.stream));
     CUDA_TRY(cudaStreamSynchronize(H.side));      // a look-ahead noise launch for the old step counter may still be in flight
-    if (step != H.step) { H.buf_step[0] = H.buf_step[1] = -1; H.ybuf_step[0] = H.ybuf_step[1] = -1; }
+    if (step != H.step) H.buf_step[0] = H.buf_step[1] = -1;
     H.step = step;
     H.corr.ring_count = 0;       // the next step follows the restored state: no temporal pair reaches back across it
 }
@@ -669,7 +700,6 @@ static int create_impl(const dfb_config* cfg, int nplanes, dfb_handle* out) {
         CUDA_TRY(cudaSetDevice(dev));
         if (cfg->noise_mode != DFB_NOISE_GENERATE && cfg->noise_mode != DFB_NOISE_INJECT) throw Error{DFB_ERR_ARG, "bad noise_mode"};
         H->noise_mode = cfg->noise_mode;
-        H->y_ahead = std::getenv("DFB_Y_AHEAD") != nullptr;
         H->seed = cfg->seed;
         H->plane_id = cfg->plane_id;
         H->nplanes = nplanes;
@@ -734,16 +764,16 @@ int dfb_info(dfb_handle h, int what, int field, int64_t* out64) {
         case 0: *out64 = h->plan.f[field].Ny_max; break;
         case 1: *out64 = h->plan.f[field].Nz_max; break;
         case 2: *out64 = h->step; break;
-        case 3: *out64 = h->tuned ? 1 : 0; break;
+        case 3: *out64 = h->sw.forms()[0]; break;
         case 4: *out64 = h->plan.taps_per_step; break;
         case 5: *out64 = h->plan.NzG; break;
         case 6: *out64 = h->device; break;
-        case 7: *out64 = h->tuned ? h->zp[0].zmode : 0; break;
-        case 8: *out64 = h->tuned ? h->n_tiles_rec : 0; break;
-        case 9: *out64 = h->tuned ? h->n_tiles_dense : 0; break;
-        case 10: *out64 = h->tuned ? h->y_form : -1; break;
+        case 7: *out64 = h->sw.forms()[1]; break;
+        case 8: *out64 = h->sw.tuned ? h->sw.n_tiles_rec : 0; break;
+        case 9: *out64 = h->sw.tuned ? h->sw.n_tiles_dense : 0; break;
+        case 10: *out64 = h->sw.forms()[2]; break;
         case 12: *out64 = h->transport; break;
-        case 11: *out64 = h->tuned ? h->yp[0].n_rtiles : 0; break;
+        case 11: *out64 = h->sw.tuned ? h->sw.y[0].n_rtiles : 0; break;
         case 13: *out64 = h->plan.periodic ? 1 : 0; break;
         case 14: *out64 = h->corr_ready ? h->corr.L[field] : 0; break;
         case 15: *out64 = h->plan.Lt_rows.empty() ? 0 : 1; break;
@@ -954,8 +984,7 @@ int dfb_attach_stream(dfb_handle h, void* stream) {
         if (h->noise_mode != DFB_NOISE_GENERATE) throw Error{DFB_ERR_STATE, "dfb_attach_stream: a handle in inject mode cannot be attached"};
         if (h->corr_on) throw Error{DFB_ERR_STATE, "dfb_attach_stream: correlation statistics are on (dfb_corr_enable(h, 0, NULL) first)"};
         if (h->timing) throw Error{DFB_ERR_STATE, "dfb_attach_stream: timing is on (dfb_set_timing(h, 0) first)"};
-        if (h->pipe_begun != h->pipe_ended || h->g_begun != h->g_ended)
-            throw Error{DFB_ERR_STATE, "dfb_attach_stream: a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first"};
+        refuse_outstanding(*h, "dfb_attach_stream");
         int dev = -1;
         CUDA_TRY(cudaStreamGetDevice(static_cast<cudaStream_t>(stream), &dev));
         if (dev != h->device)
@@ -992,9 +1021,8 @@ int dfb_filter_dev(dfb_handle h, const double* dt_dev) {
 int dfb_set_time_scales(dfb_handle h, const double* Lt_rows) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_set_time_scales") + ": set the rows before attaching");
-    if (h->pipe_begun != h->pipe_ended || h->g_begun != h->g_ended)
-        return fail(DFB_ERR_STATE, "dfb_set_time_scales: a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first");
     return guarded([&] {
+        refuse_outstanding(*h, "dfb_set_time_scales");
         Plan& P = h->plan;
         if (!Lt_rows) {
             P.Lt_rows.clear();
@@ -1047,16 +1075,12 @@ int dfb_set_filter_shape(dfb_handle h, int shape) {
         build_coef_table(P);
         const StepPlan S = plan_for_device(*h, P);        // refusals (DFB_Y_MODE / DFB_Z_MODE against the shape) throw here
         CUDA_TRY(cudaSetDevice(h->device));
-        CUDA_TRY(cudaStreamSynchronize(h->stream));
+        Sweeps sw = build_sweeps(*h, P, S);               // beside the old sweeps: a failure leaves the handle as it was
+        CUDA_TRY(cudaStreamSynchronize(h->stream));       // the new tables are uploaded, and nothing reads the old ones any more
         CUDA_TRY(cudaStreamSynchronize(h->side));
-        for (void* p : h->sweep_allocs) CUDA_TRY(cudaFree(p));
-        h->sweep_allocs.clear();
-        for (int b = 0; b < 2; ++b) { h->yp[b] = YParams{}; h->zp[b] = ZParams{}; h->maps[b] = YMaps{}; h->rmaps[b] = YRMaps{}; h->zmaps[b] = ZMaps{}; }
-        h->y_form = 0; h->n_tiles_dense = h->n_tiles_rec = 0; h->tl = nullptr;
+        install_sweeps(*h, std::move(sw));
         h->plan = std::move(P);
-        build_sweeps(*h, S);
         h->fingerprint = rst::fingerprint(h->plan);
-        CUDA_TRY(cudaStreamSynchronize(h->stream));
     });
 }
 
@@ -1065,10 +1089,9 @@ int dfb_set_flux_correction(dfb_handle h, int mode) {
     if (mode != DFB_FLUX_OFF && mode != DFB_FLUX_MASS && mode != DFB_FLUX_VOLUME)
         return fail(DFB_ERR_ARG, "unknown flux correction mode " + std::to_string(mode) + " (DFB_FLUX_OFF = 0, DFB_FLUX_MASS = 1, DFB_FLUX_VOLUME = 2)");
     if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_set_flux_correction") + ": set the mode before attaching");
-    if (h->pipe_begun != h->pipe_ended || h->g_begun != h->g_ended)
-        return fail(DFB_ERR_STATE, "dfb_set_flux_correction: a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first");
-    if (mode == DFB_FLUX_OFF) { h->flux_mode = DFB_FLUX_OFF; return DFB_OK; }
     return guarded([&] {
+        refuse_outstanding(*h, "dfb_set_flux_correction");
+        if (mode == DFB_FLUX_OFF) { h->flux_mode = DFB_FLUX_OFF; return; }
         FluxTables T = flux_tables(h->plan, mode);          // refusals (slab, R11 = 0 everywhere) throw before anything changes
         CUDA_TRY(cudaSetDevice(h->device));
         FluxParams& F = h->fx;
@@ -1293,9 +1316,8 @@ int dfb_corr_enable(dfb_handle h, int on, const int lags[3]) {
         return guarded([&] {
             CUDA_TRY(cudaSetDevice(h->device));
             CUDA_TRY(cudaStreamSynchronize(h->stream));
-            CUDA_TRY(cudaFree(h->corr.ring));
-            CUDA_TRY(cudaFree(h->corr.part));
             h->corr.ring = h->corr.part = nullptr;
+            CUDA_TRY(h->corr_work.reset());
         });
     }
     if (!lags) return fail(DFB_ERR_ARG, "lags is NULL");
@@ -1323,17 +1345,10 @@ int dfb_corr_enable(dfb_handle h, int on, const int lags[3]) {
         CorrParams& c = h->corr;
         const int NP = h->nplanes, Ny = P.Ny, W = P.NzG;
         const size_t rows = (size_t)NP * 3 * Ny;
-        auto alloc = [&](size_t n) {
-            void* q = nullptr;
-            CUDA_TRY(cudaMalloc(&q, std::max<size_t>(n, 1) * sizeof(double)));
-            return static_cast<double*>(q);
-        };
         if (!h->corr_ready || L[0] != c.L[0] || L[1] != c.L[1] || L[2] != c.L[2]) {
             CUDA_TRY(cudaStreamSynchronize(h->stream));
-            for (void* q : h->corr_mem) cudaFree(q);
-            h->corr_mem.clear();
-            cudaFree(c.ring);
-            cudaFree(c.part);
+            h->corr_sums.reset();
+            h->corr_work.reset();
             h->corr_ready = false;
             h->corr_on = false;
             c = CorrParams{};
@@ -1341,15 +1356,15 @@ int dfb_corr_enable(dfb_handle h, int on, const int lags[3]) {
             c.P = NP; c.Ny = Ny; c.W = W; c.periodic = P.periodic ? 1 : 0;
             for (int d = 0; d < 3; ++d) {
                 c.L[d] = L[d];
-                if (L[d]) { c.sum[d] = alloc(rows * (L[d] + 1)); h->corr_mem.push_back(c.sum[d]); }
+                if (L[d]) c.sum[d] = h->corr_sums.alloc<double>(rows * (L[d] + 1));
             }
             c.y_nsplit = c.y_split_cols = 1;
             if (L[1]) corr_y_split(Ny, W, &c.y_nsplit, &c.y_split_cols);
         }
         // the ring and the partial-sum scratch exist only while accumulating (on = 0 frees them)
         const size_t part = corr_part_doubles(NP, Ny, W, c.L[0], c.L[1], c.y_nsplit);
-        if (part && !c.part) c.part = alloc(part);
-        if (c.L[2] && !c.ring) c.ring = alloc((size_t)c.L[2] * rows * W);
+        if (part && !c.part) c.part = h->corr_work.alloc<double>(part);
+        if (c.L[2] && !c.ring) c.ring = h->corr_work.alloc<double>((size_t)c.L[2] * rows * W);
         for (int d = 0; d < 3; ++d)
             if (c.sum[d]) CUDA_TRY(cudaMemsetAsync(c.sum[d], 0, rows * (c.L[d] + 1) * sizeof(double), h->stream));
         CUDA_TRY(cudaStreamSynchronize(h->stream));
@@ -1454,8 +1469,7 @@ int check_restart_call(dfb_handle h, const char* path, int& what) {
     if (!h || !path) return fail(DFB_ERR_ARG, "handle/path is NULL");
     if (what & ~(DFB_RESTART_STATE | DFB_RESTART_STATS | DFB_RESTART_CORR)) return fail(DFB_ERR_ARG, "what must be a combination of DFB_RESTART_STATE, _STATS and _CORR");
     what |= DFB_RESTART_STATE;
-    if (h->pipe_begun != h->pipe_ended || h->g_begun != h->g_ended)
-        return fail(DFB_ERR_STATE, "a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first");
+    if (const int rc = guarded([&] { refuse_outstanding(*h, nullptr); }); rc != DFB_OK) return rc;
     const Plan& P = h->plan;
     if ((what & DFB_RESTART_CORR) && (P.k0 != 0 || P.k1 != P.NzG)) return fail(DFB_ERR_ARG, "correlation statistics need the whole plane");
     return DFB_OK;
@@ -1512,7 +1526,8 @@ int dfb_save_restart(dfb_handle h, const char* path, int what) {
         hd.Ny = P.Ny; hd.NzG = P.NzG; hd.plane0 = h->plane_id; hd.nplanes = h->nplanes; hd.periodic = P.periodic ? 1 : 0;
         hd.noise_mode = h->noise_mode; hd.seed = h->seed; hd.step = h->step;
         for (int f = 0; f < 3; ++f) { hd.Ny_max[f] = P.f[f].Ny_max; hd.Nz_max[f] = P.f[f].Nz_max; hd.Lt[f] = P.f[f].Lt; }
-        hd.forms[0] = h->tuned ? 1 : 0; hd.forms[1] = h->tuned ? h->zp[0].zmode : 0; hd.forms[2] = h->tuned ? h->y_form : -1;   // dfb_info 3, 7, 10
+        const std::array<int, 3> forms = h->sw.forms();
+        std::copy(forms.begin(), forms.end(), hd.forms);
         hd.fingerprint = h->fingerprint;
         hd.filter_shape = P.filter_shape;
         hd.sections = (uint32_t)what;
@@ -1728,27 +1743,10 @@ int dfb_face_map(dfb_handle h, int n, const double* yf, const double* zf, int* p
 // ---- face maps: the taps are built on the host (facemap.cpp), summed on the device (interp_kernel) ----
 namespace {
 
-void check_idle(const dfb_filter_s& H) {
-    if (H.pipe_begun != H.pipe_ended || H.g_begun != H.g_ended)
-        throw Error{DFB_ERR_STATE, "a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first"};
-}
-
 FaceMapDev& facemap_of(dfb_filter_s& H, int map_id) {
     if (map_id < 0 || map_id >= (int)H.facemaps.size() || !H.facemaps[map_id])
         throw Error{DFB_ERR_ARG, "no face map " + std::to_string(map_id) + " on this handle"};
     return *H.facemaps[map_id];
-}
-
-template <class T>
-T* upload_now(const std::vector<T>& v, cudaStream_t st) {
-    T* p = nullptr;
-    CUDA_TRY(cudaMalloc(&p, std::max<size_t>(v.size(), 1) * sizeof(T)));
-    if (!v.empty()) {
-        cudaError_t e = cudaMemcpyAsync(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        if (e != cudaSuccess) { cudaFree(p); throw Error{DFB_ERR_CUDA, std::string("face map upload: ") + cudaGetErrorString(e)}; }
-    }
-    return p;
 }
 
 // the checks and arguments dfb_interp_to_cells and dfb_interp_to_host share
@@ -1770,21 +1768,22 @@ int dfb_facemap_create(dfb_handle h, int kind, int n, const double* yf, const do
                        int own_end, int flags, int* map_id) {
     if (!h || !map_id) return fail(DFB_ERR_ARG, "handle/map_id is NULL");
     return guarded([&] {
-        check_idle(*h);
+        refuse_outstanding(*h, nullptr);
         const FaceMap M = build_face_map(h->plan, kind, n, yf, zf, hy, hz, own_begin, own_end, flags);
         CUDA_TRY(cudaSetDevice(h->device));
         auto F = std::make_unique<FaceMapDev>();
         F->kind = kind; F->n = n; F->n_served = M.n_served; F->served = M.served;
         for (int i = 0; i < n; ++i)
             if (M.served[i]) F->faces.push_back(i);
-        F->idx = upload_now(M.idx, h->stream);
-        F->w = upload_now(M.w, h->stream);
-        if (kind == DFB_MAP_AREA) F->ptr = upload_now(M.ptr, h->stream);
+        F->idx = F->mem.upload(M.idx, h->stream);
+        F->w = F->mem.upload(M.w, h->stream);
+        if (kind == DFB_MAP_AREA) F->ptr = F->mem.upload(M.ptr, h->stream);
         if (M.n_served < n) {
             std::vector<int> slot(n, -1);
             for (int r = 0; r < M.n_served; ++r) slot[F->faces[r]] = r;
-            F->slot = upload_now(slot, h->stream);
+            F->slot = F->mem.upload(slot, h->stream);
         }
+        CUDA_TRY(cudaStreamSynchronize(h->stream));
         int id = 0;
         while (id < (int)h->facemaps.size() && h->facemaps[id]) ++id;
         if (id == (int)h->facemaps.size()) h->facemaps.emplace_back();
@@ -1816,7 +1815,7 @@ int dfb_interp_to_cells(dfb_handle h, int map_id, int plane, int fields, const i
                         const double scale[5], double* const dst[5], int stride) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     return guarded([&] {
-        check_idle(*h);
+        refuse_outstanding(*h, nullptr);
         const FaceMapDev& F = facemap_of(*h, map_id);
         InterpArgs a = interp_args(*h, F, plane, fields);
         if (stride < 1) throw Error{DFB_ERR_ARG, "stride must be >= 1"};
@@ -1839,14 +1838,14 @@ int dfb_interp_to_cells(dfb_handle h, int map_id, int plane, int fields, const i
 int dfb_interp_to_host(dfb_handle h, int map_id, int plane, int fields, double* out) {
     if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
     return guarded([&] {
-        check_idle(*h);
+        refuse_outstanding(*h, nullptr);
         sync_record(*h);
         FaceMapDev& F = facemap_of(*h, map_id);
         InterpArgs a = interp_args(*h, F, plane, fields);
         if (F.n > 0 && !out) throw Error{DFB_ERR_ARG, "out is NULL"};
         CUDA_TRY(cudaSetDevice(h->device));
         const size_t ns = (size_t)F.n_served;
-        if (!F.stage) CUDA_TRY(cudaMalloc(&F.stage, std::max<size_t>(5 * ns, 1) * sizeof(double)));
+        if (!F.stage) F.stage = F.mem.alloc<double>(5 * ns);
         int nf = 0;
         for (int f = 0; f < 5; ++f)
             if ((fields >> f) & 1) a.dst[f] = F.stage + ns * nf++;
@@ -1869,9 +1868,9 @@ int dfb_debug_yprof(dfb_handle h, unsigned long long* out8) {
     if (!h || !out8) return fail(DFB_ERR_ARG, "bad argument");
     return guarded([&] {
         CUDA_TRY(cudaStreamSynchronize(h->stream));
-        if (!h->yp[0].prof) throw Error{DFB_ERR_STATE, "no profile buffer"};
-        CUDA_TRY(cudaMemcpy(out8, h->yp[0].prof, 64, cudaMemcpyDeviceToHost));
-        CUDA_TRY(cudaMemset(h->yp[0].prof, 0, 64));
+        if (!h->sw.y[0].prof) throw Error{DFB_ERR_STATE, "no profile buffer"};
+        CUDA_TRY(cudaMemcpy(out8, h->sw.y[0].prof, 64, cudaMemcpyDeviceToHost));
+        CUDA_TRY(cudaMemset(h->sw.y[0].prof, 0, 64));
     });
 }
 
@@ -1879,11 +1878,11 @@ int dfb_debug_timeline(dfb_handle h, unsigned long long* out512) {
     // development aid: DFB_TIMELINE=1 at create; returns and clears 64 step slots x {noise, y, z, -} x {start, end} (ns)
     if (!h || !out512) return fail(DFB_ERR_ARG, "bad argument");
     return guarded([&] {
-        if (!h->tl) throw Error{DFB_ERR_STATE, "DFB_TIMELINE was not set when the handle was created"};
+        if (!h->sw.tl) throw Error{DFB_ERR_STATE, "DFB_TIMELINE was not set when the handle was created"};
         CUDA_TRY(cudaStreamSynchronize(h->stream));
         CUDA_TRY(cudaStreamSynchronize(h->side));
-        CUDA_TRY(cudaMemcpy(out512, h->tl, 512 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-        timeline_reset(*h);
+        CUDA_TRY(cudaMemcpy(out512, h->sw.tl, 512 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+        timeline_reset(h->sw.tl);
     });
 }
 
@@ -1891,9 +1890,9 @@ int dfb_debug_zprof(dfb_handle h, unsigned long long* out8) {
     if (!h || !out8) return fail(DFB_ERR_ARG, "bad argument");
     return guarded([&] {
         CUDA_TRY(cudaStreamSynchronize(h->stream));
-        if (!h->zp[0].prof) throw Error{DFB_ERR_STATE, "no profile buffer"};
-        CUDA_TRY(cudaMemcpy(out8, h->zp[0].prof, 1024, cudaMemcpyDeviceToHost));     // 128 counters
-        CUDA_TRY(cudaMemset(h->zp[0].prof, 0, 1024));
+        if (!h->sw.z[0].prof) throw Error{DFB_ERR_STATE, "no profile buffer"};
+        CUDA_TRY(cudaMemcpy(out8, h->sw.z[0].prof, 1024, cudaMemcpyDeviceToHost));     // 128 counters
+        CUDA_TRY(cudaMemset(h->sw.z[0].prof, 0, 1024));
     });
 }
 
@@ -2095,13 +2094,13 @@ int dfb_comm_init(dfb_handle h, const void* id128, int rank, int world) {
             CUDA_TRY(cudaGetDeviceProperties(&prop, h->device));
             const int reserve = std::getenv("DFB_COMM_SMS") ? std::atoi(std::getenv("DFB_COMM_SMS")) : (h->transport == 2 ? 0 : 8);
             const int sms = std::max(1, prop.multiProcessorCount - std::max(0, reserve));
-            if (world > 1 && h->tuned)
+            if (world > 1 && h->sw.tuned)
                 for (int b = 0; b < 2; ++b) {
-                    if (h->yp[b].r_grid > sms) h->yp[b].r_grid = sms;
-                    const int per_sm = std::max(1, h->zp[b].nblocks / prop.multiProcessorCount);
-                    if (h->zp[b].nblocks > per_sm * sms) h->zp[b].nblocks = per_sm * sms;
+                    if (h->sw.y[b].r_grid > sms) h->sw.y[b].r_grid = sms;
+                    const int per_sm = std::max(1, h->sw.z[b].nblocks / prop.multiProcessorCount);
+                    if (h->sw.z[b].nblocks > per_sm * sms) h->sw.z[b].nblocks = per_sm * sms;
                 }
-            reset_run_queues(*h);
+            reset_run_queues(*h, h->sw);
         }
     });
 }

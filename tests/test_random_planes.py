@@ -39,7 +39,7 @@ TOTAL_TAPS = 1.2e11                      # ... of both chains (values, term magn
 DT_MENU = (5e-8, 2e-7, 4.5e-7, 1.2e-6, 3e-6)   # Lt is 1.2e-6 (u) and 4.5e-7 (v, w)
 OVERRIDES = {"DFB_Y_MODE": "y_mode", "DFB_Y_TK": "y_tk", "DFB_Y_COLGROUP": "y_colgroup", "DFB_ZK": "zk", "DFB_Z_MODE": "z_mode"}
 assert tuple(OVERRIDES.values()) == OVR
-KNOBS = {"DFB_Z_BLOCKS_PER_SM": ("1", "2", "3"), "DFB_Y_PERSIST": ("1", "2", "7"), "DFB_Y_AHEAD": ("1",)}
+KNOBS = {"DFB_Z_BLOCKS_PER_SM": ("1", "2", "3"), "DFB_Y_PERSIST": ("1", "2", "7")}
 
 
 @pytest.fixture(scope="module")
@@ -213,7 +213,7 @@ FEATURES = {
     "periodic", "periodic:wrap",                                        # a periodic plane; one whose noise window wraps
     "slab:aligned:halo", "slab:aligned:no-halo", "slab:unaligned:halo", "slab:unaligned:no-halo",
     "mode:inject", "mode:generate",
-    "knob:DFB_Z_BLOCKS_PER_SM", "knob:DFB_Y_PERSIST", "knob:DFB_Y_AHEAD",
+    "knob:DFB_Z_BLOCKS_PER_SM", "knob:DFB_Y_PERSIST",
     "refused",
 }
 
@@ -277,8 +277,6 @@ def features(case, sp):
         out.add("knob:DFB_Z_BLOCKS_PER_SM")
     if "DFB_Y_PERSIST" in env and sp.s("n_tiles_dense"):
         out.add("knob:DFB_Y_PERSIST")
-    if "DFB_Y_AHEAD" in env and case["mode"] == "generate":
-        out.add("knob:DFB_Y_AHEAD")
     return out
 
 
@@ -286,7 +284,7 @@ def features(case, sp):
 # one seed alone (y form 3, a batch in it and one run window buffer: 329; more than one column group: 279; DFB_Y_PERSIST on dense
 # tiles: 172; an unaligned slab that draws no halo: 112).
 SEEDS = list(range(60)) + [112, 172, 279, 329]
-DIGEST = "5bfdc67cb7bdce268d776e13bef1eb4edf5e91330e2fb38276f884fdb84e806b"
+DIGEST = "d1cb6fe3b1d6f862a6089487cfacac791e83b789b8a2be8065a6c529aa60f999"
 
 
 @pytest.fixture(scope="module")

@@ -357,7 +357,6 @@ CONFIGS = {
     "simple": ((64, 130, 16, 12), {}, {"kernel_variant": 1}, 1, -1),
     "periodic": ((64, 130, 16, 12), {"DFB_Y_MODE": "2"}, {"periodic_z": 1}, 1, 2),
     "batch3": ((64, 130, 16, 12), {"DFB_Y_MODE": "2"}, {}, 3, 2),
-    "y-ahead": ((72, 530, 20, 16), {"DFB_Y_MODE": "2", "DFB_Y_AHEAD": "1"}, {}, 1, 2),
 }
 
 
@@ -379,7 +378,7 @@ def _driver(dfb, O, W, monkeypatch, name):
 # ---------------------------------------------------------------------------------------------
 def sc_prefetch_every_step(d):
     """run_step: `buf_step[b] != H.step` -- a long run of plain steps, every one of them reading the set the look-ahead filled
-    after the step before (and, with DFB_Y_AHEAD, its y-sweep: `ybuf_step[b] == H.step`)"""
+    after the step before"""
     for i in range(12):
         d.filter(DT[i % 4])
 
