@@ -153,6 +153,7 @@ def lib():
         L.dfb_attach_stream.argtypes = [C.c_void_p, C.c_void_p]
         L.dfb_filter_dev.argtypes = [C.c_void_p, C.c_void_p]
         L.dfb_set_time_scales.argtypes = [C.c_void_p, c_dp]
+        L.dfb_set_profiles.argtypes = [C.c_void_p, c_dp]
         L.dfb_time_scales_from_lengths.argtypes = [C.c_void_p, c_dp, C.c_double, c_dp]
         L.dfb_set_filter_shape.argtypes = [C.c_void_p, C.c_int]
         L.dfb_set_flux_correction.argtypes = [C.c_void_p, C.c_int]
@@ -453,6 +454,28 @@ class DIGITAL_FILTER:
         out = np.zeros(3)
         _check(lib().dfb_flux_info(self._h, int(plane), _dptr(out)))
         return float(out[0]), float(out[1]), float(out[2])
+
+    # ---- per-cell profiles (include/dfb200.h, dfb_set_profiles) ----
+    def set_profiles(self, cells):
+        """Per-cell R11, R21, R22, R33, Us, Ts, rhos, Ms from the next step on: cells = [8][Ny][Nz_global] for the whole plane, in the
+        order of DFConfig rows (a slab uses its own columns, a batch the same table for every plane); None returns to the row tables.
+        Refused (DfbError) for a value that is not finite or whose epilogue constant is not, while attached, with a communicator, or
+        while a filter_to_host_begin / gather_begin is outstanding."""
+        if cells is None:
+            _check(lib().dfb_set_profiles(self._h, None))
+            return
+        a = np.ascontiguousarray(cells, dtype=np.float64)
+        nzg = self.info(5)
+        if a.shape != (8, self.Ny, nzg):
+            raise ValueError("profiles must be [8][Ny][Nz_global] = [8][%d][%d], got %s" % (self.Ny, nzg, a.shape))
+        _check(lib().dfb_set_profiles(self._h, _dptr(a)))
+
+    @property
+    def profiles(self):
+        """the [8][Ny][Nz] profiles in use for this handle's columns (dfb_get_table 16), or None without per-cell profiles (dfb_info 19)"""
+        if not self.info(19):
+            return None
+        return np.stack([self.table(16, q, self.Ny * self.Nz).reshape(self.Ny, self.Nz) for q in range(8)])
 
     # ---- per-row temporal scales (include/dfb200.h, dfb_set_time_scales) ----
     def set_time_scales(self, rows):

@@ -212,6 +212,10 @@ struct dfb_filter_s {
     int flux_mode = DFB_FLUX_OFF;
     FluxTables flux_tab;
     FluxParams fx{};
+    double* fx_wz = nullptr;          // [Ny][W] the per-cell weights of flux_tab (per-cell profiles), allocated by the first need
+    // per-cell profiles (dfb_set_profiles; the quantities themselves are plan.cells): the epilogue's constants of this handle's cells,
+    // [7][Ny][W], allocated by the first dfb_set_profiles
+    double* prof_dev = nullptr;
     // timing
     bool timing = false;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -455,13 +459,16 @@ void launch_noise_for(dfb_filter_s& H, int64_t step, int b, cudaStream_t st) {
 }
 
 // The sweeps of one step on the main stream, after its noise: the y-sweep (band-matrix tiles, if any, first, then the run-recursive
-// tiles: disjoint rows of r_zs), the z-sweep, the flux correction and N2 where the z-sweep's epilogue does not accumulate it.  Buffer set
-// b; rec: the step record of an attached step (nullptr host-driven); tl: the step's timeline slot (DFB_TIMELINE) or nullptr.
+// tiles: disjoint rows of r_zs), the z-sweep, the per-cell profiles' rescale, the flux correction and N2 where the z-sweep's epilogue
+// does not accumulate it.  Buffer set b; rec: the step record of an attached step (nullptr host-driven); tl: the step's timeline slot
+// (DFB_TIMELINE) or nullptr.
 void enqueue_sweeps(dfb_filter_s& H, int b, const StepConsts& S, const double2* rows, const StepRecord* rec, unsigned long long* tl) {
     const Sweeps& sw = H.sw;
     const bool first = S.first_step != 0;
     const bool accumulate = H.stats_on && !first;                  // rms_add, df.cpp:606
     const bool flux = H.flux_mode != DFB_FLUX_OFF && !first;      // the constructor's step is never corrected
+    const bool profiles = H.plan.cells != nullptr;
+    const bool after = flux || profiles;                           // u', T', rho' change after the z-sweep: N2 from stats_kernel after them
     if (sw.tuned) {
         YParams Y = sw.y[b];
         Y.tl = tl ? tl + 2 : nullptr;
@@ -478,13 +485,17 @@ void enqueue_sweeps(dfb_filter_s& H, int b, const StepConsts& S, const double2* 
         Z.rec = rec;
         Z.rows = rows;
         Z.tl = tl ? tl + 4 : nullptr;
-        Z.stats = (accumulate && !flux) ? H.stats : nullptr;       // N2 fused into the epilogue, unless the correction changes u', T', rho' after it
+        Z.stats = (accumulate && !after) ? H.stats : nullptr;      // N2 fused into the epilogue, unless u', T', rho' change after it
         CUDA_TRY(launch_zsweep_tuned(sw.zmaps[b], Z, H.stream));
     } else {
         CUDA_TRY(launch_zsweep_simple(H.D[b], S, rec, rows, H.stream));
     }
-    if (flux) CUDA_TRY(launch_flux(H.fx, rec, H.stream));
-    if (accumulate && (!sw.tuned || flux)) CUDA_TRY(launch_stats(H.D[0], H.stats, rec, H.stream));
+    if (profiles) CUDA_TRY(launch_profiles(H.D[0], H.prof_dev, first ? 1 : 0, rec, H.stream));
+    if (flux) {
+        const FluxCells cells{H.fx_wz, H.prof_dev};
+        CUDA_TRY(launch_flux(H.fx, profiles ? &cells : nullptr, rec, H.stream));
+    }
+    if (accumulate && (!sw.tuned || after)) CUDA_TRY(launch_stats(H.D[0], H.stats, rec, H.stream));
 }
 
 // A step of a handle attached to a caller's stream (dfb_attach_stream): advance -> noise -> y-sweep(s) -> z-sweep (-> N2 for the
@@ -601,6 +612,30 @@ void refuse_outstanding(const dfb_filter_s& H, const char* call) {
     if (H.pipe_begun == H.pipe_ended && H.g_begun == H.g_ended) return;
     const std::string prefix = call ? std::string(call) + ": " : "";
     throw Error{DFB_ERR_STATE, prefix + "a dfb_filter_to_host_begin or dfb_gather_begin is outstanding: end it first"};
+}
+
+// Makes T the flux correction's tables: the device buffers on the first call, then the weights (steps enqueued before read the previous
+// ones on this stream).
+void install_flux(dfb_filter_s& H, FluxTables&& T) {
+    CUDA_TRY(cudaSetDevice(H.device));
+    FluxParams& F = H.fx;
+    const int NP = H.nplanes, Ny = H.plan.Ny, W = H.plan.NzG;
+    if (!F.out) {
+        CUDA_TRY(flux_prepare());
+        F.u = H.D[0].f[0].fluc; F.T = H.D[0].T_fluc; F.rho = H.D[0].rho_fluc; F.rowc = H.D[0].rowc;
+        F.Ny = Ny; F.W = W; F.P = NP; F.ps_cells = H.D[0].ps_cells;
+        F.wy = H.dalloc<double>(Ny, false);
+        F.hz = H.upload(T.hz);
+        F.part = H.dalloc<double>((size_t)NP * Ny, false);
+        F.counter = H.dalloc<unsigned>(NP);
+        F.out = H.dalloc<double2>(NP);
+    }
+    if (!T.wz.empty() && !H.fx_wz) H.fx_wz = H.dalloc<double>(T.wz.size(), false);
+    CUDA_TRY(cudaMemcpyAsync(const_cast<double*>(F.wy), T.wy.data(), Ny * sizeof(double), cudaMemcpyHostToDevice, H.stream));
+    if (!T.wz.empty()) CUDA_TRY(cudaMemcpyAsync(H.fx_wz, T.wz.data(), T.wz.size() * sizeof(double), cudaMemcpyHostToDevice, H.stream));
+    CUDA_TRY(cudaStreamSynchronize(H.stream));
+    F.D = T.D;
+    H.flux_tab = std::move(T);
 }
 
 // Attached: waits for the caller's stream and reads the device step record back into the host's step counter and N2 count.  A void
@@ -779,6 +814,7 @@ int dfb_info(dfb_handle h, int what, int field, int64_t* out64) {
         case 15: *out64 = h->plan.Lt_rows.empty() ? 0 : 1; break;
         case 17: *out64 = h->plan.filter_shape; break;
         case 18: *out64 = h->flux_mode; break;
+        case 19: *out64 = h->plan.cells ? 1 : 0; break;
         default: return fail(DFB_ERR_ARG, "unknown info selector");
     }
     return DFB_OK;
@@ -804,6 +840,15 @@ int dfb_get_table(dfb_handle h, int which, int arg, double* dst, int cap) {
         if (P.Lt_rows.empty()) { tmp.assign(P.Ny, P.f[arg].Lt); src = tmp.data(); }
         else src = P.Lt_rows.data() + (size_t)arg * P.Ny;
         n = P.Ny;
+    } else if (which == 16) {
+        if (arg < 0 || arg > 7) return fail(DFB_ERR_ARG, "table 16: quantity must be 0..7");
+        n = P.Ny * P.Nz();
+        if (P.cells) src = P.cells->data() + (size_t)arg * n;
+        else {
+            tmp.resize(n);
+            for (int j = 0; j < P.Ny; ++j) std::fill_n(tmp.begin() + (size_t)j * P.Nz(), P.Nz(), P.rows[(size_t)arg * P.Ny + j]);
+            src = tmp.data();
+        }
     }
     else return fail(DFB_ERR_ARG, "unknown table selector");
     if (cap < n) return fail(DFB_ERR_ARG, "dst too small");
@@ -1093,27 +1138,43 @@ int dfb_set_flux_correction(dfb_handle h, int mode) {
         refuse_outstanding(*h, "dfb_set_flux_correction");
         if (mode == DFB_FLUX_OFF) { h->flux_mode = DFB_FLUX_OFF; return; }
         FluxTables T = flux_tables(h->plan, mode);          // refusals (slab, R11 = 0 everywhere) throw before anything changes
-        CUDA_TRY(cudaSetDevice(h->device));
-        FluxParams& F = h->fx;
-        const int NP = h->nplanes, Ny = h->plan.Ny, W = h->plan.NzG;
-        if (!F.out) {
-            CUDA_TRY(flux_prepare());
-            F.u = h->D[0].f[0].fluc; F.T = h->D[0].T_fluc; F.rho = h->D[0].rho_fluc; F.rowc = h->D[0].rowc;
-            F.Ny = Ny; F.W = W; F.P = NP; F.ps_cells = h->D[0].ps_cells;
-            F.wy = h->dalloc<double>(Ny, false);
-            F.hz = h->upload(T.hz);
-            F.part = h->dalloc<double>((size_t)NP * Ny, false);
-            F.counter = h->dalloc<unsigned>(NP);
-            F.out = h->dalloc<double2>(NP);
+        install_flux(*h, std::move(T));
+        h->flux_mode = mode;
+    });
+}
+
+int dfb_set_profiles(dfb_handle h, const double* cells) {
+    if (!h) return fail(DFB_ERR_ARG, "handle is NULL");
+    if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_set_profiles") + ": set the profiles before attaching");
+    if (h->comm)
+        return fail(DFB_ERR_STATE, "dfb_set_profiles: the handle has a communicator (dfb_comm_init): the gathered plane is rebuilt with the row tables");
+    return guarded([&] {
+        refuse_outstanding(*h, "dfb_set_profiles");
+        Plan P = h->plan;
+        std::vector<double> pc;
+        if (cells) {
+            pc = profile_consts(P, cells);                  // refusals (DFB_ERR_ARG) throw before anything changes
+            P.cells = std::make_shared<const std::vector<double>>(profile_columns(P, cells));
+            P.cells_hash = rst::hash_f64(cells, (size_t)8 * P.Ny * P.NzG);
+        } else {
+            P.cells.reset();
+            P.cells_hash = 0;
         }
-        if (h->flux_tab.mode != mode) {
+        FluxTables T;
+        if (h->flux_mode != DFB_FLUX_OFF) T = flux_tables(P, h->flux_mode);
+        CUDA_TRY(cudaSetDevice(h->device));
+        if (cells) {
+            if (!h->prof_dev) {
+                CUDA_TRY(profiles_prepare());
+                h->prof_dev = h->dalloc<double>(pc.size(), false);
+            }
             // steps enqueued before read the previous table on this stream
-            CUDA_TRY(cudaMemcpyAsync(const_cast<double*>(F.wy), T.wy.data(), Ny * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+            CUDA_TRY(cudaMemcpyAsync(h->prof_dev, pc.data(), pc.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
             CUDA_TRY(cudaStreamSynchronize(h->stream));
         }
-        F.D = T.D;
-        h->flux_tab = std::move(T);
-        h->flux_mode = mode;
+        h->plan = std::move(P);
+        if (h->flux_mode != DFB_FLUX_OFF) install_flux(*h, std::move(T));
+        h->fingerprint = rst::fingerprint(h->plan);
     });
 }
 
@@ -1530,6 +1591,7 @@ int dfb_save_restart(dfb_handle h, const char* path, int what) {
         std::copy(forms.begin(), forms.end(), hd.forms);
         hd.fingerprint = h->fingerprint;
         hd.filter_shape = P.filter_shape;
+        hd.profiles = P.cells_hash;
         hd.sections = (uint32_t)what;
         if (what & DFB_RESTART_STATS) { hd.stats_count = h->stats_count; hd.stats_on = h->stats_on ? 1 : 0; }
         if (what & DFB_RESTART_CORR) {
@@ -1581,6 +1643,10 @@ int dfb_load_restart(dfb_handle h, const char* path, int what) {
             throw arg(std::string("filter shape differs: file ") + shape_name[hd.filter_shape] + ", handle " + shape_name[P.filter_shape] +
                       " (dfb_set_filter_shape)");
         }
+        if (hd.profiles != P.cells_hash)
+            throw arg(!P.cells_hash ? "the file was saved with per-cell profiles (dfb_set_profiles), the handle has none"
+                      : !hd.profiles ? "the handle has per-cell profiles (dfb_set_profiles), the file was saved without them"
+                                     : "the per-cell profiles (dfb_set_profiles) differ from the file's");
         if (hd.fingerprint != h->fingerprint) throw arg("the filter tables differ (half-widths, row tables or time scales)");
         if (h->noise_mode == DFB_NOISE_GENERATE && hd.seed != h->seed)
             throw arg("seed differs: file " + std::to_string(hd.seed) + ", handle " + std::to_string(h->seed));
@@ -2012,6 +2078,8 @@ int dfb_comm_init(dfb_handle h, const void* id128, int rank, int world) {
     if (h->comm) return fail(DFB_ERR_STATE, "dfb_comm_init was already called on this handle");
     if (h->attached) return fail(DFB_ERR_STATE, attached_msg("dfb_comm_init"));
     if (h->nplanes != 1) return fail(DFB_ERR_STATE, "slab communication is defined for single-plane handles");
+    if (h->plan.cells)
+        return fail(DFB_ERR_STATE, "dfb_comm_init: the handle has per-cell profiles (dfb_set_profiles): the gathered plane is rebuilt with the row tables");
     return guarded([&] {
         CUDA_TRY(cudaSetDevice(h->device));
         ncclUniqueId id;
@@ -2315,6 +2383,9 @@ int dfb_set_filter_shape_f(const dfb_handle* h, const int* shape) {
 }
 int dfb_set_flux_correction_f(const dfb_handle* h, const int* mode) {
     return (h && mode) ? dfb_set_flux_correction(*h, *mode) : fail(DFB_ERR_ARG, "NULL argument");
+}
+int dfb_set_profiles_f(const dfb_handle* h, const double* const* cells) {
+    return (h && cells) ? dfb_set_profiles(*h, *cells) : fail(DFB_ERR_ARG, "NULL argument");
 }
 int dfb_flux_info_f(const dfb_handle* h, const int* plane, double* out) {
     return (h && plane) ? dfb_flux_info(*h, *plane, out) : fail(DFB_ERR_ARG, "NULL argument");

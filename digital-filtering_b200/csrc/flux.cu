@@ -1,5 +1,6 @@
 // csrc/flux.cu -- inflow mass-flux correction (dfb_set_flux_correction): per plane and step, the plane sum m' = sum_j wy_j sum_k hz_k u'_jk
 // in a fixed order, c = m' / D, then u' <- fma(-c, rc0_j, u') and T', rho' rebuilt from it.  The tables come from fluxtables.cpp.
+// With per-cell profiles (dfb_set_profiles) the weights hz_k and the constants rc0_j, rc4_j, Ts_j, rhos_j are per cell.
 #include "kernels.hpp"
 
 namespace dfb {
@@ -31,12 +32,15 @@ __device__ __forceinline__ double block_sum(double s) {
 // One CTA per (row, plane): the row's partial wy_j * sum_k hz_k u'_jk (each thread a strided sum in k, then block_sum).  The last CTA
 // of a plane to finish (ticket counter) sums the plane's Ny partials in row order the same way, writes {c, m'} and puts the counter
 // back to 0, so that the next step (or graph replay) needs no memset.  Neither order depends on the batch size or the launch.
-__global__ void __launch_bounds__(FLUX_THREADS) flux_rows_kernel(const FluxParams F, const StepRecord* rec) {
+// CELL: per-cell profiles, the weight of cell (j, k) is wz_jk instead of hz_k.
+template <bool CELL>
+__device__ __forceinline__ void flux_rows(const FluxParams& F, const double* wz, const StepRecord* rec) {
     if (rec && rec->void_step) return;
     const int j = blockIdx.x, p = blockIdx.y;
     const double* u = F.u + (size_t)p * F.ps_cells + (size_t)j * F.W;
+    const double* w = CELL ? wz + (size_t)j * F.W : F.hz;
     double s = 0.0;
-    for (int k = threadIdx.x; k < F.W; k += FLUX_THREADS) s = __fma_rn(__ldg(F.hz + k), u[k], s);
+    for (int k = threadIdx.x; k < F.W; k += FLUX_THREADS) s = __fma_rn(__ldg(w + k), u[k], s);
     const double row = __dmul_rn(block_sum(s), __ldg(F.wy + j));
     __shared__ bool last;
     if (threadIdx.x == 0) {
@@ -56,6 +60,11 @@ __global__ void __launch_bounds__(FLUX_THREADS) flux_rows_kernel(const FluxParam
     }
 }
 
+__global__ void __launch_bounds__(FLUX_THREADS) flux_rows_kernel(const FluxParams F, const StepRecord* rec) { flux_rows<false>(F, nullptr, rec); }
+__global__ void __launch_bounds__(FLUX_THREADS) flux_rows_cell_kernel(const FluxParams F, const FluxCells C, const StepRecord* rec) {
+    flux_rows<true>(F, C.wz, rec);
+}
+
 // One thread per cell: u' <- fma(-c_p, rc0_j, u'), then T', rho' from it with the epilogue's roundings (as rebuild_kernel).
 __global__ void __launch_bounds__(FLUX_THREADS) flux_apply_kernel(const FluxParams F, const StepRecord* rec) {
     if (rec && rec->void_step) return;
@@ -72,9 +81,25 @@ __global__ void __launch_bounds__(FLUX_THREADS) flux_apply_kernel(const FluxPara
     F.rho[idx] = __dmul_rn(-t2, __ldg(rc + 6));
 }
 
+// flux_apply_kernel with the constants of every cell (per-cell profiles): pc [7][Ny][W]
+__global__ void __launch_bounds__(FLUX_THREADS) flux_apply_cell_kernel(const FluxParams F, const FluxCells C, const StepRecord* rec) {
+    if (rec && rec->void_step) return;
+    const int k = blockIdx.x * FLUX_THREADS + threadIdx.x;
+    const int j = blockIdx.y, p = blockIdx.z;
+    if (k >= F.W) return;
+    const size_t n = (size_t)F.Ny * F.W, c = (size_t)j * F.W + k, idx = (size_t)p * F.ps_cells + c;
+    const double cp = F.out[p].x;
+    const double u = __fma_rn(-cp, __ldg(C.pc + c), F.u[idx]);
+    const double t2 = __dmul_rn(__ldg(C.pc + 4 * n + c), u);
+    F.u[idx] = u;
+    F.T[idx] = __dmul_rn(t2, __ldg(C.pc + 5 * n + c));
+    F.rho[idx] = __dmul_rn(-t2, __ldg(C.pc + 6 * n + c));
+}
+
 cudaError_t flux_prepare() {
     // load both kernels now, not while an attached handle's stream is being captured
-    const void* fns[] = {(const void*)flux_rows_kernel, (const void*)flux_apply_kernel};
+    const void* fns[] = {(const void*)flux_rows_kernel, (const void*)flux_apply_kernel, (const void*)flux_rows_cell_kernel,
+                         (const void*)flux_apply_cell_kernel};
     for (const void* fn : fns) {
         cudaFuncAttributes a;
         const cudaError_t e = cudaFuncGetAttributes(&a, fn);
@@ -83,9 +108,15 @@ cudaError_t flux_prepare() {
     return cudaSuccess;
 }
 
-cudaError_t launch_flux(const FluxParams& F, const StepRecord* rec, cudaStream_t st) {
-    flux_rows_kernel<<<dim3((unsigned)F.Ny, (unsigned)F.P), FLUX_THREADS, 0, st>>>(F, rec);
-    flux_apply_kernel<<<dim3((unsigned)((F.W + FLUX_THREADS - 1) / FLUX_THREADS), (unsigned)F.Ny, (unsigned)F.P), FLUX_THREADS, 0, st>>>(F, rec);
+cudaError_t launch_flux(const FluxParams& F, const FluxCells* cells, const StepRecord* rec, cudaStream_t st) {
+    const dim3 rows((unsigned)F.Ny, (unsigned)F.P), grid((unsigned)((F.W + FLUX_THREADS - 1) / FLUX_THREADS), (unsigned)F.Ny, (unsigned)F.P);
+    if (cells) {
+        flux_rows_cell_kernel<<<rows, FLUX_THREADS, 0, st>>>(F, *cells, rec);
+        flux_apply_cell_kernel<<<grid, FLUX_THREADS, 0, st>>>(F, *cells, rec);
+    } else {
+        flux_rows_kernel<<<rows, FLUX_THREADS, 0, st>>>(F, rec);
+        flux_apply_kernel<<<grid, FLUX_THREADS, 0, st>>>(F, rec);
+    }
     return cudaGetLastError();
 }
 

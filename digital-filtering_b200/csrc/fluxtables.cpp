@@ -30,18 +30,43 @@ FluxTables flux_tables(const Plan& P, int mode) {
         Z += T.hz[k];
     }
     double d = 0.0, mean = 0.0;
-    for (int j = 0; j < Ny; ++j) {
-        const double hy = P.vert_y[j + 1] - P.vert_y[j];
-        const double g = mode == DFB_FLUX_MASS ? rhos[j] * (1.0 + 0.2 * Ms[j] * Ms[j]) : 1.0;
-        T.rc0[j] = std::sqrt(R11[j]);                       // the epilogue's rowc[0] (stepplan.cpp), bit for bit
-        T.wy[j] = g * hy;
-        d += T.wy[j] * T.rc0[j];
-        mean += hy * (mode == DFB_FLUX_MASS ? rhos[j] * Us[j] : Us[j]);
+    if (P.cells) {
+        // per-cell profiles: wy_j = hy_j, and g_jk hz_k per cell in wz
+        const double* C = P.cells->data();
+        const size_t n = (size_t)Ny * NzG;
+        T.wz.resize(n);
+        for (int j = 0; j < Ny; ++j) {
+            const double hy = P.vert_y[j + 1] - P.vert_y[j];
+            double dj = 0.0, mj = 0.0;
+            for (int k = 0; k < NzG; ++k) {
+                const size_t i = (size_t)j * NzG + k;
+                const double r11 = C[i], us = C[4 * n + i], rho = C[6 * n + i], ms = C[7 * n + i];
+                const double g = mode == DFB_FLUX_MASS ? rho * (1.0 + 0.2 * ms * ms) : 1.0;
+                T.wz[i] = g * T.hz[k];
+                dj += T.wz[i] * std::sqrt(r11);             // sqrt(R11): the per-cell constant rc0 (profile_consts), bit for bit
+                mj += T.hz[k] * (mode == DFB_FLUX_MASS ? rho * us : us);
+            }
+            T.wy[j] = hy;
+            d += hy * dj;
+            mean += hy * mj;
+        }
+        T.rc0.clear();
+        T.D = d;
+        T.mean = mean;
+    } else {
+        for (int j = 0; j < Ny; ++j) {
+            const double hy = P.vert_y[j + 1] - P.vert_y[j];
+            const double g = mode == DFB_FLUX_MASS ? rhos[j] * (1.0 + 0.2 * Ms[j] * Ms[j]) : 1.0;
+            T.rc0[j] = std::sqrt(R11[j]);                       // the epilogue's rowc[0] (stepplan.cpp), bit for bit
+            T.wy[j] = g * hy;
+            d += T.wy[j] * T.rc0[j];
+            mean += hy * (mode == DFB_FLUX_MASS ? rhos[j] * Us[j] : Us[j]);
+        }
+        T.D = d * Z;
+        T.mean = mean * Z;
     }
-    T.D = d * Z;
-    T.mean = mean * Z;
     if (!(T.D > 0.0) || !std::isfinite(T.D))
-        throw Error{DFB_ERR_ARG, "the flux correction needs sum A g sqrt(R11) > 0: R11 is zero on every row of this plane"};
+        throw Error{DFB_ERR_ARG, std::string("the flux correction needs sum A g sqrt(R11) > 0: R11 is zero on every ") + (P.cells ? "cell" : "row") + " of this plane"};
     return T;
 }
 

@@ -56,8 +56,19 @@ struct FluxParams {
     int Ny, W, P;
     size_t ps_cells;
 };
+// per-cell profiles (dfb_set_profiles): then wy_j = hy_j, the weights are wz and the constants pc
+struct FluxCells {
+    const double* wz;                 // [Ny][W] g_jk hz_k
+    const double* pc;                 // [7][Ny][W] the epilogue's constants per cell (profile_consts): rc0, rc4, Ts, rhos at 0, 4, 5, 6
+};
 cudaError_t flux_prepare();
-cudaError_t launch_flux(const FluxParams& F, const StepRecord* rec, cudaStream_t st);   // a void attached step (rec) changes nothing
+// cells: nullptr for the row tables; a void attached step (rec) changes nothing
+cudaError_t launch_flux(const FluxParams& F, const FluxCells* cells, const StepRecord* rec, cudaStream_t st);
+
+// per-cell profiles (profiles.cu, dfb_set_profiles): u', v', w' and, unless first, T', rho' of D[0]'s planes rescaled from filt_old with
+// the constants pc [7][Ny][W] of every cell; a void attached step (rec) changes nothing
+cudaError_t profiles_prepare();
+cudaError_t launch_profiles(const PlaneDev& D, const double* pc, int first, const StepRecord* rec, cudaStream_t st);
 
 // correlation statistics (corr.cu, dfb_corr_enable): sums [P][3][Ny][L_d + 1] per direction d = 0 z, 1 y, 2 t
 struct CorrParams {

@@ -1,7 +1,9 @@
 // csrc/plan.hpp -- host-side description of one inflow plane: everything the constructor of the
 // reference computes once (df.cpp:4-66) in the shape the device wants it.
 #pragma once
+#include <cmath>
 #include <cstdint>
+#include <memory>
 #include <optional>
 #include <string>
 #include <vector>
@@ -48,6 +50,10 @@ struct Plan {
     CoefTable coef;
     int64_t taps_per_step = 0;                   // sum over fields and LOCAL cells of (2Ny+1)+(2Nz+1)
     std::vector<double> Lt_rows;                 // [3][Ny] per-row time scales (dfb_set_time_scales); empty: f[].Lt for every row
+    // per-cell profiles (dfb_set_profiles): the eight quantities of `rows` for the cells of this handle's columns, [8][Ny][Nz()], and the
+    // hash of the whole-plane table they came from (restart fingerprint).  Null: `rows` for every column.
+    std::shared_ptr<const std::vector<double>> cells;
+    uint64_t cells_hash = 0;
     int Nz() const { return k1 - k0; }
 };
 
@@ -95,6 +101,28 @@ StepPlan plan_step(const Plan& plan, int nplanes, const DeviceLimits& dev, const
 // batch draws from stream group plane_id + p).  The advance kernel of attached steps computes the same states with noise_step_state.
 void fill_noise_states(NoiseParams& np, const uint64_t* npairs, uint64_t seed, int plane_id, int nplanes, int64_t step);
 
+// The epilogue's constants (df.cpp:425-438, 474) of one row or cell from its eight profile values q = R11, R21, R22, R33, Us, Ts, rhos,
+// Ms: rc = sqrt(R11), b, sqrt(R22 - b^2), sqrt(R33), -0.2 Ms^2 / Us, Ts, rhos.  The row tables (plan_step) and the per-cell profiles
+// (profile_consts) both use it, so that a cell whose values equal a row's gets that row's constants bit for bit.
+inline void epilogue_consts(const double q[8], double rc[7]) {
+    const double b = (q[0] < 1e-10) ? 0.0 : q[1] / std::sqrt(q[0]);
+    rc[0] = std::sqrt(q[0]);
+    rc[1] = b;
+    rc[2] = std::sqrt(q[2] - b * b);
+    rc[3] = std::sqrt(q[3]);
+    rc[4] = -0.5 * (1.4 - 1) * q[7] * q[7] / q[4];
+    rc[5] = q[5];
+    rc[6] = q[6];
+}
+constexpr int PROFILE_CONSTS = 7;                // epilogue_consts per cell
+
+// dfb_set_profiles (profiles.cpp): checks a whole-plane table [8][Ny][NzG] and returns the epilogue constants of the cells of the plan's
+// columns, [PROFILE_CONSTS][Ny][Nz()].  Throws DFB_ERR_ARG naming the quantity, row and column of the first value that is not finite
+// or whose constant is not (R11 < 0, R22 < b^2, Us = 0, ...).
+std::vector<double> profile_consts(const Plan& plan, const double* cells);
+// the plan's columns of a whole-plane table: [8][Ny][Nz()]
+std::vector<double> profile_columns(const Plan& plan, const double* cells);
+
 // Per-row time scales [3][Ny]: throws DFB_ERR_ARG naming the first entry that is not finite or not > 0.
 void check_time_scales(const Plan& plan, const double* Lt_rows);
 // dfb_time_scales_from_lengths: Lt_f(j) = Ix_f(y_j) / max(Us_j, u_min), Ix_f blended from Ix[2f] to Ix[2f+1] like Iz.  Throws dfb::Error.
@@ -103,10 +131,13 @@ void time_scales_from_lengths(const Plan& plan, const double Ix[6], double u_min
 // Inflow mass-flux correction (dfb_set_flux_correction, fluxtables.cpp): per plane and step c = m' / D with m' = sum_j wy_j sum_k hz_k u'_jk,
 // and u' <- u' - c rc0_j.  wy_j = g_j hy_j, g_j = rhos_j (1 + 0.2 Ms_j^2) (DFB_FLUX_MASS) or 1 (DFB_FLUX_VOLUME); rc0_j = sqrt(R11_j);
 // D = sum_jk hy_j hz_k g_j rc0_j; mean = sum_jk hy_j hz_k rhos_j Us_j (mass) or hy_j hz_k Us_j (volume).
+// With per-cell profiles (plan.cells) g, rc0 and the mean flux are per cell: m' = sum_j wy_j sum_k wz_jk u'_jk with wy_j = hy_j and
+// wz_jk = g_jk hz_k, u' <- u' - c rc0_jk, D = sum_j hy_j sum_k wz_jk rc0_jk.
 struct FluxTables {
     int mode = 0;
-    std::vector<double> wy, rc0;                 // [Ny]
+    std::vector<double> wy, rc0;                 // [Ny]; rc0 empty with per-cell profiles
     std::vector<double> hz;                      // [NzG]
+    std::vector<double> wz;                      // [Ny][NzG] per-cell profiles only, else empty
     double D = 0, mean = 0;
 };
 // Throws DFB_ERR_ARG for a mode other than DFB_FLUX_MASS / DFB_FLUX_VOLUME, a slab plan, or D = 0.

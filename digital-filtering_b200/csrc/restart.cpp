@@ -153,6 +153,17 @@ uint64_t fingerprint(const Plan& P) {
         H.word(0x67617573736961ull);             // "gaussia"
         H.word((uint64_t)P.filter_shape);
     }
+    if (P.cells_hash) {                          // per-cell profiles: hashed only when set, so a handle without them keeps its fingerprint
+        H.word(0x70726f66696c6573ull);           // "profiles"
+        H.word(P.cells_hash);
+    }
+    return H.h;
+}
+
+uint64_t hash_f64(const double* v, size_t n) {
+    Hash H;
+    H.word(n);
+    for (size_t i = 0; i < n; ++i) H.f64(v[i]);
     return H.h;
 }
 
@@ -190,6 +201,7 @@ void encode_header(const Header& h, unsigned char* out) {
     for (int s = 0; s < N_SECTIONS; ++s) o.i64(h.off[s]);
     o.i64(h.file_bytes);
     o.i32(h.filter_shape);
+    o.u64(h.profiles);
 }
 
 Header decode_header(const unsigned char* in_) {
@@ -216,6 +228,7 @@ Header decode_header(const unsigned char* in_) {
     for (int s = 0; s < N_SECTIONS; ++s) off[s] = in.i64();
     const int64_t bytes = in.i64();
     h.filter_shape = in.i32();
+    h.profiles = in.u64();
     if (h.Ny <= 0 || h.NzG <= 0 || h.nplanes <= 0 || h.nplanes > DFB_MAXP || h.corr_L[2] < 0 || h.corr_L[2] > MAX_LT || h.n_ring < 0 ||
         h.n_ring > h.corr_L[2] || h.filter_shape < 0 || h.filter_shape > DFB_FILTER_GAUSSIAN || h.corr_L[0] < 0 || h.corr_L[0] >= h.NzG || h.corr_L[1] < 0 || h.corr_L[1] >= h.Ny)
         throw io("corrupt restart header (sizes)");

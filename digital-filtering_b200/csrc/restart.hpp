@@ -47,6 +47,7 @@ struct Header {
     int64_t corr_count = 0;
     int64_t corr_tsteps[MAX_LT + 1] = {};
     int32_t filter_shape = 0;                     // DFB_FILTER_*; stored after file_bytes, so files written before it read 0 (exponential)
+    uint64_t profiles = 0;                        // Plan::cells_hash (0: no per-cell profiles); stored after filter_shape, older files read 0
     // derived by layout(): byte offset of each section (0 when absent) and the file's size
     int64_t off[N_SECTIONS] = {};
     int64_t file_bytes = 0;
@@ -60,8 +61,10 @@ struct Record {
 
 // Everything that decides the numbers of the next steps besides the seed and the plane range: Ny, NzG, periodic_z, the whole-plane
 // half-width tables of each field (per row when row-uniform, per cell otherwise), Lt of each field and the [8][Ny] row tables,
-// the per-row time scales when set, and the filter shape when it is Gaussian.
+// the per-row time scales when set, the filter shape when it is Gaussian, and the hash of the per-cell profiles when set.
 uint64_t fingerprint(const Plan& P);
+// the hash fingerprint() uses, of n doubles by their bits (Plan::cells_hash of a whole-plane profile table)
+uint64_t hash_f64(const double* v, size_t n);
 
 void layout(Header& h);                                       // fills off[] and file_bytes from the sizes and sections
 void encode_header(const Header& h, unsigned char* out);      // HEADER_BYTES bytes

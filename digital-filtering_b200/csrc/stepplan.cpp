@@ -580,18 +580,10 @@ StepPlan plan_step(const Plan& P, int NP, const DeviceLimits& dev, const Overrid
 
     // ---- per-row epilogue constants, reference expressions (df.cpp:425-438, 474) ----
     S.rowc.assign((size_t)Ny * ROWC, 0.0);
-    const double* R11 = P.rows.data(); const double* R21 = R11 + Ny; const double* R22 = R21 + Ny; const double* R33 = R22 + Ny;
-    const double* Us = R33 + Ny; const double* Ts = Us + Ny; const double* rhos = Ts + Ny; const double* Ms = rhos + Ny;
     for (int j = 0; j < Ny; ++j) {
-        double b = (R11[j] < 1e-10) ? 0.0 : R21[j] / std::sqrt(R11[j]);
-        double* rc = &S.rowc[(size_t)j * ROWC];
-        rc[0] = std::sqrt(R11[j]);
-        rc[1] = b;
-        rc[2] = std::sqrt(R22[j] - b * b);
-        rc[3] = std::sqrt(R33[j]);
-        rc[4] = -0.5 * (1.4 - 1) * Ms[j] * Ms[j] / Us[j];
-        rc[5] = Ts[j];
-        rc[6] = rhos[j];
+        double q[8];
+        for (int i = 0; i < 8; ++i) q[i] = P.rows[(size_t)i * Ny + j];
+        epilogue_consts(q, &S.rowc[(size_t)j * ROWC]);
     }
     for (int f = 0; f < 3; ++f) {
         const FieldPlan& FP = P.f[f];

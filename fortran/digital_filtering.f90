@@ -29,6 +29,8 @@
 !   set_filter_shape                                scales Iz / Iy (include/dfb200.h, dfb_set_filter_shape)
 !   set_flux_correction, flux_info                each step's plane-integrated mass (or volume) flux of the inflow held at its mean
 !                                                   (include/dfb200.h, dfb_set_flux_correction)
+!   set_profiles, clear_profiles                  per-cell Reynolds stresses and mean state, for boundary layers that vary along the
+!                                                   span (include/dfb200.h, dfb_set_profiles)
 !
 ! NOTE: NEVER COMPILED -- no Fortran compiler exists in the build image or on the GPU boxes.  The binding is exercised through
 ! tests/fortran_abi_mimic.c, a C program that makes exactly these calls with exactly this struct layout and by-reference
@@ -47,6 +49,7 @@ module DIGITAL_FILTERING
     public :: set_time_scales, clear_time_scales, time_scales_from_lengths
     public :: set_filter_shape, FILTER_EXPONENTIAL, FILTER_GAUSSIAN
     public :: set_flux_correction, flux_info, FLUX_OFF, FLUX_MASS, FLUX_VOLUME
+    public :: set_profiles, clear_profiles
 
     integer, parameter :: RESTART_STATE = 1, RESTART_STATS = 2, RESTART_CORR = 4   ! DFB_RESTART_* (what to save / load; added together)
     integer, parameter :: FILTER_EXPONENTIAL = 0, FILTER_GAUSSIAN = 1                ! DFB_FILTER_* (DFConfig%filter_shape)
@@ -281,6 +284,10 @@ module DIGITAL_FILTERING
             import :: c_int, c_ptr
             type(c_ptr), intent(in) :: handle
             integer(c_int), intent(in) :: mode
+        end function
+        integer(c_int) function dfb_set_profiles_f(handle, cells) bind(C, name='dfb_set_profiles_f')
+            import :: c_int, c_ptr
+            type(c_ptr), intent(in) :: handle, cells
         end function
         integer(c_int) function dfb_flux_info_f(handle, plane, out) bind(C, name='dfb_flux_info_f')
             import :: c_int, c_ptr, c_double
@@ -530,6 +537,21 @@ contains
         p = plane
         call check(dfb_flux_info_f(DF%handle, p, out), 'flux_info')
     end subroutine flux_info
+
+    ! per-cell profiles from the next step on: cells(k, j, q), k = 1..Nz (the whole plane), j = 1..Ny (after the trim), q = 1..8 in the
+    ! order R11, R21, R22, R33, Us, Ts, rhos, Ms of config%rows; set them before attach_stream and before load_restart of a file saved
+    ! with them
+    subroutine set_profiles(DF, cells)
+        type(digital_filter_type), intent(in) :: DF
+        real(c_double), intent(in), target, contiguous :: cells(:, :, :)
+        call check(dfb_set_profiles_f(DF%handle, c_loc(cells)), 'set_profiles')
+    end subroutine set_profiles
+
+    ! back to the row tables
+    subroutine clear_profiles(DF)
+        type(digital_filter_type), intent(in) :: DF
+        call check(dfb_set_profiles_f(DF%handle, c_null_ptr), 'clear_profiles')
+    end subroutine clear_profiles
 
     ! back to the scalar Lt of the configuration
     subroutine clear_time_scales(DF)

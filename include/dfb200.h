@@ -131,12 +131,15 @@ int dfb_dims(dfb_handle h, int* Ny, int* Nz);
  *    send/recv, 0 = no communicator, 13 spanwise-periodic plane (dfb_config.periodic_z) in use (0/1),
  * 14 lags of correlation direction `field` (0 z, 1 y, 2 t; dfb_corr_enable), 0 when that direction is off or before any enable,
  * 15 per-row time scales in use (dfb_set_time_scales, 0/1), 17 filter shape (dfb_set_filter_shape: DFB_FILTER_EXPONENTIAL /
- *    DFB_FILTER_GAUSSIAN), 18 flux correction mode (dfb_set_flux_correction: DFB_FLUX_OFF / _MASS / _VOLUME) */
+ *    DFB_FILTER_GAUSSIAN), 18 flux correction mode (dfb_set_flux_correction: DFB_FLUX_OFF / _MASS / _VOLUME),
+ * 19 per-cell profiles in use (dfb_set_profiles, 0/1) */
 int dfb_info(dfb_handle h, int what, int field, int64_t* out64);
 /* host copies of the setup tables (for parity tests): which = 0..7 rows R11,R21,R22,R33,Us,Ts,rhos,Ms [Ny];
  * 8 yc row [Ny]; 9 dy row [Ny]; 10 Lt[3]; 11 coefficients of half-width `arg` [2*arg+1], in the handle's filter shape;
  * 12 y of the vertex rows [Ny+1]; 13 z of the vertex columns [Nz_global+1] (df.cpp:99-100: the y / z the writers print);
- * 14 time scales Lt of field `arg` (0..2) per row in use [Ny]: the rows of dfb_set_time_scales, or the scalar Lt repeated */
+ * 14 time scales Lt of field `arg` (0..2) per row in use [Ny]: the rows of dfb_set_time_scales, or the scalar Lt repeated;
+ * 16 quantity `arg` (0..7, the order of 0..7) of the profiles in use for this handle's columns [Ny][Nz]: those of dfb_set_profiles, or
+ *    the row table repeated along the span.  Tables 0..7 are the row tables whatever the profiles. */
 int dfb_get_table(dfb_handle h, int which, int arg, double* dst, int cap);
 /* N_y / N_z of field f (dir 0 = y, 1 = z) for the local slab, [Ny*Nz] */
 int dfb_get_half_widths(dfb_handle h, int field, int dir, int* dst);
@@ -273,6 +276,26 @@ int dfb_set_filter_shape(dfb_handle h, int shape);
 enum { DFB_FLUX_OFF = 0, DFB_FLUX_MASS = 1, DFB_FLUX_VOLUME = 2 };
 int dfb_set_flux_correction(dfb_handle h, int mode);
 int dfb_flux_info(dfb_handle h, int plane, double out[3]);
+/* Per-cell profiles (opt-in), for planes whose boundary layer varies along the span (a cone at angle of attack, an elliptic cone, a
+ * swept fin, a corner or duct inflow).  By default the eight quantities R11, R21, R22, R33, Us, Ts, rhos, Ms that scale the filtered
+ * fields are one per row (dfb_config.rows, or interpolated from the data files at column 0's wall distance), so every column gets the
+ * same boundary layer.  dfb_set_profiles(h, cells) gives every cell its own: cells is [8][Ny][Nz_global], the quantities in the order
+ * of dfb_config.rows, Ny after the trim, for the whole plane (a slab handle uses its own columns; every plane of a batch the same table).
+ * The epilogue's constants of each cell are derived on the host with the row path's expressions (b = R11 < 1e-10 ? 0 : R21 / sqrt(R11),
+ * sqrt(R22 - b^2), -0.2 Ms^2 / Us, ...), so a cell whose eight values equal a row's gets that row's constants bit for bit.  After the
+ * z-sweep each step rescales u', v', w' and T', rho' from filt_old with them (T', rho' stay untouched on the constructor's step and
+ * dfb_first_step, quirk 3).  filt_old, the noise and the step counter do not depend on the profiles: a handle whose profiles equal its
+ * rows delivers its own fields bit for bit.  N2 sums are then accumulated after the rescale; the flux correction uses g, sqrt(R11) and
+ * the mean flux per cell.  The constructor's step is taken before any call, with the rows; on a handle created with skip_first_step,
+ * dfb_first_step uses the profiles.
+ * dfb_set_profiles(h, NULL) returns to the row tables.  Takes effect from the next step.  Refused, leaving the handle as it was: a value
+ * that is not finite, or whose constant is not (R11 < 0, R22 < b^2, Us = 0, ...), naming the quantity, row and column (DFB_ERR_ARG);
+ * with the flux correction on, profiles that make its D zero (DFB_ERR_ARG); an attached handle, a handle with a communicator
+ * (dfb_comm_init, which refuses a handle with profiles in turn) or an outstanding dfb_filter_to_host_begin / dfb_gather_begin
+ * (DFB_ERR_STATE).  dfb_info 19 tells whether profiles are in use, dfb_get_table 16 returns them.  The row tables (dfb_get_table 0..7),
+ * the writers and dfb_time_scales_from_lengths keep using the rows.  A restart file saved with profiles loads only into a handle with
+ * the same profiles; one saved without them only into a handle without. */
+int dfb_set_profiles(dfb_handle h, const double* cells);
 /* page-lock (cudaHostRegister) / release a caller-owned host array: dfb_filter_to_host into registered arrays runs at the PCIe
  * rate; pageable arrays cost an extra staging pass inside the driver.  The C++ facade does this for its std::vectors. */
 int dfb_host_register(void* ptr, size_t bytes);
@@ -497,6 +520,7 @@ int dfb_set_time_scales_f(const dfb_handle* h, const double* const* Lt_rows);
 int dfb_time_scales_from_lengths_f(const dfb_handle* h, const double* Ix, const double* u_min, double* Lt_rows);
 int dfb_set_filter_shape_f(const dfb_handle* h, const int* shape);
 int dfb_set_flux_correction_f(const dfb_handle* h, const int* mode);
+int dfb_set_profiles_f(const dfb_handle* h, const double* const* cells);
 int dfb_flux_info_f(const dfb_handle* h, const int* plane, double* out);
 /* path: Fortran character variable (c_loc) + its len_trim, as the file names of dfb_config (path_len < 0: NUL-terminated) */
 int dfb_save_restart_f(const dfb_handle* h, const char* path, const int* path_len, const int* what);

@@ -159,6 +159,20 @@ class DIGITAL_FILTER {
         check(dfb_flux_info(h_, plane, out.data()));
         return out;
     }
+    // per-cell profiles (dfb_set_profiles): cells = [8][Ny][Nz of the whole plane], the quantities of DFConfig rows in their order, from
+    // the next step on; clear_profiles returns to the row tables; profiles() tells whether they are in use (dfb_info 19)
+    void set_profiles(const std::vector<double>& cells) {
+        std::int64_t nzg = 0;
+        check(dfb_info(h_, 5, 0, &nzg));
+        if (cells.size() != (size_t)8 * Ny * (size_t)nzg) throw std::invalid_argument("set_profiles: cells must hold 8 * Ny * Nz values (the whole plane)");
+        check(dfb_set_profiles(h_, cells.data()));
+    }
+    void clear_profiles() { check(dfb_set_profiles(h_, nullptr)); }
+    bool profiles() const {
+        std::int64_t v = 0;
+        check(dfb_info(h_, 19, 0, &v));
+        return v != 0;
+    }
     // explicit fetch for fetch_every_step = false (also refreshes .filt)
     void fetch() {
         FilterField* F[3] = {&u, &v, &w};
